@@ -9,6 +9,7 @@ primary rays of this rank's image tiles, closest-hit traversal, one cosine bounc
 traversal, RGBA8 — then the framebuffer gather to rank 0 (the path's one exchange step) and its assembly.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (under torchrun for N > 1)
+  python bench.py ... --dump-outputs DIR                        also write the last timed step's frame to DIR/*.npy
   python bench.py --impl reference ...                          the reference's CPU algorithm (oracle port) on host cores
 
 Weak scaling: the frame holds ~N x 1920x1080 pixels (same camera, finer sampling), tiles interleaved over N ranks,
@@ -136,6 +137,26 @@ def ncu_figure(key):
         return None
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_frame(path, frame, w, h):
+    """--dump-outputs: the RGBA8 frame a step hands its caller (a device tensor or a host array), as float32 [h, w, 4] in
+    `path`/frame_rgba.npy.  A frame larger than DUMP_BYTES is cut to a fixed, seeded sample of pixels, [n, 4], with their
+    row-major pixel indices in frame_pixel_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    frame = frame.cpu().numpy() if hasattr(frame, "cpu") else np.ascontiguousarray(frame)
+    rgba = frame.view(np.uint8).reshape(h, w, 4).astype(np.float32)
+    if rgba.nbytes <= DUMP_BYTES - 4096:
+        np.save(os.path.join(path, "frame_rgba.npy"), rgba)
+        if os.path.exists(os.path.join(path, "frame_pixel_index.npy")):     # left by an earlier, sampled dump into DIR
+            os.remove(os.path.join(path, "frame_pixel_index.npy"))
+        return
+    idx = np.sort(np.random.default_rng(0).choice(h * w, size=(DUMP_BYTES - 4096) // (16 + 8), replace=False))
+    np.save(os.path.join(path, "frame_rgba.npy"), rgba.reshape(-1, 4)[idx])
+    np.save(os.path.join(path, "frame_pixel_index.npy"), idx.astype(np.float64))
+
+
 def build_scene(nthreads=0):
     from tray_racing_b200 import host
     mesh = host.Mesh.generate(WL["scene"], WL["seed"], 1.0)
@@ -197,10 +218,13 @@ def run_reference(args):
         orc.render(view, w, h, 0, nthreads=threads)
     t0 = time.perf_counter()
     rays = 0
-    for _ in range(args.steps):
-        r = orc.render(view, w, h, 0, nthreads=threads)
+    for i in range(args.steps):
+        # with --dump-outputs the last step also shades the RGBA8 frame our arm's steps produce
+        r = orc.render(view, w, h, 0, nthreads=threads, rgba=bool(args.dump_outputs) and i == args.steps - 1)
         rays += r["primary_totals"]["rays"] + r["bounce_totals"]["rays"]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, r["rgba"], w, h)
     val = rays / dt / 1e6
     sample = f"each step = one whole {w}x{h} frame of the workload (same scene, camera and size as our arm), primary+bounce"
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -608,9 +632,13 @@ def run_ours(args):
         sampler.start()
         time.sleep(0.25)
     t_wall0 = time.time()
-    total_ms = rig.timed_run(steps, flush_buf)
-    t_wall1 = time.time()
-    clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    try:
+        total_ms = rig.timed_run(steps, flush_buf)
+    finally:                                           # no nvidia-smi left running when the timed run fails
+        t_wall1 = time.time()
+        clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_frame(args.dump_outputs, rig.last_frame_tensor(rig.k - 1), w, h)
     total_ms = max_over_ranks(torch, dist, world, total_ms)
     rays_step = torch.tensor([cp["rays"] + cb["rays"], cp["rays"], cb["rays"]], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -914,6 +942,8 @@ def run_single_process(args):
         g.sync()
         ms = (time.perf_counter() - t0) * 1e3 / steps
         res[nf] = {"ms_per_step": ms, "value": rays / ms / 1e3, "frame_equals_single_gpu_frame": same}
+    if args.dump_outputs:                              # the frame of the last timed step (three frames in flight)
+        dump_frame(args.dump_outputs, g.frame(), w, h)
     nf = min(res, key=lambda q: res[q]["ms_per_step"])
     g.set_frames_in_flight(nf)
     per_frame_ms = [g.render(view, w, h, 0, flags, timed=True) for _ in range(12)][2:]
@@ -965,7 +995,12 @@ def main():
                     help="one process drives all --gpus N devices through tray_cuda_group_* (no torchrun)")
     ap.add_argument("--exchange", default="auto", choices=["auto", "push", "peer", "peer-nccl", "nccl"],
                     help="how shards reach rank 0's frame: peer-mapped frame written by the kernels, or NCCL gather + untile")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame of the last one to DIR/frame_rgba.npy (float32; a seeded "
+                         "sample of pixels when the frame exceeds 64 MB), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global WL
     WL = WORKLOADS[args.workload]
     claim_stdout()

@@ -1,5 +1,6 @@
-"""Regenerates tests/golden/*.npz from the reference's in-tree assets.  Run in the build container
-(needs /root/reference); the GPU box only reads the committed .npz files.
+"""Regenerates tests/golden/*.npz from the reference's in-tree assets; the tests only read the committed .npz files.
+
+  python tests/golden/make_fixtures.py <checkout of the reference>
 
   cornell_box.npz  triangles (n,9) f32 + per-object offsets of assets/obj/cornell_box.obj parsed with
                    `load_meshs` semantics (reference src/main.rs:530-559), camera of
@@ -15,7 +16,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from tray_racing_b200 import host  # noqa: E402
 
-REF = "/root/reference/assets"
+if len(sys.argv) != 2:
+    sys.exit("usage: python tests/golden/make_fixtures.py <checkout of the reference>")
+REF = os.path.join(sys.argv[1], "assets")
 for name, eye, look, fov in (("cornell_box", (0.0, 1.0, 2.1), (0.0, 1.0, 0.0), 90.0),
                              ("box", (3.0, 1.5, 1.4), (-3.9438584, 1.5, -1.7303504), 90.0)):
     m = host.Mesh.load_obj(f"{REF}/obj/{name}.obj")
