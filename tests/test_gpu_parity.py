@@ -358,18 +358,6 @@ def test_start_slot_runs_the_reference_protocol(cornell):
     assert st.frames >= 1 and st.traversal_ms > 0
 
 
-@pytest.mark.parametrize("use_tlas,stride", [(False, 48), (True, 64)])
-def test_pooled_kernel_is_bit_identical_too(cornell, monkeypatch, use_tlas, stride):
-    """TRAY_CUDA_POOL=1 selects the pooled kernel (traverse_pool.cuh): another lane assignment, the same per-ray
-    sequence of node and triangle tests — so the same hits AND the same visit counters."""
-    monkeypatch.setenv("TRAY_CUDA_POOL", "1")
-    render_and_compare(cornell, 640, 360, use_tlas, stride)
-    render_and_compare(host.Mesh.generate("hairball", 3, 0.1), 480, 270)
-    monkeypatch.setenv("TRAY_CUDA_POOL_REFILL_MIN", "1")
-    monkeypatch.setenv("TRAY_CUDA_POOL_TRI_WEIGHT", "3")
-    render_and_compare(cornell, 101, 37, use_tlas, stride)
-
-
 @pytest.mark.parametrize("w,h,shards", [(640, 360, 1), (101, 37, 1), (333, 130, 3)])
 def test_frame_target_receives_the_same_pixels(cornell, w, h, shards):
     """Fused framebuffer exchange (include/tray_cuda.h, tray_cuda_scene_set_frame_target): the kernels store RGBA

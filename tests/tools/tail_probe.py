@@ -4,7 +4,7 @@ Test infrastructure (it uses the CPU oracle for the step counts): takes the long
   (a) the L longest rays packed 32 to a warp,
   (b) the same rays one per warp: every aligned group of 32 rays is 1 long ray + 31 rays that miss the root (tmax = 0),
 for each setting of the knobs given on the command line, e.g.
-  python tests/tools/tail_probe.py hairball '{"TRAY_CUDA_NARROW_MAX": [0, 4], "TRAY_CUDA_LOOKAHEAD": [0, 1, 3]}'"""
+  python tests/tools/tail_probe.py hairball '{"TRAY_CUDA_REFILL_MIN": [4, 6], "TRAY_CUDA_TRI_WEIGHT": [3, 4]}'"""
 import itertools, os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -13,7 +13,7 @@ import oracle_binding as ob
 from tray_racing_b200 import cuda, host
 
 scene = sys.argv[1] if len(sys.argv) > 1 else "hairball"
-knobs = eval(sys.argv[2]) if len(sys.argv) > 2 else {"TRAY_CUDA_NARROW_MAX": [0, 4]}
+knobs = eval(sys.argv[2]) if len(sys.argv) > 2 else {"TRAY_CUDA_REFILL_MIN": [4, 6]}
 m = host.Mesh.generate(scene, 3, 1.0)
 p = host.PackedScene(m)
 w, h = 1920, 1080

@@ -38,18 +38,6 @@ constexpr int BLOCK_THREADS = TRAY_BLOCK_THREADS;
 #ifndef TRAY_STACK_SMEM
 #define TRAY_STACK_SMEM 12
 #endif
-#ifndef TRAY_STK_PTX
-#define TRAY_STK_PTX 1       // traversal stack in a PTX-declared shared array (see trace_kernel)
-#endif
-#ifndef TRAY_PUSH_LATE
-#define TRAY_PUSH_LATE 1     // the node step pushes the remaining siblings AFTER it has issued the node fetch
-#endif
-#ifndef TRAY_MASK_IMAD
-#define TRAY_MASK_IMAD 1     // hit-mask accumulation as a predicated IMAD (FMA pipe) instead of a LOP3 (ALU pipe): +1.1 % (profiles/experiments/r2_pipe_balance_ab.log)
-#endif
-#ifndef TRAY_TRI2
-#define TRAY_TRI2 1          // two triangles of a lane's pending group per triangle step (bit-exact; -2.5 % frame time, profiles/experiments/r2_ab_*)
-#endif
 constexpr int STACK_SMEM = TRAY_STACK_SMEM;      // entries per thread in shared memory
 constexpr int STACK_SPILL = 48 - STACK_SMEM;     // further entries per thread in local memory (total 48 > obvhs' 32, cwbvh.rs:88)
 constexpr unsigned FULL = 0xffffffffu;
@@ -61,18 +49,6 @@ constexpr uint32_t WIDE_BIT = 0x40000000u;       // trace_kernel: bit 30 of a la
 constexpr float F32_MAX_ = 3.402823466e+38f;
 constexpr float F32_EPS_ = 1.1920929e-7f;     // sampling.hlsl:3
 constexpr float BOX_EPS_ = 0.0001f;           // query.hlsl:274
-#ifndef TRAY_I2F_Z
-#define TRAY_I2F_Z 1
-#endif
-#ifndef TRAY_I2F_Y
-#define TRAY_I2F_Y 2         // r2: with the slot-space node test the ALU pipe is the node test's bottleneck again; all y-plane bytes through
-#endif                       //     I2F.U8 as well (32 conversions per node on the XU pipe) is the balance point: 24 -> +1.6 %, 32 -> +3.1 %, 40 -> -1.5 %
-#ifndef TRAY_I2F_X
-#define TRAY_I2F_X 0
-#endif
-constexpr int I2F_X = TRAY_I2F_X;             // the same for the x-plane bytes (lane kernel only): measured slower, the XU pipe saturates
-constexpr int I2F_Y = TRAY_I2F_Y;             // 0: no y-plane bytes via I2F.U8, 1: children 0-3 only, 2: all children
-constexpr bool I2F_Z = TRAY_I2F_Z != 0;       // convert the z-plane bytes on the XU pipe (I2F.U8) instead of PRMT+bias
 
 struct FrameParams {
     tray_view view;
@@ -99,11 +75,11 @@ struct TraceParams {
     uint32_t* __restrict__ cursor;            // work cursor
     unsigned long long* __restrict__ counters;// rays, nodes, tris, instances, hits (COUNT builds)
     uint32_t* __restrict__ overflow;
-    uint2* __restrict__ spill;                // pooled kernel: global scratch for stack entries past the shared-memory ones
+    unsigned long long* __restrict__ dev_log; // -DTRAY_EXIT_LOG / -DTRAY_STEP_CLOCK builds: per-warp records
     uint32_t k4b;                             // 0x4B000000, passed at run time (see byte_f32)
     uint32_t force_exact;                     // scene has node scales >= 2^40: always take the unfused node test
     float zero;                               // 0.0f, passed at run time (see child_test_fast)
-    uint32_t one;                             // 1, passed at run time (TRAY_MASK_IMAD: keeps the mask accumulation an IMAD on the FMA pipe)
+    uint32_t one;                             // 1, passed at run time: keeps the hit-mask accumulation an IMAD on the FMA pipe (see child_test_fast)
     uint32_t refill_min;                      // idle lanes needed before a partial warp refills
     uint32_t tri_weight;                      // vote: triangle phase when n_tri * tri_weight >= n_node
     uint32_t variant;                         // MODE 1 kernels only: TRAY_VARIANT_* switches (tray_cuda_scene_set_variant)
@@ -149,14 +125,6 @@ template <int J> __device__ __forceinline__ uint32_t byte_u32(uint32_t w) {
     return r;
 }
 
-// Optional L1 prefetch of the record a lane will need on its NEXT step, issued as soon as the step that decides it
-// ends.  MEASURED SLOWER on B200 (hairball primary 0.968 vs 0.906 ms, kitchen bounce 0.96 vs 0.60 ms): the extra
-// address arithmetic costs issue slots and the two 128-byte line fills per node evict useful L1 lines.  Off.
-#ifndef TRAY_PREFETCH
-#define TRAY_PREFETCH 0
-#endif
-__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" :: "l"(p)); }
-
 // dev instrumentation (-DTRAY_STEP_CLOCK, tests/tools/step_clock.py): where do the cycles of one dependent step go?
 #ifdef TRAY_STEP_CLOCK
 __device__ __forceinline__ long long clk() { long long c; asm volatile("mov.u64 %0, %%clock64;" : "=l"(c)); return c; }
@@ -193,60 +161,6 @@ __device__ __forceinline__ void prepare_ray(RayConst& r, float ox, float oy, flo
     r.wide = !(fmaxf(fmaxf(fabsf(r.ix), fabsf(r.iy)), fabsf(r.iz)) < 1.8446744e19f);
 }
 
-// ---- node test: CwBvhNode::intersect_ray, twin query.hlsl:213-303 -------------------------------
-template <int J>
-__device__ __forceinline__ uint32_t child_test(uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
-                                               float ax, float ay, float az, float bx, float by, float bz, float tmax,
-                                               uint32_t child_bits4, uint32_t bit_index4, uint32_t k4b, float box_tmin) {
-    // tmin3 = q_near * adj_inv + adj_org, tmax3 = q_far * adj_inv + adj_org: mul, then add (query.hlsl:285-286)
-    const float tnx = add(mul(byte_f32<J>(nx, k4b), ax), bx), tfx = add(mul(byte_f32<J>(fx, k4b), ax), bx);
-    const float tny = add(mul(byte_f32<J>(ny, k4b), ay), by), tfy = add(mul(byte_f32<J>(fy, k4b), ay), by);
-    const float tnz = add(mul(byte_f32<J>(nz, k4b), az), bz), tfz = add(mul(byte_f32<J>(fz, k4b), az), bz);
-    const float tmin = fmaxf(fmaxf(fmaxf(tnx, tny), tnz), box_tmin);      // query.hlsl:288
-    const float tfar = fminf(fminf(fminf(tfx, tfy), tfz), tmax);          // query.hlsl:289
-    // child_bits << bit_index (query.hlsl:291-298); bit_index bytes are < 32, so the shifter's wrap is harmless
-    const uint32_t contrib = byte_u32<J>(child_bits4) << ((bit_index4 >> (8 * J)) & 31u);
-    return tmin <= tfar ? contrib : 0u;
-}
-
-// `box_tmin` / `divide`: the slab test's lower clamp and the HLSL's divide-by-direction form (query.hlsl:237-242) — MODE 1 only
-__device__ __forceinline__ uint32_t node_test(const RayConst& r, float tmax, const uint4& n0, const uint4& n1,
-                                              const uint4& n2, const uint4& n3, const uint4& n4, uint32_t k4b,
-                                              float box_tmin = BOX_EPS_, bool divide = false) {
-    const uint32_t e = n0.w;
-    // adj_inv = 2^(e-127) * inv_dir ; adj_org = (p - origin) * inv_dir  (CPU path: cached reciprocal; SURVEY §8c vi)
-    const float sx_ = __uint_as_float((e & 0xffu) << 23), sy_ = __uint_as_float(((e >> 8) & 0xffu) << 23), sz_ = __uint_as_float(((e >> 16) & 0xffu) << 23);
-    const float px_ = sub(__uint_as_float(n0.x), r.ox), py_ = sub(__uint_as_float(n0.y), r.oy), pz_ = sub(__uint_as_float(n0.z), r.oz);
-    const float ax = divide ? __fdiv_rn(sx_, r.dx) : mul(sx_, r.ix);
-    const float ay = divide ? __fdiv_rn(sy_, r.dy) : mul(sy_, r.iy);
-    const float az = divide ? __fdiv_rn(sz_, r.dz) : mul(sz_, r.iz);
-    const float bx = divide ? __fdiv_rn(px_, r.dx) : mul(px_, r.ix);
-    const float by = divide ? __fdiv_rn(py_, r.dy) : mul(py_, r.iy);
-    const float bz = divide ? __fdiv_rn(pz_, r.dz) : mul(pz_, r.iz);
-    const bool sx = r.dx < 0.0f, sy = r.dy < 0.0f, sz = r.dz < 0.0f;
-    uint32_t mask = 0;
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-        const uint32_t meta4 = i == 0 ? n1.z : n1.w;
-        const uint32_t is_inner4 = (meta4 & (meta4 << 1)) & 0x10101010u;          // query.hlsl:251
-        const uint32_t inner_mask4 = (is_inner4 >> 4) * 0xffu;
-        const uint32_t bit_index4 = (meta4 ^ (r.oct_inv4 & inner_mask4)) & 0x1f1f1f1fu;
-        const uint32_t child_bits4 = (meta4 >> 5) & 0x07070707u;
-        const uint32_t lox = i == 0 ? n2.x : n2.y, hix = i == 0 ? n2.z : n2.w;
-        const uint32_t loy = i == 0 ? n3.x : n3.y, hiy = i == 0 ? n3.z : n3.w;
-        const uint32_t loz = i == 0 ? n4.x : n4.y, hiz = i == 0 ? n4.z : n4.w;
-        const uint32_t nx = sx ? hix : lox, fx = sx ? lox : hix;                   // query.hlsl:266-273
-        const uint32_t ny = sy ? hiy : loy, fy = sy ? loy : hiy;
-        const uint32_t nz = sz ? hiz : loz, fz = sz ? loz : hiz;
-        mask |= child_test<0>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, bit_index4, k4b, box_tmin);
-        mask |= child_test<1>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, bit_index4, k4b, box_tmin);
-        mask |= child_test<2>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, bit_index4, k4b, box_tmin);
-        mask |= child_test<3>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, bit_index4, k4b, box_tmin);
-    }
-    return mask;
-}
-
-
 // ---- packed f32x2 helpers (Blackwell FFMA2 / FADD2: two IEEE-rounded results per issue slot) --------
 __device__ __forceinline__ unsigned long long pack2(uint32_t lo, uint32_t hi) {
     unsigned long long r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "r"(lo), "r"(hi)); return r;
@@ -264,83 +178,11 @@ __device__ __forceinline__ unsigned long long fadd2(unsigned long long a, unsign
 template <int J> __device__ __forceinline__ uint32_t byte_biased(uint32_t w, uint32_t k4b) {   // 0x4B0000bb = 2^23 + byte
     uint32_t r; asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(w), "r"(k4b), "n"(0x7440 + J)); return r;
 }
-
-// Fast node test, BIT-IDENTICAL to node_test: with f = 2^23 + q (exact, straight out of PRMT) and C = 2^23 * A
-// (exact: a power-of-two scaling),  fma(f, A, -C) rounds the exact real value (f - 2^23) * A = q * A once, i.e. it
-// IS fl(q * A) — the conversion FADD and the FMUL collapse into one FFMA with no change of rounding.  The
-// following "+ adj_org" stays a separate, separately rounded add (query.hlsl:285-286).  (near, far) of one child
-// and axis travel as an f32x2 pair: FFMA2 + FADD2 = 2 issue slots for what took 6.
-// Requires 2^23 * A finite: rays with |1/d| >= 2^64 take node_test instead (RayConst::wide).
 // byte J of w as an exact float on the conversion (XU) pipe: I2F.U8 with a byte selector.  Quarter-rate, but
 // that pipe is otherwise idle here, so a few conversions per child run there concurrently with the ALU pipe.
 template <int J> __device__ __forceinline__ float byte_i2f(uint32_t w) { return (float)((w >> (8 * J)) & 0xffu); }
 
-template <int J, bool YI2F>
-__device__ __forceinline__ void child_test_fast(uint32_t& mask, uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
-                                                unsigned long long AX, unsigned long long AY, unsigned long long AZ,
-                                                unsigned long long CX, unsigned long long CY, unsigned long long CZ,
-                                                unsigned long long BX, unsigned long long BY, unsigned long long BZ,
-                                                unsigned long long Z0, float tmax, uint32_t child_bits4, uint32_t bit_index4, uint32_t k4b) {
-    float tnx, tfx, tny, tfy, tnz, tfz;
-    unpack2f(fadd2(ffma2(pack2(byte_biased<J>(nx, k4b), byte_biased<J>(fx, k4b)), AX, CX), BX), tnx, tfx);
-    if (YI2F) unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(ny), byte_i2f<J>(fy)), AY, Z0), BY), tny, tfy);
-    else unpack2f(fadd2(ffma2(pack2(byte_biased<J>(ny, k4b), byte_biased<J>(fy, k4b)), AY, CY), BY), tny, tfy);
-    if (I2F_Z) {
-        // z pair through I2F.U8: q is already the plain float, fma(q, A, 0) = fl(q * A)  (Z0 is a run-time zero so
-        // that the assembler cannot turn fma+add back into one fused op)
-        unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(nz), byte_i2f<J>(fz)), AZ, Z0), BZ), tnz, tfz);
-    } else {
-        unpack2f(fadd2(ffma2(pack2(byte_biased<J>(nz, k4b), byte_biased<J>(fz, k4b)), AZ, CZ), BZ), tnz, tfz);
-    }
-    const float tmin = fmaxf(fmaxf(fmaxf(tnx, tny), tnz), BOX_EPS_);
-    const float tfar = fminf(fminf(fminf(tfx, tfy), tfz), tmax);
-    const uint32_t contrib = byte_u32<J>(child_bits4) << ((bit_index4 >> (8 * J)) & 31u);
-    // if (tmin <= tfar) mask |= contrib   — as one compare + one predicated OR
-    asm("{.reg .pred p; setp.le.f32 p, %1, %2; @p or.b32 %0, %0, %3;}" : "+r"(mask) : "f"(tmin), "f"(tfar), "r"(contrib));
-}
-
-struct NodeConsts { unsigned long long AX, AY, AZ, CX, CY, CZ, BX, BY, BZ, Z0; };
-
-template <int I>
-__device__ __forceinline__ void node_half_fast(uint32_t& mask, const RayConst& r, float tmax, const NodeConsts& c, uint32_t meta4,
-                                               uint32_t lox, uint32_t hix, uint32_t loy, uint32_t hiy, uint32_t loz, uint32_t hiz,
-                                               uint32_t k4b) {
-    const uint32_t is_inner4 = (meta4 & (meta4 << 1)) & 0x10101010u;                 // query.hlsl:251
-    const uint32_t inner_mask4 = (is_inner4 >> 4) * 0xffu;
-    const uint32_t bit_index4 = (meta4 ^ (r.oct_inv4 & inner_mask4)) & 0x1f1f1f1fu;
-    const uint32_t child_bits4 = (meta4 >> 5) & 0x07070707u;
-    const bool sx = r.dx < 0.0f, sy = r.dy < 0.0f, sz = r.dz < 0.0f;
-    const uint32_t nx = sx ? hix : lox, fx = sx ? lox : hix;                          // query.hlsl:266-273
-    const uint32_t ny = sy ? hiy : loy, fy = sy ? loy : hiy;
-    const uint32_t nz = sz ? hiz : loz, fz = sz ? loz : hiz;
-    constexpr bool YI = I2F_Y == 2 || (I2F_Y == 1 && I == 0);
-    child_test_fast<0, YI>(mask, nx, fx, ny, fy, nz, fz, c.AX, c.AY, c.AZ, c.CX, c.CY, c.CZ, c.BX, c.BY, c.BZ, c.Z0, tmax, child_bits4, bit_index4, k4b);
-    child_test_fast<1, YI>(mask, nx, fx, ny, fy, nz, fz, c.AX, c.AY, c.AZ, c.CX, c.CY, c.CZ, c.BX, c.BY, c.BZ, c.Z0, tmax, child_bits4, bit_index4, k4b);
-    child_test_fast<2, YI>(mask, nx, fx, ny, fy, nz, fz, c.AX, c.AY, c.AZ, c.CX, c.CY, c.CZ, c.BX, c.BY, c.BZ, c.Z0, tmax, child_bits4, bit_index4, k4b);
-    child_test_fast<3, YI>(mask, nx, fx, ny, fy, nz, fz, c.AX, c.AY, c.AZ, c.CX, c.CY, c.CZ, c.BX, c.BY, c.BZ, c.Z0, tmax, child_bits4, bit_index4, k4b);
-}
-
-__device__ __forceinline__ uint32_t node_test_fast(const RayConst& r, float tmax, const uint4& n0, const uint4& n1,
-                                                   const uint4& n2, const uint4& n3, const uint4& n4, uint32_t k4b, float zero) {
-    const uint32_t e = n0.w;
-    const float ax = mul(__uint_as_float((e & 0xffu) << 23), r.ix);
-    const float ay = mul(__uint_as_float(((e >> 8) & 0xffu) << 23), r.iy);
-    const float az = mul(__uint_as_float(((e >> 16) & 0xffu) << 23), r.iz);
-    const float bx = mul(sub(__uint_as_float(n0.x), r.ox), r.ix);
-    const float by = mul(sub(__uint_as_float(n0.y), r.oy), r.iy);
-    const float bz = mul(sub(__uint_as_float(n0.z), r.oz), r.iz);
-    const float cx = mul(ax, -8388608.0f), cy = mul(ay, -8388608.0f), cz = mul(az, -8388608.0f);   // -2^23 * A, exact
-    NodeConsts c;
-    c.AX = pack2f(ax, ax); c.AY = pack2f(ay, ay); c.AZ = pack2f(az, az);
-    c.CX = pack2f(cx, cx); c.CY = pack2f(cy, cy); c.CZ = pack2f(cz, cz);
-    c.BX = pack2f(bx, bx); c.BY = pack2f(by, by); c.BZ = pack2f(bz, bz); c.Z0 = pack2f(zero, zero);
-    uint32_t mask = 0;
-    node_half_fast<0>(mask, r, tmax, c, n1.z, n2.x, n2.z, n3.x, n3.z, n4.x, n4.z, k4b);
-    node_half_fast<1>(mask, r, tmax, c, n1.w, n2.y, n2.w, n3.y, n3.w, n4.y, n4.w, k4b);
-    return mask;
-}
-
-// ---- node test in slot space ------------------------------------------------------------------------
+// ---- node test: CwBvhNode::intersect_ray, twin query.hlsl:213-303, in slot space ------------------------------
 // The lane kernel keeps the top byte of the hit mask / node group word in SLOT space: an inner child (bit_index = 24 + slot,
 // query.hlsl:251-262) sets bit 24 + slot, WITHOUT the octant XOR.  That XOR exists so that firstbithigh (query.hlsl:358) finds
 // the hit child nearest along the ray, and `slot = bit ^ oct_inv` (:370) undoes it; here the pair becomes ONE lookup when the
@@ -363,11 +205,11 @@ __device__ __forceinline__ void child_order_fill(uint8_t* lut, unsigned tid, uns
     }
 }
 
-// exact (unfused) form: CwBvhNode::intersect_ray, twin query.hlsl:213-303 (wide rays, huge node scales, MODE 1)
+// exact (unfused) form (wide rays, huge node scales, MODE 1)
 template <int J>
-__device__ __forceinline__ uint32_t child_test_s(uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
-                                                 float ax, float ay, float az, float bx, float by, float bz, float tmax,
-                                                 uint32_t child_bits4, uint32_t meta4, uint32_t k4b, float box_tmin) {
+__device__ __forceinline__ uint32_t child_test(uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
+                                               float ax, float ay, float az, float bx, float by, float bz, float tmax,
+                                               uint32_t child_bits4, uint32_t meta4, uint32_t k4b, float box_tmin) {
     const float tnx = add(mul(byte_f32<J>(nx, k4b), ax), bx), tfx = add(mul(byte_f32<J>(fx, k4b), ax), bx);
     const float tny = add(mul(byte_f32<J>(ny, k4b), ay), by), tfy = add(mul(byte_f32<J>(fy, k4b), ay), by);
     const float tnz = add(mul(byte_f32<J>(nz, k4b), az), bz), tfz = add(mul(byte_f32<J>(fz, k4b), az), bz);
@@ -376,8 +218,9 @@ __device__ __forceinline__ uint32_t child_test_s(uint32_t nx, uint32_t fx, uint3
     const uint32_t contrib = byte_u32<J>(child_bits4) << ((meta4 >> (8 * J)) & 31u);       // query.hlsl:291-298, slot space
     return tmin <= tfar ? contrib : 0u;
 }
-__device__ __forceinline__ uint32_t node_test_s(const RayConst& r, float tmax, const uint4& n0, const uint4& n1, const uint4& n2,
-                                                const uint4& n3, const uint4& n4, uint32_t k4b, float box_tmin = BOX_EPS_, bool divide = false) {
+// `box_tmin` / `divide`: the slab test's lower clamp and the HLSL's divide-by-direction form (query.hlsl:237-242) — MODE 1 only
+__device__ __forceinline__ uint32_t node_test(const RayConst& r, float tmax, const uint4& n0, const uint4& n1, const uint4& n2,
+                                              const uint4& n3, const uint4& n4, uint32_t k4b, float box_tmin = BOX_EPS_, bool divide = false) {
     const uint32_t e = n0.w;
     const float sx_ = __uint_as_float((e & 0xffu) << 23), sy_ = __uint_as_float(((e >> 8) & 0xffu) << 23), sz_ = __uint_as_float(((e >> 16) & 0xffu) << 23);
     const float px_ = sub(__uint_as_float(n0.x), r.ox), py_ = sub(__uint_as_float(n0.y), r.oy), pz_ = sub(__uint_as_float(n0.z), r.oz);
@@ -399,52 +242,54 @@ __device__ __forceinline__ uint32_t node_test_s(const RayConst& r, float tmax, c
         const uint32_t nx = sx ? hix : lox, fx = sx ? lox : hix;                   // query.hlsl:266-273
         const uint32_t ny = sy ? hiy : loy, fy = sy ? loy : hiy;
         const uint32_t nz = sz ? hiz : loz, fz = sz ? loz : hiz;
-        mask |= child_test_s<0>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
-        mask |= child_test_s<1>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
-        mask |= child_test_s<2>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
-        mask |= child_test_s<3>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
+        mask |= child_test<0>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
+        mask |= child_test<1>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
+        mask |= child_test<2>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
+        mask |= child_test<3>(nx, fx, ny, fy, nz, fz, ax, ay, az, bx, by, bz, tmax, child_bits4, meta4, k4b, box_tmin);
     }
     return mask;
 }
 
-// fused form (the arithmetic of child_test_fast, bit-identical to node_test_s)
-template <int J, bool YI2F, bool XI2F>
-__device__ __forceinline__ void child_test_fast_s(uint32_t& mask, uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
-                                                  const NodeConsts& c, float tmax, uint32_t child_bits4, uint32_t meta4, uint32_t k4b, uint32_t one) {
+// Fused form, BIT-IDENTICAL to node_test: with f = 2^23 + q (exact, straight out of PRMT) and C = 2^23 * A (exact: a
+// power-of-two scaling),  fma(f, A, -C) rounds the exact real value (f - 2^23) * A = q * A once, i.e. it IS fl(q * A) — the
+// conversion FADD and the FMUL collapse into one FFMA with no change of rounding.  The following "+ adj_org" stays a separate,
+// separately rounded add (query.hlsl:285-286).  (near, far) of one child and axis travel as an f32x2 pair: FFMA2 + FADD2 = 2
+// issue slots for what took 6.
+// Requires 2^23 * A finite: rays with |1/d| >= 2^64 take node_test instead (RayConst::wide).
+// Pipe balance: the ALU pipe is the node test's bottleneck, so the y- and z-plane bytes go through I2F.U8 on the XU pipe instead
+// of PRMT (32 conversions per node is the balance point: 24 -> +1.6 %, 32 -> +3.1 %, 40 -> -1.5 %; the x-plane bytes as well is
+// slower, the XU pipe saturates).  There q is already the plain float and fma(q, A, 0) = fl(q * A)  (Z0 is a run-time zero so
+// that the assembler cannot turn fma+add back into one fused op).
+struct NodeConsts { unsigned long long AX, AY, AZ, CX, BX, BY, BZ, Z0; };
+
+template <int J>
+__device__ __forceinline__ void child_test_fast(uint32_t& mask, uint32_t nx, uint32_t fx, uint32_t ny, uint32_t fy, uint32_t nz, uint32_t fz,
+                                                const NodeConsts& c, float tmax, uint32_t child_bits4, uint32_t meta4, uint32_t k4b, uint32_t one) {
     float tnx, tfx, tny, tfy, tnz, tfz;
-    if (XI2F) unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(nx), byte_i2f<J>(fx)), c.AX, c.Z0), c.BX), tnx, tfx);
-    else unpack2f(fadd2(ffma2(pack2(byte_biased<J>(nx, k4b), byte_biased<J>(fx, k4b)), c.AX, c.CX), c.BX), tnx, tfx);
-    if (YI2F) unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(ny), byte_i2f<J>(fy)), c.AY, c.Z0), c.BY), tny, tfy);
-    else unpack2f(fadd2(ffma2(pack2(byte_biased<J>(ny, k4b), byte_biased<J>(fy, k4b)), c.AY, c.CY), c.BY), tny, tfy);
-    if (I2F_Z) unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(nz), byte_i2f<J>(fz)), c.AZ, c.Z0), c.BZ), tnz, tfz);
-    else unpack2f(fadd2(ffma2(pack2(byte_biased<J>(nz, k4b), byte_biased<J>(fz, k4b)), c.AZ, c.CZ), c.BZ), tnz, tfz);
+    unpack2f(fadd2(ffma2(pack2(byte_biased<J>(nx, k4b), byte_biased<J>(fx, k4b)), c.AX, c.CX), c.BX), tnx, tfx);
+    unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(ny), byte_i2f<J>(fy)), c.AY, c.Z0), c.BY), tny, tfy);
+    unpack2f(fadd2(ffma2(pack2f(byte_i2f<J>(nz), byte_i2f<J>(fz)), c.AZ, c.Z0), c.BZ), tnz, tfz);
     const float tmin = fmaxf(fmaxf(fmaxf(tnx, tny), tnz), BOX_EPS_);
     const float tfar = fminf(fminf(fminf(tfx, tfy), tfz), tmax);
     const uint32_t contrib = byte_u32<J>(child_bits4) << ((meta4 >> (8 * J)) & 31u);
-#if TRAY_MASK_IMAD
-    // the children's bits are disjoint, so OR = ADD = contrib * 1 + mask: an IMAD on the FMA pipe instead of a LOP3 on the ALU pipe
+    // if (tmin <= tfar) mask |= contrib.  The children's bits are disjoint, so OR = ADD = contrib * 1 + mask: a predicated IMAD on
+    // the FMA pipe instead of a LOP3 on the ALU pipe, +1.1 % (profiles/experiments/r2_pipe_balance_ab.log)
     asm("{.reg .pred p; setp.le.f32 p, %1, %2; @p mad.lo.u32 %0, %3, %4, %0;}" : "+r"(mask) : "f"(tmin), "f"(tfar), "r"(contrib), "r"(one));
-#else
-    asm("{.reg .pred p; setp.le.f32 p, %1, %2; @p or.b32 %0, %0, %3;}" : "+r"(mask) : "f"(tmin), "f"(tfar), "r"(contrib));
-#endif
 }
-template <int I>
-__device__ __forceinline__ void node_half_fast_s(uint32_t& mask, const RayConst& r, float tmax, const NodeConsts& c, uint32_t meta4,
-                                                 uint32_t lox, uint32_t hix, uint32_t loy, uint32_t hiy, uint32_t loz, uint32_t hiz, uint32_t k4b, uint32_t one) {
+__device__ __forceinline__ void node_half_fast(uint32_t& mask, const RayConst& r, float tmax, const NodeConsts& c, uint32_t meta4,
+                                               uint32_t lox, uint32_t hix, uint32_t loy, uint32_t hiy, uint32_t loz, uint32_t hiz, uint32_t k4b, uint32_t one) {
     const uint32_t child_bits4 = (meta4 >> 5) & 0x07070707u;
     const bool sx = r.dx < 0.0f, sy = r.dy < 0.0f, sz = r.dz < 0.0f;
     const uint32_t nx = sx ? hix : lox, fx = sx ? lox : hix;                          // query.hlsl:266-273
     const uint32_t ny = sy ? hiy : loy, fy = sy ? loy : hiy;
     const uint32_t nz = sz ? hiz : loz, fz = sz ? loz : hiz;
-    constexpr bool YI = I2F_Y == 2 || (I2F_Y == 1 && I == 0);
-    constexpr bool XI = I2F_X == 2 || (I2F_X == 1 && I == 0);
-    child_test_fast_s<0, YI, XI>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
-    child_test_fast_s<1, YI, XI>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
-    child_test_fast_s<2, YI, XI>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
-    child_test_fast_s<3, YI, XI>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
+    child_test_fast<0>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
+    child_test_fast<1>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
+    child_test_fast<2>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
+    child_test_fast<3>(mask, nx, fx, ny, fy, nz, fz, c, tmax, child_bits4, meta4, k4b, one);
 }
-__device__ __forceinline__ uint32_t node_test_fast_s(const RayConst& r, float tmax, const uint4& n0, const uint4& n1, const uint4& n2,
-                                                     const uint4& n3, const uint4& n4, uint32_t k4b, float zero, uint32_t one) {
+__device__ __forceinline__ uint32_t node_test_fast(const RayConst& r, float tmax, const uint4& n0, const uint4& n1, const uint4& n2,
+                                                   const uint4& n3, const uint4& n4, uint32_t k4b, float zero, uint32_t one) {
     const uint32_t e = n0.w;
     const float ax = mul(__uint_as_float((e & 0xffu) << 23), r.ix);
     const float ay = mul(__uint_as_float(((e >> 8) & 0xffu) << 23), r.iy);
@@ -452,14 +297,13 @@ __device__ __forceinline__ uint32_t node_test_fast_s(const RayConst& r, float tm
     const float bx = mul(sub(__uint_as_float(n0.x), r.ox), r.ix);
     const float by = mul(sub(__uint_as_float(n0.y), r.oy), r.iy);
     const float bz = mul(sub(__uint_as_float(n0.z), r.oz), r.iz);
-    const float cx = mul(ax, -8388608.0f), cy = mul(ay, -8388608.0f), cz = mul(az, -8388608.0f);   // -2^23 * A, exact
+    const float cx = mul(ax, -8388608.0f);                                                          // -2^23 * A, exact
     NodeConsts c;
-    c.AX = pack2f(ax, ax); c.AY = pack2f(ay, ay); c.AZ = pack2f(az, az);
-    c.CX = pack2f(cx, cx); c.CY = pack2f(cy, cy); c.CZ = pack2f(cz, cz);
+    c.AX = pack2f(ax, ax); c.AY = pack2f(ay, ay); c.AZ = pack2f(az, az); c.CX = pack2f(cx, cx);
     c.BX = pack2f(bx, bx); c.BY = pack2f(by, by); c.BZ = pack2f(bz, bz); c.Z0 = pack2f(zero, zero);
     uint32_t mask = 0;
-    node_half_fast_s<0>(mask, r, tmax, c, n1.z, n2.x, n2.z, n3.x, n3.z, n4.x, n4.z, k4b, one);
-    node_half_fast_s<1>(mask, r, tmax, c, n1.w, n2.y, n2.w, n3.y, n3.w, n4.y, n4.w, k4b, one);
+    node_half_fast(mask, r, tmax, c, n1.z, n2.x, n2.z, n3.x, n3.z, n4.x, n4.z, k4b, one);
+    node_half_fast(mask, r, tmax, c, n1.w, n2.y, n2.w, n3.y, n3.w, n4.y, n4.w, k4b, one);
     return mask;
 }
 
@@ -764,10 +608,7 @@ __device__ __forceinline__ bool poll_hit(const tray_hit* src, float2& ph) {     
 // hand at once; nothing was postponed, nothing mismatched, and the extra vote cost 3 %.  profiles/experiments/r2_relaxed_*.)
 template <bool TLAS, bool COUNT, int TRI_STRIDE, bool ANYHIT = false, bool FRAME = false, int MODE = 0>
 __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(const __grid_constant__ TraceParams P) {
-#if !TRAY_STK_PTX
-    __shared__ uint2 s_stack[STACK_SMEM * BLOCK_THREADS];
-#endif
-    __shared__ uint8_t s_lut[LUT_BYTES];          // child_order[oct_inv][hit byte] (see node_test_s)
+    __shared__ uint8_t s_lut[LUT_BYTES];          // child_order[oct_inv][hit byte] (see node_test)
     uint2 spill[STACK_SPILL];
     child_order_fill(s_lut, threadIdx.x, BLOCK_THREADS);
     __syncthreads();
@@ -779,23 +620,18 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     float best_t = 0.f;
     uint32_t best_prim = INVALID;
     uint32_t cur_x = 0, cur_y = 0, tri_x = 0, tri_y = 0;
-    // the stack pointer IS the byte offset of the lane's next free entry in s_stack ([entry][thread]): depth * SP_STEP + thread * 8
+    // the stack pointer IS the byte offset of the lane's next free entry in tray_stack_mem ([entry][thread]): depth * SP_STEP + thread * 8
     // (one register instead of a depth and a per-thread base address)
     constexpr uint32_t SP_STEP = BLOCK_THREADS * 8u, SP_SMEM_END = STACK_SMEM * SP_STEP, SP_END = (STACK_SMEM + STACK_SPILL) * SP_STEP;
     uint32_t sp = threadIdx.x * 8u;
-#if TRAY_STK_PTX
     // the stack lives in a shared-memory array declared in PTX, so that its address is a plain CTA-local offset that ptxas keeps in a
     // uniform register (STS.64 [R + UR]) — the address of a C++ __shared__ array goes through the generic->shared conversion, which
     // on sm_90+ reads SR_CgaCtaId and rebuilds the shared window base (S2R + MOV + LEA + IADD) at EVERY push and pop: +2.3 % on C3,
-    // +1.2 % on C1 together with the late push (profiles/experiments/r2_push_late_ab.log)
+    // +1.2 % on C1 together with the late push of the node step (profiles/experiments/r2_push_late_ab.log)
     uint32_t stk_base;
     asm volatile(".shared .align 16 .b8 tray_stack_mem[%1];\n\tmov.u32 %0, tray_stack_mem;" : "=r"(stk_base) : "n"(STACK_SMEM * BLOCK_THREADS * 8));
     auto stk_store = [&](uint32_t off, uint32_t x, uint32_t y) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" :: "r"(stk_base + off), "r"(x), "r"(y) : "memory"); };
     auto stk_load = [&](uint32_t off) { uint2 e; asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(e.x), "=r"(e.y) : "r"(stk_base + off) : "memory"); return e; };
-#else
-    auto stk_store = [&](uint32_t off, uint32_t x, uint32_t y) { *reinterpret_cast<uint2*>(reinterpret_cast<char*>(s_stack) + off) = make_uint2(x, y); };
-    auto stk_load = [&](uint32_t off) { return *reinterpret_cast<uint2*>(reinterpret_cast<char*>(s_stack) + off); };
-#endif
     uint32_t tlas_sp = INVALID, bvh_off = 0;
     uint32_t ray_idx = 0;
     bool exhausted = false;                      // warp-uniform
@@ -876,9 +712,9 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                 if ((int)lane == leader) base = atomicAdd(P.cursor, n_idle);
                 base = __shfl_sync(FULL, base, leader);
 #ifdef TRAY_EXIT_LOG
-                if (base + n_idle >= n_work && !exhausted && P.spill && lane == 0) {   // ... and when it ran dry
+                if (base + n_idle >= n_work && !exhausted && P.dev_log && lane == 0) {   // ... and when it ran dry
                     unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-                    ((unsigned long long*)P.spill)[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5))] = t;
+                    P.dev_log[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5))] = t;
                 }
 #endif
                 if (base + n_idle >= n_work) exhausted = true;
@@ -984,9 +820,9 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         }
 
 #ifdef TRAY_EXIT_LOG
-        if (exhausted && P.spill) {       // first time the warp is down to <= 8 / 4 / 2 / 1 rays after the cursor ran dry
+        if (exhausted && P.dev_log) {       // first time the warp is down to <= 8 / 4 / 2 / 1 rays after the cursor ran dry
             const int nb = __popc(busy);
-            unsigned long long* rec = (unsigned long long*)P.spill + 6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
+            unsigned long long* rec = P.dev_log + 6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
             if (lane == 0 && nb <= 8) {
                 unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
                 if (rec[2] == 0) rec[2] = t;
@@ -1003,21 +839,20 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         if (!tri_phase) {
             if (want_node) {
                 const uint32_t hits_imask = cur_y;
-                uint32_t slot;                                                                 // query.hlsl:358 + :370 in one lookup (see node_test_s)
+                uint32_t slot;                                                                 // query.hlsl:358 + :370 in one lookup (see node_test)
                 asm("ld.shared.u8 %0, [%1];" : "=r"(slot) : "r"(r.lut_off + (hits_imask >> 24)));
                 cur_y = hits_imask ^ (0x01000000u << slot);                                    // :362
-                if (!TRAY_PUSH_LATE && (cur_y & 0xff000000u)) push(cur_x, cur_y);              // :365-368
                 const uint32_t rel = (uint32_t)__popc(hits_imask & ((1u << slot) - 1u));       // :371 (slot < 8: imask bits only)
                 const uint4* np = P.nodes + (size_t)(bvh_off + cur_x + rel) * 5u;              // :373, tlas:383
                 SC(const long long sc_a = clk_after(rel); sc_acc[1] += sc_a - sc_voted;)
                 const uint4 n0 = __ldg(np), n1 = __ldg(np + 1), n2 = __ldg(np + 2), n3 = __ldg(np + 3), n4 = __ldg(np + 4);
-                if (TRAY_PUSH_LATE && (cur_y & 0xff000000u)) push(cur_x, cur_y);               // :365-368, in the shadow of the node fetch
+                if (cur_y & 0xff000000u) push(cur_x, cur_y);                                   // :365-368, in the shadow of the node fetch
                 SC(const long long sc_b = clk_after(n0.x ^ n1.x ^ n2.x ^ n3.x ^ n4.x); sc_acc[2] += sc_b - sc_a;)
                 TRAY_CNT(nodes);
-                uint32_t hitmask;                                                              // slot space (see node_test_s)
-                if (MODE == 1) hitmask = node_test_s(r, best_t, n0, n1, n2, n3, n4, k4b, r.box_tmin, (P.variant & TRAY_VARIANT_BOX_DIVIDE) != 0u);
-                else hitmask = ((ray_idx & WIDE_BIT) || P.force_exact) ? node_test_s(r, best_t, n0, n1, n2, n3, n4, k4b)
-                                                : node_test_fast_s(r, best_t, n0, n1, n2, n3, n4, k4b, P.zero, P.one);   // :380
+                uint32_t hitmask;                                                              // slot space (see node_test)
+                if (MODE == 1) hitmask = node_test(r, best_t, n0, n1, n2, n3, n4, k4b, r.box_tmin, (P.variant & TRAY_VARIANT_BOX_DIVIDE) != 0u);
+                else hitmask = ((ray_idx & WIDE_BIT) || P.force_exact) ? node_test(r, best_t, n0, n1, n2, n3, n4, k4b)
+                                                : node_test_fast(r, best_t, n0, n1, n2, n3, n4, k4b, P.zero, P.one);   // :380
                 SC(const long long sc_c = clk_after(hitmask); sc_acc[3] += sc_c - sc_b; sc_n[0]++;)
                 cur_x = n1.x; tri_x = n1.y;                                                    // :383-384
                 cur_y = (hitmask & 0xff000000u) | (n0.w >> 24);                                // :386 (top byte: hit inner children, slot space)
@@ -1044,28 +879,25 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     SC({ const uint4 q0 = __ldg(P.tris + (size_t)g * (TRI_STRIDE / 16)), q2 = __ldg(P.tris + (size_t)g * (TRI_STRIDE / 16) + 2);
                          sc_acc[6] -= sc_a; sc_acc[6] += clk_after(q0.x ^ q2.x); })
                     SC(const long long sc_b = clk();)
-#if TRAY_TRI2
                     // Two triangles of the lane's pending group per iteration (82 % of the groups hold >= 2): both records are
                     // fetched together and the two tests run side by side.  The second test's only use of tmax is its final
                     // `tt <= tmax` (query.hlsl:119), so running it against the OLD tmax and comparing with the updated best_t
-                    // afterwards accepts exactly what the sequential order accepts — bit-exact, ties included.
+                    // afterwards accepts exactly what the sequential order accepts — bit-exact, ties included.  -2.5 % frame time
+                    // (profiles/experiments/r2_ab_tri2_*).
                     const bool two = MODE != 1 && tri_y != 0u;
-                    const uint32_t local2 = two ? 31u - (uint32_t)__clz((int)tri_y) : local;
+                    const uint32_t local2 = 31u - (uint32_t)__clz((int)tri_y);                  // read only when `two`
                     const uint32_t g2 = tri_x + local2;
                     if (two) tri_y &= ~(1u << local2);
                     float t2 = __int_as_float(0x7f800000);
                     if (two) t2 = tri_test<TRI_STRIDE, false>(r, best_t, P.tris, g2);
-#endif
                     const float t = tri_test<TRI_STRIDE, MODE == 1>(r, best_t, P.tris, g);
                     // CPU tie rule: first of equal t wins (§8a a11); TRAY_VARIANT_TIE_LAST: the HLSL's `tt <= t` (query.hlsl:120)
                     const bool closer = (MODE == 1 && (P.variant & TRAY_VARIANT_TIE_LAST)) ? (t <= best_t && t < __int_as_float(0x7f800000)) : (t < best_t);
                     if (closer) { best_t = t; best_prim = g; }
-#if TRAY_TRI2
                     if (two && !(ANYHIT && best_prim != INVALID)) {      // (any-hit: the reference never runs the second test after a hit)
                         TRAY_CNT(tris);
                         if (t2 < best_t) { best_t = t2; best_prim = g2; }
                     }
-#endif
                     if (ANYHIT && best_prim != INVALID) { sp &= SP_STEP - 1u; tri_y = 0u; cur_y = 0u; }   // drop the rest of the traversal
                     if (tri_y == 0u && cur_y < 0x01000000u) pop_or_retire();
                     SC(sc_acc[7] += clk_after(cur_y ^ tri_y ^ __float_as_uint(best_t)) - sc_b; sc_n[1]++;)
@@ -1075,16 +907,16 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     }
 
 #ifdef TRAY_STEP_CLOCK
-    if (P.spill && lane == 0) {       // per warp: cycles in [vote, node pre, node load wait, node test, node post, tri pre, tri load wait, tri test+post], steps, total
-        long long* o = (long long*)P.spill + 12 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
+    if (P.dev_log && lane == 0) {     // per warp: cycles in [vote, node pre, node load wait, node test, node post, tri pre, tri load wait, tri test+post], steps, total
+        long long* o = (long long*)P.dev_log + 12 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
         for (int i = 0; i < 8; i++) o[i] = sc_acc[i];
         o[8] = sc_n[0]; o[9] = sc_n[1]; o[10] = clk() - sc_t0; o[11] = 1;
     }
 #endif
 #ifdef TRAY_EXIT_LOG
-    if (P.spill && lane == 0) {       // dev instrumentation (scripts/exit_log.py): when this warp exited (ns)
+    if (P.dev_log && lane == 0) {     // dev instrumentation (scripts/exit_log.py): when this warp exited (ns)
         unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-        ((unsigned long long*)P.spill)[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5)) + 1] = t;
+        P.dev_log[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5)) + 1] = t;
     }
 #endif
     if (COUNT) {

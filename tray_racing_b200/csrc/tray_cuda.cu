@@ -13,7 +13,6 @@
 #include "build_gpu.h"
 #include "host_copy.h"
 #include "traverse.cuh"
-#include "traverse_pool.cuh"
 
 static_assert(sizeof(tray_cwbvh_node) == 80, "CwBvhNode is 80 bytes (bvh_embree_to_cwbvh.rs:91, rt_gpu/mod.rs:70)");
 static_assert(sizeof(tray_tri48) == 48 && sizeof(tray_tri64) == 64 && sizeof(tray_tri24) == 24, "triangle record strides");
@@ -90,10 +89,7 @@ struct tray_scene {
     uint32_t variant = 0;                    // TRAY_VARIANT_* (tray_cuda_scene_set_variant): the MODE 1 kernels
     uint32_t refill_min = 6, tri_weight = 3, gen_min = 4;
     bool overlap_default = false;            // TRAY_CUDA_OVERLAP=1: tray_cuda_render always takes the one-launch frame kernel
-    bool pool = false;                       // pooled kernel (traverse_pool.cuh) or one-ray-per-lane kernel (traverse.cuh)
-    uint32_t pool_refill_min = 8, pool_tri_weight = 1;
-    uint2* d_spill = nullptr; uint64_t spill_cap = 0;
-    int blocks_per_sm[3] = { 0, 0, 0 };      // resident CTAs per SM of the lane kernel [0], the pooled kernel [1], the MODE 1 kernel [2]
+    int blocks_per_sm[2] = { 0, 0 };         // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1]
     // ray-batch staging
     tray_ray* d_rays = nullptr; tray_hit* d_hits = nullptr; uint64_t batch_cap = 0;
     // host <-> device pipeline of tray_cuda_trace: two pinned staging slots per direction, copy streams, events
@@ -137,41 +133,22 @@ void free_pipeline(tray_scene* s) {
 
 typedef void (*kernel_fn)(const TraceParams);
 
-template <bool TLAS, bool COUNT, bool ANYHIT>
-kernel_fn pick_stride(uint32_t stride) {
-    return stride == 64 ? (kernel_fn)trace_kernel<TLAS, COUNT, 64, ANYHIT>
-         : stride == 24 ? (kernel_fn)trace_kernel<TLAS, COUNT, 24, ANYHIT> : (kernel_fn)trace_kernel<TLAS, COUNT, 48, ANYHIT>;
+// The trace_kernel instantiation of a launch. MODE 0: every (tlas, count, stride) x {closest hit, any hit, frame}.
+// MODE 1 (variant) exists without counters only, so it ignores `count` (launch() rejects that combination).
+template <bool TLAS, bool COUNT, int STRIDE>
+kernel_fn pick_kernel(bool anyhit, bool frame, bool variant) {
+    if (variant) return (kernel_fn)trace_kernel<TLAS, false, STRIDE, false, false, 1>;
+    if (frame) return (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, false, true>;
+    return anyhit ? (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, true> : (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, false>;
 }
 template <bool TLAS, bool COUNT>
-kernel_fn pick_frame_stride(uint32_t stride) {
-    return stride == 64 ? (kernel_fn)trace_kernel<TLAS, COUNT, 64, false, true>
-         : stride == 24 ? (kernel_fn)trace_kernel<TLAS, COUNT, 24, false, true> : (kernel_fn)trace_kernel<TLAS, COUNT, 48, false, true>;
+kernel_fn pick_kernel(uint32_t stride, bool anyhit, bool frame, bool variant) {
+    return stride == 64 ? pick_kernel<TLAS, COUNT, 64>(anyhit, frame, variant)
+         : stride == 24 ? pick_kernel<TLAS, COUNT, 24>(anyhit, frame, variant) : pick_kernel<TLAS, COUNT, 48>(anyhit, frame, variant);
 }
-kernel_fn pick_frame_kernel(bool tlas, bool count, uint32_t stride) {
-    if (tlas) return count ? pick_frame_stride<true, true>(stride) : pick_frame_stride<true, false>(stride);
-    return count ? pick_frame_stride<false, true>(stride) : pick_frame_stride<false, false>(stride);
-}
-template <bool TLAS>
-kernel_fn pick_variant_stride(uint32_t stride) {
-    return stride == 64 ? (kernel_fn)trace_kernel<TLAS, false, 64, false, false, 1>
-         : stride == 24 ? (kernel_fn)trace_kernel<TLAS, false, 24, false, false, 1> : (kernel_fn)trace_kernel<TLAS, false, 48, false, false, 1>;
-}
-kernel_fn pick_variant_kernel(bool tlas, uint32_t stride) { return tlas ? pick_variant_stride<true>(stride) : pick_variant_stride<false>(stride); }
-kernel_fn pick_kernel(bool tlas, bool count, uint32_t stride, bool anyhit) {
-    if (anyhit) {
-        if (tlas) return count ? pick_stride<true, true, true>(stride) : pick_stride<true, false, true>(stride);
-        return count ? pick_stride<false, true, true>(stride) : pick_stride<false, false, true>(stride);
-    }
-    if (tlas) return count ? pick_stride<true, true, false>(stride) : pick_stride<true, false, false>(stride);
-    return count ? pick_stride<false, true, false>(stride) : pick_stride<false, false, false>(stride);
-}
-template <bool TLAS, bool COUNT>
-kernel_fn pick_pool_stride(uint32_t stride) {
-    return stride == 64 ? (kernel_fn)trace_pool_kernel<TLAS, COUNT, 64> : (kernel_fn)trace_pool_kernel<TLAS, COUNT, 48>;
-}
-kernel_fn pick_pool_kernel(bool tlas, bool count, uint32_t stride) {
-    if (tlas) return count ? pick_pool_stride<true, true>(stride) : pick_pool_stride<true, false>(stride);
-    return count ? pick_pool_stride<false, true>(stride) : pick_pool_stride<false, false>(stride);
+kernel_fn pick_kernel(bool tlas, bool count, uint32_t stride, bool anyhit, bool frame, bool variant) {
+    if (tlas) return count ? pick_kernel<true, true>(stride, anyhit, frame, variant) : pick_kernel<true, false>(stride, anyhit, frame, variant);
+    return count ? pick_kernel<false, true>(stride, anyhit, frame, variant) : pick_kernel<false, false>(stride, anyhit, frame, variant);
 }
 
 uint64_t local_items(uint32_t w, uint32_t h, uint32_t shard, uint32_t shards) {
@@ -193,16 +170,11 @@ void base_params(const tray_scene* s, TraceParams& P) {
 int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* cur, int counter_slot, bool anyhit = false, bool keep_counters = false, bool frame = false) {
     if (s->variant && (anyhit || frame || s->counting))
         return fail(TRAY_ERR_ARG, "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only");
-    const bool pool = s->pool && !anyhit && !frame && s->tri_stride != 24 && !s->variant;      // the pooled kernel covers closest hit on f32 records
-    kernel_fn k = s->variant ? pick_variant_kernel(s->tlas, s->tri_stride)
-                : pool ? pick_pool_kernel(s->tlas, s->counting, s->tri_stride)
-                : frame ? pick_frame_kernel(s->tlas, s->counting, s->tri_stride) : pick_kernel(s->tlas, s->counting, s->tri_stride, anyhit);
-    const int threads = pool ? POOL_WARPS * 32 : BLOCK_THREADS;
-    const uint64_t rays_per_block = pool ? (uint64_t)POOL_WARPS * POOL_SLOTS : (uint64_t)BLOCK_THREADS;
-    int& bps = s->blocks_per_sm[s->variant ? 2 : pool ? 1 : 0];
+    kernel_fn k = pick_kernel(s->tlas, s->counting, s->tri_stride, anyhit, frame, s->variant != 0);
+    int& bps = s->blocks_per_sm[s->variant ? 1 : 0];
     if (bps == 0) {
         int nb = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, threads, 0));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, BLOCK_THREADS, 0));
         bps = nb > 0 ? nb : 1;
         int cap = env_int("TRAY_CUDA_BLOCKS_PER_SM", 0);
         if (cap > 0 && cap < bps) bps = cap;
@@ -211,25 +183,13 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
     P.counters = cur + 1 + 5 * counter_slot;
     CU(cudaMemsetAsync(cur, 0, sizeof(unsigned long long), st));
     if (s->counting && !keep_counters) CU(cudaMemsetAsync(P.counters, 0, (frame ? 10 : 5) * sizeof(unsigned long long), st));
-    const uint64_t blocks_needed = ((uint64_t)P.n_work + rays_per_block - 1) / rays_per_block;
+    const uint64_t blocks_needed = ((uint64_t)P.n_work + BLOCK_THREADS - 1) / BLOCK_THREADS;
     uint64_t grid = (uint64_t)s->sm_count * bps;
     if (blocks_needed < grid) grid = blocks_needed;
     if (grid == 0) return TRAY_OK;
-    if (pool) {
-        P.refill_min = s->pool_refill_min; P.tri_weight = s->pool_tri_weight;
-        const uint64_t need = grid * POOL_WARPS * POOL_STACK_SPILL * POOL_SLOTS;      // uint2 entries
-        if (need > s->spill_cap) {
-            CU(cudaStreamSynchronize(st));
-            cudaFree(s->d_spill); s->d_spill = nullptr; s->spill_cap = 0;
-            const uint64_t cap = (uint64_t)s->sm_count * bps * POOL_WARPS * POOL_STACK_SPILL * POOL_SLOTS;
-            CU(cudaMalloc(&s->d_spill, cap * sizeof(uint2)));
-            s->spill_cap = cap;
-        }
-        P.spill = s->d_spill;
-    }
     // the persisting-L2 window over the node array travels with the launch, so it holds on any stream
     cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof cfg);
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)threads); cfg.stream = st;
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)BLOCK_THREADS); cfg.stream = st;
     cudaLaunchAttribute attr[1];
     if (s->have_window) {
         attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
@@ -239,21 +199,19 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
 #if defined(TRAY_EXIT_LOG) || defined(TRAY_STEP_CLOCK)
 #ifdef TRAY_STEP_CLOCK
 #define TRAY_EXIT_LOG 1              // from here on: the host side of both dev logs is the same dump
-    const size_t log_n = 12 * grid * (threads / 32);
+    const size_t log_n = 12 * grid * (BLOCK_THREADS / 32);
 #else
-    const size_t log_n = 6 * grid * (threads / 32);
+    const size_t log_n = 6 * grid * (BLOCK_THREADS / 32);
 #endif
     static unsigned long long* d_log = nullptr;
-    if (!pool) {
-        if (!d_log) CU(cudaMalloc(&d_log, 1 << 24));
-        CU(cudaMemsetAsync(d_log, 0, log_n * 8, st));
-        P.spill = (uint2*)d_log;
-    }
+    if (!d_log) CU(cudaMalloc(&d_log, 1 << 24));
+    CU(cudaMemsetAsync(d_log, 0, log_n * 8, st));
+    P.dev_log = d_log;
 #endif
     void* args[1] = { (void*)&P };
     CU(cudaLaunchKernelExC(&cfg, (const void*)k, args));
 #ifdef TRAY_EXIT_LOG
-    if (!pool && getenv("TRAY_EXIT_LOG_FILE")) {
+    if (getenv("TRAY_EXIT_LOG_FILE")) {
         std::vector<unsigned long long> h(log_n);
         CU(cudaStreamSynchronize(st));
         CU(cudaMemcpy(h.data(), d_log, log_n * 8, cudaMemcpyDeviceToHost));
@@ -393,7 +351,7 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
     cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
-    cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_spill); cudaFree(s->d_geom_offsets);
+    cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_geom_offsets);
     free_pipeline(s);
     cudaFree(s->d_untiled);
     for (auto& f : s->slot) {
@@ -449,11 +407,6 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     s->tri_weight = (uint32_t)env_int("TRAY_CUDA_TRI_WEIGHT", 3);     // 3: +0.6 ... 1.2 % over 4 with two triangles per step (profiles/experiments/r2_triweight_ab.log)
     s->gen_min = (uint32_t)env_int("TRAY_CUDA_GEN_MIN", 4);
     s->overlap_default = env_int("TRAY_CUDA_OVERLAP", 0) != 0;
-    s->pool = env_int("TRAY_CUDA_POOL", 0) != 0;
-    s->pool_refill_min = (uint32_t)env_int("TRAY_CUDA_POOL_REFILL_MIN", 8);
-    s->pool_tri_weight = (uint32_t)env_int("TRAY_CUDA_POOL_TRI_WEIGHT", 1);
-    if (s->pool_refill_min < 1) s->pool_refill_min = 1;
-    if (s->pool_refill_min > POOL_SLOTS) s->pool_refill_min = POOL_SLOTS;
     int rc = TRAY_OK;
     bool adopted = false;
     auto body = [&]() -> int {
@@ -611,7 +564,7 @@ int tray_cuda_scene_info(const tray_scene* s, tray_scene_info* o) {
 
 int tray_cuda_set_counting(tray_scene* s, int enabled) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
-    if (s->counting != (enabled != 0)) { s->counting = enabled != 0; s->blocks_per_sm[0] = s->blocks_per_sm[1] = 0; }
+    if (s->counting != (enabled != 0)) { s->counting = enabled != 0; s->blocks_per_sm[0] = 0; }
     return TRAY_OK;
 }
 
