@@ -53,8 +53,7 @@ struct FrameSlot {
     uint32_t* d_units = nullptr;             // FRAME kernel: cursor over the 32-item groups of bounce work
     cudaEvent_t ev[4] = { nullptr, nullptr, nullptr, nullptr };
     cudaEvent_t done = nullptr;              // recorded behind the frame's last launch (fences, group completion)
-    uint32_t fw = 0, fh = 0, fshard = 0, fshards = 1;
-    uint64_t f_items = 0, f_cap = 0;
+    uint64_t f_cap = 0;
     bool f_has_bounce = false, f_has_rgba = false, f_has_rays = false;
     uchar4* f_target = nullptr;              // the frame target the last frame was rendered into (NULL: compact d_rgba)
     tray_hit* d_primary = nullptr; tray_hit* d_bounce = nullptr; uchar4* d_rgba = nullptr;
@@ -62,7 +61,7 @@ struct FrameSlot {
     tray_ray* d_brays = nullptr;             // generated bounce rays, COMPACT (hit pixels only)
     uint32_t* d_bitem = nullptr;             // local item of compact bounce ray i
     tray_ray* d_brays_item = nullptr;        // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
-    tray::FrameParams last_frame;
+    tray::FrameParams last_frame{};          // width 0: no frame rendered yet
 };
 
 struct tray_scene {
@@ -81,7 +80,7 @@ struct tray_scene {
     uint32_t* d_overflow = nullptr;
     cudaStream_t stream = nullptr;          // the stream work is enqueued on
     cudaStream_t own_stream = nullptr;      // created with the scene
-    cudaEvent_t ev[4] = { nullptr, nullptr, nullptr, nullptr };
+    cudaEvent_t ev[2] = { nullptr, nullptr };
     bool have_window = false;                // persisting-L2 access-policy window over the node array, applied per launch
     cudaAccessPolicyWindow window{};
     uint64_t device_bytes = 0, l2_bytes = 0, l2_persist = 0;
@@ -224,8 +223,33 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
 }
 
 cudaStream_t slot_stream(const tray_scene* s, int k) { return k == 0 ? s->stream : s->slot[k].own_stream; }
-int sync_slot_streams(const tray_scene* s) {          // the scene's own frame streams (slot 0 runs on tray_scene::stream)
+int next_slot(const tray_scene* s) { return (s->cur + 1) % s->n_slots; }     // the slot the next tray_cuda_render takes
+// waits for the scene stream and the scene's own frame streams (slot 0 runs on tray_scene::stream), in the order asked for
+int sync_streams(const tray_scene* s, bool scene_stream_first) {
+    if (scene_stream_first) CU(cudaStreamSynchronize(s->stream));
     for (int k = 1; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) CU(cudaStreamSynchronize(s->slot[k].own_stream));
+    if (!scene_stream_first) CU(cudaStreamSynchronize(s->stream));
+    return TRAY_OK;
+}
+
+// the per-frame buffers of a slot (not its cursor block); the caller has synchronised the slot's stream
+void free_frame_buffers(FrameSlot& f) {
+    cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
+    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item);
+    f.d_primary = nullptr; f.d_bounce = nullptr; f.d_brays = nullptr; f.d_rgba = nullptr;
+    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.f_cap = 0;
+}
+
+int check_tri_stride(uint32_t tri_stride) {
+    if (tri_stride != 48 && tri_stride != 64 && tri_stride != 24) return fail(TRAY_ERR_ARG, "tri_stride must be 48, 64 or 24 (got %u)", tri_stride);
+    return TRAY_OK;
+}
+// after the argument checks, so that a bad argument is reported as such on a machine without a GPU too
+int select_device(int device) {
+    const int ndev = tray_cuda_device_count();
+    if (ndev == 0) return fail(TRAY_ERR_NO_DEVICE, "no CUDA device (tray_cuda has no CPU fallback)");
+    if (device < 0 || device >= ndev) return fail(TRAY_ERR_ARG, "device %d out of range (0..%d)", device, ndev - 1);
+    CU(cudaSetDevice(device));
     return TRAY_OK;
 }
 
@@ -237,7 +261,7 @@ void frame_params(FrameParams& F, const tray_view* view, uint32_t w, uint32_t h,
     F.n_items = (uint32_t)local_items(w, h, shard, shards);
 }
 
-int read_counters(tray_scene* s, const unsigned long long* cur, cudaStream_t st, int slot, tray_counters* out) {
+int read_counters(const unsigned long long* cur, cudaStream_t st, int slot, tray_counters* out) {
     unsigned long long c[5];
     CU(cudaMemcpyAsync(c, cur + 1 + 5 * slot, sizeof c, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -245,19 +269,52 @@ int read_counters(tray_scene* s, const unsigned long long* cur, cudaStream_t st,
     return TRAY_OK;
 }
 
+// a word of the device error flag as a status (4: the frame kernel's watchdog, other bits: stack overflow); clears a set flag
+int flag_status(tray_scene* s, uint32_t f) {
+    if (!f) return TRAY_OK;
+    cudaMemsetAsync(s->d_overflow, 0, 4, s->stream);
+    if (f & 4u) return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
+    return fail(TRAY_ERR_OVERFLOW, "traversal stack overflow: BVH needs more than %d stack entries", STACK_SMEM + STACK_SPILL);
+}
 int check_overflow(tray_scene* s, cudaStream_t st = nullptr) {
     if (!st) st = s->stream;
     uint32_t f = 0;
     CU(cudaMemcpyAsync(&f, s->d_overflow, 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    if (f & 4u) {
-        cudaMemsetAsync(s->d_overflow, 0, 4, s->stream);
-        return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
+    return flag_status(s, f);
+}
+
+// the start protocol's arguments (the reference asserts these strides at src/rt_gpu/mod.rs:70,86,105,107)
+int check_start_args(const tray_view* view, uint64_t bvh_len, uint64_t tri_len, uint32_t tri_stride, uint64_t instance_len) {
+    if (!view) return fail(TRAY_ERR_ARG, "NULL view");
+    if (bvh_len % 80 != 0) return fail(TRAY_ERR_ARG, "bvh_bytes length %llu is not a multiple of 80", (unsigned long long)bvh_len);
+    if (tri_stride == 0 || tri_len % tri_stride != 0) return fail(TRAY_ERR_ARG, "tri_bytes length is not a multiple of tri_stride");
+    if (instance_len % 4 != 0) return fail(TRAY_ERR_ARG, "instance_bytes length is not a multiple of 4");
+    return TRAY_OK;
+}
+
+// the timed loop of the start protocol over one scene or a group: render(frame_count), render_timed(frame_count, &ms), sync()
+template <typename Render, typename RenderTimed, typename Sync>
+int start_loop(Render render, RenderTimed render_timed, Sync sync, float render_time_s, int benchmark, int animate,
+               float* out_min_ms, float* out_mean_ms, uint32_t* out_frames) {
+    float min_ms = 3.402823466e+38f; double sum = 0; uint32_t frames = 0, frame_count = 0;
+    const auto t0 = std::chrono::steady_clock::now();
+    for (;;) {
+        if (benchmark) {   // untimed warm-up dispatch right before the timed one (rt_gpu_software.rs:289-295)
+            if (const int rc = render(frame_count)) return rc;
+        }
+        float ms = 0.f;       // the whole dispatch, as the reference's timestamp queries bracket it (rt_gpu_software.rs:296-301)
+        if (const int rc = render_timed(frame_count, &ms)) return rc;
+        if (ms < min_ms) min_ms = ms;
+        sum += ms; frames++;
+        if (animate) frame_count = frames;                                   // rt_cpu.rs:95-97
+        const float el = std::chrono::duration<float>(std::chrono::steady_clock::now() - t0).count();
+        if (el > render_time_s) break;                                       // rt_cpu.rs:98-100, rt_gpu_software.rs:354-359
     }
-    if (f) {
-        cudaMemsetAsync(s->d_overflow, 0, 4, s->stream);
-        return fail(TRAY_ERR_OVERFLOW, "traversal stack overflow: BVH needs more than %d stack entries", STACK_SMEM + STACK_SPILL);
-    }
+    if (const int rc = sync()) return rc;
+    if (out_min_ms) *out_min_ms = min_ms;
+    if (out_mean_ms) *out_mean_ms = frames ? (float)(sum / frames) : 0.f;
+    if (out_frames) *out_frames = frames;
     return TRAY_OK;
 }
 
@@ -356,8 +413,8 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     cudaFree(s->d_untiled);
     for (auto& f : s->slot) {
         if (f.own_stream) cudaStreamSynchronize(f.own_stream);
-        cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
-        cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item); cudaFree(f.d_cursor); cudaFree(f.d_units);
+        free_frame_buffers(f);
+        cudaFree(f.d_cursor); cudaFree(f.d_units);
         for (auto& e : f.ev) if (e) cudaEventDestroy(e);
         if (f.done) cudaEventDestroy(f.done);
         if (f.own_stream) cudaStreamDestroy(f.own_stream);
@@ -386,14 +443,11 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     if (!out) return fail(TRAY_ERR_ARG, "out_scene is NULL");
     *out = nullptr;
     if (!built && ((n_nodes && !nodes) || (n_tris && !tris))) return fail(TRAY_ERR_ARG, "NULL node / triangle buffer");
-    if (tri_stride != 48 && tri_stride != 64 && tri_stride != 24) return fail(TRAY_ERR_ARG, "tri_stride must be 48, 64 or 24 (got %u)", tri_stride);
+    if (const int rc = check_tri_stride(tri_stride)) return rc;
     if (n_instances && !blas_offsets && !built) return fail(TRAY_ERR_ARG, "n_instances > 0 but blas_offsets is NULL");
     if (n_instances && tlas_start >= n_nodes) return fail(TRAY_ERR_ARG, "tlas_start %u outside %llu nodes", tlas_start, (unsigned long long)n_nodes);
     if (n_nodes >= 0xffffffffull || n_tris >= 0xffffffffull) return fail(TRAY_ERR_ARG, "node / triangle indices are 32-bit");
-    const int ndev = tray_cuda_device_count();
-    if (ndev == 0) return fail(TRAY_ERR_NO_DEVICE, "no CUDA device (tray_cuda has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(TRAY_ERR_ARG, "device %d out of range (0..%d)", device, ndev - 1);
-    CU(cudaSetDevice(device));
+    if (const int rc = select_device(device)) return rc;
     tray_scene* s = new (std::nothrow) tray_scene();
     if (!s) return fail(TRAY_ERR_ARG, "out of host memory");
     s->device = device; s->n_nodes = n_nodes; s->n_tris = n_tris; s->tri_stride = tri_stride;
@@ -407,8 +461,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     s->tri_weight = (uint32_t)env_int("TRAY_CUDA_TRI_WEIGHT", 3);     // 3: +0.6 ... 1.2 % over 4 with two triangles per step (profiles/experiments/r2_triweight_ab.log)
     s->gen_min = (uint32_t)env_int("TRAY_CUDA_GEN_MIN", 4);
     s->overlap_default = env_int("TRAY_CUDA_OVERLAP", 0) != 0;
-    int rc = TRAY_OK;
-    bool adopted = false;
+    const bool adopted = built && built->d_nodes;
     auto body = [&]() -> int {
         cudaDeviceProp prop;
         CU(cudaGetDeviceProperties(&prop, device));
@@ -427,12 +480,11 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
             CU(cudaEventCreateWithFlags(&s->ev_copied[i], cudaEventDisableTiming));
         }
         const size_t nb = (size_t)(n_nodes ? n_nodes : 1) * 80, tb = (size_t)(n_tris ? n_tris : 1) * tri_stride;
-        if (built && built->d_nodes) {
+        if (adopted) {
             s->d_nodes = (uint4*)built->d_nodes; s->d_tris = (uint4*)built->d_tris; s->d_prim_indices = built->d_prim_indices;
             s->d_blas = built->d_blas_offsets;
             // ownership moves to the scene HERE: from now on tray_cuda_scene_destroy is the one place that frees them
             built->d_nodes = nullptr; built->d_tris = nullptr; built->d_prim_indices = nullptr; built->d_blas_offsets = nullptr;
-            adopted = true;
         } else {
             CU(cudaMalloc(&s->d_nodes, nb));
             CU(cudaMalloc(&s->d_tris, tb));
@@ -452,10 +504,11 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         }
         CU(cudaMemsetAsync(s->d_overflow, 0, 4, s->stream));
         s->device_bytes = nb + tb + (size_t)n_instances * 4;
-        if (adopted) {}
-        else if (n_nodes) CU(tray::upload_pipelined(s->d_nodes, nodes, (size_t)n_nodes * 80, s->stream));
-        else CU(cudaMemsetAsync(s->d_nodes, 0, 80, s->stream));   // empty scene: a root with no children, every ray misses
-        if (!adopted && n_tris) CU(tray::upload_pipelined(s->d_tris, tris, (size_t)n_tris * tri_stride, s->stream));
+        if (!adopted) {
+            if (n_nodes) CU(tray::upload_pipelined(s->d_nodes, nodes, (size_t)n_nodes * 80, s->stream));
+            else CU(cudaMemsetAsync(s->d_nodes, 0, 80, s->stream));   // empty scene: a root with no children, every ray misses
+            if (n_tris) CU(tray::upload_pipelined(s->d_tris, tris, (size_t)n_tris * tri_stride, s->stream));
+        }
         if (n_instances && blas_offsets) CU(cudaMemcpyAsync(s->d_blas, blas_offsets, (size_t)n_instances * 4, cudaMemcpyHostToDevice, s->stream));
         // keep the node array hot in the 126 MB L2: persisting access-policy window, attached to every traversal launch
         if (env_int("TRAY_CUDA_L2_PERSIST", 1) && prop.persistingL2CacheMaxSize > 0 && n_nodes) {
@@ -477,7 +530,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         CU(cudaStreamSynchronize(s->stream));
         return TRAY_OK;
     };
-    rc = body();
+    const int rc = body();
     if (rc != TRAY_OK) { tray_cuda_scene_destroy(s); return rc; }
     *out = s;
     return TRAY_OK;
@@ -500,14 +553,11 @@ int scene_build_impl(const float* tris9, uint64_t n_tris, const uint64_t* object
     if (!out) return fail(TRAY_ERR_ARG, "out_scene is NULL");
     *out = nullptr;
     if (n_tris && !tris9) return fail(TRAY_ERR_ARG, "NULL triangle buffer");
-    if (tri_stride != 48 && tri_stride != 64 && tri_stride != 24) return fail(TRAY_ERR_ARG, "tri_stride must be 48, 64 or 24 (got %u)", tri_stride);
+    if (const int rc = check_tri_stride(tri_stride)) return rc;
     if (max_prims_per_leaf < 1 || max_prims_per_leaf > 3) return fail(TRAY_ERR_ARG, "max_prims_per_leaf must be 1..3");
     if (search_radius > 64) return fail(TRAY_ERR_ARG, "search_radius must be 0 (default 14) or 1..64");
     if (object_offsets && n_tris == 0) return fail(TRAY_ERR_ARG, "a two-level scene needs triangles");
-    const int ndev = tray_cuda_device_count();
-    if (ndev == 0) return fail(TRAY_ERR_NO_DEVICE, "no CUDA device (tray_cuda has no CPU fallback)");
-    if (device < 0 || device >= ndev) return fail(TRAY_ERR_ARG, "device %d out of range (0..%d)", device, ndev - 1);
-    CU(cudaSetDevice(device));
+    if (const int rc = select_device(device)) return rc;
     tray_build::Result r;
     char msg[400] = "";
     const int brc = tray_build::build_tlas(tris9, n_tris, object_offsets, n_objects, tri_stride, max_prims_per_leaf,
@@ -578,8 +628,7 @@ int tray_cuda_scene_set_variant(tray_scene* s, uint32_t flags) {
 int tray_cuda_scene_set_stream(tray_scene* s, void* stream) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     CU(cudaSetDevice(s->device));
-    CU(cudaStreamSynchronize(s->stream));
-    { const int rc_ = sync_slot_streams(s); if (rc_) return rc_; }
+    if (const int rc = sync_streams(s, /*scene_stream_first=*/true)) return rc;
     s->stream = stream ? (cudaStream_t)stream : s->own_stream;
     return TRAY_OK;
 }
@@ -600,9 +649,9 @@ int tray_cuda_untile_rgba(tray_scene* s, const void* d_compact, uint32_t w, uint
 int tray_cuda_frame_push(tray_scene* s, void* d_dst) {
     if (!s || !d_dst) return fail(TRAY_ERR_ARG, "NULL argument");
     const FrameSlot& f = s->slot[s->cur];
-    if (f.fw == 0 || !f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA (or into a frame target)");
+    if (f.last_frame.width == 0 || !f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA (or into a frame target)");
     CU(cudaSetDevice(s->device));
-    if (f.f_items) CU(cudaMemcpyAsync(d_dst, f.d_rgba, (size_t)f.f_items * sizeof(uchar4), cudaMemcpyDeviceToDevice, slot_stream(s, s->cur)));
+    if (f.last_frame.n_items) CU(cudaMemcpyAsync(d_dst, f.d_rgba, (size_t)f.last_frame.n_items * sizeof(uchar4), cudaMemcpyDeviceToDevice, slot_stream(s, s->cur)));
     return TRAY_OK;
 }
 
@@ -670,8 +719,7 @@ int tray_cuda_scene_set_frame_target(tray_scene* s, void* d_frame) {
 int tray_cuda_sync(tray_scene* s) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     CU(cudaSetDevice(s->device));
-    { const int rc_ = sync_slot_streams(s); if (rc_) return rc_; }
-    CU(cudaStreamSynchronize(s->stream));
+    if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
     return check_overflow(s);
 }
 
@@ -786,7 +834,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         CU(cudaStreamSynchronize(s->stream));
         CU(cudaEventElapsedTime(&k, s->ev[0], s->ev[1]));       // span of the GPU work, uploads it waited for included
     }
-    if (s->counting) { rc = read_counters(s, s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc; memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce); }
+    if (s->counting) { rc = read_counters(s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc; memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce); }
     rc = check_overflow(s);
     if (rc) return rc;
     if (ms_kernel) *ms_kernel = k;
@@ -829,8 +877,7 @@ uint64_t tray_cuda_shard_items(uint32_t w, uint32_t h, uint32_t shard, uint32_t 
 int tray_cuda_scene_set_frames_in_flight(tray_scene* s, uint32_t n) {
     if (!s || n < 1 || n > TRAY_MAX_FRAMES_IN_FLIGHT) return fail(TRAY_ERR_ARG, "frames in flight must be 1 .. %d", TRAY_MAX_FRAMES_IN_FLIGHT);
     CU(cudaSetDevice(s->device));
-    { const int rc_ = sync_slot_streams(s); if (rc_) return rc_; }
-    CU(cudaStreamSynchronize(s->stream));
+    if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
     if ((int)n != s->n_slots) { s->n_slots = (int)n; s->cur = 0; }
     return TRAY_OK;
 }
@@ -887,7 +934,7 @@ int tray_cuda_frame_wait_flag(tray_scene* s, const void* d_flag, uint32_t value,
     if (!s || !d_flag) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     int rc = resolve_memops(); if (rc) return rc;
-    const int k = before_next_frame ? (s->n_slots > 1 ? (s->cur + 1) % s->n_slots : 0) : s->cur;
+    const int k = before_next_frame ? next_slot(s) : s->cur;
     const int e = g_wait32((void*)slot_stream(s, k), (unsigned long long)(uintptr_t)d_flag, value, 0u /* CU_STREAM_WAIT_VALUE_GEQ */);
     if (e) return fail(TRAY_ERR_CUDA, "cuStreamWaitValue32 failed (CUresult %d)", e);
     return TRAY_OK;
@@ -911,7 +958,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     CU(cudaSetDevice(s->device));
     const bool want_count = (flags & TRAY_RENDER_COUNTERS) != 0;
     if (want_count != s->counting) tray_cuda_set_counting(s, want_count);
-    s->cur = s->n_slots > 1 ? (s->cur + 1) % s->n_slots : 0;           // the next frame goes to the other slot
+    s->cur = next_slot(s);
     FrameSlot& f = s->slot[s->cur];
     cudaStream_t st = slot_stream(s, s->cur);
     const uint64_t items_cap = local_items(w, h, 0, shards);   // every shard's buffers have the size of the largest (gather)
@@ -922,10 +969,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item)) {
         const uint64_t cap = items_cap > f.f_cap ? items_cap : f.f_cap;
         CU(cudaStreamSynchronize(st));
-        cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
-        cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item);
-        f.d_primary = nullptr; f.d_bounce = nullptr; f.d_brays = nullptr; f.d_rgba = nullptr;
-        f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.f_cap = 0;
+        free_frame_buffers(f);
         const uint64_t c1 = cap ? cap : 1;
         CU(cudaMalloc(&f.d_primary, c1 * sizeof(tray_hit)));
         CU(cudaMalloc(&f.d_bounce, c1 * sizeof(tray_hit)));
@@ -940,7 +984,6 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         f.f_cap = cap;
     }
     FrameParams F; frame_params(F, view, w, h, frame_count, shard, shards);
-    f.fw = w; f.fh = h; f.fshard = shard; f.fshards = shards; f.f_items = F.n_items;
     f.f_has_bounce = bounce; f.f_has_rgba = rgba && !s->frame_target; f.f_has_rays = keep_rays && bounce;
     f.f_target = rgba ? s->frame_target : nullptr;
     f.last_frame = F;
@@ -1002,8 +1045,8 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         rc = check_overflow(s, st); if (rc) return rc;
     }
     if (s->counting) {
-        rc = read_counters(s, f.d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
-        if (bounce) { rc = read_counters(s, f.d_cursor, st, 1, &s->cnt_bounce); if (rc) return rc; }
+        rc = read_counters(f.d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
+        if (bounce) { rc = read_counters(f.d_cursor, st, 1, &s->cnt_bounce); if (rc) return rc; }
         else memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
         // rays generated for pixels outside the frame (tmax = 0) are not rays of the workload
         const uint64_t pad = (uint64_t)F.n_items - tray_cuda_shard_pixels(w, h, shard, shards);
@@ -1016,7 +1059,7 @@ int tray_cuda_render_timed(tray_scene* s, const tray_view* view, uint32_t w, uin
                            uint32_t shard, uint32_t shards, float* ms_frame) {
     if (!s || !view || !ms_frame) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
-    const int k = s->n_slots > 1 ? (s->cur + 1) % s->n_slots : 0;          // the slot tray_cuda_render is about to take
+    const int k = next_slot(s);                                               // the slot tray_cuda_render is about to take
     cudaStream_t st = slot_stream(s, k);
     CU(cudaEventRecord(s->slot[k].ev[0], st));
     int rc = tray_cuda_render(s, view, w, h, frame_count, flags, shard, shards, nullptr, nullptr);
@@ -1046,22 +1089,30 @@ int tray_cuda_frame_device_ptrs(tray_scene* s, void** d_primary, void** d_bounce
 }  // extern "C"
 
 namespace {
+// the last frame's compact buffer `d_src`, untiled into the row-major `d_dst` on the frame's stream
+template <typename T>
+int untile_last_frame(tray_scene* s, const T* d_src, T* d_dst) {
+    const FrameParams& F = s->slot[s->cur].last_frame;
+    cudaStream_t st = slot_stream(s, s->cur);
+    if (F.shard_count > 1) CU(cudaMemsetAsync(d_dst, 0, (uint64_t)F.width * F.height * sizeof(T), st));   // pixels of other shards read as zero
+    if (F.n_items) {
+        tray::untile_kernel<T><<<(F.n_items + 255) / 256, 256, 0, st>>>(F, d_src, d_dst);
+        CU(cudaGetLastError());
+    }
+    return TRAY_OK;
+}
+
 template <typename T>
 int download(tray_scene* s, const T* d_src, T* host_dst) {
-    const FrameSlot& f = s->slot[s->cur];
+    const FrameParams& F = s->slot[s->cur].last_frame;
     cudaStream_t st = slot_stream(s, s->cur);
-    const uint64_t n = (uint64_t)f.fw * f.fh, bytes = n * sizeof(T);
+    const uint64_t bytes = (uint64_t)F.width * F.height * sizeof(T);
     if (bytes > s->untiled_cap) {
         cudaFree(s->d_untiled); s->d_untiled = nullptr; s->untiled_cap = 0;
         CU(cudaMalloc(&s->d_untiled, bytes));
         s->untiled_cap = bytes;
     }
-    if (f.fshards > 1) CU(cudaMemsetAsync(s->d_untiled, 0, bytes, st));   // pixels of other shards read as zero
-    if (f.f_items) {
-        const unsigned grid = (unsigned)((f.f_items + 255) / 256);
-        tray::untile_kernel<T><<<grid, 256, 0, st>>>(f.last_frame, d_src, (T*)s->d_untiled);
-        CU(cudaGetLastError());
-    }
+    if (const int rc = untile_last_frame(s, d_src, (T*)s->d_untiled)) return rc;
     CU(cudaMemcpyAsync(host_dst, s->d_untiled, bytes, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return TRAY_OK;
@@ -1073,7 +1124,7 @@ extern "C" {
 int tray_cuda_frame_download(tray_scene* s, tray_hit* primary, tray_hit* bounce, tray_ray* bounce_rays, uint8_t* rgba) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     const FrameSlot& f = s->slot[s->cur];
-    if (f.fw == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
+    if (f.last_frame.width == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
     CU(cudaSetDevice(s->device));
     int rc;
     if (primary) { rc = download<tray_hit>(s, f.d_primary, primary); if (rc) return rc; }
@@ -1096,9 +1147,9 @@ int tray_cuda_frame_readback_begin(tray_scene* s, uint8_t* rgba, uint32_t slot) 
     if (!s || !rgba || slot >= TRAY_READBACK_SLOTS) return fail(TRAY_ERR_ARG, "bad argument");
     const FrameSlot& f = s->slot[s->cur];
     cudaStream_t st = slot_stream(s, s->cur);
-    if (f.fw == 0 || (!f.f_has_rgba && !f.f_target)) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA");
+    if (f.last_frame.width == 0 || (!f.f_has_rgba && !f.f_target)) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA");
     CU(cudaSetDevice(s->device));
-    const uint64_t bytes = (uint64_t)f.fw * f.fh * sizeof(uchar4);
+    const uint64_t bytes = (uint64_t)f.last_frame.width * f.last_frame.height * sizeof(uchar4);
     if (s->stage_busy[slot]) {                       // the previous copy out of this staging buffer must have landed
         CU(cudaEventSynchronize(s->ev_copied[slot]));
         s->stage_busy[slot] = false;
@@ -1112,13 +1163,8 @@ int tray_cuda_frame_readback_begin(tray_scene* s, uint8_t* rgba, uint32_t slot) 
         // the frame was rendered into a row-major frame target (all shards' pixels, once the caller's barrier has passed):
         // snapshot it, so that the next frame may overwrite the target while this one travels to the host
         CU(cudaMemcpyAsync(s->d_stage[slot], f.f_target, bytes, cudaMemcpyDeviceToDevice, st));
-    } else {
-        if (f.fshards > 1) CU(cudaMemsetAsync(s->d_stage[slot], 0, bytes, st));
-        if (f.f_items) {
-            const unsigned grid = (unsigned)((f.f_items + 255) / 256);
-            tray::untile_kernel<uchar4><<<grid, 256, 0, st>>>(f.last_frame, f.d_rgba, s->d_stage[slot]);
-            CU(cudaGetLastError());
-        }
+    } else if (const int rc = untile_last_frame(s, f.d_rgba, s->d_stage[slot])) {
+        return rc;
     }
     CU(cudaEventRecord(s->ev_untiled[slot], st));
     CU(cudaStreamWaitEvent(s->copy_stream, s->ev_untiled[slot], 0));
@@ -1137,24 +1183,15 @@ int tray_cuda_frame_readback_wait(tray_scene* s, uint32_t slot) {
     CU(cudaEventSynchronize(s->ev_copied[slot]));
     s->stage_busy[slot] = false;
     const uint32_t fl = s->h_flag[slot];
-    if (fl) {
-        s->h_flag[slot] = 0u;
-        cudaMemsetAsync(s->d_overflow, 0, 4, s->stream);
-        if (fl & 4u) return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
-        return fail(TRAY_ERR_OVERFLOW, "traversal stack overflow: BVH needs more than %d stack entries", STACK_SMEM + STACK_SPILL);
-    }
-    return TRAY_OK;
+    s->h_flag[slot] = 0u;
+    return flag_status(s, fl);
 }
 
 int tray_cuda_start(const void* bvh_bytes, uint64_t bvh_len, const void* instance_bytes, uint64_t instance_len,
                     const void* tri_bytes, uint64_t tri_len, uint32_t tri_stride, uint32_t tlas_start, int use_tlas,
                     const tray_view* view, uint32_t width, uint32_t height, float render_time_s, int benchmark,
                     int animate, int device, float* out_min_ms, float* out_mean_ms, uint32_t* out_frames) {
-    if (!view) return fail(TRAY_ERR_ARG, "NULL view");
-    // the reference asserts these strides at src/rt_gpu/mod.rs:70,86,105,107
-    if (bvh_len % 80 != 0) return fail(TRAY_ERR_ARG, "bvh_bytes length %llu is not a multiple of 80", (unsigned long long)bvh_len);
-    if (tri_stride == 0 || tri_len % tri_stride != 0) return fail(TRAY_ERR_ARG, "tri_bytes length is not a multiple of tri_stride");
-    if (instance_len % 4 != 0) return fail(TRAY_ERR_ARG, "instance_bytes length is not a multiple of 4");
+    if (const int rc = check_start_args(view, bvh_len, tri_len, tri_stride, instance_len)) return rc;
     tray_scene* s = nullptr;
     int rc = tray_cuda_scene_create(bvh_bytes, bvh_len / 80, tri_bytes, tri_len / tri_stride, tri_stride,
                                     use_tlas ? (const uint32_t*)instance_bytes : nullptr,
@@ -1174,29 +1211,12 @@ int tray_cuda_start(const void* bvh_bytes, uint64_t bvh_len, const void* instanc
         if (rc) { tray_cuda_scene_destroy(s); return rc; }
         if (best[1] < best[0]) flags |= TRAY_RENDER_OVERLAP;
     }
-    float min_ms = 3.402823466e+38f; double sum = 0; uint32_t frames = 0, frame_count = 0;
-    const auto t0 = std::chrono::steady_clock::now();
-    for (;;) {
-        if (benchmark) {   // untimed warm-up dispatch right before the timed one (rt_gpu_software.rs:289-295)
-            rc = tray_cuda_render(s, view, width, height, frame_count, flags, 0, 1, nullptr, nullptr);
-            if (rc) break;
-        }
-        float ms = 0.f;       // the whole dispatch, as the reference's timestamp queries bracket it (rt_gpu_software.rs:296-301)
-        rc = tray_cuda_render_timed(s, view, width, height, frame_count, flags, 0, 1, &ms);
-        if (rc) break;
-        if (ms < min_ms) min_ms = ms;
-        sum += ms; frames++;
-        if (animate) frame_count = frames;                                   // rt_cpu.rs:95-97
-        const float el = std::chrono::duration<float>(std::chrono::steady_clock::now() - t0).count();
-        if (el > render_time_s) break;                                       // rt_cpu.rs:98-100, rt_gpu_software.rs:354-359
-    }
-    if (!rc) rc = tray_cuda_sync(s);
+    rc = start_loop([&](uint32_t fc) { return tray_cuda_render(s, view, width, height, fc, flags, 0, 1, nullptr, nullptr); },
+                    [&](uint32_t fc, float* ms) { return tray_cuda_render_timed(s, view, width, height, fc, flags, 0, 1, ms); },
+                    [&] { return tray_cuda_sync(s); },
+                    render_time_s, benchmark, animate, out_min_ms, out_mean_ms, out_frames);
     tray_cuda_scene_destroy(s);
-    if (rc) return rc;
-    if (out_min_ms) *out_min_ms = min_ms;
-    if (out_mean_ms) *out_mean_ms = frames ? (float)(sum / frames) : 0.f;
-    if (out_frames) *out_frames = frames;
-    return TRAY_OK;
+    return rc;
 }
 
 }  // extern "C"
@@ -1410,13 +1430,13 @@ int tray_cuda_group_render(tray_group* g, const tray_view* view, uint32_t w, uin
     const int n = (int)g->scenes.size();
     const bool push = g->exchange == 1 && n > 1;
     if (push) { rc = group_ensure_staging(g, w, h); if (rc) return rc; }
-    g->cur = g->in_flight > 1 ? (g->cur + 1) % g->in_flight : 0;
+    g->cur = (g->cur + 1) % g->in_flight;
     uchar4* const target = g->target[g->cur];
     const uint64_t items = local_items(w, h, 0, (uint32_t)n);
     const bool snap = g->snap_pending[g->cur];             // the frame this target held last is still being copied out
     for (int i = 0; i < n; i++) {
         tray_scene* sc = g->scenes[i];
-        const int k = sc->n_slots > 1 ? (sc->cur + 1) % sc->n_slots : 0;          // the slot this frame will take on device i
+        const int k = next_slot(sc);                       // the slot this frame will take on device i
         if (!push && i > 0 && snap) {                      // the previous frame in this target must have been copied out first
             CU(cudaSetDevice(sc->device));
             CU(cudaStreamWaitEvent(slot_stream(sc, k), g->ev_snap[g->cur], 0));
@@ -1429,8 +1449,8 @@ int tray_cuda_group_render(tray_group* g, const tray_view* view, uint32_t w, uin
             // one DMA copy of the compact shard into devices[0]'s staging (behind the untile of the frame that used it last)
             if (g->staged_pending[g->cur]) CU(cudaStreamWaitEvent(st, g->ev_staged[g->cur], 0));
             const FrameSlot& f = sc->slot[sc->cur];
-            if (f.f_items)
-                CU(cudaMemcpyPeerAsync(g->staging[g->cur] + (uint64_t)i * items, g->devices[0], f.d_rgba, sc->device, (size_t)f.f_items * sizeof(uchar4), st));
+            if (f.last_frame.n_items)
+                CU(cudaMemcpyPeerAsync(g->staging[g->cur] + (uint64_t)i * items, g->devices[0], f.d_rgba, sc->device, (size_t)f.last_frame.n_items * sizeof(uchar4), st));
         }
         if (i > 0) CU(cudaEventRecord(sc->slot[sc->cur].done, st));
     }
@@ -1457,14 +1477,12 @@ int tray_cuda_group_render_timed(tray_group* g, const tray_view* view, uint32_t 
     int rc = group_ensure_target(g, w, h);
     if (rc) return rc;
     tray_scene* s0 = g->scenes[0];
-    const int k0 = s0->n_slots > 1 ? (s0->cur + 1) % s0->n_slots : 0;
     CU(cudaSetDevice(s0->device));
-    CU(cudaEventRecord(g->ev_t0, slot_stream(s0, k0)));
+    CU(cudaEventRecord(g->ev_t0, slot_stream(s0, next_slot(s0))));
     for (size_t i = 1; i < g->scenes.size(); i++) {      // nobody starts before the clock does
         tray_scene* sc = g->scenes[i];
-        const int k = sc->n_slots > 1 ? (sc->cur + 1) % sc->n_slots : 0;
         CU(cudaSetDevice(sc->device));
-        CU(cudaStreamWaitEvent(slot_stream(sc, k), g->ev_t0, 0));
+        CU(cudaStreamWaitEvent(slot_stream(sc, next_slot(sc)), g->ev_t0, 0));
     }
     rc = tray_cuda_group_render(g, view, w, h, frame_count, flags);
     if (rc) return rc;
@@ -1508,39 +1526,19 @@ int tray_cuda_start_multi(const int* devices, int n_devices,
                           const void* tri_bytes, uint64_t tri_len, uint32_t tri_stride, uint32_t tlas_start, int use_tlas,
                           const tray_view* view, uint32_t width, uint32_t height, float render_time_s, int benchmark,
                           int animate, float* out_min_ms, float* out_mean_ms, uint32_t* out_frames) {
-    if (!view) return fail(TRAY_ERR_ARG, "NULL view");
-    if (bvh_len % 80 != 0) return fail(TRAY_ERR_ARG, "bvh_bytes length %llu is not a multiple of 80", (unsigned long long)bvh_len);
-    if (tri_stride == 0 || tri_len % tri_stride != 0) return fail(TRAY_ERR_ARG, "tri_bytes length is not a multiple of tri_stride");
-    if (instance_len % 4 != 0) return fail(TRAY_ERR_ARG, "instance_bytes length is not a multiple of 4");
+    if (const int rc = check_start_args(view, bvh_len, tri_len, tri_stride, instance_len)) return rc;
     tray_group* g = nullptr;
     int rc = tray_cuda_group_create(bvh_bytes, bvh_len / 80, tri_bytes, tri_len / tri_stride, tri_stride,
                                     use_tlas ? (const uint32_t*)instance_bytes : nullptr, use_tlas ? (uint32_t)(instance_len / 4) : 0u,
                                     tlas_start, devices, n_devices, &g);
     if (rc) return rc;
     const uint32_t flags = TRAY_RENDER_BOUNCE | TRAY_RENDER_RGBA;
-    float min_ms = 3.402823466e+38f; double sum = 0; uint32_t frames = 0, frame_count = 0;
-    const auto t0 = std::chrono::steady_clock::now();
-    for (;;) {
-        if (benchmark) {   // untimed warm-up dispatch right before the timed one (rt_gpu_software.rs:289-295)
-            rc = tray_cuda_group_render(g, view, width, height, frame_count, flags);
-            if (rc) break;
-        }
-        float ms = 0.f;
-        rc = tray_cuda_group_render_timed(g, view, width, height, frame_count, flags, &ms);
-        if (rc) break;
-        if (ms < min_ms) min_ms = ms;
-        sum += ms; frames++;
-        if (animate) frame_count = frames;
-        const float el = std::chrono::duration<float>(std::chrono::steady_clock::now() - t0).count();
-        if (el > render_time_s) break;
-    }
-    if (!rc) rc = tray_cuda_group_sync(g);
+    rc = start_loop([&](uint32_t fc) { return tray_cuda_group_render(g, view, width, height, fc, flags); },
+                    [&](uint32_t fc, float* ms) { return tray_cuda_group_render_timed(g, view, width, height, fc, flags, ms); },
+                    [&] { return tray_cuda_group_sync(g); },
+                    render_time_s, benchmark, animate, out_min_ms, out_mean_ms, out_frames);
     tray_cuda_group_destroy(g);
-    if (rc) return rc;
-    if (out_min_ms) *out_min_ms = min_ms;
-    if (out_mean_ms) *out_mean_ms = frames ? (float)(sum / frames) : 0.f;
-    if (out_frames) *out_frames = frames;
-    return TRAY_OK;
+    return rc;
 }
 
 }  // extern "C"
