@@ -243,7 +243,8 @@ int tray_cuda_trace(tray_scene* scene, const tray_ray* rays, uint64_t n, tray_hi
 
 /* Same with DEVICE pointers (rays and hits already resident in HBM); launches on `stream`
  * (a cudaStream_t passed as void*, NULL = the scene's own stream) and does NOT synchronise unless
- * ms_kernel != NULL.                                                                             */
+ * ms_kernel != NULL; when it does, it also reports a stack overflow of the batch (TRAY_ERR_OVERFLOW).  Without
+ * ms_kernel the overflow is reported by the next synchronising call on the scene (tray_cuda_sync).   */
 int tray_cuda_trace_device(tray_scene* scene, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits,
                            void* stream, float* ms_kernel);
 
@@ -294,7 +295,10 @@ int tray_cuda_frame_download(tray_scene* scene, tray_hit* primary, tray_hit* bou
  * through two or three of them, and `wait` for a slot before reading its host frame (begin on a slot still in flight waits for
  * it first).
  * After a frame rendered into a frame target (tray_cuda_scene_set_frame_target) the WHOLE target is read back — every
- * shard's pixels: call it on the device that owns the frame, stream-ordered after the barrier that completes the frame. */
+ * shard's pixels: call it on the device that owns the frame, stream-ordered after the barrier that completes the frame.
+ * The error status travels with the frame: every frame slot has its own device error word, `begin` takes the word of the
+ * frame it reads (on that frame's stream, so a later frame on the slot is not affected) and `wait` reports it — a stack
+ * overflow as TRAY_ERR_OVERFLOW, once, for that frame alone, also with two frames in flight (tests/test_deep_stack.py). */
 #define TRAY_READBACK_SLOTS 4
 int tray_cuda_frame_readback_begin(tray_scene* scene, uint8_t* rgba_host, uint32_t slot);
 int tray_cuda_frame_readback_wait(tray_scene* scene, uint32_t slot);

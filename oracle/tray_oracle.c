@@ -37,7 +37,14 @@
 
 static uint32_t g_variant = ORC_VARIANT_DEFAULT;
 void orc_set_variant(uint32_t flags) { g_variant = flags; }
-unsigned orc_abi_version(void) { return 2u; }
+static uint32_t g_stack_limit = ORC_STACK;
+int orc_set_stack_limit(uint32_t entries) {
+    if (entries < 1 || entries > ORC_STACK_MAX) return -1;
+    g_stack_limit = entries;
+    return 0;
+}
+uint32_t orc_stack_limit(void) { return g_stack_limit; }
+unsigned orc_abi_version(void) { return 3u; }
 int orc_max_threads(void) {
 #ifdef _OPENMP
     return omp_get_max_threads();
@@ -257,11 +264,13 @@ static inline int closer(float t, float tmax) {
 /* `any_hit`: stop at the first accepted triangle (the "faster anyhit query" rt_cpu.rs:78-79 asks for; the reference's
  * own intersects_bl_bvh, query.hlsl:440-445, runs the full closest-hit loop).  Same order of tests up to that point. */
 static int g_oplog_detail = 0;   /* step log flavour (orc_trace_oplog_detail): 'T'/'U' first / later triangle of a group, lower case = the test moved tmax */
-static int trace_one_ex(const orc_scene* s, const orc_ray* ray, orc_hit* out, orc_count* cnt, uint8_t* oplog, int any_hit) {
+/* `cap`: stack entries the traversal may hold; `peak` (optional): the most it held at once */
+static int trace_one_ex(const orc_scene* s, const orc_ray* ray, orc_hit* out, orc_count* cnt, uint8_t* oplog, int any_hit,
+                        uint32_t cap, uint32_t* peak) {
     uint32_t n_ops = 0;   /* optional step log: 'N' node fetch+test, 'T' triangle test, 'I' instance entry */
     prep_ray r; prepare_ray(ray, &r);
-    uint32_t stack[ORC_STACK][2];
-    uint32_t size = 0;
+    uint32_t stack[ORC_STACK_MAX][2];
+    uint32_t size = 0, max_size = 0;
     const int tlas = s->use_tlas;
     uint32_t tlas_stack_size = 0xFFFFFFFFu;                /* query_tlas.hlsl:343 INVALID = in the TLAS */
     uint32_t bvh_offset = tlas ? s->tlas_start : 0u;       /* query_tlas.hlsl:344 */
@@ -280,8 +289,9 @@ static int trace_one_ex(const orc_scene* s, const orc_ray* ray, orc_hit* out, or
             uint32_t child_index_base = cur_x;
             cur_y &= ~(1u << child_index_offset);                          /* :362 */
             if (cur_y & 0xff000000u) {                                     /* :365-368 */
-                if (size >= ORC_STACK) { overflow = 1; break; }
+                if (size >= cap) { overflow = 1; break; }
                 stack[size][0] = cur_x; stack[size][1] = cur_y; size++;
+                if (size > max_size) max_size = size;
             }
             uint32_t slot_index = (child_index_offset - 24u) ^ (r.oct_inv4 & 0xffu);      /* :370 */
             uint32_t relative_index = (uint32_t)__builtin_popcount(hits_imask & ~(0xffffffffu << slot_index)); /* :371 */
@@ -308,12 +318,14 @@ static int trace_one_ex(const orc_scene* s, const orc_ray* ray, orc_hit* out, or
             if (tlas && tlas_stack_size == 0xFFFFFFFFu) {
                 /* TLAS leaf: `global` is an instance slot (query_tlas.hlsl:410-446) */
                 if (tri_y != 0) {
-                    if (size >= ORC_STACK) { overflow = 1; break; }
+                    if (size >= cap) { overflow = 1; break; }
                     stack[size][0] = tri_x; stack[size][1] = tri_y; size++;       /* tlas:420-423 */
+                    if (size > max_size) max_size = size;
                 }
                 if (cur_y & 0xff000000u) {
-                    if (size >= ORC_STACK) { overflow = 1; break; }
+                    if (size >= cap) { overflow = 1; break; }
                     stack[size][0] = cur_x; stack[size][1] = cur_y; size++;       /* tlas:425-428 */
+                    if (size > max_size) max_size = size;
                 }
                 tlas_stack_size = size;                                           /* tlas:431 */
                 bvh_offset = s->blas_offsets[global];                             /* tlas:439 */
@@ -348,11 +360,12 @@ static int trace_one_ex(const orc_scene* s, const orc_ray* ray, orc_hit* out, or
     if (best_prim != ORC_INVALID_PRIM) { out->t = best_t; out->prim = best_prim; }
     else { out->t = INFINITY; out->prim = ORC_INVALID_PRIM; }              /* RayHit::none() */
     if (cnt) { cnt->nodes = n_nodes; cnt->tris = n_tris; cnt->insts = n_insts; }
+    if (peak) *peak = max_size;
     return overflow ? -4 : 0;
 }
 
 static int trace_one(const orc_scene* s, const orc_ray* ray, orc_hit* out, orc_count* cnt, uint8_t* oplog) {
-    return trace_one_ex(s, ray, out, cnt, oplog, 0);
+    return trace_one_ex(s, ray, out, cnt, oplog, 0, g_stack_limit, NULL);
 }
 
 int orc_trace_any(const orc_scene* s, const orc_ray* rays, uint64_t n, orc_hit* hits, orc_count* counts,
@@ -363,7 +376,7 @@ int orc_trace_any(const orc_scene* s, const orc_ray* rays, uint64_t n, orc_hit* 
 #pragma omp parallel for schedule(dynamic, 2048) num_threads(nthreads) reduction(+:tn,tt,ti,th) reduction(min:rc)
     for (int64_t i = 0; i < (int64_t)n; i++) {
         orc_count c;
-        int e = trace_one_ex(s, &rays[i], &hits[i], &c, NULL, 1);
+        int e = trace_one_ex(s, &rays[i], &hits[i], &c, NULL, 1, g_stack_limit, NULL);
         if (e < rc) rc = e;
         if (counts) counts[i] = c;
         tn += c.nodes; tt += c.tris; ti += c.insts; th += hits[i].prim != ORC_INVALID_PRIM;
@@ -387,6 +400,18 @@ int orc_trace(const orc_scene* s, const orc_ray* rays, uint64_t n, orc_hit* hits
         tn += c.nodes; tt += c.tris; ti += c.insts; th += hits[i].prim != ORC_INVALID_PRIM;
     }
     if (totals) { totals->rays = n; totals->nodes = tn; totals->tris = tt; totals->insts = ti; totals->hits = th; }
+    return rc;
+}
+
+int orc_stack_need(const orc_scene* s, const orc_ray* rays, uint64_t n, uint32_t* need, int any_hit, int nthreads) {
+    int rc = 0;
+    if (nthreads <= 0) nthreads = orc_max_threads();
+#pragma omp parallel for schedule(dynamic, 2048) num_threads(nthreads) reduction(min:rc)
+    for (int64_t i = 0; i < (int64_t)n; i++) {
+        orc_hit h;
+        int e = trace_one_ex(s, &rays[i], &h, NULL, NULL, any_hit, ORC_STACK_MAX, &need[i]);
+        if (e < rc) rc = e;
+    }
     return rc;
 }
 

@@ -64,7 +64,19 @@ void orc_set_simd(int on);
 int orc_simd(void);
 int orc_max_threads(void);
 
-/* closest hit for n rays; returns 0, or -4 if any ray overflowed the 32-entry stack (cwbvh.rs:88) */
+/* Traversal stack capacity of orc_trace, orc_trace_any, orc_trace_oplog* and orc_render: 1 .. ORC_STACK_MAX entries, default
+ * 32 (obvhs, cwbvh.rs:88); the CUDA kernels hold 48.  Returns 0, or -1 (unchanged) when `entries` is out of range. */
+#define ORC_STACK_MAX 64
+int orc_set_stack_limit(uint32_t entries);
+uint32_t orc_stack_limit(void);
+
+/* Per ray, the most entries its traversal holds on the stack at once, counted as the kernels count them: node groups pushed
+ * behind a node's first child, and at a TLAS instance entry the rest of the instance group and the node group.  Closest-hit
+ * (any_hit = 0) or any-hit traversal, traversed with ORC_STACK_MAX entries whatever orc_set_stack_limit says.
+ * Returns 0, or -4 if a ray needs more than ORC_STACK_MAX (its need is then not meaningful). */
+int orc_stack_need(const orc_scene* s, const orc_ray* rays, uint64_t n, uint32_t* need, int any_hit, int nthreads);
+
+/* closest hit for n rays; returns 0, or -4 if any ray overflowed the stack (orc_set_stack_limit) */
 int orc_trace(const orc_scene* s, const orc_ray* rays, uint64_t n, orc_hit* hits, orc_count* counts,
               orc_totals* totals, int nthreads);
 

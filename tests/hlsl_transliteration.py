@@ -118,7 +118,8 @@ def intersect_ray_tri(org, d, v0, e1_stored, e2, t):                  # :89-129;
     return None
 
 
-def traverse_bvh(scene, origin, direction):                           # :328-438; returns (t, triangle_id, nodes, tris)
+def traverse_bvh(scene, origin, direction, stack_peak=False):         # :328-438; returns (t, triangle_id, nodes, tris)
+    """stack_peak=True: the tuple ends with the most entries the stack held at once"""
     org = [f32(x) for x in origin]
     d = [f32(x) for x in direction]
     d = [F32_EPSILON if x == 0.0 else x for x in d]                   # :334
@@ -126,7 +127,7 @@ def traverse_bvh(scene, origin, direction):                           # :328-438
     oct_inv4 = ray_get_octant_inv4(d)
     current_group = [0, 0x80000000]
     t, triangle_id = F32_MAX, -1
-    n_nodes = n_tris = 0
+    n_nodes = n_tris = peak = 0
     while True:
         if current_group[1] & 0xff000000:
             hits_imask = current_group[1]
@@ -135,6 +136,7 @@ def traverse_bvh(scene, origin, direction):                           # :328-438
             current_group[1] &= ~(1 << child_index_offset) & 0xffffffff
             if current_group[1] & 0xff000000:
                 stack.append(list(current_group))
+                peak = max(peak, len(stack))
             slot_index = (child_index_offset - 24) ^ (oct_inv4 & 0xff)
             relative_index = bin(hits_imask & ~(0xffffffff << slot_index) & 0xffffffff).count("1")
             node = scene.nodes[child_index_base + relative_index]
@@ -160,14 +162,15 @@ def traverse_bvh(scene, origin, direction):                           # :328-438
             if not stack:
                 break
             current_group = stack.pop()
-    return t, triangle_id, n_nodes, n_tris
+    return (t, triangle_id, n_nodes, n_tris) + ((peak,) if stack_peak else ())
 
 
 INVALID = 0xFFFFFFFF
 
 
-def traverse_bvh_tlas(scene, origin, direction):
-    """rt_gpu_software_query_tlas.hlsl:333-500; returns (t, triangle_id, nodes, tris, instances entered)"""
+def traverse_bvh_tlas(scene, origin, direction, stack_peak=False):
+    """rt_gpu_software_query_tlas.hlsl:333-500; returns (t, triangle_id, nodes, tris, instances entered), and with
+    stack_peak=True the most entries the stack held at once"""
     org = [f32(x) for x in origin]
     d = [f32(x) for x in direction]
     d = [F32_EPSILON if x == 0.0 else x for x in d]                   # :339
@@ -177,7 +180,7 @@ def traverse_bvh_tlas(scene, origin, direction):
     oct_inv4 = ray_get_octant_inv4(d)
     current_group = [0, 0x80000000]
     t, triangle_id = F32_MAX, -1
-    n_nodes = n_tris = n_inst = 0
+    n_nodes = n_tris = n_inst = peak = 0
     while True:
         if current_group[1] & 0xff000000:
             hits_imask = current_group[1]
@@ -186,6 +189,7 @@ def traverse_bvh_tlas(scene, origin, direction):
             current_group[1] &= ~(1 << child_index_offset) & 0xffffffff
             if current_group[1] & 0xff000000:
                 stack.append(list(current_group))
+                peak = max(peak, len(stack))
             slot_index = (child_index_offset - 24) ^ (oct_inv4 & 0xff)
             relative_index = bin(hits_imask & ~(0xffffffff << slot_index) & 0xffffffff).count("1")
             node = scene.nodes[current_bvh_offset + child_index_base + relative_index]          # :383
@@ -207,6 +211,7 @@ def traverse_bvh_tlas(scene, origin, direction):
                     stack.append(list(triangle_group))                                           # :420-423
                 if (current_group[1] & 0xff000000) != 0:
                     stack.append(list(current_group))                                            # :425-428
+                peak = max(peak, len(stack))
                 tlas_stack_size = len(stack)                                                     # :431
                 current_bvh_offset = scene.blas_offsets[g]                                       # :439
                 n_inst += 1
@@ -227,4 +232,4 @@ def traverse_bvh_tlas(scene, origin, direction):
                 tlas_stack_size = INVALID
                 current_bvh_offset = scene.tlas_start
             current_group = stack.pop()
-    return t, triangle_id, n_nodes, n_tris, n_inst
+    return (t, triangle_id, n_nodes, n_tris, n_inst) + ((peak,) if stack_peak else ())

@@ -2,6 +2,7 @@
 __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs — never from the package."""
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 import subprocess
@@ -22,6 +23,8 @@ VARIANT_BOX_TMIN_RAY = 4
 VARIANT_ZERODIR_BOX_ONLY = 8
 RENDER_BOUNCE = 1
 RENDER_RGBA = 2
+STACK_DEFAULT = 32          # obvhs' traversal stack (cwbvh.rs:88)
+STACK_MAX = 64              # ORC_STACK_MAX
 
 
 class OrcView(C.Structure):
@@ -57,6 +60,11 @@ def lib() -> C.CDLL:
         L = C.CDLL(_LIB_PATH)
         vp, u64, u32, i32 = C.c_void_p, C.c_uint64, C.c_uint32, C.c_int
         L.orc_set_variant.argtypes = [u32]
+        L.orc_set_stack_limit.restype = i32
+        L.orc_set_stack_limit.argtypes = [u32]
+        L.orc_stack_limit.restype = u32
+        L.orc_stack_need.restype = i32
+        L.orc_stack_need.argtypes = [C.POINTER(OrcScene), vp, u64, vp, i32, i32]
         L.orc_max_threads.restype = i32
         L.orc_set_simd.argtypes = [i32]
         L.orc_simd.restype = i32
@@ -85,6 +93,17 @@ def lib() -> C.CDLL:
     return _lib
 
 
+@contextlib.contextmanager
+def _stack_limit(entries):
+    """the oracle's stack capacity for the calls inside the block (1 .. STACK_MAX), the default again after it"""
+    if lib().orc_set_stack_limit(int(entries)) != 0:
+        raise ValueError(f"stack_limit must be 1 .. {STACK_MAX} (got {entries})")
+    try:
+        yield
+    finally:
+        lib().orc_set_stack_limit(STACK_DEFAULT)
+
+
 def _view(view) -> OrcView:
     v = OrcView()
     C.memmove(C.byref(v), C.byref(view), C.sizeof(OrcView))
@@ -110,18 +129,30 @@ class Oracle:
     def from_packed(cls, p) -> "Oracle":
         return cls(p.bvh_bytes, p.tri_bytes, p.tri_stride, p.blas_offsets if p.use_tlas else None, p.tlas_start, p.use_tlas)
 
-    def trace(self, rays, counts=False, nthreads=0, any_hit=False):
-        """closest hit per ray; any_hit=True stops each ray at the first accepted triangle (orc_trace_any)"""
+    def trace(self, rays, counts=False, nthreads=0, any_hit=False, stack_limit=STACK_DEFAULT):
+        """closest hit per ray; any_hit=True stops each ray at the first accepted triangle (orc_trace_any).
+        Raises when a ray needs more than `stack_limit` stack entries (obvhs' 32 by default; the kernels hold 48)."""
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
         hits = np.empty(rays.shape[0], dtype=HIT_DTYPE)
         cnt = np.empty(rays.shape[0], dtype=COUNT_DTYPE) if counts else None
         tot = OrcTotals()
         fn = lib().orc_trace_any if any_hit else lib().orc_trace
-        rc = fn(C.byref(self.scene), rays.ctypes.data, rays.shape[0], hits.ctypes.data,
-                             None if cnt is None else cnt.ctypes.data, C.byref(tot), nthreads)
+        with _stack_limit(stack_limit):
+            rc = fn(C.byref(self.scene), rays.ctypes.data, rays.shape[0], hits.ctypes.data,
+                    None if cnt is None else cnt.ctypes.data, C.byref(tot), nthreads)
         if rc != 0:
             raise RuntimeError(f"oracle traversal stack overflow ({rc})")
         return (hits, cnt, tot.as_dict()) if counts else hits
+
+    def stack_need(self, rays, any_hit=False, nthreads=0) -> np.ndarray:
+        """per ray, the most stack entries its traversal holds at once (node groups, and the two pushes of a TLAS instance
+        entry), whatever the stack capacity; raises when a ray needs more than STACK_MAX"""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        need = np.empty(rays.shape[0], dtype=np.uint32)
+        rc = lib().orc_stack_need(C.byref(self.scene), rays.ctypes.data, rays.shape[0], need.ctypes.data, int(any_hit), nthreads)
+        if rc != 0:
+            raise RuntimeError(f"a ray needs more than {STACK_MAX} stack entries ({rc})")
+        return need
 
     def brute_force(self, rays, nthreads=0):
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
@@ -134,7 +165,7 @@ class Oracle:
         r = np.ascontiguousarray(ray, dtype=RAY_DTYPE).reshape(1)
         return lib().orc_intersect_tri(C.byref(self.scene), int(prim), r.ctypes.data)
 
-    def render(self, view, w, h, frame_count=0, flags=RENDER_BOUNCE, nthreads=0, rgba=False):
+    def render(self, view, w, h, frame_count=0, flags=RENDER_BOUNCE, nthreads=0, rgba=False, stack_limit=STACK_DEFAULT):
         n = w * h
         primary = np.empty(n, dtype=HIT_DTYPE)
         bounce = np.empty(n, dtype=HIT_DTYPE)
@@ -142,9 +173,10 @@ class Oracle:
         img = np.zeros((n, 4), dtype=np.uint8) if rgba else None
         pt, bt = OrcTotals(), OrcTotals()
         v = _view(view)
-        rc = lib().orc_render(C.byref(self.scene), C.byref(v), w, h, frame_count, flags | (RENDER_RGBA if rgba else 0),
-                              primary.ctypes.data, bounce.ctypes.data, brays.ctypes.data,
-                              None if img is None else img.ctypes.data, C.byref(pt), C.byref(bt), nthreads)
+        with _stack_limit(stack_limit):
+            rc = lib().orc_render(C.byref(self.scene), C.byref(v), w, h, frame_count, flags | (RENDER_RGBA if rgba else 0),
+                                  primary.ctypes.data, bounce.ctypes.data, brays.ctypes.data,
+                                  None if img is None else img.ctypes.data, C.byref(pt), C.byref(bt), nthreads)
         if rc != 0:
             raise RuntimeError(f"oracle traversal stack overflow ({rc})")
         return dict(primary=primary, bounce=bounce, bounce_rays=brays, rgba=img, primary_totals=pt.as_dict(), bounce_totals=bt.as_dict())

@@ -61,6 +61,7 @@ struct FrameSlot {
     tray_ray* d_brays = nullptr;             // generated bounce rays, COMPACT (hit pixels only)
     uint32_t* d_bitem = nullptr;             // local item of compact bounce ray i
     tray_ray* d_brays_item = nullptr;        // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
+    uint32_t* d_flag = nullptr;              // the device error word of this slot's launches (a word of tray_scene::d_overflow)
     tray::FrameParams last_frame{};          // width 0: no frame rendered yet
 };
 
@@ -77,6 +78,8 @@ struct tray_scene {
     uint32_t* d_prim_indices = nullptr;      // BVH slot -> input triangle (scenes made by tray_cuda_scene_build)
     uint32_t* d_geom_offsets = nullptr; uint32_t n_geometries = 0;   // first global triangle of BLAS / object g (tray_cuda_scene_set_geometry_offsets)
     unsigned long long* d_cursor = nullptr;     // [0] cursor (u32), [1..10] 2 x 5 counters, [11] bounce-ray count (u32)
+    // device error words (TraceParams::overflow): [0] batch traces, [1 + k] the launches of frame slot k — one word per slot, so
+    // that a frame's error is reported for that frame and cleared in the order of that slot's stream
     uint32_t* d_overflow = nullptr;
     cudaStream_t stream = nullptr;          // the stream work is enqueued on
     cudaStream_t own_stream = nullptr;      // created with the scene
@@ -105,7 +108,7 @@ struct tray_scene {
     cudaEvent_t ev_untiled[TRAY_READBACK_SLOTS] = {}, ev_copied[TRAY_READBACK_SLOTS] = {};
     cudaEvent_t ev_after = nullptr;          // tray_cuda_scene_after
     uint32_t bounce_sort = 1;                // raygen_bounce_kernel: 0 append in pixel order, 1 group by direction octant, 2 octant x major axis
-    uint32_t* h_flag = nullptr;              // pinned, one word per staging slot: the device error flag as it was when staging slot i was filled
+    uint32_t* h_flag = nullptr;              // pinned, one word per staging slot: the error word of the frame staging slot i was filled from
     uchar4* frame_target = nullptr;          // borrowed: row-major RGBA8 frame (this or a peer device), see tray_cuda_scene_set_frame_target
     tray_counters cnt_primary{}, cnt_bounce{};
 };
@@ -269,19 +272,20 @@ int read_counters(const unsigned long long* cur, cudaStream_t st, int slot, tray
     return TRAY_OK;
 }
 
-// a word of the device error flag as a status (4: the frame kernel's watchdog, other bits: stack overflow); clears a set flag
-int flag_status(tray_scene* s, uint32_t f) {
+// a device error word as a status (4: the frame kernel's watchdog, other bits: stack overflow)
+int flag_status(uint32_t f) {
     if (!f) return TRAY_OK;
-    cudaMemsetAsync(s->d_overflow, 0, 4, s->stream);
     if (f & 4u) return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
     return fail(TRAY_ERR_OVERFLOW, "traversal stack overflow: BVH needs more than %d stack entries", STACK_SMEM + STACK_SPILL);
 }
-int check_overflow(tray_scene* s, cudaStream_t st = nullptr) {
-    if (!st) st = s->stream;
+// the error word `flag` behind the work enqueued on `st`, as a status; a set word is cleared there, in stream order, so that an
+// error is reported once, by the first synchronising call that covers the launch that raised it
+int check_overflow(uint32_t* flag, cudaStream_t st) {
     uint32_t f = 0;
-    CU(cudaMemcpyAsync(&f, s->d_overflow, 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&f, flag, 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    return flag_status(s, f);
+    if (f) cudaMemsetAsync(flag, 0, 4, st);
+    return flag_status(f);
 }
 
 // the start protocol's arguments (the reference asserts these strides at src/rt_gpu/mod.rs:70,86,105,107)
@@ -491,18 +495,19 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         }
         if (!s->d_blas) CU(cudaMalloc(&s->d_blas, (size_t)(n_instances ? n_instances : 1) * 4));
         CU(cudaMalloc(&s->d_cursor, 16 * sizeof(unsigned long long)));
-        CU(cudaMalloc(&s->d_overflow, 4));
+        CU(cudaMalloc(&s->d_overflow, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t)));
         CU(cudaMemsetAsync(s->d_cursor, 0, 16 * sizeof(unsigned long long), s->stream));
         for (int k = 0; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) {
             FrameSlot& f = s->slot[k];
             if (k >= 1) CU(cudaStreamCreateWithFlags(&f.own_stream, cudaStreamNonBlocking));
             CU(cudaMalloc(&f.d_cursor, 16 * sizeof(unsigned long long)));
             CU(cudaMalloc(&f.d_units, sizeof(uint32_t)));
+            f.d_flag = s->d_overflow + 1 + k;
             CU(cudaMemsetAsync(f.d_cursor, 0, 16 * sizeof(unsigned long long), s->stream));
             for (auto& e : f.ev) CU(cudaEventCreate(&e));
             CU(cudaEventCreateWithFlags(&f.done, cudaEventDisableTiming));
         }
-        CU(cudaMemsetAsync(s->d_overflow, 0, 4, s->stream));
+        CU(cudaMemsetAsync(s->d_overflow, 0, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t), s->stream));
         s->device_bytes = nb + tb + (size_t)n_instances * 4;
         if (!adopted) {
             if (n_nodes) CU(tray::upload_pipelined(s->d_nodes, nodes, (size_t)n_nodes * 80, s->stream));
@@ -720,7 +725,15 @@ int tray_cuda_sync(tray_scene* s) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     CU(cudaSetDevice(s->device));
     if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
-    return check_overflow(s);
+    // every error word a launch of the scene can have set: batch traces and each frame slot; a set word is cleared on its own
+    // stream, ahead of whatever is enqueued there next
+    uint32_t f[1 + TRAY_MAX_FRAMES_IN_FLIGHT];
+    CU(cudaMemcpyAsync(f, s->d_overflow, sizeof f, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    uint32_t all = 0;
+    for (int k = 0; k <= TRAY_MAX_FRAMES_IN_FLIGHT; k++)
+        if (f[k]) { all |= f[k]; cudaMemsetAsync(s->d_overflow + k, 0, 4, k ? slot_stream(s, k - 1) : s->stream); }
+    return flag_status(all);
 }
 
 }  // extern "C"
@@ -742,6 +755,7 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
         CU(cudaEventRecord(s->ev[1], st));
         CU(cudaEventSynchronize(s->ev[1]));
         CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+        return check_overflow(s->d_overflow, st);         // synchronised: an overflow of this batch is reported by this call
     }
     return TRAY_OK;
 }
@@ -835,7 +849,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         CU(cudaEventElapsedTime(&k, s->ev[0], s->ev[1]));       // span of the GPU work, uploads it waited for included
     }
     if (s->counting) { rc = read_counters(s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc; memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce); }
-    rc = check_overflow(s);
+    rc = check_overflow(s->d_overflow, s->stream);
     if (rc) return rc;
     if (ms_kernel) *ms_kernel = k;
     if (ms_total) *ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -997,7 +1011,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     tray::raygen_primary_kernel<<<gen_grid, 256, 0, st>>>(F, f.d_prays);
     CU(cudaGetLastError());
     TraceParams P; base_params(s, P);
-    P.rays = f.d_prays; P.n_work = F.n_items; P.hits_out = f.d_primary;
+    P.rays = f.d_prays; P.n_work = F.n_items; P.hits_out = f.d_primary; P.overflow = f.d_flag;
     uchar4* const rgba_dst = s->frame_target ? s->frame_target : f.d_rgba;
     auto set_frame = [&](TraceParams& T) {
         if (!s->frame_target) return;
@@ -1029,6 +1043,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         CU(cudaGetLastError());
         TraceParams B; base_params(s, B);
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
+        B.overflow = f.d_flag;
         B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
         if (B.rgba_out) set_frame(B);
         rc = launch(s, B, st, f.d_cursor, 1, any_ao);
@@ -1042,7 +1057,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         if (bounce) CU(cudaEventElapsedTime(&b, f.ev[1], f.ev[2]));
         if (ms_primary) *ms_primary = a;
         if (ms_bounce) *ms_bounce = b;
-        rc = check_overflow(s, st); if (rc) return rc;
+        rc = check_overflow(f.d_flag, st); if (rc) return rc;
     }
     if (s->counting) {
         rc = read_counters(f.d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
@@ -1067,7 +1082,7 @@ int tray_cuda_render_timed(tray_scene* s, const tray_view* view, uint32_t w, uin
     CU(cudaEventRecord(s->slot[k].ev[3], st));
     CU(cudaEventSynchronize(s->slot[k].ev[3]));
     CU(cudaEventElapsedTime(ms_frame, s->slot[k].ev[0], s->slot[k].ev[3]));
-    return check_overflow(s, st);             // synchronising point: a stack overflow / watchdog flag must not pass as TRAY_OK
+    return check_overflow(s->slot[k].d_flag, st);    // synchronising point: a stack overflow / watchdog flag must not pass as TRAY_OK
 }
 
 int tray_cuda_counters(tray_scene* s, tray_counters* primary, tray_counters* bounce) {
@@ -1140,7 +1155,7 @@ int tray_cuda_frame_download(tray_scene* s, tray_hit* primary, tray_hit* bounce,
         if (!f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA");
         rc = download<uchar4>(s, f.d_rgba, (uchar4*)rgba); if (rc) return rc;
     }
-    return check_overflow(s, slot_stream(s, s->cur));
+    return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 
 int tray_cuda_frame_readback_begin(tray_scene* s, uint8_t* rgba, uint32_t slot) {
@@ -1166,11 +1181,13 @@ int tray_cuda_frame_readback_begin(tray_scene* s, uint8_t* rgba, uint32_t slot) 
     } else if (const int rc = untile_last_frame(s, f.d_rgba, s->d_stage[slot])) {
         return rc;
     }
+    // the error word travels with the frame (a stream synchronise here would undo the overlap): taken on the frame's stream,
+    // behind the frame's launches and ahead of the next frame on that slot, and reported by _wait
+    CU(cudaMemcpyAsync(s->h_flag + slot, f.d_flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemsetAsync(f.d_flag, 0, sizeof(uint32_t), st));
     CU(cudaEventRecord(s->ev_untiled[slot], st));
     CU(cudaStreamWaitEvent(s->copy_stream, s->ev_untiled[slot], 0));
     CU(cudaMemcpyAsync(rgba, s->d_stage[slot], bytes, cudaMemcpyDeviceToHost, s->copy_stream));
-    // the error flag travels with the frame (a stream synchronise here would undo the overlap): checked in _wait
-    CU(cudaMemcpyAsync(s->h_flag + slot, s->d_overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s->copy_stream));
     CU(cudaEventRecord(s->ev_copied[slot], s->copy_stream));
     s->stage_busy[slot] = true;
     return TRAY_OK;
@@ -1184,7 +1201,7 @@ int tray_cuda_frame_readback_wait(tray_scene* s, uint32_t slot) {
     s->stage_busy[slot] = false;
     const uint32_t fl = s->h_flag[slot];
     s->h_flag[slot] = 0u;
-    return flag_status(s, fl);
+    return flag_status(fl);
 }
 
 int tray_cuda_start(const void* bvh_bytes, uint64_t bvh_len, const void* instance_bytes, uint64_t instance_len,
@@ -1490,7 +1507,7 @@ int tray_cuda_group_render_timed(tray_group* g, const tray_view* view, uint32_t 
     CU(cudaEventRecord(g->ev_t1, slot_stream(s0, s0->cur)));
     CU(cudaEventSynchronize(g->ev_t1));
     CU(cudaEventElapsedTime(ms_frame, g->ev_t0, g->ev_t1));
-    for (auto* sc : g->scenes) { CU(cudaSetDevice(sc->device)); rc = check_overflow(sc, slot_stream(sc, sc->cur)); if (rc) return rc; }
+    for (auto* sc : g->scenes) { CU(cudaSetDevice(sc->device)); rc = check_overflow(sc->slot[sc->cur].d_flag, slot_stream(sc, sc->cur)); if (rc) return rc; }
     return TRAY_OK;
 }
 
