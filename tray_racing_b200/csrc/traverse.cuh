@@ -45,7 +45,16 @@ constexpr uint32_t INVALID = 0xffffffffu;
 // rows are LUT_ROW = 260 bytes apart: the same hit byte under different octants then falls into different banks (lanes of an
 // incoherent warp mostly hold one-bit hit bytes; at a 256-byte pitch they would all collide in banks 0, 1, 2, 4, ...)
 constexpr uint32_t LUT_ROW = 260u, LUT_BYTES = 8u * LUT_ROW;
-constexpr uint32_t WIDE_BIT = 0x40000000u;       // trace_kernel: bit 30 of a lane's ray index = RayConst::wide
+// trace_kernel's ray index: the ray's place in its launch (the host keeps launches below 2^30 rays) and two tag bits
+constexpr uint32_t BOUNCE_BIT = 0x80000000u;     // FRAME kernel: a bounce ray, its index is the work item
+constexpr uint32_t WIDE_BIT = 0x40000000u;       // RayConst::wide
+constexpr uint32_t INDEX_MASK = 0x3fffffffu;
+// bits of the device error word (TraceParams::overflow)
+constexpr uint32_t ERR_STACK_OVERFLOW = 1u;      // a push past the last of the STACK_SMEM + STACK_SPILL entries
+constexpr uint32_t ERR_WATCHDOG = 4u;            // FRAME kernel: the primary hits of a group never arrived
+// a launch's cursor block, CURSOR_WORDS 64-bit words: [0] the work cursor (u32), [CURSOR_COUNTERS + N_COUNTERS * k ..] counter slot k
+// (rays, nodes, tris, instances, hits; slot 1: the bounce rays of a frame), [CURSOR_N_BOUNCE] the bounce-ray count of a frame (u32)
+constexpr uint32_t CURSOR_COUNTERS = 1, N_COUNTERS = 5, CURSOR_N_BOUNCE = 11, CURSOR_WORDS = 16;
 constexpr float F32_MAX_ = 3.402823466e+38f;
 constexpr float F32_EPS_ = 1.1920929e-7f;     // sampling.hlsl:3
 constexpr float BOX_EPS_ = 0.0001f;           // query.hlsl:274
@@ -69,12 +78,12 @@ struct TraceParams {
     uint32_t n_work;
     const uint32_t* __restrict__ n_work_dev;  // optional: ray count produced on the device (overrides n_work)
     tray_hit* __restrict__ hits_out;
-    uchar4* __restrict__ rgba_out;            // optional: compact (item order), or a row-major frame when frame_w != 0
-    uint32_t frame_w, frame_h, frame_tiles_x, frame_shard, frame_shards;   // frame target geometry (item -> pixel)
+    uchar4* __restrict__ rgba_out;            // optional: compact (item order), or the row-major frame of `frame` when row_major
+    uint32_t row_major;
     uint32_t shade_mode;
     uint32_t* __restrict__ cursor;            // work cursor
-    unsigned long long* __restrict__ counters;// rays, nodes, tris, instances, hits (COUNT builds)
-    uint32_t* __restrict__ overflow;
+    unsigned long long* __restrict__ counters;// counter slot (N_COUNTERS; FRAME: two slots) of the cursor block (COUNT builds)
+    uint32_t* __restrict__ overflow;          // device error word (ERR_*)
     unsigned long long* __restrict__ dev_log; // -DTRAY_EXIT_LOG / -DTRAY_STEP_CLOCK builds: per-warp records
     uint32_t k4b;                             // 0x4B000000, passed at run time (see byte_f32)
     uint32_t force_exact;                     // scene has node scales >= 2^40: always take the unfused node test
@@ -83,8 +92,8 @@ struct TraceParams {
     uint32_t refill_min;                      // idle lanes needed before a partial warp refills
     uint32_t tri_weight;                      // vote: triangle phase when n_tri * tri_weight >= n_node
     uint32_t variant;                         // MODE 1 kernels only: TRAY_VARIANT_* switches (tray_cuda_scene_set_variant)
+    FrameParams frame;                        // frame launches: camera, frame geometry, frame_count (item -> pixel)
     // FRAME kernel only (one launch per frame: bounce rays of finished 32-item groups start while the primary pass drains)
-    FrameParams frame;                        // camera, frame geometry, frame_count (rays = the primary rays in item order)
     tray_hit* __restrict__ bounce_out;        // bounce hits by item
     tray_ray* __restrict__ rays_by_item;      // optional: the generated bounce rays by item (checkers)
     tray_ray* gen_rays;                       // bounce rays by item: written full-width when a group is claimed, read back lane by lane
@@ -376,12 +385,11 @@ __device__ __forceinline__ bool item_to_pixel(const FrameParams& P, uint32_t j, 
 
 // where the RGBA of work item `item` goes: slot `item` of the compact buffer, or its pixel of a row-major frame target
 // (possibly peer memory: the store then travels over NVLink while the warp keeps tracing); -1 = pixel outside the frame
-__device__ __forceinline__ long long rgba_slot(uint32_t item, uint32_t w, uint32_t h, uint32_t tiles_x, uint32_t shard, uint32_t shards) {
-    if (w == 0u) return (long long)item;
-    FrameParams F; F.width = w; F.height = h; F.tiles_x = tiles_x; F.shard_index = shard; F.shard_count = shards;
+__device__ __forceinline__ long long rgba_slot(const FrameParams& F, uint32_t item, bool row_major) {
+    if (!row_major) return (long long)item;
     uint32_t px, py;
     if (!item_to_pixel(F, item, px, py)) return -1;
-    return (long long)py * w + px;
+    return (long long)py * F.width + px;
 }
 
 // glam Mat4 * Vec4 (column-major): ((c0*x + c1*y) + c2*z) + c3*w
@@ -465,11 +473,41 @@ __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __
     normalize3(dx, dy, dz);
 }
 
-__device__ __forceinline__ uchar4 shade(float col) {                           // rt_cpu.rs:104-106
+// the colour of a result of kind `mode` (ShadeMode), gamma-encoded as rt_cpu.rs:104-106
+__device__ __forceinline__ uchar4 shade(uint32_t mode, float t) {
+    float col;
+    if (mode == SHADE_PRIMARY) col = __fdiv_rn(1.0f, t);                                   // rt_cpu.rs:59 (1/inf = 0)
+    else if (mode == SHADE_OCCLUSION) col = t < F32_MAX_ ? 0.0f : 1.0f;                   // any-hit AO: visibility only
+    else col = t < F32_MAX_ ? __fdiv_rn(t, add(1.0f, t)) : 1.0f;                          // rt_cpu.rs:82-87
     float g = powf(col, 2.2f) * 255.0f;
     g = g < 0.0f ? 0.0f : (g > 255.0f ? 255.0f : g);
     const unsigned char v = (unsigned char)g;
     return make_uchar4(v, v, v, 255);
+}
+__device__ __forceinline__ void store_rgba(uchar4* rgba_out, const FrameParams& F, bool row_major, uint32_t item, uint32_t mode, float t) {
+    if (!rgba_out) return;
+    const long long o = rgba_slot(F, item, row_major);
+    if (o >= 0) rgba_out[o] = shade(mode, t);
+}
+
+// a tray_ray as two 16-byte stores: {origin, tmin}, {direction, tmax}
+__device__ __forceinline__ void store_ray(tray_ray* dst, const float4& a, const float4& b) {
+    float4* o = reinterpret_cast<float4*>(dst);
+    o[0] = a; o[1] = b;
+}
+// the bounce ray of work item `item` as generated, for checkers (optional buffer, TRAY_RENDER_KEEP_RAYS)
+__device__ __forceinline__ void keep_ray(tray_ray* rays_by_item, uint32_t item, const float4& a, const float4& b) {
+    if (rays_by_item) store_ray(rays_by_item + item, a, b);
+}
+// a pixel that shoots no bounce ray (primary miss, or outside the frame) gets its final results at once: a bounce miss, the
+// primary shade, a zero ray
+__device__ __forceinline__ void finish_no_bounce(const FrameParams& F, bool row_major, uint32_t item, float t_primary, tray_hit* bounce_out,
+                                                 uchar4* rgba_out, tray_ray* rays_by_item) {
+    tray_hit miss; miss.t = __int_as_float(0x7f800000); miss.prim = INVALID;
+    bounce_out[item] = miss;
+    store_rgba(rgba_out, F, row_major, item, SHADE_PRIMARY, t_primary);
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    keep_ray(rays_by_item, item, z, z);
 }
 
 // ---- ray generation ---------------------------------------------------------------------------------
@@ -483,8 +521,7 @@ __global__ void __launch_bounds__(256) raygen_primary_kernel(const __grid_consta
         a = make_float4(F.view.eye[0], F.view.eye[1], F.view.eye[2], 0.0f);            // Ray::new(eye, dir, 0.0, f32::MAX)
         b = make_float4(dx, dy, dz, F32_MAX_);
     }
-    float4* out = reinterpret_cast<float4*>(rays + j);
-    out[0] = a; out[1] = b;
+    store_ray(rays + j, a, b);
 }
 
 // One thread per pixel of the shard.  Hit pixels append their bounce ray to a compact list (warp-aggregated
@@ -495,7 +532,7 @@ __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __gri
                                                             const tray_hit* __restrict__ primary, tray_ray* __restrict__ rays,
                                                             uint32_t* __restrict__ ray_item, uint32_t* __restrict__ n_rays,
                                                             tray_hit* __restrict__ bounce_out, uchar4* __restrict__ rgba_out,
-                                                            tray_ray* __restrict__ rays_by_item, uint32_t rgba_row_major, uint32_t sort_octant) {
+                                                            tray_ray* __restrict__ rays_by_item, uint32_t row_major, uint32_t sort_octant) {
     __shared__ uint32_t s_cnt[24], s_base[24];
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned lane = threadIdx.x & 31u;
@@ -536,8 +573,7 @@ __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __gri
         __syncthreads();
         if (shoot) {
             const uint32_t slot = s_base[oct] + pos;
-            float4* out = reinterpret_cast<float4*>(rays + slot);
-            out[0] = a; out[1] = b;
+            store_ray(rays + slot, a, b);
             ray_item[slot] = j;
         }
     } else {
@@ -549,22 +585,14 @@ __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __gri
         base = __shfl_sync(FULL, base, leader);
         if (shoot) {
             const uint32_t slot = base + (uint32_t)__popc(m & ((1u << lane) - 1u));
-            float4* out = reinterpret_cast<float4*>(rays + slot);
-            out[0] = a; out[1] = b;
+            store_ray(rays + slot, a, b);
             ray_item[slot] = j;
         }
     }
     }
     if (j < F.n_items) {
-        if (!shoot) {
-            tray_hit miss; miss.t = __int_as_float(0x7f800000); miss.prim = INVALID;
-            bounce_out[j] = miss;
-            if (rgba_out) {                                                             // rt_cpu.rs:59 (1/inf = 0)
-                if (!rgba_row_major) rgba_out[j] = shade(__fdiv_rn(1.0f, ph.t));
-                else if (item_to_pixel(F, j, px, py)) rgba_out[(size_t)py * F.width + px] = shade(__fdiv_rn(1.0f, ph.t));
-            }
-        }
-        if (rays_by_item) { float4* o2 = reinterpret_cast<float4*>(rays_by_item + j); o2[0] = a; o2[1] = b; }
+        if (!shoot) finish_no_bounce(F, row_major, j, ph.t, bounce_out, rgba_out, rays_by_item);
+        else keep_ray(rays_by_item, j, a, b);
     }
 }
 
@@ -579,6 +607,21 @@ __device__ __forceinline__ bool poll_hit(const tray_hit* src, float2& ph) {     
     asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(src) : "memory");
     ph.x = __uint_as_float((uint32_t)v); ph.y = __uint_as_float((uint32_t)(v >> 32));
     return v != 0xffffffffffffffffull;
+}
+
+// one counter slot += the warp's counts (COUNT builds)
+__device__ __forceinline__ void flush_counters(unsigned long long* dst, unsigned lane, unsigned long long rays, unsigned long long nodes,
+                                               unsigned long long tris, unsigned long long insts, unsigned long long hits) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        rays += __shfl_xor_sync(FULL, rays, o); nodes += __shfl_xor_sync(FULL, nodes, o);
+        tris += __shfl_xor_sync(FULL, tris, o); insts += __shfl_xor_sync(FULL, insts, o);
+        hits += __shfl_xor_sync(FULL, hits, o);
+    }
+    if (lane == 0) {
+        atomicAdd(dst + 0, rays); atomicAdd(dst + 1, nodes); atomicAdd(dst + 2, tris);
+        atomicAdd(dst + 3, insts); atomicAdd(dst + 4, hits);
+    }
 }
 
 // ---- the traversal kernel ---------------------------------------------------------------------------
@@ -597,7 +640,7 @@ __device__ __forceinline__ bool poll_hit(const tray_hit* src, float2& ph) {     
 // The hand-shake needs neither counters nor fences: the host fills the primary-hit buffer with 0xFFFFFFFF'FFFFFFFF before the
 // launch, no hit record looks like that (its t would be a NaN), and a lane publishes its record with ONE aligned 8-byte store;
 // a reader that sees something else than the fill pattern sees the whole record.  A warp with nothing else in hand polls with
-// __nanosleep and a watchdog (the device is never hung: after ~2 s it raises the overflow flag and leaves).
+// __nanosleep and a watchdog (the device is never hung: after ~2 s it sets ERR_WATCHDOG in the error word and leaves).
 // Per ray nothing changes: same node order, same triangle order, same (prim, t).
 // MODE 1: the three semantics of the reference's CPU path that are sourced from memory of the un-vendored obvhs crate (tie
 // rule, slab-test lower clamp, reach of the zero-direction patch) and the HLSL's divide-form box test become RUN-TIME switches
@@ -637,17 +680,24 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     bool exhausted = false;                      // warp-uniform
     unsigned long long c_rays = 0, c_nodes = 0, c_tris = 0, c_insts = 0, c_hits = 0;
     unsigned long long b_rays = 0, b_nodes = 0, b_tris = 0, b_insts = 0, b_hits = 0;    // FRAME && COUNT: the bounce rays' share
-    // FRAME: bit 31 of ray_idx marks a bounce ray; bit 30 (WIDE_BIT) a ray that must take the unfused node test (RayConst::wide) —
-    // the host keeps batches and frames below 2^30 rays per launch, so the index itself fits in 30 bits
-#define TRAY_CNT(name) do { if (COUNT) { if (FRAME && (ray_idx >> 31)) b_##name++; else c_##name++; } } while (0)
+    // ray_idx: INDEX_MASK bits of index, BOUNCE_BIT, WIDE_BIT
+#define TRAY_CNT(name) do { if (COUNT) { if (FRAME && (ray_idx & BOUNCE_BIT)) b_##name++; else c_##name++; } } while (0)
     uint32_t cur_unit = INVALID, cand_unit = INVALID, H = 0, sleeps = 0;   // FRAME, warp-uniform: 32-pixel group being fed from, claimed group, its pixels still to shoot
     bool units_done = false;
 
     auto push = [&](uint32_t x, uint32_t y) {
         if (sp < SP_SMEM_END) stk_store(sp, x, y);
         else if (sp < SP_END) spill[sp / SP_STEP - STACK_SMEM] = make_uint2(x, y);
-        else { atomicOr(P.overflow, 1u); return; }
+        else { atomicOr(P.overflow, ERR_STACK_OVERFLOW); return; }
         sp += SP_STEP;
+    };
+    // the lane takes up the ray ray_idx holds, at the root group (query.hlsl:343)
+    auto start_ray = [&](float ox, float oy, float oz, float dx, float dy, float dz, float tmin, float tmax, uint32_t variant) {
+        prepare_ray(r, ox, oy, oz, dx, dy, dz, tmin, variant, (uint32_t)__cvta_generic_to_shared(s_lut));
+        if (r.wide) ray_idx |= WIDE_BIT;
+        best_t = tmax; best_prim = INVALID;
+        cur_x = 0; cur_y = 0x80000000u; tri_x = 0; tri_y = 0; sp &= SP_STEP - 1u;
+        tlas_sp = INVALID; bvh_off = TLAS ? P.tlas_start : 0u;
     };
     // called when the lane has neither triangles nor nodes left in hand: pop the stack, or retire the ray
     // (query.hlsl:417-427; tlas:480-486; the popped-triangle-group case is query.hlsl:389-393)
@@ -657,32 +707,21 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
             h.t = best_prim != INVALID ? best_t : __int_as_float(0x7f800000);   // RayHit::none()
             h.prim = best_prim;
             if (FRAME) {
-                const uint32_t it = ray_idx & 0x3fffffffu;
+                const uint32_t it = ray_idx & INDEX_MASK;
                 if (COUNT && best_prim != INVALID) TRAY_CNT(hits);
-                if (!(ray_idx >> 31))      // ONE 64-bit scalar store (single-copy atomic, unlike a .v2 pair): the record itself tells a reader that it is there
+                if (!(ray_idx & BOUNCE_BIT))      // ONE 64-bit scalar store (single-copy atomic, unlike a .v2 pair): the record itself tells a reader that it is there
                     publish_hit(P.hits_out + it, h);
                 else {
                     P.bounce_out[it] = h;
-                    if (P.rgba_out) {
-                        const float col = h.t < F32_MAX_ ? __fdiv_rn(h.t, add(1.0f, h.t)) : 1.0f;    // rt_cpu.rs:82-87
-                        const long long o = rgba_slot(it, P.frame_w, P.frame_h, P.frame_tiles_x, P.frame_shard, P.frame_shards);
-                        if (o >= 0) P.rgba_out[o] = shade(col);
-                    }
+                    store_rgba(P.rgba_out, P.frame, P.row_major, it, SHADE_BOUNCE, h.t);
                 }
                 cur_x = 0; cur_y = 0;
                 return;
             }
-            const uint32_t ri = ray_idx & 0x3fffffffu;
+            const uint32_t ri = ray_idx & INDEX_MASK;
             const uint32_t item = P.ray_item ? __ldg(P.ray_item + ri) : ri;
             P.hits_out[item] = h;
-            if (P.rgba_out) {
-                float col;
-                if (P.shade_mode == SHADE_PRIMARY) col = __fdiv_rn(1.0f, h.t);                       // rt_cpu.rs:59
-                else if (P.shade_mode == SHADE_OCCLUSION) col = h.t < F32_MAX_ ? 0.0f : 1.0f;        // any-hit AO: visibility only
-                else col = h.t < F32_MAX_ ? __fdiv_rn(h.t, add(1.0f, h.t)) : 1.0f;                   // rt_cpu.rs:82-87
-                const long long o = rgba_slot(item, P.frame_w, P.frame_h, P.frame_tiles_x, P.frame_shard, P.frame_shards);
-                if (o >= 0) P.rgba_out[o] = shade(col);
-            }
+            store_rgba(P.rgba_out, P.frame, P.row_major, item, P.shade_mode, h.t);
             if (COUNT && best_prim != INVALID) c_hits++;
             cur_x = 0; cur_y = 0;                                                                    // IDLE
         } else {
@@ -723,11 +762,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     if (base < n_work && ray_idx < n_work) {
                         const float4* rp = reinterpret_cast<const float4*>(P.rays + ray_idx);
                         const float4 a = __ldg(rp), b = __ldg(rp + 1);
-                        prepare_ray(r, a.x, a.y, a.z, b.x, b.y, b.z, a.w, MODE == 1 ? P.variant : 0u, (uint32_t)__cvta_generic_to_shared(s_lut));
-                        if (r.wide) ray_idx |= WIDE_BIT;
-                        best_t = b.w; best_prim = INVALID;
-                        cur_x = 0; cur_y = 0x80000000u; tri_x = 0; tri_y = 0; sp &= SP_STEP - 1u;   // root group, query.hlsl:343
-                        tlas_sp = INVALID; bvh_off = TLAS ? P.tlas_start : 0u;
+                        start_ray(a.x, a.y, a.z, b.x, b.y, b.z, a.w, b.w, MODE == 1 ? P.variant : 0u);
                         if (COUNT) c_rays++;
                     }
                 }
@@ -748,12 +783,8 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                             const uint32_t item = cur_unit * 32u + pix;
                             const float4* gp = reinterpret_cast<const float4*>(P.gen_rays + item);     // written by this warp at the claim
                             const float4 ga = __ldcg(gp), gb = __ldcg(gp + 1);
-                            const float ox = ga.x, oy = ga.y, oz = ga.z, dx = gb.x, dy = gb.y, dz = gb.z;
-                            prepare_ray(r, ox, oy, oz, dx, dy, dz, 0.0f, 0u, (uint32_t)__cvta_generic_to_shared(s_lut));   // Ray::new(o, dir, 0.0, f32::MAX)
-                            best_t = F32_MAX_; best_prim = INVALID;
-                            cur_x = 0; cur_y = 0x80000000u; tri_x = 0; tri_y = 0; sp &= SP_STEP - 1u;
-                            tlas_sp = INVALID; bvh_off = TLAS ? P.tlas_start : 0u;
-                            ray_idx = item | 0x80000000u | (r.wide ? WIDE_BIT : 0u);
+                            ray_idx = item | BOUNCE_BIT;
+                            start_ray(ga.x, ga.y, ga.z, gb.x, gb.y, gb.z, 0.0f, F32_MAX_, 0u);   // Ray::new(o, dir, 0.0, f32::MAX)
                             if (COUNT) b_rays++;
                         }
                         int n_take = min(__popc(idle), __popc(H));
@@ -781,28 +812,14 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                             uint32_t px, py;
                             const bool inside = item_to_pixel(P.frame, item, px, py);
                             const bool shoot = inside && ph.x < F32_MAX_;                     // rt_cpu.rs:61
-                            if (!shoot) {
-                                tray_hit miss; miss.t = __int_as_float(0x7f800000); miss.prim = INVALID;
-                                P.bounce_out[item] = miss;
-                                if (P.rgba_out) {
-                                    const long long o = rgba_slot(item, P.frame_w, P.frame_h, P.frame_tiles_x, P.frame_shard, P.frame_shards);
-                                    if (o >= 0) P.rgba_out[o] = shade(__fdiv_rn(1.0f, ph.x));
-                                }
-                                if (P.rays_by_item) {
-                                    float4* o2 = reinterpret_cast<float4*>(P.rays_by_item + item);
-                                    o2[0] = make_float4(0.f, 0.f, 0.f, 0.f); o2[1] = make_float4(0.f, 0.f, 0.f, 0.f);
-                                }
-                            }
+                            if (!shoot) finish_no_bounce(P.frame, P.row_major, item, ph.x, P.bounce_out, P.rgba_out, P.rays_by_item);
                             else {
                                 const float4 pb = __ldg(reinterpret_cast<const float4*>(P.rays + item) + 1);   // the primary direction as generated
                                 float ox, oy, oz, dx, dy, dz;
                                 bounce_ray<TRI_STRIDE>(P.frame, P.tris, px, py, pb.x, pb.y, pb.z, ph.x, __float_as_uint(ph.y), ox, oy, oz, dx, dy, dz);
-                                float4* go = reinterpret_cast<float4*>(P.gen_rays + item);
-                                go[0] = make_float4(ox, oy, oz, 0.0f); go[1] = make_float4(dx, dy, dz, F32_MAX_);
-                                if (P.rays_by_item) {
-                                    float4* o2 = reinterpret_cast<float4*>(P.rays_by_item + item);
-                                    o2[0] = make_float4(ox, oy, oz, 0.0f); o2[1] = make_float4(dx, dy, dz, F32_MAX_);
-                                }
+                                const float4 a = make_float4(ox, oy, oz, 0.0f), b = make_float4(dx, dy, dz, F32_MAX_);
+                                store_ray(P.gen_rays + item, a, b);
+                                keep_ray(P.rays_by_item, item, a, b);
                             }
                             __syncwarp();                      // the group's rays are read back by other lanes of this warp
                             H = __ballot_sync(FULL, shoot);
@@ -810,7 +827,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                         }
                         if (busy == 0u) {                     // nothing else in hand: wait for the tile's last primary rays
                             __nanosleep(500);
-                            if (++sleeps > 4000000u) { atomicOr(P.overflow, 4u); break; }       // watchdog: never hang the device
+                            if (++sleeps > 4000000u) { atomicOr(P.overflow, ERR_WATCHDOG); break; }       // watchdog: never hang the device
                             continue;
                         }
                     } else if (busy == 0u) break;             // no group left, nothing in flight
@@ -920,28 +937,8 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     }
 #endif
     if (COUNT) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            c_rays += __shfl_xor_sync(FULL, c_rays, o); c_nodes += __shfl_xor_sync(FULL, c_nodes, o);
-            c_tris += __shfl_xor_sync(FULL, c_tris, o); c_insts += __shfl_xor_sync(FULL, c_insts, o);
-            c_hits += __shfl_xor_sync(FULL, c_hits, o);
-        }
-        if (lane == 0) {
-            atomicAdd(P.counters + 0, c_rays); atomicAdd(P.counters + 1, c_nodes); atomicAdd(P.counters + 2, c_tris);
-            atomicAdd(P.counters + 3, c_insts); atomicAdd(P.counters + 4, c_hits);
-        }
-        if (FRAME) {          // the bounce rays' counters live in the next counter slot
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                b_rays += __shfl_xor_sync(FULL, b_rays, o); b_nodes += __shfl_xor_sync(FULL, b_nodes, o);
-                b_tris += __shfl_xor_sync(FULL, b_tris, o); b_insts += __shfl_xor_sync(FULL, b_insts, o);
-                b_hits += __shfl_xor_sync(FULL, b_hits, o);
-            }
-            if (lane == 0) {
-                atomicAdd(P.counters + 5, b_rays); atomicAdd(P.counters + 6, b_nodes); atomicAdd(P.counters + 7, b_tris);
-                atomicAdd(P.counters + 8, b_insts); atomicAdd(P.counters + 9, b_hits);
-            }
-        }
+        flush_counters(P.counters, lane, c_rays, c_nodes, c_tris, c_insts, c_hits);
+        if (FRAME) flush_counters(P.counters + N_COUNTERS, lane, b_rays, b_nodes, b_tris, b_insts, b_hits);   // the bounce rays' slot
     }
 #undef TRAY_CNT
 }

@@ -49,7 +49,7 @@ int env_int(const char* name, int dflt) {
 // the kernels of frame k+1 fill the SM slots the drain phase of frame k leaves empty.
 struct FrameSlot {
     cudaStream_t own_stream = nullptr;       // slot 1 only
-    unsigned long long* d_cursor = nullptr;  // [0] cursor (u32), [1..10] 2 x 5 counters, [11] bounce-ray count (u32)
+    unsigned long long* d_cursor = nullptr;  // cursor block (tray::CURSOR_WORDS)
     uint32_t* d_units = nullptr;             // FRAME kernel: cursor over the 32-item groups of bounce work
     cudaEvent_t ev[4] = { nullptr, nullptr, nullptr, nullptr };
     cudaEvent_t done = nullptr;              // recorded behind the frame's last launch (fences, group completion)
@@ -77,7 +77,7 @@ struct tray_scene {
     uint32_t* d_blas = nullptr;
     uint32_t* d_prim_indices = nullptr;      // BVH slot -> input triangle (scenes made by tray_cuda_scene_build)
     uint32_t* d_geom_offsets = nullptr; uint32_t n_geometries = 0;   // first global triangle of BLAS / object g (tray_cuda_scene_set_geometry_offsets)
-    unsigned long long* d_cursor = nullptr;     // [0] cursor (u32), [1..10] 2 x 5 counters, [11] bounce-ray count (u32)
+    unsigned long long* d_cursor = nullptr;     // cursor block of batch traces (tray::CURSOR_WORDS)
     // device error words (TraceParams::overflow): [0] batch traces, [1 + k] the launches of frame slot k — one word per slot, so
     // that a frame's error is reported for that frame and cleared in the order of that slot's stream
     uint32_t* d_overflow = nullptr;
@@ -168,7 +168,7 @@ void base_params(const tray_scene* s, TraceParams& P) {
 }
 
 // one launch: reset the cursor, run the persistent grid (sized to the chip, or to the work if that is smaller)
-// `cur` = the cursor block the launch works on: [0] cursor, [1..10] counters ([1 + 5 * counter_slot ..])
+// `cur` = the cursor block the launch works on; its counters go to slot `counter_slot` (and the next, for the frame kernel)
 int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* cur, int counter_slot, bool anyhit = false, bool keep_counters = false, bool frame = false) {
     if (s->variant && (anyhit || frame || s->counting))
         return fail(TRAY_ERR_ARG, "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only");
@@ -182,9 +182,9 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
         if (cap > 0 && cap < bps) bps = cap;
     }
     P.cursor = (uint32_t*)cur;
-    P.counters = cur + 1 + 5 * counter_slot;
+    P.counters = cur + CURSOR_COUNTERS + N_COUNTERS * counter_slot;
     CU(cudaMemsetAsync(cur, 0, sizeof(unsigned long long), st));
-    if (s->counting && !keep_counters) CU(cudaMemsetAsync(P.counters, 0, (frame ? 10 : 5) * sizeof(unsigned long long), st));
+    if (s->counting && !keep_counters) CU(cudaMemsetAsync(P.counters, 0, (frame ? 2 : 1) * N_COUNTERS * sizeof(unsigned long long), st));
     const uint64_t blocks_needed = ((uint64_t)P.n_work + BLOCK_THREADS - 1) / BLOCK_THREADS;
     uint64_t grid = (uint64_t)s->sm_count * bps;
     if (blocks_needed < grid) grid = blocks_needed;
@@ -265,17 +265,17 @@ void frame_params(FrameParams& F, const tray_view* view, uint32_t w, uint32_t h,
 }
 
 int read_counters(const unsigned long long* cur, cudaStream_t st, int slot, tray_counters* out) {
-    unsigned long long c[5];
-    CU(cudaMemcpyAsync(c, cur + 1 + 5 * slot, sizeof c, cudaMemcpyDeviceToHost, st));
+    unsigned long long c[N_COUNTERS];
+    CU(cudaMemcpyAsync(c, cur + CURSOR_COUNTERS + N_COUNTERS * slot, sizeof c, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     out->rays = c[0]; out->nodes = c[1]; out->tris = c[2]; out->instances = c[3]; out->hits = c[4];
     return TRAY_OK;
 }
 
-// a device error word as a status (4: the frame kernel's watchdog, other bits: stack overflow)
+// a device error word as a status
 int flag_status(uint32_t f) {
     if (!f) return TRAY_OK;
-    if (f & 4u) return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
+    if (f & ERR_WATCHDOG) return fail(TRAY_ERR_CUDA, "frame kernel watchdog: a group of primary hits never arrived (the frame is incomplete)");
     return fail(TRAY_ERR_OVERFLOW, "traversal stack overflow: BVH needs more than %d stack entries", STACK_SMEM + STACK_SPILL);
 }
 // the error word `flag` behind the work enqueued on `st`, as a status; a set word is cleared there, in stream order, so that an
@@ -494,16 +494,16 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
             CU(cudaMalloc(&s->d_tris, tb));
         }
         if (!s->d_blas) CU(cudaMalloc(&s->d_blas, (size_t)(n_instances ? n_instances : 1) * 4));
-        CU(cudaMalloc(&s->d_cursor, 16 * sizeof(unsigned long long)));
+        CU(cudaMalloc(&s->d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
         CU(cudaMalloc(&s->d_overflow, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t)));
-        CU(cudaMemsetAsync(s->d_cursor, 0, 16 * sizeof(unsigned long long), s->stream));
+        CU(cudaMemsetAsync(s->d_cursor, 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
         for (int k = 0; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) {
             FrameSlot& f = s->slot[k];
             if (k >= 1) CU(cudaStreamCreateWithFlags(&f.own_stream, cudaStreamNonBlocking));
-            CU(cudaMalloc(&f.d_cursor, 16 * sizeof(unsigned long long)));
+            CU(cudaMalloc(&f.d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
             CU(cudaMalloc(&f.d_units, sizeof(uint32_t)));
             f.d_flag = s->d_overflow + 1 + k;
-            CU(cudaMemsetAsync(f.d_cursor, 0, 16 * sizeof(unsigned long long), s->stream));
+            CU(cudaMemsetAsync(f.d_cursor, 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
             for (auto& e : f.ev) CU(cudaEventCreate(&e));
             CU(cudaEventCreateWithFlags(&f.done, cudaEventDisableTiming));
         }
@@ -744,7 +744,7 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (ms_kernel) CU(cudaEventRecord(s->ev[0], st));
-    const uint64_t chunk = 1ull << 30;                    // ray indices are 32-bit inside the kernel
+    const uint64_t chunk = INDEX_MASK + 1ull;             // inside the kernel a ray index keeps two tag bits above INDEX_MASK
     for (uint64_t off = 0; off < n; off += chunk) {
         TraceParams P; base_params(s, P);
         P.rays = d_rays + off; P.n_work = (uint32_t)(n - off < chunk ? n - off : chunk); P.hits_out = d_hits + off;
@@ -815,7 +815,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         if (chunk_env >= 4096 && (uint64_t)chunk_env <= PIPE_CHUNK) chunk = (uint64_t)chunk_env;
         const uint64_t n_chunks = (n + chunk - 1) / chunk;
         auto chunk_len = [&](uint64_t i) { return i + 1 < n_chunks ? chunk : n - i * chunk; };
-        if (s->counting) CU(cudaMemsetAsync(s->d_cursor + 1, 0, 5 * sizeof(unsigned long long), s->stream));
+        if (s->counting) CU(cudaMemsetAsync(s->d_cursor + CURSOR_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), s->stream));
         CU(cudaEventRecord(s->ev[0], s->stream));
         for (uint64_t i = 0; i < n_chunks + 2; i++) {
             const int slot = (int)(i & 1);
@@ -968,7 +968,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     if (!s || !view) return fail(TRAY_ERR_ARG, "NULL argument");
     if (shards == 0) shards = 1;
     if (w == 0 || h == 0 || shard >= shards) return fail(TRAY_ERR_ARG, "bad frame size / shard (%ux%u, %u of %u)", w, h, shard, shards);
-    if ((uint64_t)((w + 31) / 32) * ((h + 7) / 8) * 256ull >= 0x40000000ull) return fail(TRAY_ERR_ARG, "frame too large");
+    if ((uint64_t)((w + 31) / 32) * ((h + 7) / 8) * 256ull > INDEX_MASK) return fail(TRAY_ERR_ARG, "frame too large");
     CU(cudaSetDevice(s->device));
     const bool want_count = (flags & TRAY_RENDER_COUNTERS) != 0;
     if (want_count != s->counting) tray_cuda_set_counting(s, want_count);
@@ -1003,7 +1003,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     f.last_frame = F;
     if (F.n_items == 0) { if (ms_primary) *ms_primary = 0.f; if (ms_bounce) *ms_bounce = 0.f; return TRAY_OK; }
     const unsigned gen_grid = (F.n_items + 255) / 256;
-    uint32_t* d_nbrays = (uint32_t*)(f.d_cursor + 11);
+    uint32_t* d_nbrays = (uint32_t*)(f.d_cursor + CURSOR_N_BOUNCE);
     const bool timed = ms_primary || ms_bounce;
 
     // ---- primary: generate rays, trace ----
@@ -1012,22 +1012,18 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     CU(cudaGetLastError());
     TraceParams P; base_params(s, P);
     P.rays = f.d_prays; P.n_work = F.n_items; P.hits_out = f.d_primary; P.overflow = f.d_flag;
+    P.frame = F; P.row_major = s->frame_target ? 1u : 0u;
     uchar4* const rgba_dst = s->frame_target ? s->frame_target : f.d_rgba;
-    auto set_frame = [&](TraceParams& T) {
-        if (!s->frame_target) return;
-        T.frame_w = w; T.frame_h = h; T.frame_tiles_x = F.tiles_x; T.frame_shard = shard; T.frame_shards = shards;
-    };
     P.rgba_out = (rgba && !bounce) ? rgba_dst : nullptr; P.shade_mode = SHADE_PRIMARY;
     if (overlap) {
         // one launch for the whole frame (trace_kernel<FRAME>): the bounce rays of finished tiles fill the primary pass's drain
         CU(cudaMemsetAsync(f.d_units, 0, sizeof(uint32_t), st));
         CU(cudaMemsetAsync(f.d_primary, 0xff, (size_t)F.n_items * sizeof(tray_hit), st));     // "not there yet" for every primary hit
         P.rgba_out = rgba ? rgba_dst : nullptr;
-        P.frame = F; P.bounce_out = f.d_bounce; P.rays_by_item = keep_rays ? f.d_brays_item : nullptr; P.gen_min = s->gen_min;
+        P.bounce_out = f.d_bounce; P.rays_by_item = keep_rays ? f.d_brays_item : nullptr; P.gen_min = s->gen_min;
         P.gen_rays = f.d_brays;
         P.unit_cursor = f.d_units; P.n_units = (uint32_t)(F.n_items / 32);
     }
-    if (P.rgba_out) set_frame(P);
     int rc = launch(s, P, st, f.d_cursor, 0, false, false, overlap);
     if (rc) return rc;
     if (timed) CU(cudaEventRecord(f.ev[1], st));
@@ -1038,14 +1034,13 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         CU(cudaMemsetAsync(d_nbrays, 0, sizeof(uint32_t), st));
         auto gen = s->tri_stride == 64 ? tray::raygen_bounce_kernel<64> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24> : tray::raygen_bounce_kernel<48>;
         gen<<<(F.n_items + BOUNCE_BLOCK - 1) / BOUNCE_BLOCK, BOUNCE_BLOCK, 0, st>>>(F, s->d_tris, f.d_primary, f.d_brays, f.d_bitem, d_nbrays, f.d_bounce,
-                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, s->frame_target ? 1u : 0u,
+                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major,
                                              s->bounce_sort);
         CU(cudaGetLastError());
         TraceParams B; base_params(s, B);
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
-        B.overflow = f.d_flag;
+        B.overflow = f.d_flag; B.frame = F; B.row_major = P.row_major;
         B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
-        if (B.rgba_out) set_frame(B);
         rc = launch(s, B, st, f.d_cursor, 1, any_ao);
         if (rc) return rc;
         if (timed) CU(cudaEventRecord(f.ev[2], st));
