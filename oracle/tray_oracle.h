@@ -124,6 +124,47 @@ void orc_sincos_tau(float u, float* s, float* c);
 /* node box test alone (for known-answer tests): returns the 32-bit hit mask */
 uint32_t orc_node_intersect(const uint8_t* node80, const orc_ray* ray, float tmax);
 
+/* ---- build_ref.c: serial reference of the device builder (tray_build::build_tlas in build_gpu.cu) ----------------------
+ * Morton sort -> PLOC -> reinsertion -> 8-wide collapse -> encode, single-threaded, byte for byte what the device builds.
+ * The device reads the knobs from the environment (TRAY_CUDA_BUILD_REINSERT, _VISITS, _ROUNDS); here they are parameters.
+ * Triangle records are not written: they depend only on prim_indices. */
+typedef struct orc_build_params {
+    uint32_t max_leaf;       /* 1 .. 3 */
+    uint32_t radius;         /* PLOC search radius 1 .. 64; 0 means 14 */
+    uint32_t passes;         /* reinsertion passes (device default 4) */
+    uint32_t visits;         /* node visits per move search (192) */
+    uint32_t rounds;         /* lock / apply rounds per pass (3) */
+} orc_build_params;
+
+typedef struct orc_build_stats {
+    uint64_t n_nodes;
+    uint32_t ploc_iterations, levels;         /* two-level builds: forest + TLAS */
+    uint32_t reinsert_passes, reinsert_moves; /* the flat / forest run alone; all 0 when it ran no reinsertion */
+    double sah_before, sah_after;             /* sum of the inner nodes' half-areas before / after the reinsertion */
+} orc_build_stats;
+
+typedef struct orc_bvh2_node {                /* 40 B; leaf: left = -1, right = primitive index */
+    float lo[3], hi[3];
+    int32_t left, right;
+    uint32_t count;
+    int32_t parent;                           /* -1 at a root */
+} orc_bvh2_node;
+
+typedef struct orc_build_result {
+    uint8_t* nodes; uint64_t n_nodes;         /* 80-byte CwBvhNode records: BLAS forest | TLAS */
+    uint32_t* prim_indices; uint64_t n_prims; /* BVH slot -> input triangle */
+    uint32_t* blas_offsets; uint32_t n_instances, tlas_start;   /* two-level builds, TLAS-leaf order */
+    int force_exact;                          /* some node exponent byte >= 167 */
+    orc_build_stats stats;
+    orc_bvh2_node* bvh2; uint32_t n_bvh2, n_bvh2_leaves;        /* final BVH2 of the flat / forest run */
+} orc_build_result;
+
+/* object_offsets == NULL: one flat BVH; otherwise n_objects + 1 offsets, one BLAS per object plus a TLAS.
+ * Returns 0, -1 on bad arguments, -2 out of memory, -3 when the build fails as the device build would (a stalled PLOC). */
+int orc_build_ref(const float* tris9, uint64_t n_tris, const uint64_t* object_offsets, uint32_t n_objects,
+                  const orc_build_params* params, orc_build_result* out);
+void orc_build_free(orc_build_result* r);
+
 #ifdef __cplusplus
 }
 #endif

@@ -45,6 +45,26 @@ class OrcTotals(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class OrcBuildParams(C.Structure):
+    _fields_ = [(n, C.c_uint32) for n in ("max_leaf", "radius", "passes", "visits", "rounds")]
+
+
+class OrcBuildStats(C.Structure):
+    _fields_ = [("n_nodes", C.c_uint64), ("ploc_iterations", C.c_uint32), ("levels", C.c_uint32),
+                ("reinsert_passes", C.c_uint32), ("reinsert_moves", C.c_uint32), ("sah_before", C.c_double), ("sah_after", C.c_double)]
+
+
+class OrcBuildResult(C.Structure):
+    _fields_ = [("nodes", C.c_void_p), ("n_nodes", C.c_uint64), ("prim_indices", C.c_void_p), ("n_prims", C.c_uint64),
+                ("blas_offsets", C.c_void_p), ("n_instances", C.c_uint32), ("tlas_start", C.c_uint32), ("force_exact", C.c_int),
+                ("stats", OrcBuildStats), ("bvh2", C.c_void_p), ("n_bvh2", C.c_uint32), ("n_bvh2_leaves", C.c_uint32)]
+
+
+# orc_bvh2_node: leaf left = -1, right = primitive; parent = -1 at a root
+BVH2_DTYPE = np.dtype([("lo", "<f4", 3), ("hi", "<f4", 3), ("left", "<i4"), ("right", "<i4"), ("count", "<u4"), ("parent", "<i4")])
+assert BVH2_DTYPE.itemsize == 40
+
+
 _lib = None
 
 
@@ -89,6 +109,9 @@ def lib() -> C.CDLL:
         L.orc_sincos_tau.argtypes = [C.c_float, C.POINTER(C.c_float), C.POINTER(C.c_float)]
         L.orc_node_intersect.restype = u32
         L.orc_node_intersect.argtypes = [vp, vp, C.c_float]
+        L.orc_build_ref.restype = i32
+        L.orc_build_ref.argtypes = [vp, u64, vp, u32, C.POINTER(OrcBuildParams), C.POINTER(OrcBuildResult)]
+        L.orc_build_free.argtypes = [C.POINTER(OrcBuildResult)]
         _lib = L
     return _lib
 
@@ -180,6 +203,48 @@ class Oracle:
         if rc != 0:
             raise RuntimeError(f"oracle traversal stack overflow ({rc})")
         return dict(primary=primary, bounce=bounce, bounce_rays=brays, rgba=img, primary_totals=pt.as_dict(), bounce_totals=bt.as_dict())
+
+
+def _copy(ptr, count, dtype):
+    if not count or not ptr:
+        return np.zeros(0, dtype=dtype)
+    n = count * np.dtype(dtype).itemsize
+    return np.frombuffer((C.c_uint8 * n).from_address(ptr), dtype=dtype).copy()
+
+
+def build_reference(tris, tri_stride=48, max_leaf=3, radius=14, object_offsets=None, passes=4, visits=192, rounds=3, bvh2=False):
+    """The serial reference of the device builder (oracle/build_ref.c), shaped like what a device-built TrayCudaScene reports:
+    nodes / tri_bytes / prim_indices as download_bvh(), blas_offsets as download_instances(), `info` with the fields of
+    info() it determines, `build_stats` with the fields of build_stats it determines, force_exact, and with bvh2=True the
+    final BVH2 of the flat / forest run (BVH2_DTYPE, leaves first).  radius 0 means 14, as in the C ABI."""
+    from tray_racing_b200 import host
+    t = np.ascontiguousarray(tris, dtype=np.float32).reshape(-1, 9)
+    prm = OrcBuildParams(max_leaf, radius, passes, visits, rounds)
+    res = OrcBuildResult()
+    if object_offsets is None:
+        rc = lib().orc_build_ref(t.ctypes.data, t.shape[0], None, 0, C.byref(prm), C.byref(res))
+    else:
+        off = np.ascontiguousarray(object_offsets, dtype=np.uint64)
+        rc = lib().orc_build_ref(t.ctypes.data, t.shape[0], off.ctypes.data, off.size - 1, C.byref(prm), C.byref(res))
+    if rc != 0:
+        raise RuntimeError(f"reference build failed ({rc})")
+    try:
+        nodes = _copy(res.nodes, res.n_nodes * 80, np.uint8)
+        pi = _copy(res.prim_indices, res.n_prims, np.uint32)
+        blas = _copy(res.blas_offsets, res.n_instances, np.uint32)
+        tree = _copy(res.bvh2, res.n_bvh2, BVH2_DTYPE) if bvh2 else None
+        st = res.stats
+        out = dict(
+            nodes=nodes, tri_bytes=host.tri_records(t.reshape(-1, 3, 3)[pi], tri_stride), prim_indices=pi, blas_offsets=blas,
+            info=dict(n_nodes=res.n_nodes, n_tris=t.shape[0], tri_stride=tri_stride, n_instances=res.n_instances,
+                      tlas_start=res.tlas_start, is_tlas=int(object_offsets is not None)),
+            build_stats=dict(n_tris=t.shape[0], n_nodes=st.n_nodes, ploc_iterations=st.ploc_iterations, levels=st.levels,
+                             reinsert_passes=st.reinsert_passes, reinsert_moves=st.reinsert_moves,
+                             sah_before=st.sah_before, sah_after=st.sah_after),
+            force_exact=bool(res.force_exact), bvh2=tree, bvh2_leaves=res.n_bvh2_leaves)
+    finally:
+        lib().orc_build_free(C.byref(res))
+    return out
 
 
 def primary_rays(view, w, h, nthreads=0):

@@ -47,6 +47,12 @@ namespace {
 constexpr int TPB = 256;
 inline unsigned blocks(uint64_t n) { return (unsigned)((n + TPB - 1) / TPB); }
 
+// ---- sign of zero ----------------------------------------------------------------------------------------------
+// fminf / fmaxf (min.f32 / max.f32) order -0.0 below +0.0 whatever the argument order, and so do the ordered-int atomics of
+// the scene bounds: every box corner that is zero is -0.0 when some primitive below it has -0.0 there (minimum) and +0.0 when
+// some has +0.0 (maximum).  A node's p is therefore its primitives' minimum bit for bit.  oracle/build_ref.c states the same
+// rule, and the host producer (host/cwbvh_build.cpp) follows it.
+
 // ---- ordered-int float atomics ------------------------------------------------------------------------------
 __device__ __forceinline__ int f2o(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
 __device__ __forceinline__ float o2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }

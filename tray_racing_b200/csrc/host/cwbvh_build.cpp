@@ -25,16 +25,21 @@
 
 namespace {
 
+// min / max that order -0.0 below +0.0 whichever argument comes first, as the device builder's fminf / fmaxf do: a node's
+// p is the minimum of its primitives bit for bit, sign of zero included (std::min keeps its first argument on a tie)
+inline float min_z(float a, float b) { return (b < a || (b == a && std::signbit(b))) ? b : a; }
+inline float max_z(float a, float b) { return (b > a || (b == a && !std::signbit(b))) ? b : a; }
+
 struct Box {
     float mn[3], mx[3];
     void reset() {
         for (int a = 0; a < 3; a++) { mn[a] = std::numeric_limits<float>::max(); mx[a] = -std::numeric_limits<float>::max(); }
     }
     void grow(const Box& o) {
-        for (int a = 0; a < 3; a++) { mn[a] = std::min(mn[a], o.mn[a]); mx[a] = std::max(mx[a], o.mx[a]); }
+        for (int a = 0; a < 3; a++) { mn[a] = min_z(mn[a], o.mn[a]); mx[a] = max_z(mx[a], o.mx[a]); }
     }
     void grow(const float p[3]) {
-        for (int a = 0; a < 3; a++) { mn[a] = std::min(mn[a], p[a]); mx[a] = std::max(mx[a], p[a]); }
+        for (int a = 0; a < 3; a++) { mn[a] = min_z(mn[a], p[a]); mx[a] = max_z(mx[a], p[a]); }
     }
     float half_area() const {
         float dx = mx[0] - mn[0], dy = mx[1] - mn[1], dz = mx[2] - mn[2];
@@ -317,8 +322,8 @@ int tray_host_build_cwbvh_from_tris(const float* tris9, uint64_t n, uint32_t max
     for (uint64_t i = 0; i < n; i++) {
         const float* t = tris9 + 9 * i;
         for (int a = 0; a < 3; a++) {
-            mn[3 * i + a] = std::min(t[a], std::min(t[3 + a], t[6 + a]));
-            mx[3 * i + a] = std::max(t[a], std::max(t[3 + a], t[6 + a]));
+            mn[3 * i + a] = min_z(t[a], min_z(t[3 + a], t[6 + a]));
+            mx[3 * i + a] = max_z(t[a], max_z(t[3 + a], t[6 + a]));
         }
     }
     return tray_host_build_cwbvh_from_aabbs(mn.data(), mx.data(), n, max_prims_per_leaf, nthreads, out);
