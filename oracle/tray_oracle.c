@@ -242,6 +242,11 @@ static inline float tri_intersect(const uint8_t* rec, uint32_t stride, const pre
     float v = dot3(rr, e1) * inv_det;                                  /* :101 */
     float w = 1.0f - u - v;                                            /* :102 */
     uint32_t hit = as_uint(u) | as_uint(v) | as_uint(w);               /* :112 (-0.0 rejects) */
+    /* :116 tests the sign bit.  On x86 an invalid operation (inf - inf, 0 * inf: dot(r, e2) or dot(r, e1) overflowing with
+     * opposite signs) gives the default NaN 0xFFC00000, whose sign bit is set, so the CPU path rejects a NaN u, v or w.  Other
+     * hosts' default NaN has the sign clear (aarch64: 0x7FC00000), so the rejection is written out: same answer everywhere.
+     * (A NaN already in a record or ray is not a case the reference defines; it is rejected here as well.) */
+    if (isnan(u) || isnan(v) || isnan(w)) return INFINITY;
     if (inv_det != 0.0f && (hit & 0x80000000u) == 0) {                 /* :116 */
         float t = dot3(ng, c) * inv_det;                               /* :118 */
         if (t >= r->tmin && t <= tmax) return t;                       /* :119 (tmin = ray.tmin on the CPU path) */
@@ -565,6 +570,16 @@ void orc_bounce_ray(const orc_scene* s, const orc_view* vw, const orc_ray* pr, c
     out->d[0] = d[0]; out->d[1] = d[1]; out->d[2] = d[2]; out->tmax = F32_MAX;
 }
 
+/* the grey level of a result of kind `mode` (ORC_SHADE_*), gamma-encoded and truncated as rt_cpu.rs:104-106 */
+uint8_t orc_shade(uint32_t mode, float t) {
+    float col;
+    if (mode == ORC_SHADE_PRIMARY) col = 1.0f / t;                      /* rt_cpu.rs:59 (1/inf = 0) */
+    else if (mode == ORC_SHADE_OCCLUSION) col = t < F32_MAX ? 0.0f : 1.0f;   /* any-hit AO: visibility only */
+    else col = t < F32_MAX ? t / (1.0f + t) : 1.0f;                      /* rt_cpu.rs:82-87 */
+    float g = powf(col, 2.2f) * 255.0f;
+    return (uint8_t)(g < 0.0f ? 0.0f : (g > 255.0f ? 255.0f : g));
+}
+
 /* ---- one frame of rt_cpu::start (src/rt_cpu/rt_cpu.rs:35-91, 102-107) ------------------------ */
 int orc_render(const orc_scene* s, const orc_view* vw, uint32_t w, uint32_t h, uint32_t frame_count,
                uint32_t flags, orc_hit* primary, orc_hit* bounce, orc_ray* bounce_rays, uint8_t* rgba,
@@ -582,7 +597,7 @@ int orc_render(const orc_scene* s, const orc_view* vw, uint32_t w, uint32_t h, u
         if (e < rc) rc = e;
         pn += c.nodes; pt += c.tris; pi += c.insts; ph += hit.prim != ORC_INVALID_PRIM;
         if (primary) primary[i] = hit;
-        float col = 1.0f / hit.t;                                       /* rt_cpu.rs:59 */
+        uint32_t shade_mode = ORC_SHADE_PRIMARY; float shade_t = hit.t;  /* rt_cpu.rs:59 */
         orc_hit ao; ao.t = INFINITY; ao.prim = ORC_INVALID_PRIM;
         orc_ray aoray; memset(&aoray, 0, sizeof(aoray));
         if ((flags & ORC_RENDER_BOUNCE) && hit.t < F32_MAX) {
@@ -590,13 +605,12 @@ int orc_render(const orc_scene* s, const orc_view* vw, uint32_t w, uint32_t h, u
             e = trace_one(s, &aoray, &ao, &c, NULL);
             if (e < rc) rc = e;
             br++; bn += c.nodes; bt += c.tris; bi += c.insts; bh += ao.prim != ORC_INVALID_PRIM;
-            col = (ao.t < F32_MAX) ? ao.t / (1.0f + ao.t) : 1.0f;       /* rt_cpu.rs:82-87 */
+            shade_mode = ORC_SHADE_BOUNCE; shade_t = ao.t;              /* rt_cpu.rs:82-87 */
         }
         if (bounce) bounce[i] = ao;
         if (bounce_rays) bounce_rays[i] = aoray;
-        if (rgba && (flags & ORC_RENDER_RGBA)) {                        /* rt_cpu.rs:104-106 */
-            float g = powf(col, 2.2f) * 255.0f;
-            uint8_t v8 = (uint8_t)(g < 0.0f ? 0.0f : (g > 255.0f ? 255.0f : g));
+        if (rgba && (flags & ORC_RENDER_RGBA)) {
+            const uint8_t v8 = orc_shade(shade_mode, shade_t);
             rgba[4 * i + 0] = v8; rgba[4 * i + 1] = v8; rgba[4 * i + 2] = v8; rgba[4 * i + 3] = 255;
         }
     }

@@ -116,6 +116,13 @@ int orc_render(const orc_scene* s, const orc_view* v, uint32_t w, uint32_t h, ui
                uint32_t flags, orc_hit* primary, orc_hit* bounce, orc_ray* bounce_rays, uint8_t* rgba,
                orc_totals* primary_totals, orc_totals* bounce_totals, int nthreads);
 
+/* shading (src/rt_cpu/rt_cpu.rs:59, 82-88, 104-106): the grey level orc_render writes for a result of kind `mode` —
+ * PRIMARY: 1/t; BOUNCE: t/(1+t), 1 for a miss; OCCLUSION: 0 for a hit, 1 for a miss (the kernels' ShadeMode numbering) */
+#define ORC_SHADE_PRIMARY   1u
+#define ORC_SHADE_BOUNCE    2u
+#define ORC_SHADE_OCCLUSION 3u
+uint8_t orc_shade(uint32_t mode, float t);
+
 /* sampling utilities (src/rt_gpu/sampling.hlsl:5-51) */
 uint32_t orc_uhash(uint32_t a, uint32_t b);
 float orc_hash_noise(uint32_t x, uint32_t y, uint32_t frame);

@@ -286,6 +286,40 @@ def test_huge_scene_scale_falls_back_to_unfused_test():
     assert_hits_identical(got, ref)
 
 
+@pytest.mark.parametrize("e", [62, 64])
+def test_scene_scale_where_barycentrics_overflow_to_nan(e):
+    """Large triangles at 2^62 and 2^64 units: dot(r, e2) or dot(r, e1) can overflow with opposite signs, so u or v is NaN
+    while t stays finite (here +-0, origins in a triangle's plane).  The reference's x86 CPU path rejects a NaN barycentric
+    (its default NaN has the sign bit set); CUDA's canonical NaN has it clear, so a sign-bit test alone reported hits at
+    t = +-0 there.  Closest hit, any hit and the f16 records, against the oracle."""
+    rng = np.random.default_rng(e)
+    tris = (rng.integers(-8, 9, size=(3000, 3, 3)) / 4).astype(np.float32)
+    n = 300000
+    org = (rng.integers(-4, 5, size=(n, 3)) / 2).astype(np.float32)
+    pick = rng.integers(0, len(tris), n)
+    b = rng.random((n, 2))
+    b[b.sum(1) > 1] = 1 - b[b.sum(1) > 1]
+    tgt = tris[pick, 0] + b[:, :1] * (tris[pick, 1] - tris[pick, 0]) + b[:, 1:] * (tris[pick, 2] - tris[pick, 0])
+    d = tgt - org
+    ok = np.linalg.norm(d, axis=1) > 0
+    rays = np.zeros(int(ok.sum()), dtype=ob.RAY_DTYPE)
+    rays["d"] = (d[ok] / np.linalg.norm(d[ok], axis=1, keepdims=True)).astype(np.float32)
+    s = np.float32(2.0 ** e)
+    rays["o"] = org[ok] * s
+    rays["tmax"] = F32_MAX
+    tris = tris * s
+    nodes, pidx, _ = host.build_cwbvh(tris)
+    for stride in (48, 24):
+        rec = host.tri_records(tris[pidx], stride)
+        orc = ob.Oracle(nodes, rec, stride)
+        sc = cuda.TrayCudaScene(nodes, rec, stride)
+        try:
+            for any_hit in (False, True):
+                assert_hits_identical(sc.traverse(rays, any_hit=any_hit), orc.trace(rays, any_hit=any_hit), f"stride {stride} any_hit {any_hit}")
+        finally:
+            sc.close()
+
+
 def test_degenerate_scenes():
     """One triangle (root with a single leaf child), coincident triangles (tie rule), empty scene."""
     one = np.array([[0, 0, 0, 1, 0, 0, 0, 1, 0]], dtype=np.float32)

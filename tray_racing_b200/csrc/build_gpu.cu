@@ -593,7 +593,7 @@ __global__ void collapse_emit_kernel(const int* __restrict__ items, uint32_t n_i
         w[a] = __float_as_uint(nmn[a]);
         const int ke = quant_exponent(nmx[a] - nmn[a]);
         nb[12 + a] = (uint8_t)(ke + 127);
-        if (ke + 127 >= 167) atomicOr(flags, 1u);          // scale >= 2^40: the traversal must use its unfused node test
+        if (ke + 127 >= 167) atomicOr(flags, 1u);          // scale >= 2^40: the traversal must use its unfused node test (tray::EXACT_EXP_BYTE)
         scale[a] = ldexp(1.0, ke);
     }
     w[4] = next_base + inner_off[i] - my_root;              // child_base_idx

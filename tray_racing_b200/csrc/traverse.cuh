@@ -58,6 +58,13 @@ constexpr uint32_t CURSOR_COUNTERS = 1, N_COUNTERS = 5, CURSOR_N_BOUNCE = 11, CU
 constexpr float F32_MAX_ = 3.402823466e+38f;
 constexpr float F32_EPS_ = 1.1920929e-7f;     // sampling.hlsl:3
 constexpr float BOX_EPS_ = 0.0001f;           // query.hlsl:274
+// The fused node test needs 2^23 * scale * |1/d| finite, i.e. below 2^105 on the x axis.  Rays with |1/d| >= 2^64 on some axis
+// (RayConst::wide) and scenes with an exponent byte >= EXACT_EXP_BYTE (scale >= 2^40) take the unfused test: together the two
+// guards keep 2^23 * A below 2^23 * 2^39 * 2^64 = 2^126, two bits short of the overflow.
+constexpr uint32_t EXACT_EXP_BYTE = 167;
+__host__ __device__ __forceinline__ bool node_needs_exact(uint32_t exp_bytes3) {    // the three exponent bytes of a node (byte 12..14)
+    return (exp_bytes3 & 0xffu) >= EXACT_EXP_BYTE || ((exp_bytes3 >> 8) & 0xffu) >= EXACT_EXP_BYTE || ((exp_bytes3 >> 16) & 0xffu) >= EXACT_EXP_BYTE;
+}
 
 struct FrameParams {
     tray_view view;
@@ -364,7 +371,12 @@ __device__ __forceinline__ float tri_test(const RayConst& r, float tmax, const u
     const float w = sub(sub(1.0f, u), v);                                          // :102
     const uint32_t hit = __float_as_uint(u) | __float_as_uint(v) | __float_as_uint(w);   // :112
     float t = __int_as_float(0x7f800000);
-    if (inv_det != 0.0f && (hit & 0x80000000u) == 0u) {                            // :116
+    // :116 tests the sign bit.  An accepted triangle has u, v, w in [+0, 1], whose bits are all below 0x40000000 (2.0f), and u or
+    // v > 1 forces w < 0, so `hit < 0x40000000` accepts exactly what the sign test accepts on non-NaN values — and also rejects a
+    // NaN in any position, as the reference's x86 CPU path does (its invalid operations give the default NaN 0xFFC00000, sign
+    // set; CUDA's canonical NaN 0x7FFFFFFF has the sign clear).  u or v is NaN when dot(r, e2) or dot(r, e1) overflows with
+    // opposite signs, and tt can still be finite then.
+    if (inv_det != 0.0f && hit < 0x40000000u) {
         const float tt = mul(dot3(ngx, ngy, ngz, cx, cy, cz), inv_det);            // :118
         if (tt >= r.tmin && tt <= tmax) t = tt;                                    // :119
     }

@@ -460,7 +460,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     s->force_exact = env_int("TRAY_CUDA_FORCE_EXACT", 0) != 0 || (built && built->force_exact);
     for (uint64_t i = 0; !built && i < n_nodes && !s->force_exact; i++) {
         const uint8_t* e = (const uint8_t*)nodes + i * 80 + 12;
-        if (e[0] >= 167 || e[1] >= 167 || e[2] >= 167) s->force_exact = true;   // scale = 2^(e-127) >= 2^40
+        if (tray::node_needs_exact(e[0] | (uint32_t)e[1] << 8 | (uint32_t)e[2] << 16)) s->force_exact = true;   // scale = 2^(e-127) >= 2^40
     }
     s->tri_weight = (uint32_t)env_int("TRAY_CUDA_TRI_WEIGHT", 3);     // 3: +0.6 ... 1.2 % over 4 with two triangles per step (profiles/experiments/r2_triweight_ab.log)
     s->gen_min = (uint32_t)env_int("TRAY_CUDA_GEN_MIN", 4);
