@@ -391,8 +391,8 @@ int tray_cuda_scene_set_stream(tray_scene* scene, void* stream);
 /* Wait for everything enqueued on the scene stream. */
 int tray_cuda_sync(tray_scene* scene);
 
-/* Counters of the last tray_cuda_render / tray_cuda_trace call made with counting enabled
- * (TRAY_RENDER_COUNTERS, or tray_cuda_set_counting).                                             */
+/* Counters of the last tray_cuda_render / tray_cuda_trace call, or timed (ms_kernel != NULL) tray_cuda_trace_device /
+ * tray_cuda_trace_any_device call, made with counting enabled (TRAY_RENDER_COUNTERS, or tray_cuda_set_counting).         */
 int tray_cuda_counters(tray_scene* scene, tray_counters* primary, tray_counters* bounce);
 int tray_cuda_set_counting(tray_scene* scene, int enabled);
 

@@ -10,12 +10,11 @@ that holds it is popped from a known depth and not merely fetched and culled.
 Reference: the CPU oracle with a 48-entry stack (Oracle.trace(stack_limit=48)); Oracle.stack_need shows which depths each
 batch really reaches.  The CPU tests check the encoder, that need against the independent HLSL transliteration, and the
 oracle's capacity; the GPU tests check the kernels bit for bit against it and pin how an overflow is reported."""
-import math
-
 import numpy as np
 import pytest
 
 import oracle_binding as ob
+from cwbvh_bytes import Scene, encode_node
 from tray_racing_b200 import cuda, host
 
 R = 0.93
@@ -25,41 +24,6 @@ FLAT_DEPTHS = (12, 13, 32, 33, 48)              # needs D - 1 at the edges of sh
 FRAME_FLAGS = cuda.RENDER_BOUNCE | cuda.RENDER_RGBA | cuda.RENDER_KEEP_RAYS | cuda.RENDER_COUNTERS
 DIAGONAL_CAMERA = host.Camera((-1.2,) * 3, (0, 0, 0), 10.0)          # pixels span needs 0 .. D - 1
 SIDE_CAMERA = host.Camera((-1.2, -1.0, -1.3), (0.3, 0.5, 0.4), 20.0)  # shallow levels only: needs <= 13
-
-
-# ---- a CWBVH encoder, written the way host/cwbvh_build.cpp's Collapser writes nodes ----------------------------------------
-def quant_exponent(extent):
-    extent = max(extent, 1e-20)
-    k = math.ceil(math.log2(extent / 255.0))
-    while math.ldexp(255.0, k) < extent:
-        k += 1
-    while math.ldexp(255.0, k - 1) >= extent:
-        k -= 1
-    return k
-
-
-def encode_node(lo, hi, children, child_base=0, prim_base=0):
-    """One 80-byte CwBvhNode over the cube [lo, hi]^3.  children: (slot, child_lo, child_hi, kind), kind "inner" or the
-    triangle count of a leaf; inner children are the nodes child_base, child_base + 1, .. in slot order."""
-    n = np.zeros(80, np.uint8)
-    lo, hi = np.float32(lo), np.float32(hi)
-    n[0:12] = np.full(3, lo, np.float32).view(np.uint8)                       # p = box min
-    k = quant_exponent(float(hi) - float(lo))
-    n[12:15] = k + 127
-    scale = math.ldexp(1.0, k)
-    n[16:24] = np.array([child_base, prim_base], np.uint32).view(np.uint8)
-    tri_offset = 0
-    for slot, clo, chi, kind in children:
-        for a in range(3):
-            n[32 + 16 * a + slot] = min(255, max(0, math.floor((float(np.float32(clo)) - float(lo)) / scale)))
-            n[40 + 16 * a + slot] = min(255, max(0, math.ceil((float(np.float32(chi)) - float(lo)) / scale)))
-        if kind == "inner":
-            n[15] |= 1 << slot
-            n[24 + slot] = 0x20 | (24 + slot)
-        else:
-            n[24 + slot] = (0x20, 0x60, 0xE0)[kind - 1] | tri_offset
-            tri_offset += kind
-    return n
 
 
 def ladder_nodes(D, r=R, prim_base=0):
@@ -81,20 +45,6 @@ def ladder_tris(D, r=R):
     t = [[s[i], s[i + 1], s[i + 1], s[i + 1], s[i], s[i + 1], s[i + 1], s[i + 1], s[i]] for i in range(D - 1)]
     t.append([s[-1], 0, 0, 0, s[-1], 0, 0, 0, s[-1]])
     return np.array(t, np.float32)
-
-
-class Scene:
-    """nodes + triangle soup (+ blas_offsets, tlas_start of a two-level scene), as the oracle and the CUDA scene take them"""
-
-    def __init__(self, nodes, tris, blas=None, tlas_start=0, stride=48):
-        self.nodes, self.tris, self.blas, self.tlas_start, self.stride = nodes, tris, blas, tlas_start, stride
-        self.rec = host.tri_records(tris, stride)
-
-    def oracle(self):
-        return ob.Oracle(self.nodes, self.rec, self.stride, self.blas, self.tlas_start, self.blas is not None)
-
-    def cuda(self):
-        return cuda.TrayCudaScene(self.nodes, self.rec, self.stride, self.blas, self.tlas_start)
 
 
 def flat_ladder(D, stride=48):

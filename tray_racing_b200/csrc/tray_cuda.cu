@@ -272,6 +272,12 @@ int read_counters(const unsigned long long* cur, cudaStream_t st, int slot, tray
     return TRAY_OK;
 }
 
+// An empty scene is uploaded as one zeroed placeholder root (scene_create_impl), which every ray fetches and misses.  It is not
+// a node of the scene: its visits are not counted, as the reference visits no node there.
+void drop_placeholder_root(tray_scene* s) {
+    if (s->n_nodes == 0) { s->cnt_primary.nodes = 0; s->cnt_bounce.nodes = 0; }
+}
+
 // a device error word as a status
 int flag_status(uint32_t f) {
     if (!f) return TRAY_OK;
@@ -755,6 +761,11 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
         CU(cudaEventRecord(s->ev[1], st));
         CU(cudaEventSynchronize(s->ev[1]));
         CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+        if (s->counting) {                                // synchronised: the batch's counters, summed over its launches
+            const int rc = read_counters(s->d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
+            memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
+            drop_placeholder_root(s);
+        }
         return check_overflow(s->d_overflow, st);         // synchronised: an overflow of this batch is reported by this call
     }
     return TRAY_OK;
@@ -848,7 +859,11 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         CU(cudaStreamSynchronize(s->stream));
         CU(cudaEventElapsedTime(&k, s->ev[0], s->ev[1]));       // span of the GPU work, uploads it waited for included
     }
-    if (s->counting) { rc = read_counters(s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc; memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce); }
+    if (s->counting) {
+        rc = read_counters(s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc;
+        memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
+        drop_placeholder_root(s);
+    }
     rc = check_overflow(s->d_overflow, s->stream);
     if (rc) return rc;
     if (ms_kernel) *ms_kernel = k;
@@ -1061,6 +1076,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         // rays generated for pixels outside the frame (tmax = 0) are not rays of the workload
         const uint64_t pad = (uint64_t)F.n_items - tray_cuda_shard_pixels(w, h, shard, shards);
         s->cnt_primary.rays -= pad; s->cnt_primary.nodes -= pad;
+        drop_placeholder_root(s);
     }
     return TRAY_OK;
 }
