@@ -391,8 +391,10 @@ int tray_cuda_scene_set_stream(tray_scene* scene, void* stream);
 /* Wait for everything enqueued on the scene stream. */
 int tray_cuda_sync(tray_scene* scene);
 
-/* Counters of the last tray_cuda_render / tray_cuda_trace call, or timed (ms_kernel != NULL) tray_cuda_trace_device /
- * tray_cuda_trace_any_device call, made with counting enabled (TRAY_RENDER_COUNTERS, or tray_cuda_set_counting).         */
+/* Counters of the last call that counted: a tray_cuda_render with TRAY_RENDER_COUNTERS, or — while tray_cuda_set_counting
+ * is on — a tray_cuda_trace / tray_cuda_trace_any call or a timed (ms_kernel != NULL) tray_cuda_trace_device /
+ * tray_cuda_trace_any_device call.  The flag counts the render that carries it and nothing else; tray_cuda_set_counting
+ * governs batch traces alone.  Neither changes the other.                                                               */
 int tray_cuda_counters(tray_scene* scene, tray_counters* primary, tray_counters* bounce);
 int tray_cuda_set_counting(tray_scene* scene, int enabled);
 

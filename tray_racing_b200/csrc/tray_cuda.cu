@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <utility>
 #include <vector>
 
 #include "build_gpu.h"
@@ -87,11 +88,11 @@ struct tray_scene {
     bool have_window = false;                // persisting-L2 access-policy window over the node array, applied per launch
     cudaAccessPolicyWindow window{};
     uint64_t device_bytes = 0, l2_bytes = 0, l2_persist = 0;
-    bool counting = false;
+    bool counting = false;                   // tray_cuda_set_counting: batch traces count (a render counts with TRAY_RENDER_COUNTERS alone)
     uint32_t variant = 0;                    // TRAY_VARIANT_* (tray_cuda_scene_set_variant): the MODE 1 kernels
     uint32_t refill_min = 6, tri_weight = 3, gen_min = 4;
     bool overlap_default = false;            // TRAY_CUDA_OVERLAP=1: tray_cuda_render always takes the one-launch frame kernel
-    int blocks_per_sm[2] = { 0, 0 };         // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1]
+    int blocks_per_sm[3] = { 0, 0, 0 };      // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1], the counting lane kernel [2]
     // ray-batch staging
     tray_ray* d_rays = nullptr; tray_hit* d_hits = nullptr; uint64_t batch_cap = 0;
     // host <-> device pipeline of tray_cuda_trace: two pinned staging slots per direction, copy streams, events
@@ -167,13 +168,15 @@ void base_params(const tray_scene* s, TraceParams& P) {
     P.variant = s->variant; P.one = 1u;
 }
 
+const char* const VARIANT_REFUSAL = "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only";
+
 // one launch: reset the cursor, run the persistent grid (sized to the chip, or to the work if that is smaller)
-// `cur` = the cursor block the launch works on; its counters go to slot `counter_slot` (and the next, for the frame kernel)
-int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* cur, int counter_slot, bool anyhit = false, bool keep_counters = false, bool frame = false) {
-    if (s->variant && (anyhit || frame || s->counting))
-        return fail(TRAY_ERR_ARG, "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only");
-    kernel_fn k = pick_kernel(s->tlas, s->counting, s->tri_stride, anyhit, frame, s->variant != 0);
-    int& bps = s->blocks_per_sm[s->variant ? 1 : 0];
+// `cur` = the cursor block the launch works on; its counters go to slot `counter_slot` (and the next, for the frame kernel).
+// `count`: the counting kernels (tray_scene::counting for batch traces, TRAY_RENDER_COUNTERS for the launches of one frame)
+int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* cur, int counter_slot, bool count, bool anyhit = false, bool keep_counters = false, bool frame = false) {
+    if (s->variant && (anyhit || frame || count)) return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);
+    kernel_fn k = pick_kernel(s->tlas, count, s->tri_stride, anyhit, frame, s->variant != 0);
+    int& bps = s->blocks_per_sm[s->variant ? 1 : count ? 2 : 0];
     if (bps == 0) {
         int nb = 0;
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, BLOCK_THREADS, 0));
@@ -184,7 +187,7 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
     P.cursor = (uint32_t*)cur;
     P.counters = cur + CURSOR_COUNTERS + N_COUNTERS * counter_slot;
     CU(cudaMemsetAsync(cur, 0, sizeof(unsigned long long), st));
-    if (s->counting && !keep_counters) CU(cudaMemsetAsync(P.counters, 0, (frame ? 2 : 1) * N_COUNTERS * sizeof(unsigned long long), st));
+    if (count && !keep_counters) CU(cudaMemsetAsync(P.counters, 0, (frame ? 2 : 1) * N_COUNTERS * sizeof(unsigned long long), st));
     const uint64_t blocks_needed = ((uint64_t)P.n_work + BLOCK_THREADS - 1) / BLOCK_THREADS;
     uint64_t grid = (uint64_t)s->sm_count * bps;
     if (blocks_needed < grid) grid = blocks_needed;
@@ -625,7 +628,7 @@ int tray_cuda_scene_info(const tray_scene* s, tray_scene_info* o) {
 
 int tray_cuda_set_counting(tray_scene* s, int enabled) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
-    if (s->counting != (enabled != 0)) { s->counting = enabled != 0; s->blocks_per_sm[0] = 0; }
+    s->counting = enabled != 0;
     return TRAY_OK;
 }
 
@@ -754,7 +757,7 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
     for (uint64_t off = 0; off < n; off += chunk) {
         TraceParams P; base_params(s, P);
         P.rays = d_rays + off; P.n_work = (uint32_t)(n - off < chunk ? n - off : chunk); P.hits_out = d_hits + off;
-        int rc = launch(s, P, st, s->d_cursor, 0, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
+        int rc = launch(s, P, st, s->d_cursor, 0, s->counting, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
         if (rc) return rc;
     }
     if (ms_kernel) {
@@ -839,7 +842,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 CU(cudaStreamWaitEvent(s->stream, s->e_in[slot], 0));
                 TraceParams P; base_params(s, P);
                 P.rays = s->d_rays + off; P.n_work = (uint32_t)len; P.hits_out = s->d_hits + off;
-                rc = launch(s, P, s->stream, s->d_cursor, 0, anyhit, /*keep_counters=*/true);
+                rc = launch(s, P, s->stream, s->d_cursor, 0, s->counting, anyhit, /*keep_counters=*/true);
                 if (rc) return rc;
                 CU(cudaEventRecord(s->e_k[slot], s->stream));
             }
@@ -907,7 +910,23 @@ int tray_cuda_scene_set_frames_in_flight(tray_scene* s, uint32_t n) {
     if (!s || n < 1 || n > TRAY_MAX_FRAMES_IN_FLIGHT) return fail(TRAY_ERR_ARG, "frames in flight must be 1 .. %d", TRAY_MAX_FRAMES_IN_FLIGHT);
     CU(cudaSetDevice(s->device));
     if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
-    if ((int)n != s->n_slots) { s->n_slots = (int)n; s->cur = 0; }
+    if (s->cur >= (int)n) {
+        // The last frame's slot does not survive the switch: its frame moves to slot n - 1, and that slot's older frame moves
+        // out, so that "the last frame" is still the latest render; the next render takes slot 0.  Every stream is idle here, so
+        // buffers, cursors and events move freely.  The streams stay with their slots, and the error word follows the frame.
+        FrameSlot& a = s->slot[s->cur];
+        FrameSlot& b = s->slot[n - 1];
+        std::swap(a, b);
+        std::swap(a.own_stream, b.own_stream);
+        std::swap(a.d_flag, b.d_flag);
+        uint32_t wa = 0, wb = 0;
+        CU(cudaMemcpy(&wa, a.d_flag, 4, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(&wb, b.d_flag, 4, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(a.d_flag, &wb, 4, cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(b.d_flag, &wa, 4, cudaMemcpyHostToDevice));
+        s->cur = (int)n - 1;
+    }
+    s->n_slots = (int)n;
     return TRAY_OK;
 }
 
@@ -978,19 +997,16 @@ int tray_cuda_scene_after(tray_scene* s, void* stream) {
     return TRAY_OK;
 }
 
-int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, uint32_t frame_count, uint32_t flags,
-                     uint32_t shard, uint32_t shards, float* ms_primary, float* ms_bounce) {
-    if (!s || !view) return fail(TRAY_ERR_ARG, "NULL argument");
-    if (shards == 0) shards = 1;
-    if (w == 0 || h == 0 || shard >= shards) return fail(TRAY_ERR_ARG, "bad frame size / shard (%ux%u, %u of %u)", w, h, shard, shards);
-    if ((uint64_t)((w + 31) / 32) * ((h + 7) / 8) * 256ull > INDEX_MASK) return fail(TRAY_ERR_ARG, "frame too large");
-    CU(cudaSetDevice(s->device));
-    const bool want_count = (flags & TRAY_RENDER_COUNTERS) != 0;
-    if (want_count != s->counting) tray_cuda_set_counting(s, want_count);
-    s->cur = next_slot(s);
+}  // extern "C"
+
+namespace {
+// the frame of tray_cuda_render in slot s->cur, its arguments checked; it writes the slot's frame record before its launches
+int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, uint32_t frame_count, uint32_t flags,
+                uint32_t shard, uint32_t shards, float* ms_primary, float* ms_bounce) {
     FrameSlot& f = s->slot[s->cur];
     cudaStream_t st = slot_stream(s, s->cur);
     const uint64_t items_cap = local_items(w, h, 0, shards);   // every shard's buffers have the size of the largest (gather)
+    const bool want_count = (flags & TRAY_RENDER_COUNTERS) != 0;
     const bool bounce = (flags & TRAY_RENDER_BOUNCE) != 0, rgba = (flags & TRAY_RENDER_RGBA) != 0;
     const bool keep_rays = (flags & TRAY_RENDER_KEEP_RAYS) != 0;
     const bool any_ao = (flags & TRAY_RENDER_ANYHIT_AO) != 0;
@@ -1016,7 +1032,12 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
     f.f_has_bounce = bounce; f.f_has_rgba = rgba && !s->frame_target; f.f_has_rays = keep_rays && bounce;
     f.f_target = rgba ? s->frame_target : nullptr;
     f.last_frame = F;
-    if (F.n_items == 0) { if (ms_primary) *ms_primary = 0.f; if (ms_bounce) *ms_bounce = 0.f; return TRAY_OK; }
+    if (F.n_items == 0) {                        // a shard without tiles: no launch, and nothing to count
+        if (ms_primary) *ms_primary = 0.f;
+        if (ms_bounce) *ms_bounce = 0.f;
+        if (want_count) { memset(&s->cnt_primary, 0, sizeof s->cnt_primary); memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce); }
+        return TRAY_OK;
+    }
     const unsigned gen_grid = (F.n_items + 255) / 256;
     uint32_t* d_nbrays = (uint32_t*)(f.d_cursor + CURSOR_N_BOUNCE);
     const bool timed = ms_primary || ms_bounce;
@@ -1039,7 +1060,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         P.gen_rays = f.d_brays;
         P.unit_cursor = f.d_units; P.n_units = (uint32_t)(F.n_items / 32);
     }
-    int rc = launch(s, P, st, f.d_cursor, 0, false, false, overlap);
+    int rc = launch(s, P, st, f.d_cursor, 0, want_count, false, false, overlap);
     if (rc) return rc;
     if (timed) CU(cudaEventRecord(f.ev[1], st));
     if (overlap && timed) CU(cudaEventRecord(f.ev[2], st));
@@ -1056,7 +1077,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
         B.overflow = f.d_flag; B.frame = F; B.row_major = P.row_major;
         B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
-        rc = launch(s, B, st, f.d_cursor, 1, any_ao);
+        rc = launch(s, B, st, f.d_cursor, 1, want_count, any_ao);
         if (rc) return rc;
         if (timed) CU(cudaEventRecord(f.ev[2], st));
     }
@@ -1069,7 +1090,7 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         if (ms_bounce) *ms_bounce = b;
         rc = check_overflow(f.d_flag, st); if (rc) return rc;
     }
-    if (s->counting) {
+    if (want_count) {
         rc = read_counters(f.d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
         if (bounce) { rc = read_counters(f.d_cursor, st, 1, &s->cnt_bounce); if (rc) return rc; }
         else memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
@@ -1079,6 +1100,30 @@ int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t 
         drop_placeholder_root(s);
     }
     return TRAY_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int tray_cuda_render(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, uint32_t frame_count, uint32_t flags,
+                     uint32_t shard, uint32_t shards, float* ms_primary, float* ms_bounce) {
+    // every refusal comes before the first change of state: a refused render leaves the last frame, the slot the next render
+    // takes and the counting state of batch traces as they were
+    if (!s || !view) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (shards == 0) shards = 1;
+    if (w == 0 || h == 0 || shard >= shards) return fail(TRAY_ERR_ARG, "bad frame size / shard (%ux%u, %u of %u)", w, h, shard, shards);
+    if ((uint64_t)((w + 31) / 32) * ((h + 7) / 8) * 256ull > INDEX_MASK) return fail(TRAY_ERR_ARG, "frame too large");
+    // the launches' own check (launch()), made here: the primary launch counts with TRAY_RENDER_COUNTERS, the bounce launch is an
+    // any-hit launch with TRAY_RENDER_ANYHIT_AO (TRAY_RENDER_OVERLAP is ignored under a variant)
+    if (s->variant && ((flags & TRAY_RENDER_COUNTERS) || ((flags & TRAY_RENDER_BOUNCE) && (flags & TRAY_RENDER_ANYHIT_AO))))
+        return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);
+    CU(cudaSetDevice(s->device));
+    s->cur = next_slot(s);
+    const int rc = render_slot(s, view, w, h, frame_count, flags, shard, shards, ms_primary, ms_bounce);
+    // A frame that failed on its way is no frame: downloads of it fail rather than return what the slot held before.  A stack
+    // overflow is reported for a frame whose launches ran to the end.
+    if (rc != TRAY_OK && rc != TRAY_ERR_OVERFLOW) s->slot[s->cur].last_frame.width = 0;
+    return rc;
 }
 
 int tray_cuda_render_timed(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, uint32_t frame_count, uint32_t flags,
