@@ -124,6 +124,18 @@ typedef struct tray_counters {
     uint64_t hits;       /* rays that ended with a hit                        */
 } tray_counters;
 
+/* The cost of ONE ray, as the counting kernels see it (the reference's PROFILE_RT heat map colours each pixel by its own ray's
+ * counters, rt_gpu_software.hlsl:93-102).  nodes, tris and instances count exactly what tray_counters counts for that ray, so a
+ * batch's or a frame's records sum to the tray_counters of the same call with counting on; the rays of an empty scene report
+ * 0 nodes, as the totals do.  16 bytes, one aligned store per ray.                                                        */
+typedef struct tray_ray_cost {
+    uint32_t nodes;      /* CWBVH nodes fetched (the reference's aabb_hit_count / 8)                                  */
+    uint32_t tris;       /* triangle records tested (tri_hit_count)                                                   */
+    uint32_t instances;  /* TLAS leaf entries (blas_offsets lookups)                                                  */
+    uint32_t stack;      /* most traversal-stack entries the ray held at once: the peak of the kernel's stack pointer, at
+                          * most 48; a ray that needed more reports 48 and its call TRAY_ERR_OVERFLOW                    */
+} tray_ray_cost;         /* 16 bytes */
+
 typedef struct tray_scene_info {
     uint64_t n_nodes, n_tris;
     uint32_t tri_stride, n_instances, tlas_start, is_tlas;
@@ -397,6 +409,30 @@ int tray_cuda_sync(tray_scene* scene);
  * governs batch traces alone.  Neither changes the other.                                                               */
 int tray_cuda_counters(tray_scene* scene, tray_counters* primary, tray_counters* bounce);
 int tray_cuda_set_counting(tray_scene* scene, int enabled);
+
+/* ---- per-ray cost: which rays and pixels are expensive ------------------------------------------------------------------
+ * The counting kernels also keep each ray's tray_ray_cost.  Hits, bounce rays and RGBA are bit-identical with ray costs on or
+ * off; the kernels that do not count are not touched.  Under tray_cuda_scene_set_variant every call below that traces is
+ * refused (TRAY_ERR_ARG) before it changes any state, as counting is.
+ *
+ * tray_cuda_trace / tray_cuda_trace_any (any_hit != 0), and their _device forms, with one more output: costs[i] is the cost
+ * of rays[i].  They always run the counting kernels, and update tray_cuda_counters exactly when the plain calls would, that
+ * is, while tray_cuda_set_counting is on.  HOST buffers for tray_cuda_trace_cost, DEVICE buffers (and `stream`, ms_kernel as
+ * tray_cuda_trace_device) for tray_cuda_trace_cost_device, where d_costs must be 16-byte aligned.                          */
+int tray_cuda_trace_cost(tray_scene* scene, const tray_ray* rays, uint64_t n, int any_hit, tray_hit* hits,
+                         tray_ray_cost* costs, float* ms_kernel, float* ms_total);
+int tray_cuda_trace_cost_device(tray_scene* scene, const tray_ray* d_rays, uint64_t n, int any_hit, tray_hit* d_hits,
+                                tray_ray_cost* d_costs, void* stream, float* ms_kernel);
+/* While enabled (default: off), every tray_cuda_render with TRAY_RENDER_COUNTERS also keeps the cost of each of its rays, in
+ * buffers of the frame's slot that travel with the frame like its hits (frames in flight included).  A switch, not a render
+ * flag: the set of TRAY_RENDER_* flags stays as it is.                                                                     */
+int tray_cuda_scene_set_ray_cost(tray_scene* scene, int enabled);
+/* The last frame's costs to HOST buffers, width*height records each in row-major pixel order: `primary` the primary ray of
+ * each pixel, `bounce` its bounce ray.  Pixels of other shards, and bounce records of pixels that shot no bounce ray, are zero.
+ * Either pointer may be NULL.  TRAY_ERR_ARG if the last frame kept no costs (rendered without TRAY_RENDER_COUNTERS or with ray
+ * costs off), or bounce != NULL for a frame without TRAY_RENDER_BOUNCE.  Reports the frame's error status as
+ * tray_cuda_frame_download does.  Per device of a tray_group: download each shard from tray_cuda_group_scene(i).           */
+int tray_cuda_frame_download_cost(tray_scene* scene, tray_ray_cost* primary, tray_ray_cost* bounce);
 
 /* ---- the slot itself ------------------------------------------------------------------------- */
 

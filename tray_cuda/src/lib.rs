@@ -24,6 +24,11 @@ pub struct TrayView {
 #[derive(Clone, Copy, bytemuck::Pod, bytemuck::Zeroable)]
 pub struct TrayTri48 { pub v0: [f32; 3], pub p0: f32, pub e1: [f32; 3], pub p1: f32, pub e2: [f32; 3], pub p2: f32 }
 
+/// `tray_ray_cost` of include/tray_cuda.h: one ray's nodes fetched, triangles tested, TLAS leaf entries and peak stack entries
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug, bytemuck::Pod, bytemuck::Zeroable)]
+pub struct TrayRayCost { pub nodes: u32, pub tris: u32, pub instances: u32, pub stack: u32 }
+
 #[repr(C)] pub struct TrayScene { _private: [u8; 0] }
 #[repr(C)] pub struct TrayGroup { _private: [u8; 0] }
 
@@ -86,6 +91,12 @@ extern "C" {
     pub fn tray_cuda_sync(scene: *mut TrayScene) -> c_int;
     pub fn tray_cuda_counters(scene: *mut TrayScene, primary: *mut TrayCounters, bounce: *mut TrayCounters) -> c_int;
     pub fn tray_cuda_set_counting(scene: *mut TrayScene, enabled: c_int) -> c_int;
+    pub fn tray_cuda_trace_cost(scene: *mut TrayScene, rays: *const TrayRay, n: u64, any_hit: c_int, hits: *mut TrayHit,
+        costs: *mut TrayRayCost, ms_kernel: *mut f32, ms_total: *mut f32) -> c_int;
+    pub fn tray_cuda_trace_cost_device(scene: *mut TrayScene, d_rays: *const TrayRay, n: u64, any_hit: c_int, d_hits: *mut TrayHit,
+        d_costs: *mut TrayRayCost, stream: *mut c_void, ms_kernel: *mut f32) -> c_int;
+    pub fn tray_cuda_scene_set_ray_cost(scene: *mut TrayScene, enabled: c_int) -> c_int;
+    pub fn tray_cuda_frame_download_cost(scene: *mut TrayScene, primary: *mut TrayRayCost, bounce: *mut TrayRayCost) -> c_int;
     pub fn tray_cuda_bandwidth_probe(device: c_int, bytes: u64, iters: c_int, out_gbs: *mut f32) -> c_int;
     pub fn tray_cuda_l1_gather_probe(device: c_int, bytes: u32, iters: c_int, out_gbs: *mut f32) -> c_int;
     pub fn tray_cuda_device_count() -> c_int;

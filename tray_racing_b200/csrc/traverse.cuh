@@ -107,6 +107,10 @@ struct TraceParams {
     uint32_t* __restrict__ unit_cursor;       // next tile whose bounce rays have not been claimed (zeroed by the host)
     uint32_t n_units;                         // n_work / 32: bounce work is claimed in groups of 32 items
     uint32_t gen_min;                         // idle lanes needed before the warp generates bounce rays into them
+    // optional, COUNT builds: one cost record per ray at its output item (tray_cuda_trace_cost, tray_cuda_scene_set_ray_cost).
+    // FRAME kernel: the bounce records follow the n_work primary ones.  Last member: the offsets of every other member, and so
+    // the code of the kernels that do not count, stay as they were.
+    tray_ray_cost* __restrict__ ray_cost;
 };
 
 // ---- exact float helpers (no contraction, IEEE rounding) --------------------------------------
@@ -690,10 +694,15 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     uint32_t tlas_sp = INVALID, bvh_off = 0;
     uint32_t ray_idx = 0;
     bool exhausted = false;                      // warp-uniform
-    unsigned long long c_rays = 0, c_nodes = 0, c_tris = 0, c_insts = 0, c_hits = 0;
-    unsigned long long b_rays = 0, b_nodes = 0, b_tris = 0, b_insts = 0, b_hits = 0;    // FRAME && COUNT: the bounce rays' share
+    // a lane starts fewer than 2^30 rays per launch (INDEX_MASK), so its ray and hit counts fit 32 bits
+    uint32_t c_rays = 0, c_hits = 0, b_rays = 0, b_hits = 0;
+    unsigned long long c_nodes = 0, c_tris = 0, c_insts = 0;
+    unsigned long long b_nodes = 0, b_tris = 0, b_insts = 0;    // FRAME && COUNT: the bounce rays' share
+    // COUNT builds: the cost of the lane's ray so far, added to the warp totals above when it retires; r_peak is the highest
+    // stack pointer it reached (depth * SP_STEP + thread * 8, so r_peak / SP_STEP is its peak depth in entries)
+    uint32_t r_nodes = 0, r_tris = 0, r_insts = 0, r_peak = 0;
     // ray_idx: INDEX_MASK bits of index, BOUNCE_BIT, WIDE_BIT
-#define TRAY_CNT(name) do { if (COUNT) { if (FRAME && (ray_idx & BOUNCE_BIT)) b_##name++; else c_##name++; } } while (0)
+#define TRAY_CNT(name) do { if constexpr (COUNT) r_##name++; } while (0)
     uint32_t cur_unit = INVALID, cand_unit = INVALID, H = 0, sleeps = 0;   // FRAME, warp-uniform: 32-pixel group being fed from, claimed group, its pixels still to shoot
     bool units_done = false;
 
@@ -702,6 +711,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         else if (sp < SP_END) spill[sp / SP_STEP - STACK_SMEM] = make_uint2(x, y);
         else { atomicOr(P.overflow, ERR_STACK_OVERFLOW); return; }
         sp += SP_STEP;
+        if constexpr (COUNT) r_peak = max(r_peak, sp);
     };
     // the lane takes up the ray ray_idx holds, at the root group (query.hlsl:343)
     auto start_ray = [&](float ox, float oy, float oz, float dx, float dy, float dz, float tmin, float tmax, uint32_t variant) {
@@ -710,6 +720,17 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         best_t = tmax; best_prim = INVALID;
         cur_x = 0; cur_y = 0x80000000u; tri_x = 0; tri_y = 0; sp &= SP_STEP - 1u;
         tlas_sp = INVALID; bvh_off = TLAS ? P.tlas_start : 0u;
+        if constexpr (COUNT) { r_nodes = 0; r_tris = 0; r_insts = 0; r_peak = 0; }
+    };
+    // COUNT builds, a ray retires: its counts join the warp totals of its pass, and its record goes to slot `item` of P.ray_cost
+    // (`if constexpr` here and at every use of the r_* registers: the kernels that do not count compile to the code they had
+    // before these records existed)
+    auto retire_cost = [&](uint32_t item, bool hit) {
+        if constexpr (COUNT) {
+            if (FRAME && (ray_idx & BOUNCE_BIT)) { b_nodes += r_nodes; b_tris += r_tris; b_insts += r_insts; b_hits += hit; }
+            else { c_nodes += r_nodes; c_tris += r_tris; c_insts += r_insts; c_hits += hit; }
+            if (P.ray_cost) reinterpret_cast<uint4*>(P.ray_cost)[item] = make_uint4(r_nodes, r_tris, r_insts, r_peak / SP_STEP);
+        }
     };
     // called when the lane has neither triangles nor nodes left in hand: pop the stack, or retire the ray
     // (query.hlsl:417-427; tlas:480-486; the popped-triangle-group case is query.hlsl:389-393)
@@ -720,7 +741,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
             h.prim = best_prim;
             if (FRAME) {
                 const uint32_t it = ray_idx & INDEX_MASK;
-                if (COUNT && best_prim != INVALID) TRAY_CNT(hits);
+                if constexpr (COUNT) retire_cost((ray_idx & BOUNCE_BIT) ? P.n_work + it : it, best_prim != INVALID);
                 if (!(ray_idx & BOUNCE_BIT))      // ONE 64-bit scalar store (single-copy atomic, unlike a .v2 pair): the record itself tells a reader that it is there
                     publish_hit(P.hits_out + it, h);
                 else {
@@ -734,7 +755,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
             const uint32_t item = P.ray_item ? __ldg(P.ray_item + ri) : ri;
             P.hits_out[item] = h;
             store_rgba(P.rgba_out, P.frame, P.row_major, item, P.shade_mode, h.t);
-            if (COUNT && best_prim != INVALID) c_hits++;
+            if constexpr (COUNT) retire_cost(item, best_prim != INVALID);
             cur_x = 0; cur_y = 0;                                                                    // IDLE
         } else {
             if (TLAS && sp == tlas_sp) { tlas_sp = INVALID; bvh_off = P.tlas_start; }

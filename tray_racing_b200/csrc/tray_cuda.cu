@@ -18,6 +18,7 @@
 static_assert(sizeof(tray_cwbvh_node) == 80, "CwBvhNode is 80 bytes (bvh_embree_to_cwbvh.rs:91, rt_gpu/mod.rs:70)");
 static_assert(sizeof(tray_tri48) == 48 && sizeof(tray_tri64) == 64 && sizeof(tray_tri24) == 24, "triangle record strides");
 static_assert(sizeof(tray_ray) == 32 && sizeof(tray_hit) == 8, "ray / hit records");
+static_assert(sizeof(tray_ray_cost) == 16 && alignof(tray_ray_cost) == 4, "ray cost record: one 16-byte store per ray");
 static_assert(sizeof(tray_view) == 160, "ViewUniform is padded to 160 bytes (main.rs:589-597)");
 
 namespace {
@@ -62,6 +63,8 @@ struct FrameSlot {
     tray_ray* d_brays = nullptr;             // generated bounce rays, COMPACT (hit pixels only)
     uint32_t* d_bitem = nullptr;             // local item of compact bounce ray i
     tray_ray* d_brays_item = nullptr;        // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
+    tray_ray_cost* d_cost = nullptr;         // optional: ray costs by local item, 2 x f_cap: primary [0, n_items), bounce from n_items
+    bool f_has_cost = false;                 // the last frame kept ray costs (tray_cuda_scene_set_ray_cost + TRAY_RENDER_COUNTERS)
     uint32_t* d_flag = nullptr;              // the device error word of this slot's launches (a word of tray_scene::d_overflow)
     tray::FrameParams last_frame{};          // width 0: no frame rendered yet
 };
@@ -89,14 +92,17 @@ struct tray_scene {
     cudaAccessPolicyWindow window{};
     uint64_t device_bytes = 0, l2_bytes = 0, l2_persist = 0;
     bool counting = false;                   // tray_cuda_set_counting: batch traces count (a render counts with TRAY_RENDER_COUNTERS alone)
+    bool ray_cost = false;                   // tray_cuda_scene_set_ray_cost: counted renders keep every ray's cost
     uint32_t variant = 0;                    // TRAY_VARIANT_* (tray_cuda_scene_set_variant): the MODE 1 kernels
     uint32_t refill_min = 6, tri_weight = 3, gen_min = 4;
     bool overlap_default = false;            // TRAY_CUDA_OVERLAP=1: tray_cuda_render always takes the one-launch frame kernel
     int blocks_per_sm[3] = { 0, 0, 0 };      // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1], the counting lane kernel [2]
     // ray-batch staging
     tray_ray* d_rays = nullptr; tray_hit* d_hits = nullptr; uint64_t batch_cap = 0;
+    tray_ray_cost* d_costs = nullptr; uint64_t cost_cap = 0;   // tray_cuda_trace_cost: allocated on first use
     // host <-> device pipeline of tray_cuda_trace: two pinned staging slots per direction, copy streams, events
     tray_ray* h_rays[2] = { nullptr, nullptr }; tray_hit* h_hits[2] = { nullptr, nullptr };
+    tray_ray_cost* h_costs[2] = { nullptr, nullptr };          // pinned cost slots, allocated by the first pipelined cost call
     cudaStream_t s_in = nullptr, s_out = nullptr; bool pipeline_ready = false;
     cudaEvent_t e_in[2] = { nullptr, nullptr }, e_k[2] = { nullptr, nullptr }, e_out[2] = { nullptr, nullptr };
     // frame state: one FrameSlot per frame in flight (tray_cuda_scene_set_frames_in_flight); `cur` = the slot of the last frame
@@ -122,6 +128,8 @@ void free_pipeline(tray_scene* s) {
     for (int i = 0; i < 2; i++) {
         if (s->h_rays[i]) cudaFreeHost(s->h_rays[i]);
         if (s->h_hits[i]) cudaFreeHost(s->h_hits[i]);
+        if (s->h_costs[i]) cudaFreeHost(s->h_costs[i]);
+        s->h_costs[i] = nullptr;
         if (s->e_in[i]) cudaEventDestroy(s->e_in[i]);
         if (s->e_k[i]) cudaEventDestroy(s->e_k[i]);
         if (s->e_out[i]) cudaEventDestroy(s->e_out[i]);
@@ -241,9 +249,9 @@ int sync_streams(const tray_scene* s, bool scene_stream_first) {
 // the per-frame buffers of a slot (not its cursor block); the caller has synchronised the slot's stream
 void free_frame_buffers(FrameSlot& f) {
     cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
-    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item);
+    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item); cudaFree(f.d_cost);
     f.d_primary = nullptr; f.d_bounce = nullptr; f.d_brays = nullptr; f.d_rgba = nullptr;
-    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.f_cap = 0;
+    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.d_cost = nullptr; f.f_cap = 0;
 }
 
 int check_tri_stride(uint32_t tri_stride) {
@@ -279,6 +287,12 @@ int read_counters(const unsigned long long* cur, cudaStream_t st, int slot, tray
 // a node of the scene: its visits are not counted, as the reference visits no node there.
 void drop_placeholder_root(tray_scene* s) {
     if (s->n_nodes == 0) { s->cnt_primary.nodes = 0; s->cnt_bounce.nodes = 0; }
+}
+// The same for the cost records of n rays at d: a ray of an empty scene fetches the placeholder root and nothing else (no
+// triangle, no instance, no push), so its whole record is zero.
+int drop_placeholder_costs(const tray_scene* s, tray_ray_cost* d, uint64_t n, cudaStream_t st) {
+    if (s->n_nodes == 0 && d && n) CU(cudaMemsetAsync(d, 0, n * sizeof(tray_ray_cost), st));
+    return TRAY_OK;
 }
 
 // a device error word as a status
@@ -421,7 +435,7 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
     cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
-    cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_geom_offsets);
+    cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_costs); cudaFree(s->d_geom_offsets);
     free_pipeline(s);
     cudaFree(s->d_untiled);
     for (auto& f : s->slot) {
@@ -632,6 +646,12 @@ int tray_cuda_set_counting(tray_scene* s, int enabled) {
     return TRAY_OK;
 }
 
+int tray_cuda_scene_set_ray_cost(tray_scene* s, int enabled) {
+    if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
+    s->ray_cost = enabled != 0;
+    return TRAY_OK;
+}
+
 int tray_cuda_scene_set_variant(tray_scene* s, uint32_t flags) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     if (flags & ~0xfu) return fail(TRAY_ERR_ARG, "unknown variant flags 0x%x", flags);
@@ -748,7 +768,9 @@ int tray_cuda_sync(tray_scene* s) {
 }  // extern "C"
 
 namespace {
-int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits, void* stream, float* ms_kernel, bool anyhit) {
+// d_costs != NULL: the cost calls — the counting kernels whatever tray_scene::counting says, the counters read under it alone
+int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits, tray_ray_cost* d_costs, void* stream,
+                      float* ms_kernel, bool anyhit) {
     if (!s || (n && (!d_rays || !d_hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
@@ -757,9 +779,11 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
     for (uint64_t off = 0; off < n; off += chunk) {
         TraceParams P; base_params(s, P);
         P.rays = d_rays + off; P.n_work = (uint32_t)(n - off < chunk ? n - off : chunk); P.hits_out = d_hits + off;
-        int rc = launch(s, P, st, s->d_cursor, 0, s->counting, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
+        P.ray_cost = d_costs ? d_costs + off : nullptr;
+        int rc = launch(s, P, st, s->d_cursor, 0, s->counting || d_costs, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
         if (rc) return rc;
     }
+    if (const int rc = drop_placeholder_costs(s, d_costs, n, st)) return rc;
     if (ms_kernel) {
         CU(cudaEventRecord(s->ev[1], st));
         CU(cudaEventSynchronize(s->ev[1]));
@@ -801,7 +825,9 @@ int ensure_pipeline(tray_scene* s) {
 // over chunks of PIPE_CHUNK rays: [host threads: caller's rays -> pinned slot] [copy stream: H2D] [scene stream: traversal]
 // [copy stream: D2H into a pinned slot] [host threads: -> caller's hits]; chunk i+1 is staged and uploaded while chunk i is
 // traced and chunk i-1 is read back.  The caller's memory is only borrowed for the call and never registered.
-int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, float* ms_kernel, float* ms_total, bool anyhit) {
+// costs != NULL: the cost calls (see trace_device_impl); the records travel like the hits
+int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, tray_ray_cost* costs, float* ms_kernel, float* ms_total,
+               bool anyhit) {
     if (!s || (n && (!rays || !hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     const auto t0 = std::chrono::steady_clock::now();
@@ -811,17 +837,26 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         CU(cudaMalloc(&s->d_hits, n * sizeof(tray_hit)));
         s->batch_cap = n;
     }
+    if (costs && n > s->cost_cap) {
+        cudaFree(s->d_costs); s->d_costs = nullptr; s->cost_cap = 0;
+        CU(cudaMalloc(&s->d_costs, n * sizeof(tray_ray_cost)));
+        s->cost_cap = n;
+    }
+    tray_ray_cost* const d_costs = costs ? s->d_costs : nullptr;
     float k = 0.f;
     int rc = TRAY_OK;
     if (n < PIPE_MIN) {
         if (n) CU(cudaMemcpyAsync(s->d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, s->stream));
-        rc = trace_device_impl(s, s->d_rays, n, s->d_hits, s->stream, &k, anyhit);
+        rc = trace_device_impl(s, s->d_rays, n, s->d_hits, d_costs, s->stream, &k, anyhit);
         if (rc) return rc;
         if (n) CU(cudaMemcpyAsync(hits, s->d_hits, n * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->stream));
+        if (n && costs) CU(cudaMemcpyAsync(costs, d_costs, n * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->stream));
         CU(cudaStreamSynchronize(s->stream));
     } else {
         rc = ensure_pipeline(s);
         if (rc) return rc;
+        for (int i = 0; costs && i < 2; i++)
+            if (!s->h_costs[i]) CU(cudaMallocHost(&s->h_costs[i], PIPE_CHUNK * sizeof(tray_ray_cost)));
         // chunk size: the pipeline only pays once it has a few stages, and every stage is a kernel launch with its own
         // drain phase — 2^19 rays below 4 M rays, 2^20 above (TRAY_CUDA_PIPE_CHUNK overrides, <= 2^20)
         uint64_t chunk = n < (4ull << 20) ? (PIPE_CHUNK >> 1) : PIPE_CHUNK;
@@ -842,7 +877,10 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 CU(cudaStreamWaitEvent(s->stream, s->e_in[slot], 0));
                 TraceParams P; base_params(s, P);
                 P.rays = s->d_rays + off; P.n_work = (uint32_t)len; P.hits_out = s->d_hits + off;
-                rc = launch(s, P, s->stream, s->d_cursor, 0, s->counting, anyhit, /*keep_counters=*/true);
+                P.ray_cost = d_costs ? d_costs + off : nullptr;
+                rc = launch(s, P, s->stream, s->d_cursor, 0, s->counting || costs, anyhit, /*keep_counters=*/true);
+                if (rc) return rc;
+                rc = drop_placeholder_costs(s, P.ray_cost, len, s->stream);
                 if (rc) return rc;
                 CU(cudaEventRecord(s->e_k[slot], s->stream));
             }
@@ -850,12 +888,14 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 const uint64_t j = i - 1; const int ps = (int)(j & 1);
                 CU(cudaStreamWaitEvent(s->s_out, s->e_k[ps], 0));
                 CU(cudaMemcpyAsync(s->h_hits[ps], s->d_hits + j * chunk, chunk_len(j) * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->s_out));
+                if (costs) CU(cudaMemcpyAsync(s->h_costs[ps], d_costs + j * chunk, chunk_len(j) * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->s_out));
                 CU(cudaEventRecord(s->e_out[ps], s->s_out));
             }
             if (i >= 2) {                                                               // chunk i-2: hand its hits to the caller
                 const uint64_t j = i - 2; const int ps = (int)(j & 1);
                 CU(cudaEventSynchronize(s->e_out[ps]));
                 tray::par_copy(hits + j * chunk, s->h_hits[ps], chunk_len(j) * sizeof(tray_hit));
+                if (costs) tray::par_copy(costs + j * chunk, s->h_costs[ps], chunk_len(j) * sizeof(tray_ray_cost));
             }
         }
         CU(cudaEventRecord(s->ev[1], s->stream));
@@ -878,16 +918,29 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
 extern "C" {
 
 int tray_cuda_trace_device(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits, void* stream, float* ms_kernel) {
-    return trace_device_impl(s, d_rays, n, d_hits, stream, ms_kernel, false);
+    return trace_device_impl(s, d_rays, n, d_hits, nullptr, stream, ms_kernel, false);
 }
 int tray_cuda_trace(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, float* ms_kernel, float* ms_total) {
-    return trace_impl(s, rays, n, hits, ms_kernel, ms_total, false);
+    return trace_impl(s, rays, n, hits, nullptr, ms_kernel, ms_total, false);
 }
 int tray_cuda_trace_any_device(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits, void* stream, float* ms_kernel) {
-    return trace_device_impl(s, d_rays, n, d_hits, stream, ms_kernel, true);
+    return trace_device_impl(s, d_rays, n, d_hits, nullptr, stream, ms_kernel, true);
 }
 int tray_cuda_trace_any(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, float* ms_kernel, float* ms_total) {
-    return trace_impl(s, rays, n, hits, ms_kernel, ms_total, true);
+    return trace_impl(s, rays, n, hits, nullptr, ms_kernel, ms_total, true);
+}
+int tray_cuda_trace_cost_device(tray_scene* s, const tray_ray* d_rays, uint64_t n, int any_hit, tray_hit* d_hits, tray_ray_cost* d_costs,
+                                void* stream, float* ms_kernel) {
+    if (!s || (n && (!d_rays || !d_hits || !d_costs))) return fail(TRAY_ERR_ARG, "NULL argument");
+    if ((uintptr_t)d_costs & 15u) return fail(TRAY_ERR_ARG, "d_costs must be 16-byte aligned (one vector store per record)");
+    if (s->variant) return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);     // before any change of state
+    return trace_device_impl(s, d_rays, n, d_hits, d_costs, stream, ms_kernel, any_hit != 0);
+}
+int tray_cuda_trace_cost(tray_scene* s, const tray_ray* rays, uint64_t n, int any_hit, tray_hit* hits, tray_ray_cost* costs,
+                         float* ms_kernel, float* ms_total) {
+    if (!s || (n && (!rays || !hits || !costs))) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (s->variant) return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);
+    return trace_impl(s, rays, n, hits, costs, ms_kernel, ms_total, any_hit != 0);
 }
 
 uint64_t tray_cuda_shard_pixels(uint32_t w, uint32_t h, uint32_t shard, uint32_t shards) {
@@ -1011,7 +1064,8 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     const bool keep_rays = (flags & TRAY_RENDER_KEEP_RAYS) != 0;
     const bool any_ao = (flags & TRAY_RENDER_ANYHIT_AO) != 0;
     const bool overlap = bounce && !any_ao && !s->variant && ((flags & TRAY_RENDER_OVERLAP) != 0 || s->overlap_default);
-    if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item)) {
+    const bool keep_cost = want_count && s->ray_cost;
+    if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item) || (keep_cost && !f.d_cost)) {
         const uint64_t cap = items_cap > f.f_cap ? items_cap : f.f_cap;
         CU(cudaStreamSynchronize(st));
         free_frame_buffers(f);
@@ -1023,6 +1077,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         CU(cudaMalloc(&f.d_brays, c1 * sizeof(tray_ray)));
         CU(cudaMalloc(&f.d_bitem, c1 * sizeof(uint32_t)));
         if (keep_rays) CU(cudaMalloc(&f.d_brays_item, c1 * sizeof(tray_ray)));
+        if (keep_cost) CU(cudaMalloc(&f.d_cost, 2 * c1 * sizeof(tray_ray_cost)));
         CU(cudaMemsetAsync(f.d_primary, 0xff, c1 * sizeof(tray_hit), st));
         CU(cudaMemsetAsync(f.d_bounce, 0xff, c1 * sizeof(tray_hit), st));
         CU(cudaMemsetAsync(f.d_rgba, 0, c1 * sizeof(uchar4), st));
@@ -1031,6 +1086,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     FrameParams F; frame_params(F, view, w, h, frame_count, shard, shards);
     f.f_has_bounce = bounce; f.f_has_rgba = rgba && !s->frame_target; f.f_has_rays = keep_rays && bounce;
     f.f_target = rgba ? s->frame_target : nullptr;
+    f.f_has_cost = keep_cost;
     f.last_frame = F;
     if (F.n_items == 0) {                        // a shard without tiles: no launch, and nothing to count
         if (ms_primary) *ms_primary = 0.f;
@@ -1043,6 +1099,10 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     const bool timed = ms_primary || ms_bounce;
 
     // ---- primary: generate rays, trace ----
+    // ray costs: primary records at d_cost[item], bounce records at d_cost[n_items + item]; a pixel that shoots no bounce ray
+    // writes no bounce record, so that half starts zeroed
+    tray_ray_cost* const d_cost_bounce = keep_cost ? f.d_cost + F.n_items : nullptr;
+    if (keep_cost && bounce) CU(cudaMemsetAsync(d_cost_bounce, 0, (size_t)F.n_items * sizeof(tray_ray_cost), st));
     if (timed) CU(cudaEventRecord(f.ev[0], st));
     tray::raygen_primary_kernel<<<gen_grid, 256, 0, st>>>(F, f.d_prays);
     CU(cudaGetLastError());
@@ -1051,6 +1111,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     P.frame = F; P.row_major = s->frame_target ? 1u : 0u;
     uchar4* const rgba_dst = s->frame_target ? s->frame_target : f.d_rgba;
     P.rgba_out = (rgba && !bounce) ? rgba_dst : nullptr; P.shade_mode = SHADE_PRIMARY;
+    P.ray_cost = keep_cost ? f.d_cost : nullptr;
     if (overlap) {
         // one launch for the whole frame (trace_kernel<FRAME>): the bounce rays of finished tiles fill the primary pass's drain
         CU(cudaMemsetAsync(f.d_units, 0, sizeof(uint32_t), st));
@@ -1077,10 +1138,12 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
         B.overflow = f.d_flag; B.frame = F; B.row_major = P.row_major;
         B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
+        B.ray_cost = d_cost_bounce;
         rc = launch(s, B, st, f.d_cursor, 1, want_count, any_ao);
         if (rc) return rc;
         if (timed) CU(cudaEventRecord(f.ev[2], st));
     }
+    if (keep_cost) { rc = drop_placeholder_costs(s, f.d_cost, F.n_items, st); if (rc) return rc; }   // (an empty scene shoots no bounce ray)
     if (timed) {
         CU(cudaStreamSynchronize(st));
         float a = 0.f, b = 0.f;
@@ -1211,6 +1274,19 @@ int tray_cuda_frame_download(tray_scene* s, tray_hit* primary, tray_hit* bounce,
         if (!f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA");
         rc = download<uchar4>(s, f.d_rgba, (uchar4*)rgba); if (rc) return rc;
     }
+    return check_overflow(f.d_flag, slot_stream(s, s->cur));
+}
+
+int tray_cuda_frame_download_cost(tray_scene* s, tray_ray_cost* primary, tray_ray_cost* bounce) {
+    if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
+    const FrameSlot& f = s->slot[s->cur];
+    if (f.last_frame.width == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
+    if (!f.f_has_cost) return fail(TRAY_ERR_ARG, "last frame kept no ray costs (it needs tray_cuda_scene_set_ray_cost and TRAY_RENDER_COUNTERS)");
+    if (bounce && !f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
+    CU(cudaSetDevice(s->device));
+    int rc;
+    if (primary) { rc = download<tray_ray_cost>(s, f.d_cost, primary); if (rc) return rc; }
+    if (bounce) { rc = download<tray_ray_cost>(s, f.d_cost + f.last_frame.n_items, bounce); if (rc) return rc; }
     return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 

@@ -32,9 +32,12 @@ EXPORTS = (
     "tray_cuda_group_set_frames_in_flight", "tray_cuda_group_set_exchange", "tray_cuda_group_render", "tray_cuda_group_render_timed",
     "tray_cuda_group_readback_begin", "tray_cuda_group_readback_wait", "tray_cuda_group_frame_ptr", "tray_cuda_group_sync",
     "tray_cuda_start_multi",
+    "tray_cuda_trace_cost", "tray_cuda_trace_cost_device", "tray_cuda_scene_set_ray_cost", "tray_cuda_frame_download_cost",
 )
 # semantic switches of tray_cuda_scene_set_variant (include/tray_cuda.h TRAY_VARIANT_*)
 VARIANT_BOX_DIVIDE, VARIANT_TIE_LAST, VARIANT_BOX_TMIN_RAY, VARIANT_ZERODIR_BOX_ONLY = 1, 2, 4, 8
+# tray_ray_cost (include/tray_cuda.h): one ray's nodes fetched, triangles tested, TLAS leaf entries, peak stack entries
+COST_DTYPE = np.dtype([("nodes", "<u4"), ("tris", "<u4"), ("instances", "<u4"), ("stack", "<u4")])
 
 
 class TrayCudaError(RuntimeError):
@@ -201,6 +204,14 @@ def lib() -> C.CDLL:
         L.tray_cuda_group_frame_ptr.argtypes = [vp, C.POINTER(vp)]
         L.tray_cuda_group_sync.restype = i32
         L.tray_cuda_group_sync.argtypes = [vp]
+        L.tray_cuda_trace_cost.restype = i32
+        L.tray_cuda_trace_cost.argtypes = [vp, vp, u64, i32, vp, vp, f32p, f32p]
+        L.tray_cuda_trace_cost_device.restype = i32
+        L.tray_cuda_trace_cost_device.argtypes = [vp, vp, u64, i32, vp, vp, vp, f32p]
+        L.tray_cuda_scene_set_ray_cost.restype = i32
+        L.tray_cuda_scene_set_ray_cost.argtypes = [vp, i32]
+        L.tray_cuda_frame_download_cost.restype = i32
+        L.tray_cuda_frame_download_cost.argtypes = [vp, vp, vp]
         L.tray_cuda_start_multi.restype = i32
         L.tray_cuda_start_multi.argtypes = [vp, i32, vp, u64, vp, u64, vp, u64, u32, u32, i32, C.POINTER(TrayView), u32, u32,
                                             C.c_float, i32, i32, f32p, f32p, C.POINTER(u32)]
@@ -363,6 +374,30 @@ class TrayCudaScene:
     def set_counting(self, on: bool):
         _check(lib().tray_cuda_set_counting(self._h, int(on)))
 
+    def traverse_cost(self, rays: np.ndarray, any_hit: bool = False, timings: dict | None = None):
+        """(hits, costs): traverse() plus the cost of every ray (COST_DTYPE) — tray_cuda_trace_cost."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        hits = np.empty(rays.shape[0], dtype=HIT_DTYPE)
+        costs = np.empty(rays.shape[0], dtype=COST_DTYPE)
+        k, t = C.c_float(), C.c_float()
+        _check(lib().tray_cuda_trace_cost(self._h, rays.ctypes.data, rays.shape[0], int(any_hit), hits.ctypes.data, costs.ctypes.data,
+                                          C.byref(k), C.byref(t)))
+        if timings is not None:
+            timings["ms_kernel"], timings["ms_total"] = k.value, t.value
+        return hits, costs
+
+    def traverse_cost_device(self, d_rays_ptr: int, n: int, d_hits_ptr: int, d_costs_ptr: int, stream: int = 0, timed: bool = False,
+                             any_hit: bool = False):
+        """traverse_device() plus 16-byte cost records at `d_costs_ptr` — tray_cuda_trace_cost_device."""
+        k = C.c_float()
+        _check(lib().tray_cuda_trace_cost_device(self._h, d_rays_ptr, n, int(any_hit), d_hits_ptr, d_costs_ptr, stream or None,
+                                                 C.byref(k) if timed else None))
+        return k.value if timed else None
+
+    def set_ray_cost(self, on: bool):
+        """While on, every render with RENDER_COUNTERS keeps each ray's cost for download_cost()."""
+        _check(lib().tray_cuda_scene_set_ray_cost(self._h, int(on)))
+
     def set_variant(self, flags: int):
         """Run the other reading of the semantics that are sourced from memory of obvhs (VARIANT_* flags; 0 = default)."""
         _check(lib().tray_cuda_scene_set_variant(self._h, int(flags)))
@@ -464,18 +499,33 @@ class TrayCudaScene:
         g = buf("rgba", rgba, np.uint8, (h, w, 4))
         _check(lib().tray_cuda_frame_download(self._h, None if p is None else p.ctypes.data, None if b is None else b.ctypes.data,
                                               None if r is None else r.ctypes.data, None if g is None else g.ctypes.data))
-        if merge and into is not None:
-            shard, shards = self.frame_shard
-            own = shard_mask(w, h, shard, shards)
-            for k, v in out.items():
-                if k not in into:
-                    into[k] = v
-                elif k == "rgba":
-                    into[k][own.reshape(h, w)] = v[own.reshape(h, w)]
-                else:
-                    into[k][own] = v[own]
-            return into
-        return out
+        return self._merged(out, into) if merge and into is not None else out
+
+    def download_cost(self, primary=True, bounce=False, into: dict | None = None, merge: bool = False) -> dict:
+        """The last frame's ray costs (COST_DTYPE, row-major, w*h): "primary" and / or "bounce" (zero where a pixel shot no
+        bounce ray).  Pixels of other shards come back as zeros; merge=True as in download()."""
+        w, h = self.frame_size
+        out = into if (into is not None and not merge) else {}
+        for name, want in (("primary", primary), ("bounce", bounce)):
+            if want and name not in out:
+                out[name] = np.zeros(w * h, dtype=COST_DTYPE)
+        p, b = out.get("primary") if primary else None, out.get("bounce") if bounce else None
+        _check(lib().tray_cuda_frame_download_cost(self._h, None if p is None else p.ctypes.data, None if b is None else b.ctypes.data))
+        return self._merged(out, into) if merge and into is not None else out
+
+    def _merged(self, out: dict, into: dict) -> dict:
+        """this shard's pixels of `out` written over the arrays of `into` (arrays `into` lacks are taken whole)"""
+        w, h = self.frame_size
+        shard, shards = self.frame_shard
+        own = shard_mask(w, h, shard, shards)
+        for k, v in out.items():
+            if k not in into:
+                into[k] = v
+            elif k == "rgba":
+                into[k][own.reshape(h, w)] = v[own.reshape(h, w)]
+            else:
+                into[k][own] = v[own]
+        return into
 
     def frame_device_ptrs(self):
         a, b, c = C.c_void_p(), C.c_void_p(), C.c_void_p()
