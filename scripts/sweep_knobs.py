@@ -8,7 +8,7 @@ m = host.Mesh.generate(scene, 3, 1.0)
 p = host.PackedScene(m)
 w, h = 1920, 1080
 view = host.view_from_camera(m.camera, w, h)
-knobs = {"TRAY_CUDA_TRI_WEIGHT": [1, 2, 3, 4, 8, 64], "TRAY_CUDA_REFILL_MIN": [1, 4, 8, 16, 24], "TRAY_CUDA_BLOCKS_PER_SM": [0]}
+knobs = {"TRAY_CUDA_TRI_WEIGHT": [1, 2, 3, 4, 8, 64], "TRAY_CUDA_REFILL_MIN": [1, 4, 8, 16, 24]}
 if len(sys.argv) > 2:
     knobs = eval(sys.argv[2])
 names = list(knobs)

@@ -91,7 +91,10 @@ struct TraceParams {
     uint32_t* __restrict__ cursor;            // work cursor
     unsigned long long* __restrict__ counters;// counter slot (N_COUNTERS; FRAME: two slots) of the cursor block (COUNT builds)
     uint32_t* __restrict__ overflow;          // device error word (ERR_*)
-    unsigned long long* __restrict__ dev_log; // -DTRAY_EXIT_LOG / -DTRAY_STEP_CLOCK builds: per-warp records
+    // optional, COUNT builds: one cost record per ray at its output item (tray_cuda_trace_cost, tray_cuda_scene_set_ray_cost).
+    // FRAME kernel: the bounce records follow the n_work primary ones.  An 8-byte member in this slot keeps the 16-byte
+    // alignment of the members after it, and with it the generated code of every kernel.
+    tray_ray_cost* __restrict__ ray_cost;
     uint32_t k4b;                             // 0x4B000000, passed at run time (see byte_f32)
     uint32_t force_exact;                     // scene has node scales >= 2^40: always take the unfused node test
     float zero;                               // 0.0f, passed at run time (see child_test_fast)
@@ -107,10 +110,6 @@ struct TraceParams {
     uint32_t* __restrict__ unit_cursor;       // next tile whose bounce rays have not been claimed (zeroed by the host)
     uint32_t n_units;                         // n_work / 32: bounce work is claimed in groups of 32 items
     uint32_t gen_min;                         // idle lanes needed before the warp generates bounce rays into them
-    // optional, COUNT builds: one cost record per ray at its output item (tray_cuda_trace_cost, tray_cuda_scene_set_ray_cost).
-    // FRAME kernel: the bounce records follow the n_work primary ones.  Last member: the offsets of every other member, and so
-    // the code of the kernels that do not count, stay as they were.
-    tray_ray_cost* __restrict__ ray_cost;
 };
 
 // ---- exact float helpers (no contraction, IEEE rounding) --------------------------------------
@@ -144,15 +143,6 @@ template <int J> __device__ __forceinline__ uint32_t byte_u32(uint32_t w) {
     asm("prmt.b32 %0, %1, 0, %2;" : "=r"(r) : "r"(w), "n"(0x4440 + J));
     return r;
 }
-
-// dev instrumentation (-DTRAY_STEP_CLOCK, tests/tools/step_clock.py): where do the cycles of one dependent step go?
-#ifdef TRAY_STEP_CLOCK
-__device__ __forceinline__ long long clk() { long long c; asm volatile("mov.u64 %0, %%clock64;" : "=l"(c)); return c; }
-__device__ __forceinline__ long long clk_after(uint32_t dep) { long long c; asm volatile("mov.u64 %0, %%clock64; // %1" : "=l"(c) : "r"(dep)); return c; }
-#define SC(...) __VA_ARGS__
-#else
-#define SC(...)
-#endif
 
 // ---- per-ray constants ---------------------------------------------------------------------------
 struct RayConst {
@@ -540,18 +530,17 @@ __global__ void __launch_bounds__(256) raygen_primary_kernel(const __grid_consta
     store_ray(rays + j, a, b);
 }
 
-// One thread per pixel of the shard.  Hit pixels append their bounce ray to a compact list (warp-aggregated
-// atomicAdd; `ray_item` remembers the pixel); missed pixels get their final results here.
+// One thread per pixel of the shard.  Hit pixels append their bounce ray to a compact list (one atomicAdd per block;
+// `ray_item` remembers the pixel); missed pixels get their final results here.
 constexpr int BOUNCE_BLOCK = 1024;    // pixels per block of raygen_bounce_kernel = the group its rays are sorted in
 template <int TRI_STRIDE>
 __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __grid_constant__ FrameParams F, const uint4* __restrict__ tris,
                                                             const tray_hit* __restrict__ primary, tray_ray* __restrict__ rays,
                                                             uint32_t* __restrict__ ray_item, uint32_t* __restrict__ n_rays,
                                                             tray_hit* __restrict__ bounce_out, uchar4* __restrict__ rgba_out,
-                                                            tray_ray* __restrict__ rays_by_item, uint32_t row_major, uint32_t sort_octant) {
-    __shared__ uint32_t s_cnt[24], s_base[24];
+                                                            tray_ray* __restrict__ rays_by_item, uint32_t row_major) {
+    __shared__ uint32_t s_cnt[8], s_base[8];
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-    const unsigned lane = threadIdx.x & 31u;
     uint32_t px = 0, py = 0;
     bool shoot = false;
     tray_hit ph; ph.t = __int_as_float(0x7f800000); ph.prim = INVALID;
@@ -566,45 +555,25 @@ __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __gri
         bounce_ray<TRI_STRIDE>(F, tris, px, py, pdx, pdy, pdz, ph.t, ph.prim, ox, oy, oz, dx, dy, dz);
         a = make_float4(ox, oy, oz, 0.0f); b = make_float4(dx, dy, dz, F32_MAX_);
     }
-    if (sort_octant) {
-        // The rays of the block's 1024 pixels (4 tiles: close origins) are appended grouped by direction octant, so that the
-        // 32 rays a traversal warp fetches together share the order in which they visit a node's children.
-        const uint32_t nb = sort_octant >= 2u ? 24u : 8u;
-        if (threadIdx.x < 24) s_cnt[threadIdx.x] = 0u;
-        __syncthreads();
-        uint32_t oct = (b.x < 0.f ? 4u : 0u) | (b.y < 0.f ? 2u : 0u) | (b.z < 0.f ? 1u : 0u);
-        if (sort_octant >= 2u) {        // ... and by dominant axis inside the octant
-            const float ax = fabsf(b.x), ay = fabsf(b.y), az = fabsf(b.z);
-            oct = oct * 3u + (ax >= ay ? (ax >= az ? 0u : 2u) : (ay >= az ? 1u : 2u));
-        }
-        uint32_t pos = 0;
-        if (shoot) pos = atomicAdd(&s_cnt[oct], 1u);
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            uint32_t acc = 0;
-            for (uint32_t o = 0; o < nb; o++) { const uint32_t c = s_cnt[o]; s_base[o] = acc; acc += c; }
-            const uint32_t g = acc ? atomicAdd(n_rays, acc) : 0u;
-            for (uint32_t o = 0; o < nb; o++) s_base[o] += g;
-        }
-        __syncthreads();
-        if (shoot) {
-            const uint32_t slot = s_base[oct] + pos;
-            store_ray(rays + slot, a, b);
-            ray_item[slot] = j;
-        }
-    } else {
-    const unsigned m = __ballot_sync(FULL, shoot);
-    if (m) {
-        const int leader = __ffs(m) - 1;
-        uint32_t base = 0;
-        if ((int)lane == leader) base = atomicAdd(n_rays, (uint32_t)__popc(m));
-        base = __shfl_sync(FULL, base, leader);
-        if (shoot) {
-            const uint32_t slot = base + (uint32_t)__popc(m & ((1u << lane) - 1u));
-            store_ray(rays + slot, a, b);
-            ray_item[slot] = j;
-        }
+    // The rays of the block's 1024 pixels (4 tiles: close origins) are appended grouped by direction octant, so that the
+    // 32 rays a traversal warp fetches together share the order in which they visit a node's children.
+    if (threadIdx.x < 8) s_cnt[threadIdx.x] = 0u;
+    __syncthreads();
+    const uint32_t oct = (b.x < 0.f ? 4u : 0u) | (b.y < 0.f ? 2u : 0u) | (b.z < 0.f ? 1u : 0u);
+    uint32_t pos = 0;
+    if (shoot) pos = atomicAdd(&s_cnt[oct], 1u);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t acc = 0;
+        for (uint32_t o = 0; o < 8; o++) { const uint32_t c = s_cnt[o]; s_base[o] = acc; acc += c; }
+        const uint32_t g = acc ? atomicAdd(n_rays, acc) : 0u;
+        for (uint32_t o = 0; o < 8; o++) s_base[o] += g;
     }
+    __syncthreads();
+    if (shoot) {
+        const uint32_t slot = s_base[oct] + pos;
+        store_ray(rays + slot, a, b);
+        ray_item[slot] = j;
     }
     if (j < F.n_items) {
         if (!shoot) finish_no_bounce(F, row_major, j, ph.t, bounce_out, rgba_out, rays_by_item);
@@ -766,9 +735,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         }
     };
 
-    SC(long long sc_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; long long sc_n[2] = {0, 0}; long long sc_t0 = clk();)
     for (;;) {
-        SC(const long long sc_top = clk();)
         const bool want_tri = tri_y != 0u;
         const bool want_node = !want_tri && cur_y >= 0x01000000u;
         const unsigned m_tri = __ballot_sync(FULL, want_tri), m_node = __ballot_sync(FULL, want_node);
@@ -783,12 +750,6 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                 uint32_t base = 0;
                 if ((int)lane == leader) base = atomicAdd(P.cursor, n_idle);
                 base = __shfl_sync(FULL, base, leader);
-#ifdef TRAY_EXIT_LOG
-                if (base + n_idle >= n_work && !exhausted && P.dev_log && lane == 0) {   // ... and when it ran dry
-                    unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-                    P.dev_log[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5))] = t;
-                }
-#endif
                 if (base + n_idle >= n_work) exhausted = true;
                 if ((idle >> lane) & 1u) {
                     ray_idx = base + (uint32_t)__popc(idle & ((1u << lane) - 1u));
@@ -869,22 +830,8 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
             if (busy == 0u) { if (exhausted && units_done && cand_unit == INVALID && H == 0u) break; continue; }
         }
 
-#ifdef TRAY_EXIT_LOG
-        if (exhausted && P.dev_log) {       // first time the warp is down to <= 8 / 4 / 2 / 1 rays after the cursor ran dry
-            const int nb = __popc(busy);
-            unsigned long long* rec = P.dev_log + 6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
-            if (lane == 0 && nb <= 8) {
-                unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-                if (rec[2] == 0) rec[2] = t;
-                if (nb <= 4 && rec[3] == 0) rec[3] = t;
-                if (nb <= 2 && rec[4] == 0) rec[4] = t;
-                if (nb <= 1 && rec[5] == 0) rec[5] = t;
-            }
-        }
-#endif
         // ---- warp vote: node step or triangle step ----
         const bool tri_phase = m_node == 0u || (unsigned)__popc(m_tri) * P.tri_weight >= (unsigned)__popc(m_node);
-        SC(const long long sc_voted = clk_after(tri_phase); sc_acc[0] += sc_voted - sc_top;)
 
         if (!tri_phase) {
             if (want_node) {
@@ -894,21 +841,17 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                 cur_y = hits_imask ^ (0x01000000u << slot);                                    // :362
                 const uint32_t rel = (uint32_t)__popc(hits_imask & ((1u << slot) - 1u));       // :371 (slot < 8: imask bits only)
                 const uint4* np = P.nodes + (size_t)(bvh_off + cur_x + rel) * 5u;              // :373, tlas:383
-                SC(const long long sc_a = clk_after(rel); sc_acc[1] += sc_a - sc_voted;)
                 const uint4 n0 = __ldg(np), n1 = __ldg(np + 1), n2 = __ldg(np + 2), n3 = __ldg(np + 3), n4 = __ldg(np + 4);
                 if (cur_y & 0xff000000u) push(cur_x, cur_y);                                   // :365-368, in the shadow of the node fetch
-                SC(const long long sc_b = clk_after(n0.x ^ n1.x ^ n2.x ^ n3.x ^ n4.x); sc_acc[2] += sc_b - sc_a;)
                 TRAY_CNT(nodes);
                 uint32_t hitmask;                                                              // slot space (see node_test)
                 if (MODE == 1) hitmask = node_test(r, best_t, n0, n1, n2, n3, n4, k4b, r.box_tmin, (P.variant & TRAY_VARIANT_BOX_DIVIDE) != 0u);
                 else hitmask = ((ray_idx & WIDE_BIT) || P.force_exact) ? node_test(r, best_t, n0, n1, n2, n3, n4, k4b)
                                                 : node_test_fast(r, best_t, n0, n1, n2, n3, n4, k4b, P.zero, P.one);   // :380
-                SC(const long long sc_c = clk_after(hitmask); sc_acc[3] += sc_c - sc_b; sc_n[0]++;)
                 cur_x = n1.x; tri_x = n1.y;                                                    // :383-384
                 cur_y = (hitmask & 0xff000000u) | (n0.w >> 24);                                // :386 (top byte: hit inner children, slot space)
                 tri_y = hitmask & 0x00ffffffu;                                                 // :387
                 if (tri_y == 0u && cur_y < 0x01000000u) pop_or_retire();
-                SC(sc_acc[4] += clk_after(cur_y ^ tri_y) - sc_c;)
             }
         } else {
             if (want_tri) {
@@ -925,10 +868,6 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     cur_x = 0; cur_y = 0x80000000u; tri_y = 0;
                 } else {
                     TRAY_CNT(tris);
-                    SC(const long long sc_a = clk_after(g); sc_acc[5] += sc_a - sc_voted;)
-                    SC({ const uint4 q0 = __ldg(P.tris + (size_t)g * (TRI_STRIDE / 16)), q2 = __ldg(P.tris + (size_t)g * (TRI_STRIDE / 16) + 2);
-                         sc_acc[6] -= sc_a; sc_acc[6] += clk_after(q0.x ^ q2.x); })
-                    SC(const long long sc_b = clk();)
                     // Two triangles of the lane's pending group per iteration (82 % of the groups hold >= 2): both records are
                     // fetched together and the two tests run side by side.  The second test's only use of tmax is its final
                     // `tt <= tmax` (query.hlsl:119), so running it against the OLD tmax and comparing with the updated best_t
@@ -950,25 +889,11 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     }
                     if (ANYHIT && best_prim != INVALID) { sp &= SP_STEP - 1u; tri_y = 0u; cur_y = 0u; }   // drop the rest of the traversal
                     if (tri_y == 0u && cur_y < 0x01000000u) pop_or_retire();
-                    SC(sc_acc[7] += clk_after(cur_y ^ tri_y ^ __float_as_uint(best_t)) - sc_b; sc_n[1]++;)
                 }
             }
         }
     }
 
-#ifdef TRAY_STEP_CLOCK
-    if (P.dev_log && lane == 0) {     // per warp: cycles in [vote, node pre, node load wait, node test, node post, tri pre, tri load wait, tri test+post], steps, total
-        long long* o = (long long*)P.dev_log + 12 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5));
-        for (int i = 0; i < 8; i++) o[i] = sc_acc[i];
-        o[8] = sc_n[0]; o[9] = sc_n[1]; o[10] = clk() - sc_t0; o[11] = 1;
-    }
-#endif
-#ifdef TRAY_EXIT_LOG
-    if (P.dev_log && lane == 0) {     // dev instrumentation (scripts/exit_log.py): when this warp exited (ns)
-        unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-        P.dev_log[6 * (blockIdx.x * (BLOCK_THREADS / 32) + (threadIdx.x >> 5)) + 1] = t;
-    }
-#endif
     if (COUNT) {
         flush_counters(P.counters, lane, c_rays, c_nodes, c_tris, c_insts, c_hits);
         if (FRAME) flush_counters(P.counters + N_COUNTERS, lane, b_rays, b_nodes, b_tris, b_insts, b_hits);   // the bounce rays' slot

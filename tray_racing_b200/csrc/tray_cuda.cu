@@ -114,7 +114,6 @@ struct tray_scene {
     uchar4* d_stage[TRAY_READBACK_SLOTS] = {}; uint64_t stage_cap[TRAY_READBACK_SLOTS] = {}; bool stage_busy[TRAY_READBACK_SLOTS] = {};
     cudaEvent_t ev_untiled[TRAY_READBACK_SLOTS] = {}, ev_copied[TRAY_READBACK_SLOTS] = {};
     cudaEvent_t ev_after = nullptr;          // tray_cuda_scene_after
-    uint32_t bounce_sort = 1;                // raygen_bounce_kernel: 0 append in pixel order, 1 group by direction octant, 2 octant x major axis
     uint32_t* h_flag = nullptr;              // pinned, one word per staging slot: the error word of the frame staging slot i was filled from
     uchar4* frame_target = nullptr;          // borrowed: row-major RGBA8 frame (this or a peer device), see tray_cuda_scene_set_frame_target
     tray_counters cnt_primary{}, cnt_bounce{};
@@ -189,8 +188,6 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
         int nb = 0;
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, BLOCK_THREADS, 0));
         bps = nb > 0 ? nb : 1;
-        int cap = env_int("TRAY_CUDA_BLOCKS_PER_SM", 0);
-        if (cap > 0 && cap < bps) bps = cap;
     }
     P.cursor = (uint32_t*)cur;
     P.counters = cur + CURSOR_COUNTERS + N_COUNTERS * counter_slot;
@@ -209,30 +206,8 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
         attr[0].val.accessPolicyWindow = s->window;
         cfg.attrs = attr; cfg.numAttrs = 1;
     }
-#if defined(TRAY_EXIT_LOG) || defined(TRAY_STEP_CLOCK)
-#ifdef TRAY_STEP_CLOCK
-#define TRAY_EXIT_LOG 1              // from here on: the host side of both dev logs is the same dump
-    const size_t log_n = 12 * grid * (BLOCK_THREADS / 32);
-#else
-    const size_t log_n = 6 * grid * (BLOCK_THREADS / 32);
-#endif
-    static unsigned long long* d_log = nullptr;
-    if (!d_log) CU(cudaMalloc(&d_log, 1 << 24));
-    CU(cudaMemsetAsync(d_log, 0, log_n * 8, st));
-    P.dev_log = d_log;
-#endif
     void* args[1] = { (void*)&P };
     CU(cudaLaunchKernelExC(&cfg, (const void*)k, args));
-#ifdef TRAY_EXIT_LOG
-    if (getenv("TRAY_EXIT_LOG_FILE")) {
-        std::vector<unsigned long long> h(log_n);
-        CU(cudaStreamSynchronize(st));
-        CU(cudaMemcpy(h.data(), d_log, log_n * 8, cudaMemcpyDeviceToHost));
-        char name[512]; static int seq = 0;
-        snprintf(name, sizeof name, "%s.%d.bin", getenv("TRAY_EXIT_LOG_FILE"), seq++);
-        FILE* f = fopen(name, "wb"); if (f) { fwrite(h.data(), 8, log_n, f); fclose(f); }
-    }
-#endif
     return TRAY_OK;
 }
 
@@ -499,7 +474,6 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         for (auto& e : s->ev) CU(cudaEventCreate(&e));
         CU(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
         CU(cudaEventCreateWithFlags(&s->ev_after, cudaEventDisableTiming));
-        s->bounce_sort = (uint32_t)env_int("TRAY_CUDA_BOUNCE_SORT", 1);
         CU(cudaMallocHost(&s->h_flag, TRAY_READBACK_SLOTS * sizeof(uint32_t)));
         for (int i = 0; i < TRAY_READBACK_SLOTS; i++) {
             s->h_flag[i] = 0u;
@@ -539,7 +513,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         }
         if (n_instances && blas_offsets) CU(cudaMemcpyAsync(s->d_blas, blas_offsets, (size_t)n_instances * 4, cudaMemcpyHostToDevice, s->stream));
         // keep the node array hot in the 126 MB L2: persisting access-policy window, attached to every traversal launch
-        if (env_int("TRAY_CUDA_L2_PERSIST", 1) && prop.persistingL2CacheMaxSize > 0 && n_nodes) {
+        if (prop.persistingL2CacheMaxSize > 0 && n_nodes) {
             size_t want = (size_t)prop.persistingL2CacheMaxSize;
             if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
                 size_t win = (size_t)n_nodes * 80;
@@ -798,7 +772,7 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
     return TRAY_OK;
 }
 
-constexpr uint64_t PIPE_CHUNK = 1ull << 20;       // rays per pipeline stage (32 MiB in, 8 MiB out)
+constexpr uint64_t CHUNK_MAX = 1ull << 20;        // rays per pipeline stage (32 MiB in, 8 MiB out)
 constexpr uint64_t PIPE_MIN = 1ull << 18;         // smaller batches take the plain copy-launch-copy path
 
 int ensure_pipeline(tray_scene* s) {
@@ -807,8 +781,8 @@ int ensure_pipeline(tray_scene* s) {
         CU(cudaStreamCreateWithFlags(&s->s_in, cudaStreamNonBlocking));
         CU(cudaStreamCreateWithFlags(&s->s_out, cudaStreamNonBlocking));
         for (int i = 0; i < 2; i++) {
-            CU(cudaMallocHost(&s->h_rays[i], PIPE_CHUNK * sizeof(tray_ray)));
-            CU(cudaMallocHost(&s->h_hits[i], PIPE_CHUNK * sizeof(tray_hit)));
+            CU(cudaMallocHost(&s->h_rays[i], CHUNK_MAX * sizeof(tray_ray)));
+            CU(cudaMallocHost(&s->h_hits[i], CHUNK_MAX * sizeof(tray_hit)));
             CU(cudaEventCreateWithFlags(&s->e_in[i], cudaEventDisableTiming));
             CU(cudaEventCreateWithFlags(&s->e_k[i], cudaEventDisableTiming));
             CU(cudaEventCreateWithFlags(&s->e_out[i], cudaEventDisableTiming));
@@ -822,7 +796,7 @@ int ensure_pipeline(tray_scene* s) {
 }
 
 // Batch operator with HOST buffers (Traversable::traverse for a slice of rays).  Large batches run as a three-stage pipeline
-// over chunks of PIPE_CHUNK rays: [host threads: caller's rays -> pinned slot] [copy stream: H2D] [scene stream: traversal]
+// over chunks of up to CHUNK_MAX rays: [host threads: caller's rays -> pinned slot] [copy stream: H2D] [scene stream: traversal]
 // [copy stream: D2H into a pinned slot] [host threads: -> caller's hits]; chunk i+1 is staged and uploaded while chunk i is
 // traced and chunk i-1 is read back.  The caller's memory is only borrowed for the call and never registered.
 // costs != NULL: the cost calls (see trace_device_impl); the records travel like the hits
@@ -856,12 +830,10 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         rc = ensure_pipeline(s);
         if (rc) return rc;
         for (int i = 0; costs && i < 2; i++)
-            if (!s->h_costs[i]) CU(cudaMallocHost(&s->h_costs[i], PIPE_CHUNK * sizeof(tray_ray_cost)));
+            if (!s->h_costs[i]) CU(cudaMallocHost(&s->h_costs[i], CHUNK_MAX * sizeof(tray_ray_cost)));
         // chunk size: the pipeline only pays once it has a few stages, and every stage is a kernel launch with its own
-        // drain phase — 2^19 rays below 4 M rays, 2^20 above (TRAY_CUDA_PIPE_CHUNK overrides, <= 2^20)
-        uint64_t chunk = n < (4ull << 20) ? (PIPE_CHUNK >> 1) : PIPE_CHUNK;
-        const int chunk_env = env_int("TRAY_CUDA_PIPE_CHUNK", 0);
-        if (chunk_env >= 4096 && (uint64_t)chunk_env <= PIPE_CHUNK) chunk = (uint64_t)chunk_env;
+        // drain phase — 2^19 rays below 4 M rays, 2^20 above
+        const uint64_t chunk = n < (4ull << 20) ? (CHUNK_MAX >> 1) : CHUNK_MAX;
         const uint64_t n_chunks = (n + chunk - 1) / chunk;
         auto chunk_len = [&](uint64_t i) { return i + 1 < n_chunks ? chunk : n - i * chunk; };
         if (s->counting) CU(cudaMemsetAsync(s->d_cursor + CURSOR_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), s->stream));
@@ -1131,8 +1103,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         CU(cudaMemsetAsync(d_nbrays, 0, sizeof(uint32_t), st));
         auto gen = s->tri_stride == 64 ? tray::raygen_bounce_kernel<64> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24> : tray::raygen_bounce_kernel<48>;
         gen<<<(F.n_items + BOUNCE_BLOCK - 1) / BOUNCE_BLOCK, BOUNCE_BLOCK, 0, st>>>(F, s->d_tris, f.d_primary, f.d_brays, f.d_bitem, d_nbrays, f.d_bounce,
-                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major,
-                                             s->bounce_sort);
+                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major);
         CU(cudaGetLastError());
         TraceParams B; base_params(s, B);
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
