@@ -241,6 +241,36 @@ int tray_cuda_scene_download(tray_scene* scene, void* nodes, void* tris, uint32_
 
 int tray_cuda_scene_info(const tray_scene* scene, tray_scene_info* out_info);
 
+/* *out_exact = 1 when the scene's traversal takes the unfused (exact) node test at every node — some node has an exponent byte
+ * >= 167 (a scale >= 2^40, where the fused test could overflow), or TRAY_CUDA_FORCE_EXACT is set — and 0 when it takes the
+ * fused one.  Decided when the scene is made and again by every tray_cuda_scene_refit. */
+int tray_cuda_scene_exact_node_test(const tray_scene* scene, int* out_exact);
+
+/* ---- refit: move the triangles, keep the tree -----------------------------------------------------------------------------
+ * Rewrites the triangle records from new vertex positions and re-encodes, for every node reachable from a root (node 0, or
+ * every distinct blas_offsets entry and then tlas_start), only p, the exponents and the q bytes of the used slots
+ * (child_meta != 0), tight over the new triangles exactly as the builders encode them; imask, child / primitive bases, child_meta,
+ * empty slots, unreachable nodes, blas_offsets and prim_indices keep their bytes.  Two-level scenes: every BLAS first (a shared
+ * one once), then the TLAS over the BLAS roots' boxes.  Afterwards the scene traces exactly like tray_cuda_scene_create on its
+ * downloaded bytes, the exact node test included (on when some node's exponent byte is >= 167, or TRAY_CUDA_FORCE_EXACT).  A
+ * refit with the scene's own triangles is the identity on trees of either builder.
+ *   tris9     n_tris x 9 floats (v0, v1, v2) in the scene's triangle order: input order for scenes of tray_cuda_scene_build
+ *             (slot k takes triangle prim_indices[k]), BVH slot order for scenes of tray_cuda_scene_create
+ *   ms_refit  CUDA-event time of the refit launches (coordinate check, record pass, one launch per tree level), without the
+ *             host upload and without the topology walk of the first call (NULL ok)
+ * Synchronous.  Starts after every frame and batch trace already enqueued on the scene (every frame slot, the scene stream, the
+ * copy streams) and returns with the new bytes in place: a frame rendered before keeps its results (download, readback, ray
+ * costs), every later render or trace sees the new geometry.  tray_cuda_trace_device work on a caller's own stream is the
+ * caller's to order: pass that stream to tray_cuda_scene_refit_device.
+ * TRAY_ERR_ARG, with nothing changed: NULL scene or triangles, n_tris != the scene's, a coordinate that is not finite, triangles
+ * whose extent on some axis overflows f32 (max - min = inf: no box over them can be encoded; the builders cannot build over them
+ * either), or a tree the walk cannot refit (a node reached twice, a child or leaf index outside its array, a
+ * blas_offsets entry outside the node array).  The first call walks the topology once and keeps it with the scene
+ * (tray_scene_info.device_bytes counts it).  A scene with no triangles refits with n_tris = 0 and nothing happens. */
+int tray_cuda_scene_refit(tray_scene* scene, const float* tris9, uint64_t n_tris, float* ms_refit);
+/* the same with DEVICE memory; the refit starts after the work enqueued so far on `stream` (NULL: none) */
+int tray_cuda_scene_refit_device(tray_scene* scene, const float* d_tris9, uint64_t n_tris, void* stream, float* ms_refit);
+
 /* ---- ray-batch operator: Traversable::traverse at batch grain (traversable/src/lib.rs:20) ----- */
 
 /* Closest hit for `n` rays.  HOST buffers: the copy H2D of rays and D2H of hits are inside the
@@ -477,7 +507,9 @@ int tray_cuda_hits_to_geometry(tray_scene* scene, const tray_hit* hits, uint64_t
  *                                   (no device starts earlier) to the frame being complete
  *   tray_cuda_group_readback_begin / _wait   the complete frame -> HOST memory (pinned for overlap), double-buffered like
  *                                   tray_cuda_frame_readback_begin; with two frames in flight the group alternates two targets
- *   tray_cuda_group_scene           borrow the scene of devices[i] (counters, hit downloads of its shard, set_variant ..)   */
+ *   tray_cuda_group_scene           borrow the scene of devices[i] (counters, hit downloads of its shard, set_variant ..)
+ * Moving geometry: refit every replica, tray_cuda_scene_refit on tray_cuda_group_scene(i) for each i; the group has no refit
+ * call of its own, as its caller would still loop over the devices.                                                          */
 typedef struct tray_group tray_group;
 int  tray_cuda_group_create(const void* nodes, uint64_t n_nodes, const void* tris, uint64_t n_tris, uint32_t tri_stride,
                             const uint32_t* blas_offsets, uint32_t n_instances, uint32_t tlas_start,

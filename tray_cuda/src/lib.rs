@@ -69,6 +69,7 @@ pub const VARIANT_ZERODIR_BOX_ONLY: u32 = 0x8;
 extern "C" {
     pub fn tray_cuda_abi_version() -> u32;
     pub fn tray_cuda_scene_info(scene: *const TrayScene, out_info: *mut TraySceneInfo) -> c_int;
+    pub fn tray_cuda_scene_exact_node_test(scene: *const TrayScene, out_exact: *mut c_int) -> c_int;
     pub fn tray_cuda_scene_build_tlas(tris9: *const f32, n_tris: u64, object_offsets: *const u64, n_objects: u32, tri_stride: u32,
         max_prims_per_leaf: u32, search_radius: u32, device: c_int, out: *mut *mut TrayScene, stats: *mut TrayBuildStats) -> c_int;
     pub fn tray_cuda_scene_download_instances(scene: *mut TrayScene, blas_offsets: *mut u32) -> c_int;
@@ -117,6 +118,10 @@ extern "C" {
     pub fn tray_cuda_scene_build(tris9: *const f32, n_tris: u64, tri_stride: u32, max_prims_per_leaf: u32, search_radius: u32,
         device: c_int, out: *mut *mut TrayScene, stats: *mut TrayBuildStats) -> c_int;
     pub fn tray_cuda_scene_download(scene: *mut TrayScene, nodes: *mut c_void, tris: *mut c_void, prim_indices: *mut u32) -> c_int;
+    // same tree, new vertex positions (n_tris x 9 f32 in the scene's triangle order); synchronous, after every frame enqueued
+    pub fn tray_cuda_scene_refit(scene: *mut TrayScene, tris9: *const f32, n_tris: u64, ms_refit: *mut f32) -> c_int;
+    pub fn tray_cuda_scene_refit_device(scene: *mut TrayScene, d_tris9: *const f32, n_tris: u64, stream: *mut c_void,
+        ms_refit: *mut f32) -> c_int;
     pub fn tray_cuda_frame_download(scene: *mut TrayScene, primary: *mut TrayHit, bounce: *mut TrayHit,
         bounce_rays: *mut TrayRay, rgba: *mut u8) -> c_int;
     pub fn tray_cuda_scene_set_variant(scene: *mut TrayScene, variant_flags: u32) -> c_int;

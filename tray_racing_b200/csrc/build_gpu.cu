@@ -23,7 +23,10 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <chrono>
+#include <climits>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -525,6 +528,39 @@ __device__ int quant_exponent(float extent) {
     return k;
 }
 
+// The encoder (bvh_embree_to_cwbvh.rs:85-186), shared by the collapse and the refit: over the node box [nmn, nmx], p = its
+// minimum and one power-of-two scale per axis, then the floor / ceil q bytes (in double, clamped to 0 .. 255) of every slot in
+// `used`, whose box child_box(s, cmn, cmx) gives.  Writes nothing else of the node.  Returns whether some scale is >= 2^40
+// (exponent byte >= tray::EXACT_EXP_BYTE: the traversal must use its unfused node test).
+template <typename ChildBox>
+__device__ __forceinline__ bool encode_bounds(uint32_t w[20], const float nmn[3], const float nmx[3], uint32_t used, ChildBox child_box) {
+    uint8_t* nb = reinterpret_cast<uint8_t*>(w);
+    double scale[3];
+    bool exact = false;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        w[a] = __float_as_uint(nmn[a]);
+        const int ke = quant_exponent(nmx[a] - nmn[a]);
+        nb[12 + a] = (uint8_t)(ke + 127);
+        exact |= ke + 127 >= 167;
+        scale[a] = ldexp(1.0, ke);
+    }
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        if (!((used >> s) & 1u)) continue;
+        float cmn[3], cmx[3];
+        child_box(s, cmn, cmx);
+#pragma unroll
+        for (int a = 0; a < 3; a++) {
+            double ql = floor(((double)cmn[a] - (double)nmn[a]) / scale[a]);
+            double qh = ceil(((double)cmx[a] - (double)nmn[a]) / scale[a]);
+            ql = fmin(255.0, fmax(0.0, ql)); qh = fmin(255.0, fmax(0.0, qh));
+            nb[32 + 16 * a + s] = (uint8_t)ql; nb[40 + 16 * a + s] = (uint8_t)qh;
+        }
+    }
+    return exact;
+}
+
 template <int STRIDE>
 __device__ void write_tri_record(const float* __restrict__ tris9, uint32_t prim, uint8_t* __restrict__ out, uint64_t slot) {
     const float* t = tris9 + 9ull * prim;
@@ -588,28 +624,18 @@ __global__ void collapse_emit_kernel(const int* __restrict__ items, uint32_t n_i
 #pragma unroll
     for (int q = 0; q < 20; q++) w[q] = 0u;
     uint8_t* nb = reinterpret_cast<uint8_t*>(w);
-    double scale[3];
-    for (int a = 0; a < 3; a++) {
-        w[a] = __float_as_uint(nmn[a]);
-        const int ke = quant_exponent(nmx[a] - nmn[a]);
-        nb[12 + a] = (uint8_t)(ke + 127);
-        if (ke + 127 >= 167) atomicOr(flags, 1u);          // scale >= 2^40: the traversal must use its unfused node test (tray::EXACT_EXP_BYTE)
-        scale[a] = ldexp(1.0, ke);
-    }
+    const bool exact = encode_bounds(w, nmn, nmx, slot_used, [&](int s, float cmn[3], float cmx[3]) {
+        const int c = k.id[slot_child[s]];
+        const float4 lo = b.lo[c], hi = b.hi[c];
+        cmn[0] = lo.x; cmn[1] = lo.y; cmn[2] = lo.z; cmx[0] = hi.x; cmx[1] = hi.y; cmx[2] = hi.z;
+    });
+    if (exact) atomicOr(flags, 1u);
     w[4] = next_base + inner_off[i] - my_root;              // child_base_idx
     w[5] = prim_base + tri_off[i];                          // primitive_base_idx
     uint32_t tri_local = 0, n_in = 0, imask = 0;
     for (int s = 0; s < 8; s++) {
         if (slot_child[s] < 0) continue;
         const int c = k.id[slot_child[s]];
-        const float4 lo = b.lo[c], hi = b.hi[c];
-        const float cmn[3] = { lo.x, lo.y, lo.z }, cmx[3] = { hi.x, hi.y, hi.z };
-        for (int a = 0; a < 3; a++) {
-            double ql = floor(((double)cmn[a] - (double)nmn[a]) / scale[a]);
-            double qh = ceil(((double)cmx[a] - (double)nmn[a]) / scale[a]);
-            ql = fmin(255.0, fmax(0.0, ql)); qh = fmin(255.0, fmax(0.0, qh));
-            nb[32 + 16 * a + s] = (uint8_t)ql; nb[40 + 16 * a + s] = (uint8_t)qh;
-        }
         const uint32_t cnt = b.count[c];
         if (cnt > max_leaf) {
             imask |= 1u << s;
@@ -844,6 +870,156 @@ __global__ void blas_offsets_kernel(const uint32_t* __restrict__ tlas_prim, uint
     blas_offsets[i] = tlas_prim[i];                   // BLAS k has its root wide node at node index k (forest level 0)
 }
 
+// ---- 5. refit: the same trees, re-encoded tight over moved triangles (tray_cuda_scene_refit) ---------------------------------
+// A topology walk, once per scene, lists the nodes reachable from the roots level by level as (node, tree base) pairs: a
+// child's index is its tree base + child_base_idx + rank (the BLAS root, or tlas_start in the TLAS).  A refit then runs one
+// pass over the triangle slots (records + slot boxes) and one launch per level, deepest first, in which every node takes the
+// union of its slots' boxes and re-encodes p, exponents and the q bytes of its used slots.  Boxes are ordered ints (f2o),
+// min / max are exact, and no two threads write one node: the bytes are the same on every run.
+enum : uint32_t { WALK_LEAF_RANGE = 1u, WALK_CHILD_RANGE = 2u, WALK_TWICE = 4u };
+
+__device__ __forceinline__ uint32_t leaf_count(uint32_t meta) {   // unary triangle count of a leaf slot's meta byte
+    const uint32_t u = meta >> 5;
+    return u == 1u ? 1u : u == 3u ? 2u : u == 7u ? 3u : 0u;
+}
+__device__ __forceinline__ uint32_t node_meta(const uint4& n1, int s) { return ((s < 4 ? n1.z : n1.w) >> (8 * (s & 3))) & 0xffu; }
+
+// the coordinate check of a refit: scan[0] != 0 when a coordinate is not finite; scan[1 + a] / scan[4 + a] the minimum / maximum
+// of axis a over all vertices as ordered ints (their difference tells whether every box extent stays finite)
+__global__ void refit_scan_kernel(const float* __restrict__ tris9, uint64_t n9, int* __restrict__ scan) {
+    bool bad = false;
+    float mn[3] = { 3.4e38f, 3.4e38f, 3.4e38f }, mx[3] = { -3.4e38f, -3.4e38f, -3.4e38f };
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n9; i += (uint64_t)gridDim.x * blockDim.x) {
+        const float v = tris9[i];
+        bad |= !isfinite(v);
+        const int a = (int)(i % 3);
+#pragma unroll
+        for (int b = 0; b < 3; b++)
+            if (a == b) { mn[b] = fminf(mn[b], v); mx[b] = fmaxf(mx[b], v); }
+    }
+    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(scan, 1);
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        float lo = mn[a], hi = mx[a];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) { lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o)); hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o)); }
+        if ((threadIdx.x & 31) == 0) { atomicMin(scan + 1 + a, f2o(lo)); atomicMax(scan + 4 + a, f2o(hi)); }
+    }
+}
+
+__global__ void refit_roots_kernel(const uint2* __restrict__ items, uint32_t begin, uint32_t n, uint32_t* __restrict__ visited,
+                                   uint32_t* __restrict__ err) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && atomicExch(visited + items[begin + i].x, 1u) != 0u) atomicOr(err, WALK_TWICE);
+}
+
+// one level of the walk: checks every leaf range against `leaf_limit` and appends the inner children at `tail`
+__global__ void refit_walk_kernel(const uint4* __restrict__ nodes, uint2* __restrict__ items, uint32_t begin, uint32_t n, uint32_t cap,
+                                  uint64_t child_lo, uint64_t child_hi, uint64_t leaf_limit, uint32_t* __restrict__ tail,
+                                  uint32_t* __restrict__ visited, uint32_t* __restrict__ err) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint2 it = items[begin + i];
+    const uint4 n0 = nodes[5ull * it.x], n1 = nodes[5ull * it.x + 1];
+    const uint32_t imask = n0.w >> 24;
+    for (int s = 0; s < 8; s++) {
+        const uint32_t meta = node_meta(n1, s);
+        if (((imask >> s) & 1u) || meta == 0u) continue;
+        if ((uint64_t)n1.y + (meta & 31u) + leaf_count(meta) > leaf_limit) atomicOr(err, WALK_LEAF_RANGE);
+    }
+    const uint32_t k = __popc(imask);
+    if (!k) return;
+    const uint32_t pos = atomicAdd(tail, k);
+    for (uint32_t r = 0; r < k; r++) {
+        const uint64_t c = (uint64_t)it.y + n1.x + r;
+        if (c < child_lo || c >= child_hi) { atomicOr(err, WALK_CHILD_RANGE); continue; }
+        if (atomicExch(visited + c, 1u) != 0u) { atomicOr(err, WALK_TWICE); continue; }
+        if (pos + r < cap) items[pos + r] = make_uint2((uint32_t)c, it.y);
+        else atomicOr(err, WALK_TWICE);                  // more nodes than the array holds: some node came twice
+    }
+}
+
+// a node that no root reaches keeps its bytes through every refit: whether one of them asks for the exact node test is fixed
+__global__ void refit_unreached_exact_kernel(const uint4* __restrict__ nodes, uint64_t n_nodes, const uint32_t* __restrict__ visited,
+                                             uint32_t* __restrict__ flag) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_nodes || visited[i]) return;
+    const uint32_t e = nodes[5 * i].w;
+    if ((e & 0xffu) >= 167u || ((e >> 8) & 0xffu) >= 167u || ((e >> 16) & 0xffu) >= 167u) atomicOr(flag, 1u);
+}
+
+// records of slot k from triangle prim_indices[k] (k without the map), and the slot's box from the f32 vertices
+template <int STRIDE>
+__global__ void refit_tris_kernel(const float* __restrict__ tris9, uint32_t n, const uint32_t* __restrict__ prim_indices,
+                                  uint8_t* __restrict__ tri_out, int4* __restrict__ slot_box) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const uint32_t prim = prim_indices ? prim_indices[k] : k;
+    write_tri_record<STRIDE>(tris9, prim, tri_out, k);
+    const float* t = tris9 + 9ull * prim;
+    int lo[3], hi[3];
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        lo[a] = f2o(fminf(t[a], fminf(t[3 + a], t[6 + a])));
+        hi[a] = f2o(fmaxf(t[a], fmaxf(t[3 + a], t[6 + a])));
+    }
+    slot_box[2ull * k] = make_int4(lo[0], lo[1], lo[2], 0);
+    slot_box[2ull * k + 1] = make_int4(hi[0], hi[1], hi[2], 0);
+}
+
+// one level: a node's slots are its inner children (boxes of the level below) and its leaves (slot boxes of triangles, or, in
+// the TLAS, the boxes of the BLAS roots behind the instances).  A node with no box under it keeps its bytes.
+template <bool TLAS>
+__global__ void __launch_bounds__(TPB) refit_node_kernel(const uint2* __restrict__ items, uint32_t n, uint4* __restrict__ nodes,
+                                                         int4* __restrict__ node_box, const int4* __restrict__ slot_box,
+                                                         const uint32_t* __restrict__ blas, uint32_t* __restrict__ flag) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint2 it = items[i];
+    uint4* nd = nodes + 5ull * it.x;
+    uint32_t w[20];
+#pragma unroll
+    for (int q = 0; q < 5; q++) { const uint4 v = nd[q]; w[4 * q] = v.x; w[4 * q + 1] = v.y; w[4 * q + 2] = v.z; w[4 * q + 3] = v.w; }
+    const uint4 n1 = make_uint4(w[4], w[5], w[6], w[7]);
+    const uint32_t imask = w[3] >> 24;
+    int blo[8][3], bhi[8][3];
+    int nlo[3] = { INT_MAX, INT_MAX, INT_MAX }, nhi[3] = { INT_MIN, INT_MIN, INT_MIN };
+    uint32_t used = 0;
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        const uint32_t meta = node_meta(n1, s);
+#pragma unroll
+        for (int a = 0; a < 3; a++) { blo[s][a] = INT_MAX; bhi[s][a] = INT_MIN; }
+        if ((imask >> s) & 1u) {
+            const uint64_t c = (uint64_t)it.y + n1.x + __popc(imask & ((1u << s) - 1u));
+            const int4 l = node_box[2 * c], h = node_box[2 * c + 1];
+            blo[s][0] = l.x; blo[s][1] = l.y; blo[s][2] = l.z; bhi[s][0] = h.x; bhi[s][1] = h.y; bhi[s][2] = h.z;
+        } else if (meta != 0u) {
+            const uint32_t first = n1.y + (meta & 31u), cnt = leaf_count(meta);
+            for (uint32_t j = 0; j < cnt; j++) {
+                const uint64_t b = TLAS ? 2ull * blas[first + j] : 2ull * (first + j);
+                const int4 l = TLAS ? node_box[b] : slot_box[b], h = TLAS ? node_box[b + 1] : slot_box[b + 1];
+                blo[s][0] = min(blo[s][0], l.x); blo[s][1] = min(blo[s][1], l.y); blo[s][2] = min(blo[s][2], l.z);
+                bhi[s][0] = max(bhi[s][0], h.x); bhi[s][1] = max(bhi[s][1], h.y); bhi[s][2] = max(bhi[s][2], h.z);
+            }
+        }
+        if (meta != 0u) used |= 1u << s;
+#pragma unroll
+        for (int a = 0; a < 3; a++) { nlo[a] = min(nlo[a], blo[s][a]); nhi[a] = max(nhi[a], bhi[s][a]); }
+    }
+    node_box[2ull * it.x] = make_int4(nlo[0], nlo[1], nlo[2], 0);
+    node_box[2ull * it.x + 1] = make_int4(nhi[0], nhi[1], nhi[2], 0);
+    if (nlo[0] > nhi[0]) return;
+    const float nmn[3] = { o2f(nlo[0]), o2f(nlo[1]), o2f(nlo[2]) }, nmx[3] = { o2f(nhi[0]), o2f(nhi[1]), o2f(nhi[2]) };
+    const bool exact = encode_bounds(w, nmn, nmx, used, [&](int s, float cmn[3], float cmx[3]) {
+#pragma unroll
+        for (int a = 0; a < 3; a++) { cmn[a] = o2f(blo[s][a]); cmx[a] = o2f(bhi[s][a]); }
+    });
+    if (exact) atomicOr(flag, 1u);
+#pragma unroll
+    for (int q = 0; q < 5; q++) nd[q] = make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
+}
+
 }  // namespace
 
 int build(const float* tris9_host, uint64_t n_tris, uint32_t tri_stride, uint32_t max_leaf, uint32_t radius, cudaStream_t st,
@@ -945,6 +1121,155 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     out->stats.ms_ploc = (float)(t_ploc - t_upload); out->stats.ms_collapse = (float)(t_end - t_opt); out->stats.ms_total = (float)(t_end - t_begin);
     out->stats.ms_reinsert = (float)(t_opt - t_ploc); out->stats.reinsert_passes = os.passes; out->stats.reinsert_moves = os.moves;
     out->stats.sah_before = (float)os.cost_before; out->stats.sah_after = (float)os.cost_after;
+    return 0;
+}
+
+void refit_free(RefitTopology* t) {
+    cudaFree(t->d_items); cudaFree(t->d_node_box); cudaFree(t->d_slot_box); cudaFree(t->d_flag);
+    *t = RefitTopology();
+}
+
+int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uint32_t* d_blas, uint32_t n_instances, uint32_t tlas_start,
+               cudaStream_t st, RefitTopology* out, char* err, size_t errlen) {
+    RefitTopology t;
+    auto fail = [&](int code) { refit_free(&t); return code; };
+    // roots: node 0, or the distinct blas_offsets (a BLAS shared by two instances is one tree) and then the TLAS
+    std::vector<uint32_t> roots;
+    if (n_instances) {
+        roots.resize(n_instances);
+        if (cudaMemcpy(roots.data(), d_blas, (size_t)n_instances * 4, cudaMemcpyDeviceToHost) != cudaSuccess) {
+            snprintf(err, errlen, "blas_offsets download failed"); cudaGetLastError(); return -2;
+        }
+        std::sort(roots.begin(), roots.end());
+        roots.erase(std::unique(roots.begin(), roots.end()), roots.end());
+        if (roots.back() >= n_nodes) { snprintf(err, errlen, "blas_offsets entry %u outside %llu nodes", roots.back(), (unsigned long long)n_nodes); return -1; }
+    } else if (n_nodes) {
+        roots.push_back(0u);
+    }
+    uint32_t* visited = nullptr;
+    uint32_t* d_walk = nullptr;                       // [0] tail, [1] error bits
+    auto walk_fail = [&](int code) { cudaFree(visited); cudaFree(d_walk); return fail(code); };
+#define WCU(call)                                                                                                  \
+    do {                                                                                                           \
+        cudaError_t e_ = (call);                                                                                   \
+        if (e_ != cudaSuccess) {                                                                                   \
+            snprintf(err, errlen, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__);     \
+            return walk_fail(-2);                                                                                  \
+        }                                                                                                          \
+    } while (0)
+    const uint64_t cap = n_nodes ? n_nodes : 1;
+    WCU(cudaMalloc(&t.d_items, cap * sizeof(uint2)));
+    WCU(cudaMalloc(&t.d_node_box, cap * 2 * sizeof(int4)));
+    WCU(cudaMalloc(&t.d_slot_box, (n_tris ? n_tris : 1) * 2 * sizeof(int4)));
+    WCU(cudaMalloc(&t.d_flag, 7 * 4));                // the level flag; the coordinate check's 7 words
+    WCU(cudaMalloc(&visited, cap * 4));
+    WCU(cudaMalloc(&d_walk, 8));
+    WCU(cudaMemsetAsync(visited, 0, cap * 4, st));
+    WCU(cudaMemsetAsync(d_walk, 0, 8, st));
+    const uint4* nodes = static_cast<const uint4*>(d_nodes);
+    uint32_t tail = 0;
+    t.level_off.push_back(0);
+    // one tree part: its roots become a level, then level after level until one adds no node
+    auto walk = [&](const std::vector<uint2>& part_roots, uint64_t child_lo, uint64_t leaf_limit) -> int {
+        if (part_roots.empty()) return 0;
+        // the `tail` nodes listed so far are distinct: a part whose roots do not fit next to them repeats one (e.g. a
+        // blas_offsets entry equal to tlas_start).  Refused here, before its roots are written to the list.
+        if ((uint64_t)tail + part_roots.size() > cap) {
+            snprintf(err, errlen, "the tree cannot be refit: a node is reached twice");
+            return walk_fail(-1);
+        }
+        WCU(cudaMemcpyAsync(t.d_items + tail, part_roots.data(), part_roots.size() * sizeof(uint2), cudaMemcpyHostToDevice, st));
+        refit_roots_kernel<<<blocks(part_roots.size()), TPB, 0, st>>>(t.d_items, tail, (uint32_t)part_roots.size(), visited, d_walk + 1);
+        tail += (uint32_t)part_roots.size();
+        WCU(cudaMemcpyAsync(d_walk, &tail, 4, cudaMemcpyHostToDevice, st));
+        t.level_off.push_back(tail);
+        for (;;) {
+            const uint32_t begin = t.level_off[t.level_off.size() - 2], n = tail - begin;
+            refit_walk_kernel<<<blocks(n), TPB, 0, st>>>(nodes, t.d_items, begin, n, (uint32_t)cap, child_lo, n_nodes, leaf_limit, d_walk,
+                                                         visited, d_walk + 1);
+            uint32_t w[2];
+            WCU(cudaMemcpyAsync(w, d_walk, 8, cudaMemcpyDeviceToHost, st));
+            WCU(cudaStreamSynchronize(st));
+            WCU(cudaGetLastError());
+            if (w[1]) {
+                snprintf(err, errlen, "the tree cannot be refit: %s", (w[1] & WALK_TWICE) ? "a node is reached twice"
+                         : (w[1] & WALK_CHILD_RANGE) ? "a child index is outside the node array" : "a leaf range is outside its array");
+                return walk_fail(-1);
+            }
+            if (w[0] == tail) return 0;
+            tail = w[0];
+            t.level_off.push_back(tail);
+        }
+    };
+    std::vector<uint2> part;
+    for (uint32_t r : roots) part.push_back(make_uint2(r, r));
+    if (const int rc = walk(part, 0, n_tris)) return rc;
+    t.n_blas_levels = (uint32_t)t.level_off.size() - 1;
+    if (n_instances) {
+        part.assign(1, make_uint2(tlas_start, tlas_start));
+        if (const int rc = walk(part, tlas_start, n_instances)) return rc;
+    }
+    WCU(cudaMemsetAsync(t.d_flag, 0, 4, st));
+    if (n_nodes) refit_unreached_exact_kernel<<<blocks(n_nodes), TPB, 0, st>>>(nodes, n_nodes, visited, t.d_flag);
+    uint32_t f = 0;
+    WCU(cudaMemcpyAsync(&f, t.d_flag, 4, cudaMemcpyDeviceToHost, st));
+    WCU(cudaStreamSynchronize(st));
+    WCU(cudaGetLastError());
+#undef WCU
+    cudaFree(visited); cudaFree(d_walk);
+    t.unreached_exact = f != 0;
+    t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4;
+    *out = t;
+    return 0;
+}
+
+int refit_check(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, cudaStream_t st, bool* bad, char* err, size_t errlen) {
+    // flag 0; minima +max, maxima -max (ordered)
+    const int init[7] = { 0, 0x7f7fffff, 0x7f7fffff, 0x7f7fffff, (int)0x80800000, (int)0x80800000, (int)0x80800000 };
+    int scan[7];
+    BCU(cudaMemcpyAsync(t.d_flag, init, sizeof init, cudaMemcpyHostToDevice, st));
+    if (n_tris) refit_scan_kernel<<<blocks(n_tris * 9 < (1ull << 24) ? n_tris * 9 : (1ull << 24)), TPB, 0, st>>>(d_tris9, n_tris * 9,
+                                                                                                                  reinterpret_cast<int*>(t.d_flag));
+    BCU(cudaMemcpyAsync(scan, t.d_flag, sizeof scan, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    BCU(cudaGetLastError());
+    *bad = scan[0] != 0;
+    // every node box lies inside the vertices' bounds: if their extent is finite on every axis, so is every extent the encoder sees
+    for (int a = 0; a < 3 && n_tris && !*bad; a++) {
+        auto o2f_host = [](int i) { i = i >= 0 ? i : i ^ 0x7fffffff; float f; memcpy(&f, &i, 4); return f; };
+        const float ext = o2f_host(scan[4 + a]) - o2f_host(scan[1 + a]);
+        *bad = !std::isfinite(ext);
+    }
+    return 0;
+}
+
+int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, const uint32_t* d_prim_indices, uint32_t tri_stride,
+              void* d_nodes, void* d_tris, const uint32_t* d_blas, cudaStream_t st, bool* exact, char* err, size_t errlen) {
+    const uint32_t n = (uint32_t)n_tris;
+    uint8_t* tri_out = static_cast<uint8_t*>(d_tris);
+    BCU(cudaMemsetAsync(t.d_flag, 0, 4, st));
+    if (n) {
+#define TRIS(S) refit_tris_kernel<S><<<blocks(n), TPB, 0, st>>>(d_tris9, n, d_prim_indices, tri_out, t.d_slot_box)
+        if (tri_stride == 64) TRIS(64); else if (tri_stride == 24) TRIS(24); else TRIS(48);
+#undef TRIS
+    }
+    uint4* nodes = static_cast<uint4*>(d_nodes);
+    const uint32_t n_levels = (uint32_t)t.level_off.size() - 1;
+    // BLAS (or flat) levels deepest first, then the TLAS over the BLAS roots' boxes
+    for (uint32_t part = 0; part < 2; part++) {
+        const uint32_t first = part == 0 ? 0 : t.n_blas_levels, last = part == 0 ? t.n_blas_levels : n_levels;
+        for (uint32_t L = last; L-- > first;) {
+            const uint32_t begin = t.level_off[L], cnt = t.level_off[L + 1] - begin;
+            if (part == 0) refit_node_kernel<false><<<blocks(cnt), TPB, 0, st>>>(t.d_items + begin, cnt, nodes, t.d_node_box, t.d_slot_box, d_blas, t.d_flag);
+            else refit_node_kernel<true><<<blocks(cnt), TPB, 0, st>>>(t.d_items + begin, cnt, nodes, t.d_node_box, t.d_slot_box, d_blas, t.d_flag);
+        }
+    }
+    BCU(cudaGetLastError());
+    uint32_t f = 0;
+    BCU(cudaMemcpyAsync(&f, t.d_flag, 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    BCU(cudaGetLastError());
+    *exact = f != 0 || t.unreached_exact;
     return 0;
 }
 

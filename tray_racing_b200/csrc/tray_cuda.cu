@@ -80,6 +80,7 @@ struct tray_scene {
     uint4* d_tris = nullptr;
     uint32_t* d_blas = nullptr;
     uint32_t* d_prim_indices = nullptr;      // BVH slot -> input triangle (scenes made by tray_cuda_scene_build)
+    tray_build::RefitTopology* refit = nullptr;   // the topology walk of the first tray_cuda_scene_refit, kept for the next
     uint32_t* d_geom_offsets = nullptr; uint32_t n_geometries = 0;   // first global triangle of BLAS / object g (tray_cuda_scene_set_geometry_offsets)
     unsigned long long* d_cursor = nullptr;     // cursor block of batch traces (tray::CURSOR_WORDS)
     // device error words (TraceParams::overflow): [0] batch traces, [1 + k] the launches of frame slot k — one word per slot, so
@@ -411,6 +412,7 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     if (s->stream) cudaStreamSynchronize(s->stream);
     cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
     cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_costs); cudaFree(s->d_geom_offsets);
+    if (s->refit) { tray_build::refit_free(s->refit); delete s->refit; }
     free_pipeline(s);
     cudaFree(s->d_untiled);
     for (auto& f : s->slot) {
@@ -614,6 +616,12 @@ int tray_cuda_scene_info(const tray_scene* s, tray_scene_info* o) {
     return TRAY_OK;
 }
 
+int tray_cuda_scene_exact_node_test(const tray_scene* s, int* out_exact) {
+    if (!s || !out_exact) return fail(TRAY_ERR_ARG, "NULL argument");
+    *out_exact = s->force_exact ? 1 : 0;
+    return TRAY_OK;
+}
+
 int tray_cuda_set_counting(tray_scene* s, int enabled) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     s->counting = enabled != 0;
@@ -737,6 +745,74 @@ int tray_cuda_sync(tray_scene* s) {
     for (int k = 0; k <= TRAY_MAX_FRAMES_IN_FLIGHT; k++)
         if (f[k]) { all |= f[k]; cudaMemsetAsync(s->d_overflow + k, 0, 4, k ? slot_stream(s, k - 1) : s->stream); }
     return flag_status(all);
+}
+
+}  // extern "C"
+
+namespace {
+// tray_cuda_scene_refit(_device): `tris9` is host memory unless `device_ptr`.  Every check runs before the first write, so a
+// refused call leaves nodes, records and force_exact as they were.
+int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_ptr, void* stream, float* ms_refit) {
+    if (ms_refit) *ms_refit = 0.f;
+    if (!s || !tris9) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (n_tris != s->n_tris) return fail(TRAY_ERR_ARG, "refit with %llu triangles, the scene has %llu", (unsigned long long)n_tris, (unsigned long long)s->n_tris);
+    CU(cudaSetDevice(s->device));
+    // after every frame and batch enqueued so far: frames rendered before the refit keep their old-geometry results
+    if (stream) CU(cudaStreamSynchronize((cudaStream_t)stream));
+    if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
+    CU(cudaStreamSynchronize(s->copy_stream));
+    if (s->pipeline_ready) { CU(cudaStreamSynchronize(s->s_in)); CU(cudaStreamSynchronize(s->s_out)); }
+    if (n_tris == 0) return TRAY_OK;
+    char msg[400] = "";
+    if (!s->refit) {
+        tray_build::RefitTopology t;
+        const int rc = tray_build::refit_walk(s->d_nodes, s->n_nodes, s->n_tris, s->tlas ? s->d_blas : nullptr, s->tlas ? s->n_instances : 0u,
+                                              s->tlas_start, s->stream, &t, msg, sizeof msg);
+        if (rc) return fail(rc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "refit: %s", msg);
+        s->refit = new (std::nothrow) tray_build::RefitTopology(t);
+        if (!s->refit) { tray_build::refit_free(&t); return fail(TRAY_ERR_ARG, "out of host memory"); }
+        s->device_bytes += t.bytes;
+    }
+    const float* d_tris9 = tris9;
+    float* d_upload = nullptr;
+    if (!device_ptr) {
+        CU(cudaMalloc(&d_upload, (size_t)n_tris * 36));
+        const cudaError_t e = tray::upload_pipelined(d_upload, tris9, (size_t)n_tris * 36, s->stream);
+        if (e != cudaSuccess) { cudaFree(d_upload); return fail(TRAY_ERR_CUDA, "refit upload failed: %s", cudaGetErrorString(e)); }
+        d_tris9 = d_upload;
+    }
+    auto body = [&]() -> int {
+        float ms_check = 0.f, ms_run = 0.f;
+        bool bad = false, exact = false;
+        CU(cudaEventRecord(s->ev[0], s->stream));
+        if (tray_build::refit_check(*s->refit, d_tris9, n_tris, s->stream, &bad, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+        CU(cudaEventRecord(s->ev[1], s->stream));
+        CU(cudaEventSynchronize(s->ev[1]));
+        CU(cudaEventElapsedTime(&ms_check, s->ev[0], s->ev[1]));
+        if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
+        CU(cudaEventRecord(s->ev[0], s->stream));
+        if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, s->d_nodes, s->d_tris, s->d_blas, s->stream,
+                                  &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+        CU(cudaEventRecord(s->ev[1], s->stream));
+        CU(cudaEventSynchronize(s->ev[1]));
+        CU(cudaEventElapsedTime(&ms_run, s->ev[0], s->ev[1]));
+        s->force_exact = env_int("TRAY_CUDA_FORCE_EXACT", 0) != 0 || exact;      // as scene creation decides it
+        if (ms_refit) *ms_refit = ms_check + ms_run;
+        return TRAY_OK;
+    };
+    const int rc = body();
+    cudaFree(d_upload);
+    return rc;
+}
+}  // namespace
+
+extern "C" {
+
+int tray_cuda_scene_refit(tray_scene* s, const float* tris9, uint64_t n_tris, float* ms_refit) {
+    return refit_impl(s, tris9, n_tris, false, nullptr, ms_refit);
+}
+int tray_cuda_scene_refit_device(tray_scene* s, const float* d_tris9, uint64_t n_tris, void* stream, float* ms_refit) {
+    return refit_impl(s, d_tris9, n_tris, true, stream, ms_refit);
 }
 
 }  // extern "C"

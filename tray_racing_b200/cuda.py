@@ -33,6 +33,7 @@ EXPORTS = (
     "tray_cuda_group_readback_begin", "tray_cuda_group_readback_wait", "tray_cuda_group_frame_ptr", "tray_cuda_group_sync",
     "tray_cuda_start_multi",
     "tray_cuda_trace_cost", "tray_cuda_trace_cost_device", "tray_cuda_scene_set_ray_cost", "tray_cuda_frame_download_cost",
+    "tray_cuda_scene_refit", "tray_cuda_scene_refit_device", "tray_cuda_scene_exact_node_test",
 )
 # semantic switches of tray_cuda_scene_set_variant (include/tray_cuda.h TRAY_VARIANT_*)
 VARIANT_BOX_DIVIDE, VARIANT_TIE_LAST, VARIANT_BOX_TMIN_RAY, VARIANT_ZERODIR_BOX_ONLY = 1, 2, 4, 8
@@ -215,6 +216,12 @@ def lib() -> C.CDLL:
         L.tray_cuda_start_multi.restype = i32
         L.tray_cuda_start_multi.argtypes = [vp, i32, vp, u64, vp, u64, vp, u64, u32, u32, i32, C.POINTER(TrayView), u32, u32,
                                             C.c_float, i32, i32, f32p, f32p, C.POINTER(u32)]
+        L.tray_cuda_scene_refit.restype = i32
+        L.tray_cuda_scene_refit.argtypes = [vp, vp, u64, f32p]
+        L.tray_cuda_scene_refit_device.restype = i32
+        L.tray_cuda_scene_refit_device.argtypes = [vp, vp, u64, vp, f32p]
+        L.tray_cuda_scene_exact_node_test.restype = i32
+        L.tray_cuda_scene_exact_node_test.argtypes = [vp, C.POINTER(i32)]
         _lib = L
     return _lib
 
@@ -334,6 +341,28 @@ class TrayCudaScene:
         if out.size:
             _check(lib().tray_cuda_scene_download_instances(self._h, out.ctypes.data))
         return out
+
+    def exact_node_test(self) -> bool:
+        """Whether traversal takes the unfused node test everywhere (a node scale >= 2^40, or TRAY_CUDA_FORCE_EXACT)."""
+        e = C.c_int()
+        _check(lib().tray_cuda_scene_exact_node_test(self._h, C.byref(e)))
+        return bool(e.value)
+
+    def refit(self, tris, timings: dict | None = None):
+        """Same tree, new vertex positions: `tris` (n x 3 x 3 or n x 9 float32) in the scene's triangle order — input order for
+        a built scene, BVH slot order for one made from bytes (tray_cuda_scene_refit).  timings["ms_refit"]: the refit launches."""
+        t = np.ascontiguousarray(tris, dtype=np.float32).reshape(-1, 9)
+        ms = C.c_float()
+        _check(lib().tray_cuda_scene_refit(self._h, t.ctypes.data, t.shape[0], C.byref(ms)))
+        if timings is not None:
+            timings["ms_refit"] = ms.value
+
+    def refit_device(self, d_ptr: int, n: int, stream: int = 0, timed: bool = False):
+        """refit() from n x 9 float32 in device memory, after the work enqueued so far on `stream` (tray_cuda_scene_refit_device);
+        returns ms_refit when `timed`."""
+        ms = C.c_float()
+        _check(lib().tray_cuda_scene_refit_device(self._h, d_ptr, n, stream or None, C.byref(ms) if timed else None))
+        return ms.value if timed else None
 
     @classmethod
     def from_packed(cls, p, device=0) -> "TrayCudaScene":

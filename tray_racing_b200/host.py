@@ -273,3 +273,23 @@ def tri_records(tris: np.ndarray, stride: int = 48) -> np.ndarray:
         rec[:, 13] = e1[:, 2] * e2[:, 0] - e1[:, 0] * e2[:, 2]
         rec[:, 14] = e1[:, 0] * e2[:, 1] - e1[:, 1] * e2[:, 0]
     return rec.view(np.uint8).reshape(-1)
+
+
+def jitter(tris: np.ndarray, seed: int, frac: float = 0.01) -> np.ndarray:
+    """(n, 3, 3) float32: every vertex moved by up to `frac` of the mean triangle size (a small deformation, as a skinned or
+    simulated mesh moves between two frames)"""
+    t = np.asarray(tris, np.float32).reshape(-1, 3, 3)
+    size = float(np.mean(np.linalg.norm(t.max(axis=1) - t.min(axis=1), axis=1)))
+    rng = np.random.default_rng(seed)
+    return (t + rng.uniform(-frac * size, frac * size, t.shape).astype(np.float32)).astype(np.float32)
+
+
+def rigid(tris: np.ndarray, object_offsets, seed: int, frac: float = 0.05) -> np.ndarray:
+    """(n, 3, 3) float32: object k (triangles object_offsets[k] .. [k + 1]) translated as a whole by up to `frac` of the scene's
+    extent"""
+    t = np.asarray(tris, np.float32).reshape(-1, 3, 3)
+    offs = np.asarray(object_offsets, np.int64)
+    ext = float((t.reshape(-1, 3).max(axis=0) - t.reshape(-1, 3).min(axis=0)).max())
+    rng = np.random.default_rng(seed)
+    shift = rng.uniform(-frac * ext, frac * ext, (offs.size - 1, 3)).astype(np.float32)
+    return (t + np.repeat(shift, np.diff(offs), axis=0)[:, None, :]).astype(np.float32)
