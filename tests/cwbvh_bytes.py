@@ -21,7 +21,7 @@ import numpy as np
 import oracle_binding as ob
 from tray_racing_b200 import cuda, host
 
-EXACT_EXP_BYTE = 167                  # traverse.cuh: an exponent byte >= 167 sends the scene to the unfused node test
+EXACT_EXP_BYTE = 167                  # build_gpu.h: an exponent byte >= 167 sends the scene to the unfused node test
 POISON_SPAN = 100.0                   # half-size of a poison triangle (scenes live in [-1, 1]^3; f16 edges stay finite)
 POISON_BOX = float(2 ** 12)           # poison nodes cover [-POISON_BOX, POISON_BOX]^3
 

@@ -1,10 +1,11 @@
 // device_probe.cu — batch entry points onto the traversal's device primitives, one thread per case.  TEST INFRASTRUCTURE ONLY:
 // built by `make -C tray_racing_b200/csrc probe` into libtray_probe.so, loaded by tests/test_device_primitives.py, never linked by
-// the product.  Every kernel calls the product's own tray:: functions from traverse.cuh (no copies), with k4b, zero and one passed
-// at run time as TraceParams passes them.  The host wrappers take host arrays, copy them to the device, launch, copy the results
-// back and return a cudaError_t (0 = success).
+// the product.  Every kernel calls the product's own tray:: functions from traverse.cuh and build_gpu.h (no copies), with k4b, zero
+// and one passed at run time as TraceParams passes them.  The host wrappers take host arrays, copy them to the device, launch, copy
+// the results back and return a cudaError_t (0 = success).
 #include <cstring>
 
+#include "build_gpu.h"
 #include "traverse.cuh"
 
 namespace {

@@ -542,6 +542,37 @@ def test_refusals_change_nothing(cornell, kind):
 
 
 @gpu
+def test_refused_walks_release_their_device_memory():
+    """A topology walk that refuses a tree frees what it allocated: ten refusals of a builder tree of 200k triangles in which a
+    node is reached twice take no more free device memory than the buffers of one walk."""
+    import torch
+    tris = soup(200000, seed=83)
+    built = cuda.TrayCudaScene.build(tris)
+    nodes, rec, _ = built.download_bvh(prim_indices=False)
+    built.close()
+    nodes = nodes.reshape(-1, 80).copy()
+    assert nodes[1, 15] != 0                      # node 1 (a child of the root) has inner children
+    nodes[1, 16:20] = 0                           # ... whose block now starts at node 0: the root is reached twice
+    n_nodes, n_tris = nodes.shape[0], tris.shape[0]
+    # one walk's buffers: per node its entry (8 B), its box (32 B) and its visited word (4 B); per triangle slot a box (32 B); the
+    # flag and check words (28 B) and the walk's tail / error words (8 B); each rounded up to the 2 MiB pages device memory is mapped in
+    page = 2 << 20
+    walk_bytes = sum(-(-b // page) * page for b in (n_nodes * 8, n_nodes * 32, n_nodes * 4, n_tris * 32, 28, 8))
+    sc = cuda.TrayCudaScene(nodes, rec, 48)
+    try:
+        with pytest.raises(cuda.TrayCudaError, match="error -1"):
+            sc.refit(tris)                        # loads the walk's kernels before anything is measured
+        torch.cuda.synchronize()
+        free = torch.cuda.mem_get_info()[0]
+        for _ in range(10):
+            with pytest.raises(cuda.TrayCudaError, match="error -1"):
+                sc.refit(tris)
+        assert free - torch.cuda.mem_get_info()[0] <= walk_bytes
+    finally:
+        sc.close()
+
+
+@gpu
 def test_large_coordinates_refit_while_every_extent_is_finite(cornell):
     """a coordinate near the top of the f32 range is taken as long as the extent on its axis stays finite"""
     p = host.PackedScene(cornell)

@@ -30,6 +30,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <utility>
 
 #include "build_gpu.h"
 #include "host_copy.h"
@@ -43,6 +44,7 @@ namespace {
         cudaError_t e_ = (call);                                                                                   \
         if (e_ != cudaSuccess) {                                                                                   \
             snprintf(err, errlen, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__);     \
+            cudaGetLastError();                                                                                    \
             return -2;                                                                                             \
         }                                                                                                          \
     } while (0)
@@ -57,8 +59,26 @@ inline unsigned blocks(uint64_t n) { return (unsigned)((n + TPB - 1) / TPB); }
 // rule, and the host producer (host/cwbvh_build.cpp) follows it.
 
 // ---- ordered-int float atomics ------------------------------------------------------------------------------
-__device__ __forceinline__ int f2o(float f) { int i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
-__device__ __forceinline__ float o2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
+__host__ __device__ __forceinline__ int f2o(float f) { int i; memcpy(&i, &f, 4); return i >= 0 ? i : i ^ 0x7fffffff; }
+__host__ __device__ __forceinline__ float o2f(int i) { i = i >= 0 ? i : i ^ 0x7fffffff; float f; memcpy(&f, &i, 4); return f; }
+// bounds before the first box: minima +max, maxima -max (ordered)
+constexpr int EMPTY_BOUNDS[6] = { 0x7f7fffff, 0x7f7fffff, 0x7f7fffff, (int)0x80800000, (int)0x80800000, (int)0x80800000 };
+
+// the warp's minimum of mn and maximum of mx per axis, merged into lo[0..2] / hi[0..2] by one ordered-int atomic per warp
+__device__ __forceinline__ void warp_bounds(const float mn[3], const float mx[3], int* lo, int* hi) {
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        float l = mn[a], h = mx[a];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) { l = fminf(l, __shfl_xor_sync(0xffffffffu, l, o)); h = fmaxf(h, __shfl_xor_sync(0xffffffffu, h, o)); }
+        if ((threadIdx.x & 31) == 0) { atomicMin(lo + a, f2o(l)); atomicMax(hi + a, f2o(h)); }
+    }
+}
+
+__device__ __forceinline__ void tri_box(const float* t, float mn[3], float mx[3]) {
+#pragma unroll
+    for (int a = 0; a < 3; a++) { mn[a] = fminf(t[a], fminf(t[3 + a], t[6 + a])); mx[a] = fmaxf(t[a], fmaxf(t[3 + a], t[6 + a])); }
+}
 
 // BVH2 node: lo = (min.xyz, left), hi = (max.xyz, right).  Leaf i (< n_prims): left = -1, right = primitive index.
 struct Bvh2 {
@@ -70,18 +90,23 @@ __device__ __forceinline__ float half_area(const float4& lo, const float4& hi) {
     const float dx = hi.x - lo.x, dy = hi.y - lo.y, dz = hi.z - lo.z;
     return dx * dy + dy * dz + dz * dx;
 }
+__device__ __forceinline__ float union_area(const float4& alo, const float4& ahi, const float4& blo, const float4& bhi) {
+    const float dx = fmaxf(ahi.x, bhi.x) - fminf(alo.x, blo.x), dy = fmaxf(ahi.y, bhi.y) - fminf(alo.y, blo.y), dz = fmaxf(ahi.z, bhi.z) - fminf(alo.z, blo.z);
+    return dx * dy + dy * dz + dz * dx;
+}
+// inner node `id` over children l and r with boxes (alo, ahi), (blo, bhi): the union of the boxes, the children in w
+__device__ __forceinline__ void write_union(const Bvh2& b, int id, int l, int r, const float4& alo, const float4& ahi, const float4& blo,
+                                            const float4& bhi) {
+    b.lo[id] = make_float4(fminf(alo.x, blo.x), fminf(alo.y, blo.y), fminf(alo.z, blo.z), __int_as_float(l));
+    b.hi[id] = make_float4(fmaxf(ahi.x, bhi.x), fmaxf(ahi.y, bhi.y), fmaxf(ahi.z, bhi.z), __int_as_float(r));
+}
 
 // ---- 1. boxes and scene bounds -----------------------------------------------------------------------------------
 __global__ void tri_boxes_kernel(const float* __restrict__ tris9, uint32_t n, float4* __restrict__ plo, float4* __restrict__ phi) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const float* t = tris9 + 9ull * i;
     float mn[3], mx[3];
-#pragma unroll
-    for (int a = 0; a < 3; a++) {
-        mn[a] = fminf(t[a], fminf(t[3 + a], t[6 + a]));
-        mx[a] = fmaxf(t[a], fmaxf(t[3 + a], t[6 + a]));
-    }
+    tri_box(tris9 + 9ull * i, mn, mx);
     plo[i] = make_float4(mn[0], mn[1], mn[2], 0.f);
     phi[i] = make_float4(mx[0], mx[1], mx[2], 0.f);
 }
@@ -93,13 +118,7 @@ __global__ void box_bounds_kernel(const float4* __restrict__ plo, const float4* 
         const float4 lo = plo[i], hi = phi[i];
         mn[0] = lo.x; mn[1] = lo.y; mn[2] = lo.z; mx[0] = hi.x; mx[1] = hi.y; mx[2] = hi.z;
     }
-#pragma unroll
-    for (int a = 0; a < 3; a++) {
-        float lo = mn[a], hi = mx[a];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) { lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o)); hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o)); }
-        if ((threadIdx.x & 31) == 0) { atomicMin(scene + a, f2o(lo)); atomicMax(scene + 3 + a, f2o(hi)); }
-    }
+    warp_bounds(mn, mx, scene, scene + 3);
 }
 
 __device__ __forceinline__ unsigned long long spread21(unsigned long long v) {
@@ -148,8 +167,38 @@ __global__ void leaf_init_kernel(const float4* __restrict__ plo, const float4* _
 }
 
 // ---- 3. PLOC ----------------------------------------------------------------------------------------------------
-// nearest neighbour of cluster i among positions [i - r, i + r]: smallest half-area of the merged box, ties to the
-// lower position (so that "mutual" is well defined and the build is deterministic)
+// One step, run by the multi-kernel loop and by ploc_tail_kernel alike: nearest neighbours, keep / lead flags, parents.
+// nearest neighbour of position i among positions [i - r, i + r] (box(j, lo, hi) and seg(j) read position j): smallest half-area
+// of the merged box, ties to the lower position (so that "mutual" is well defined and the build is deterministic)
+template <typename Box, typename Seg>
+__device__ __forceinline__ int ploc_nearest(int i, uint32_t m, int r, Box box, Seg seg) {
+    float4 lo, hi, l2, h2;
+    box(i, lo, hi);
+    const uint32_t s = seg(i);
+    float best = 3.4e38f; int best_j = -1;
+    const int j0 = max(0, i - r), j1 = min((int)m - 1, i + r);
+    for (int j = j0; j <= j1; j++) {
+        if (j == i || seg(j) != s) continue;          // clusters of different objects never merge
+        box(j, l2, h2);
+        const float a = union_area(lo, hi, l2, h2);
+        if (a < best) { best = a; best_j = j; }
+    }
+    return best_j;
+}
+__device__ __forceinline__ void ploc_flags(const int* nn, uint32_t i, uint32_t& keep, uint32_t& lead) {
+    const int j = nn[i];
+    const bool mutual = j >= 0 && nn[j] == (int)i;
+    keep = (mutual && (int)i > j) ? 0u : 1u;          // the higher position of a merged pair disappears
+    lead = (mutual && (int)i < j) ? 1u : 0u;          // the lower one creates the parent
+}
+// node `id` over clusters l and r (boxes (alo, ahi), (blo, bhi)); its segment, when there are segments, is that of l: seg[k]
+__device__ __forceinline__ void ploc_parent(const Bvh2& b, uint32_t* node_seg, int id, int l, int r, const float4& alo, const float4& ahi,
+                                            const float4& blo, const float4& bhi, const uint32_t* seg, int k) {
+    write_union(b, id, l, r, alo, ahi, blo, bhi);
+    b.count[id] = b.count[l] + b.count[r];
+    if (node_seg) node_seg[id] = seg[k];
+}
+
 __global__ void __launch_bounds__(TPB) ploc_nn_kernel(const int* __restrict__ cluster, uint32_t m, int r, Bvh2 b, const uint32_t* __restrict__ node_seg,
                                                       int* __restrict__ nn) {
     extern __shared__ float4 s_box[];                 // [(TPB + 2r) x 2] boxes, then [(TPB + 2r)] segments
@@ -166,27 +215,16 @@ __global__ void __launch_bounds__(TPB) ploc_nn_kernel(const int* __restrict__ cl
     __syncthreads();
     const int i = (int)(blockIdx.x * TPB + threadIdx.x);
     if (i >= (int)m) return;
-    const float4 lo = s_box[2 * (threadIdx.x + r)], hi = s_box[2 * (threadIdx.x + r) + 1];
-    const uint32_t seg = s_seg[threadIdx.x + r];
-    float best = 3.4e38f; int best_j = -1;
-    const int j0 = max(0, i - r), j1 = min((int)m - 1, i + r);
-    for (int j = j0; j <= j1; j++) {
-        if (j == i || s_seg[j - base] != seg) continue;      // clusters of different objects never merge
-        const float4 l2 = s_box[2 * (j - base)], h2 = s_box[2 * (j - base) + 1];
-        const float dx = fmaxf(hi.x, h2.x) - fminf(lo.x, l2.x), dy = fmaxf(hi.y, h2.y) - fminf(lo.y, l2.y), dz = fmaxf(hi.z, h2.z) - fminf(lo.z, l2.z);
-        const float a = dx * dy + dy * dz + dz * dx;
-        if (a < best) { best = a; best_j = j; }
-    }
-    nn[i] = best_j;
+    nn[i] = ploc_nearest(i, m, r, [&](int j, float4& lo, float4& hi) { lo = s_box[2 * (j - base)]; hi = s_box[2 * (j - base) + 1]; },
+                         [&](int j) { return s_seg[j - base]; });
 }
 
 __global__ void ploc_flag_kernel(const int* __restrict__ nn, uint32_t m, uint32_t* __restrict__ keep, uint32_t* __restrict__ lead) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= m) return;
-    const int j = nn[i];
-    const bool mutual = j >= 0 && nn[j] == (int)i;
-    keep[i] = (mutual && (int)i > j) ? 0u : 1u;       // the higher position of a merged pair disappears
-    lead[i] = (mutual && (int)i < j) ? 1u : 0u;       // the lower one creates the parent
+    uint32_t k, l;
+    ploc_flags(nn, i, k, l);
+    keep[i] = k; lead[i] = l;
 }
 
 __global__ void ploc_merge_kernel(const int* __restrict__ cluster, const int* __restrict__ nn, uint32_t m, const uint32_t* __restrict__ keep,
@@ -199,10 +237,7 @@ __global__ void ploc_merge_kernel(const int* __restrict__ cluster, const int* __
         const int l = c, rgt = cluster[nn[i]];
         const float4 a0 = b.lo[l], a1 = b.hi[l], b0 = b.lo[rgt], b1 = b.hi[rgt];
         const int id = (int)(next_node + lead_pos[i]);
-        b.lo[id] = make_float4(fminf(a0.x, b0.x), fminf(a0.y, b0.y), fminf(a0.z, b0.z), __int_as_float(l));
-        b.hi[id] = make_float4(fmaxf(a1.x, b1.x), fmaxf(a1.y, b1.y), fmaxf(a1.z, b1.z), __int_as_float(rgt));
-        b.count[id] = b.count[l] + b.count[rgt];
-        if (node_seg) node_seg[id] = node_seg[l];
+        ploc_parent(b, node_seg, id, l, rgt, a0, a1, b0, b1, node_seg, l);
         c = id;
     }
     cluster_out[keep_pos[i]] = c;
@@ -210,8 +245,8 @@ __global__ void ploc_merge_kernel(const int* __restrict__ cluster, const int* __
 
 // The last iterations of a PLOC run work on a handful of clusters each and are pure launch + synchronisation latency
 // (68 iterations for 2.88 M triangles, ~55 of them below a thousand clusters).  Once m <= PLOC_TAIL they all run in ONE block:
-// the same nearest-neighbour rule, the same flags, the same prefix-sum numbering of clusters and new nodes as the
-// three kernels above, so the BVH2 is the one the multi-kernel loop would have produced.
+// the same step, the same prefix-sum numbering of clusters and new nodes as the three kernels above, so the BVH2 is the one
+// the multi-kernel loop would have produced.
 constexpr int PLOC_TAIL = 1024;
 struct PlocTailOut { uint32_t m, next_node, iters, stalled; };
 
@@ -223,6 +258,9 @@ __global__ void __launch_bounds__(PLOC_TAIL) ploc_tail_kernel(int* __restrict__ 
     __shared__ uint32_t s_tot[2];
     typedef cub::BlockScan<uint32_t, PLOC_TAIL> Scan;
     __shared__ typename Scan::TempStorage s_scan;
+    const auto box = [&](int j, float4& lo, float4& hi) {
+        lo = make_float4(s_b[0][j], s_b[1][j], s_b[2][j], 0.f); hi = make_float4(s_b[3][j], s_b[4][j], s_b[5][j], 0.f);
+    };
     const int i = (int)threadIdx.x;
     if (i < (int)m) s_cl[i] = cluster[i];
     __syncthreads();
@@ -234,28 +272,10 @@ __global__ void __launch_bounds__(PLOC_TAIL) ploc_tail_kernel(int* __restrict__ 
             s_seg[i] = node_seg ? node_seg[c] : 0u;
         }
         __syncthreads();
-        if (i < (int)m) {
-            const float3 lo = make_float3(s_b[0][i], s_b[1][i], s_b[2][i]), hi = make_float3(s_b[3][i], s_b[4][i], s_b[5][i]);
-            const uint32_t seg = s_seg[i];
-            float best = 3.4e38f; int best_j = -1;
-            const int j0 = max(0, i - r), j1 = min((int)m - 1, i + r);
-            for (int j = j0; j <= j1; j++) {
-                if (j == i || s_seg[j] != seg) continue;
-                const float dx = fmaxf(hi.x, s_b[3][j]) - fminf(lo.x, s_b[0][j]), dy = fmaxf(hi.y, s_b[4][j]) - fminf(lo.y, s_b[1][j]),
-                            dz = fmaxf(hi.z, s_b[5][j]) - fminf(lo.z, s_b[2][j]);
-                const float a = dx * dy + dy * dz + dz * dx;
-                if (a < best) { best = a; best_j = j; }
-            }
-            s_nn[i] = best_j;
-        }
+        if (i < (int)m) s_nn[i] = ploc_nearest(i, m, r, box, [&](int j) { return s_seg[j]; });
         __syncthreads();
         uint32_t keep = 0, lead = 0;
-        if (i < (int)m) {
-            const int j = s_nn[i];
-            const bool mutual = j >= 0 && s_nn[j] == i;
-            keep = (mutual && i > j) ? 0u : 1u;
-            lead = (mutual && i < j) ? 1u : 0u;
-        }
+        if (i < (int)m) ploc_flags(s_nn, (uint32_t)i, keep, lead);
         uint32_t keep_pos, lead_pos, tot_keep, tot_lead;
         Scan(s_scan).ExclusiveSum(keep, keep_pos, tot_keep);
         __syncthreads();
@@ -263,13 +283,11 @@ __global__ void __launch_bounds__(PLOC_TAIL) ploc_tail_kernel(int* __restrict__ 
         if (i < (int)m && keep) {
             int c = s_cl[i];
             if (lead) {
-                const int l = c, rgt = s_cl[s_nn[i]];
                 const int j = s_nn[i];
                 const int id = (int)(next_node + lead_pos);
-                b.lo[id] = make_float4(fminf(s_b[0][i], s_b[0][j]), fminf(s_b[1][i], s_b[1][j]), fminf(s_b[2][i], s_b[2][j]), __int_as_float(l));
-                b.hi[id] = make_float4(fmaxf(s_b[3][i], s_b[3][j]), fmaxf(s_b[4][i], s_b[4][j]), fmaxf(s_b[5][i], s_b[5][j]), __int_as_float(rgt));
-                b.count[id] = b.count[l] + b.count[rgt];
-                if (node_seg) node_seg[id] = s_seg[i];
+                float4 alo, ahi, blo, bhi;
+                box(i, alo, ahi); box(j, blo, bhi);
+                ploc_parent(b, node_seg, id, c, s_cl[j], alo, ahi, blo, bhi, s_seg, i);
                 c = id;
             }
             s_cl2[keep_pos] = c;
@@ -306,10 +324,6 @@ __global__ void opt_parent_kernel(Bvh2 b, uint32_t first_inner, uint32_t n_nodes
     parent[node_left(b.lo[i])] = (int)i; parent[node_right(b.hi[i])] = (int)i;
 }
 
-__device__ __forceinline__ float union_area(const float4& alo, const float4& ahi, const float4& blo, const float4& bhi) {
-    const float dx = fmaxf(ahi.x, bhi.x) - fminf(alo.x, blo.x), dy = fmaxf(ahi.y, bhi.y) - fminf(alo.y, blo.y), dz = fmaxf(ahi.z, bhi.z) - fminf(alo.z, blo.z);
-    return dx * dy + dy * dz + dz * dx;
-}
 __device__ __forceinline__ int sibling_of(const Bvh2& b, const int* parent, int x) {
     const int p = parent[x];
     const int l = node_left(b.lo[p]);
@@ -462,8 +476,8 @@ __global__ void opt_refit_kernel(Bvh2 b, uint32_t n_leaves, const int* __restric
         const volatile float4* vlo = b.lo; const volatile float4* vhi = b.hi;
         const float lx0 = vlo[l].x, ly0 = vlo[l].y, lz0 = vlo[l].z, lx1 = vhi[l].x, ly1 = vhi[l].y, lz1 = vhi[l].z;
         const float rx0 = vlo[r].x, ry0 = vlo[r].y, rz0 = vlo[r].z, rx1 = vhi[r].x, ry1 = vhi[r].y, rz1 = vhi[r].z;
-        b.lo[x] = make_float4(fminf(lx0, rx0), fminf(ly0, ry0), fminf(lz0, rz0), __int_as_float(l));
-        b.hi[x] = make_float4(fmaxf(lx1, rx1), fmaxf(ly1, ry1), fmaxf(lz1, rz1), __int_as_float(r));
+        write_union(b, x, l, r, make_float4(lx0, ly0, lz0, 0.f), make_float4(lx1, ly1, lz1, 0.f), make_float4(rx0, ry0, rz0, 0.f),
+                    make_float4(rx1, ry1, rz1, 0.f));
         b.count[x] = ((volatile uint32_t*)b.count)[l] + ((volatile uint32_t*)b.count)[r];
         x = parent[x];
     }
@@ -542,7 +556,7 @@ __device__ __forceinline__ bool encode_bounds(uint32_t w[20], const float nmn[3]
         w[a] = __float_as_uint(nmn[a]);
         const int ke = quant_exponent(nmx[a] - nmn[a]);
         nb[12 + a] = (uint8_t)(ke + 127);
-        exact |= ke + 127 >= 167;
+        exact |= ke + 127 >= (int)tray::EXACT_EXP_BYTE;
         scale[a] = ldexp(1.0, ke);
     }
 #pragma unroll
@@ -667,11 +681,11 @@ __global__ void collapse_emit_kernel(const int* __restrict__ items, uint32_t n_i
     for (int q = 0; q < 5; q++) dst[q] = make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
 }
 
-// Device scratch of one build: ONE cudaMalloc (reserve) carved up by a bump allocator — a build makes ~35 allocations, and
-// in a process that already holds a lot of device memory each cudaMalloc / cudaFree costs up to a millisecond.  Requests
+// Device scratch of one build: ONE cudaMalloc (reserve) carved up by a bump allocator — a two-level build makes ~80 allocations,
+// and in a process that already holds a lot of device memory each cudaMalloc / cudaFree costs up to a millisecond.  Requests
 // that do not fit the arena fall back to their own cudaMalloc.  Everything is freed on scope exit.
 struct Scratch {
-    void* p[64]; int n = 0;
+    void* p[128]; int n = 0;
     char* arena = nullptr; size_t cap = 0, used = 0;
     cudaError_t reserve(size_t bytes) {
         if (cudaMalloc((void**)&arena, bytes) != cudaSuccess) { arena = nullptr; cap = 0; cudaGetLastError(); }   // fall back to per-array allocations
@@ -681,13 +695,31 @@ struct Scratch {
     template <typename T> cudaError_t alloc(T** out, size_t bytes) {
         const size_t need = ((bytes ? bytes : 16) + 255) & ~(size_t)255;
         if (arena && used + need <= cap) { *out = (T*)(arena + used); used += need; return cudaSuccess; }
-        if (n >= 64) return cudaErrorMemoryAllocation;
+        if (n >= 128) return cudaErrorMemoryAllocation;
         void* q = nullptr; cudaError_t e = cudaMalloc(&q, need);
         if (e == cudaSuccess) { p[n++] = q; *out = (T*)q; }
         return e;
     }
     ~Scratch() { for (int i = 0; i < n; i++) cudaFree(p[i]); if (arena) cudaFree(arena); }
 };
+
+template <typename T> cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) { T* q = nullptr; const cudaError_t e = cudaMalloc(&q, bytes); p.reset(q); return e; }
+
+// Exclusive sums of the flag arrays a and b over m + 1 entries, entry m zeroed first so that the sum there is the total.
+// `consume` enqueues the work that reads the sums; then tot = the two totals, read back once the stream has drained.
+template <typename F>
+int scan_totals(void* d_tmp, size_t tmp_bytes, uint32_t* a, uint32_t* a_pos, uint32_t* b, uint32_t* b_pos, uint32_t m, cudaStream_t st,
+                F consume, uint32_t tot[2], char* err, size_t errlen) {
+    BCU(cudaMemsetAsync(a + m, 0, 4, st)); BCU(cudaMemsetAsync(b + m, 0, 4, st));
+    BCU(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, a, a_pos, (int)m + 1, st));
+    BCU(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, b, b_pos, (int)m + 1, st));
+    consume();
+    BCU(cudaMemcpyAsync(&tot[0], a_pos + m, 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaMemcpyAsync(&tot[1], b_pos + m, 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    BCU(cudaGetLastError());
+    return 0;
+}
 
 double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
@@ -707,8 +739,7 @@ int ploc_run(Scratch& sc, const float4* plo, const float4* phi, uint32_t n, cons
     BCU(sc.alloc(&keep, (size_t)(n + 1) * 4)); BCU(sc.alloc(&keep_pos, (size_t)(n + 1) * 4));
     BCU(sc.alloc(&lead, (size_t)(n + 1) * 4)); BCU(sc.alloc(&lead_pos, (size_t)(n + 1) * 4));
     if (prim_seg) BCU(sc.alloc(&node_seg, (size_t)2 * n * 4));
-    const int scene_init[6] = { 0x7f7fffff, 0x7f7fffff, 0x7f7fffff, (int)0x80800000, (int)0x80800000, (int)0x80800000 };   // +max x3, -max x3 (ordered)
-    BCU(cudaMemcpyAsync(d_scene, scene_init, sizeof scene_init, cudaMemcpyHostToDevice, st));
+    BCU(cudaMemcpyAsync(d_scene, EMPTY_BOUNDS, sizeof EMPTY_BOUNDS, cudaMemcpyHostToDevice, st));
     box_bounds_kernel<<<blocks(n), TPB, 0, st>>>(plo, phi, n, d_scene);
     morton_kernel<<<blocks(n), TPB, 0, st>>>(plo, phi, n, d_scene, prim_seg, keys, vals);
     size_t tmp_bytes = 0, tmp2 = 0;
@@ -738,16 +769,11 @@ int ploc_run(Scratch& sc, const float4* plo, const float4* phi, uint32_t n, cons
         }
         ploc_nn_kernel<<<blocks(m), TPB, (size_t)(TPB + 2 * r) * 36, st>>>(cl_in, m, r, b, node_seg, nn);
         ploc_flag_kernel<<<blocks(m), TPB, 0, st>>>(nn, m, keep, lead);
-        // scans run over m + 1 entries so that entry m holds the total (the extra input element is never a keeper)
-        BCU(cudaMemsetAsync(keep + m, 0, 4, st)); BCU(cudaMemsetAsync(lead + m, 0, 4, st));
-        BCU(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, keep, keep_pos, (int)m + 1, st));
-        BCU(cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, lead, lead_pos, (int)m + 1, st));
-        ploc_merge_kernel<<<blocks(m), TPB, 0, st>>>(cl_in, nn, m, keep, keep_pos, lead, lead_pos, next_node, b, node_seg, cl_out);
         uint32_t tot[2];
-        BCU(cudaMemcpyAsync(&tot[0], keep_pos + m, 4, cudaMemcpyDeviceToHost, st));
-        BCU(cudaMemcpyAsync(&tot[1], lead_pos + m, 4, cudaMemcpyDeviceToHost, st));
-        BCU(cudaStreamSynchronize(st));
-        BCU(cudaGetLastError());
+        const int rc = scan_totals(d_tmp, tmp_bytes, keep, keep_pos, lead, lead_pos, m, st, [&] {
+            ploc_merge_kernel<<<blocks(m), TPB, 0, st>>>(cl_in, nn, m, keep, keep_pos, lead, lead_pos, next_node, b, node_seg, cl_out);
+        }, tot, err, errlen);
+        if (rc) return rc;
         if (tot[1] == 0) {
             if (prim_seg) break;                      // every segment is down to one cluster
             snprintf(err, errlen, "PLOC made no progress at %u clusters", m); return -3;
@@ -762,15 +788,13 @@ int ploc_run(Scratch& sc, const float4* plo, const float4* phi, uint32_t n, cons
 
 // reinsertion passes over the BVH2 of a PLOC run (3b above); `stats` (optional) receives the SAH cost before / after and the moves
 struct OptStats { double cost_before, cost_after; uint32_t moves, passes; };
-int optimize_run(Scratch& sc, const PlocOut& pl, uint32_t n_leaves, uint32_t passes, uint32_t max_visits, cudaStream_t st, OptStats* stats,
-                 char* err, size_t errlen) {
+int optimize_run(Scratch& sc, const PlocOut& pl, uint32_t n_leaves, uint32_t passes, uint32_t max_visits, uint32_t rounds, cudaStream_t st,
+                 OptStats* stats, char* err, size_t errlen) {
     const uint32_t nn = pl.n_nodes;
     if (stats) memset(stats, 0, sizeof *stats);
     if (passes == 0 || nn <= n_leaves + 2) return 0;
     OptArrays o; o.visits = nullptr;
     uint32_t* arrived; uint32_t* d_count; double* d_cost; uint8_t* drop; uint8_t* dirty;
-    const char* rr_env = getenv("TRAY_CUDA_BUILD_REINSERT_ROUNDS");
-    const uint32_t rounds = rr_env && *rr_env ? (uint32_t)atoi(rr_env) : 3u;
     BCU(sc.alloc(&o.parent, (size_t)nn * 4)); BCU(sc.alloc(&o.gain, (size_t)nn * 4)); BCU(sc.alloc(&o.target, (size_t)nn * 4));
     BCU(sc.alloc(&o.lock, (size_t)nn * 8)); BCU(sc.alloc(&arrived, (size_t)nn * 4));
     BCU(sc.alloc(&d_count, 4)); BCU(sc.alloc(&d_cost, 16)); BCU(sc.alloc(&drop, (size_t)nn)); BCU(sc.alloc(&dirty, (size_t)nn)); BCU(sc.alloc(&o.win, (size_t)nn));
@@ -825,19 +849,15 @@ int collapse_run(Scratch& sc, const PlocOut& pl, uint32_t n_prims, bool forest, 
     while (n_items) {
         if ((uint64_t)level_base + n_items > node_cap) { snprintf(err, errlen, "node count exceeds its bound"); return -3; }
         collapse_count_kernel<<<blocks(n_items), TPB, 0, st>>>(it_in, n_items, pl.b, max_leaf, n_inner, n_tri);
-        BCU(cudaMemsetAsync(n_inner + n_items, 0, 4, st)); BCU(cudaMemsetAsync(n_tri + n_items, 0, 4, st));
-        BCU(cub::DeviceScan::ExclusiveSum(pl.d_tmp, const_cast<size_t&>(pl.tmp_bytes), n_inner, inner_off, (int)n_items + 1, st));
-        BCU(cub::DeviceScan::ExclusiveSum(pl.d_tmp, const_cast<size_t&>(pl.tmp_bytes), n_tri, tri_off, (int)n_items + 1, st));
         const uint32_t next_base = level_base + n_items;
+        uint32_t tot[2];
+        const int rc = scan_totals(pl.d_tmp, pl.tmp_bytes, n_inner, inner_off, n_tri, tri_off, n_items, st, [&] {
 #define EMIT(S) collapse_emit_kernel<S><<<blocks(n_items), TPB, 0, st>>>(it_in, n_items, pl.b, max_leaf, inner_off, tri_off, level_base, next_base, \
                     prim_base, d_tris9, nodes, tri_out, prim_idx, it_out, d_flags, forest ? rt_in : nullptr, forest ? rt_out : nullptr)
-        if (tri_stride == 64) EMIT(64); else if (tri_stride == 24) EMIT(24); else if (tri_stride == 48) EMIT(48); else EMIT(0);
+            if (tri_stride == 64) EMIT(64); else if (tri_stride == 24) EMIT(24); else if (tri_stride == 48) EMIT(48); else EMIT(0);
 #undef EMIT
-        uint32_t tot[2];
-        BCU(cudaMemcpyAsync(&tot[0], inner_off + n_items, 4, cudaMemcpyDeviceToHost, st));
-        BCU(cudaMemcpyAsync(&tot[1], tri_off + n_items, 4, cudaMemcpyDeviceToHost, st));
-        BCU(cudaStreamSynchronize(st));
-        BCU(cudaGetLastError());
+        }, tot, err, errlen);
+        if (rc) return rc;
         level_base = next_base; prim_base += tot[1]; n_items = tot[0]; levels++;
         int* t = it_in; it_in = it_out; it_out = t;
         uint32_t* u = rt_in; rt_in = rt_out; rt_out = u;
@@ -858,16 +878,11 @@ __global__ void seg_of_prims_kernel(const uint64_t* __restrict__ offsets, uint32
     prim_seg[i] = lo;
 }
 
-// boxes of the BLAS roots (TLAS primitives), and which node each object's BLAS starts at
+// boxes of the BLAS roots (TLAS primitives)
 __global__ void blas_boxes_kernel(const int* __restrict__ roots, uint32_t n_obj, Bvh2 b, float4* __restrict__ plo, float4* __restrict__ phi) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_obj) return;
     plo[i] = b.lo[roots[i]]; phi[i] = b.hi[roots[i]];
-}
-__global__ void blas_offsets_kernel(const uint32_t* __restrict__ tlas_prim, uint32_t n_obj, uint32_t* __restrict__ blas_offsets) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_obj) return;
-    blas_offsets[i] = tlas_prim[i];                   // BLAS k has its root wide node at node index k (forest level 0)
 }
 
 // ---- 5. refit: the same trees, re-encoded tight over moved triangles (tray_cuda_scene_refit) ---------------------------------
@@ -898,13 +913,7 @@ __global__ void refit_scan_kernel(const float* __restrict__ tris9, uint64_t n9, 
             if (a == b) { mn[b] = fminf(mn[b], v); mx[b] = fmaxf(mx[b], v); }
     }
     if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(scan, 1);
-#pragma unroll
-    for (int a = 0; a < 3; a++) {
-        float lo = mn[a], hi = mx[a];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) { lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o)); hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o)); }
-        if ((threadIdx.x & 31) == 0) { atomicMin(scan + 1 + a, f2o(lo)); atomicMax(scan + 4 + a, f2o(hi)); }
-    }
+    warp_bounds(mn, mx, scan + 1, scan + 4);
 }
 
 __global__ void refit_roots_kernel(const uint2* __restrict__ items, uint32_t begin, uint32_t n, uint32_t* __restrict__ visited,
@@ -944,8 +953,7 @@ __global__ void refit_unreached_exact_kernel(const uint4* __restrict__ nodes, ui
                                              uint32_t* __restrict__ flag) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_nodes || visited[i]) return;
-    const uint32_t e = nodes[5 * i].w;
-    if ((e & 0xffu) >= 167u || ((e >> 8) & 0xffu) >= 167u || ((e >> 16) & 0xffu) >= 167u) atomicOr(flag, 1u);
+    if (tray::node_needs_exact(nodes[5 * i].w)) atomicOr(flag, 1u);
 }
 
 // records of slot k from triangle prim_indices[k] (k without the map), and the slot's box from the f32 vertices
@@ -956,13 +964,11 @@ __global__ void refit_tris_kernel(const float* __restrict__ tris9, uint32_t n, c
     if (k >= n) return;
     const uint32_t prim = prim_indices ? prim_indices[k] : k;
     write_tri_record<STRIDE>(tris9, prim, tri_out, k);
-    const float* t = tris9 + 9ull * prim;
+    float mn[3], mx[3];
+    tri_box(tris9 + 9ull * prim, mn, mx);
     int lo[3], hi[3];
 #pragma unroll
-    for (int a = 0; a < 3; a++) {
-        lo[a] = f2o(fminf(t[a], fminf(t[3 + a], t[6 + a])));
-        hi[a] = f2o(fmaxf(t[a], fmaxf(t[3 + a], t[6 + a])));
-    }
+    for (int a = 0; a < 3; a++) { lo[a] = f2o(mn[a]); hi[a] = f2o(mx[a]); }
     slot_box[2ull * k] = make_int4(lo[0], lo[1], lo[2], 0);
     slot_box[2ull * k + 1] = make_int4(hi[0], hi[1], hi[2], 0);
 }
@@ -1022,11 +1028,6 @@ __global__ void __launch_bounds__(TPB) refit_node_kernel(const uint2* __restrict
 
 }  // namespace
 
-int build(const float* tris9_host, uint64_t n_tris, uint32_t tri_stride, uint32_t max_leaf, uint32_t radius, cudaStream_t st,
-          Result* out, char* err, size_t errlen) {
-    return build_tlas(tris9_host, n_tris, nullptr, 0, tri_stride, max_leaf, radius, st, out, err, errlen);
-}
-
 // object_offsets == NULL: one flat BVH.  Otherwise (n_objects + 1 offsets into the triangle array): one BLAS per object —
 // built together, as a forest, by a PLOC run that never merges across objects — plus a TLAS over the BLAS boxes, laid out
 // as cwbvh_gpu_runner lays them out (src/rt_gpu/mod.rs:53-100): BLAS nodes | TLAS nodes, tlas_start, blas_offsets in
@@ -1047,7 +1048,8 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     const int r = (int)(radius < 1 ? 1 : (radius > 64 ? 64 : radius));
     const double t_begin = now_ms();
     Scratch sc;
-    sc.reserve((size_t)n * 344 + (size_t)(tlas ? n_objects : 0) * 16 + (64u << 20));      // every array of the run (~320 B per triangle) + slack
+    // every array of the run (~320 B per triangle) + slack, then those of the TLAS
+    sc.reserve((size_t)n * 344 + (size_t)(tlas ? n_objects : 0) * 16 + (64u << 20) + (tlas ? (size_t)n_objects * 344 + (16u << 20) : 0));
     float* d_tris9; float4 *plo, *phi; uint32_t* prim_seg = nullptr; uint64_t* d_off = nullptr;
     BCU(sc.alloc(&d_tris9, (size_t)n * 36));
     BCU(sc.alloc(&plo, (size_t)n * 16)); BCU(sc.alloc(&phi, (size_t)n * 16));
@@ -1067,54 +1069,52 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     BCU(cudaStreamSynchronize(st));
     const double t_ploc = now_ms();
     // reinsertion passes (obvhs: `reinsertion_batch_ratio`, reference src/main.rs:563-587); TRAY_CUDA_BUILD_REINSERT=0 turns them off
-    const char* re_env = getenv("TRAY_CUDA_BUILD_REINSERT");
-    const char* rv_env = getenv("TRAY_CUDA_BUILD_REINSERT_VISITS");
-    const uint32_t re_passes = re_env && *re_env ? (uint32_t)atoi(re_env) : 4u;
-    const uint32_t re_visits = rv_env && *rv_env ? (uint32_t)atoi(rv_env) : 192u;
+    const auto env_u32 = [](const char* name, uint32_t dflt) { const char* v = getenv(name); return v && *v ? (uint32_t)atoi(v) : dflt; };
+    const uint32_t re_passes = env_u32("TRAY_CUDA_BUILD_REINSERT", 4u), re_visits = env_u32("TRAY_CUDA_BUILD_REINSERT_VISITS", 192u),
+                   re_rounds = env_u32("TRAY_CUDA_BUILD_REINSERT_ROUNDS", 3u);
     OptStats os;
-    rc = optimize_run(sc, pl, n, re_passes, re_visits, st, &os, err, errlen);
+    rc = optimize_run(sc, pl, n, re_passes, re_visits, re_rounds, st, &os, err, errlen);
     if (rc) return rc;
     BCU(cudaStreamSynchronize(st));
     const double t_opt = now_ms();
 
     // node count of a BLAS is bounded by its triangle count (>= 1 node); the TLAS by the object count
     const uint64_t blas_cap = (uint64_t)n + (tlas ? n_objects : 1), tlas_cap = tlas ? (uint64_t)n_objects + 1 : 0;
-    uint8_t *d_nodes = nullptr, *d_tri_out = nullptr; uint32_t *d_prim_idx = nullptr, *d_blas = nullptr;
-    if (cudaMalloc(&d_nodes, (blas_cap + tlas_cap) * 80) != cudaSuccess || cudaMalloc(&d_tri_out, (size_t)n * tri_stride) != cudaSuccess ||
-        cudaMalloc(&d_prim_idx, (size_t)n * 4) != cudaSuccess || (tlas && cudaMalloc(&d_blas, (size_t)n_objects * 4) != cudaSuccess)) {
-        cudaFree(d_nodes); cudaFree(d_tri_out); cudaFree(d_prim_idx); cudaFree(d_blas);
-        snprintf(err, errlen, "out of device memory for the BVH"); cudaGetLastError(); return -2;
-    }
-    auto bail = [&](int code) { cudaFree(d_nodes); cudaFree(d_tri_out); cudaFree(d_prim_idx); cudaFree(d_blas); return code; };
+    // the outputs: handed to `out` on success, freed on every other return
+    DevPtr<uint8_t> d_nodes, d_tri_out; DevPtr<uint32_t> d_prim_idx, d_blas;
+    BCU(dev_alloc(d_nodes, (blas_cap + tlas_cap) * 80));
+    BCU(dev_alloc(d_tri_out, (size_t)n * tri_stride));
+    BCU(dev_alloc(d_prim_idx, (size_t)n * 4));
+    if (tlas) BCU(dev_alloc(d_blas, (size_t)n_objects * 4));
     CollapseOut co;
-    rc = collapse_run(sc, pl, n, tlas, max_leaf, tri_stride, d_tris9, d_nodes, blas_cap, d_tri_out, d_prim_idx, 0, st, &co, err, errlen);
-    if (rc) return bail(rc);
+    rc = collapse_run(sc, pl, n, tlas, max_leaf, tri_stride, d_tris9, d_nodes.get(), blas_cap, d_tri_out.get(), d_prim_idx.get(), 0, st, &co,
+                      err, errlen);
+    if (rc) return rc;
     uint32_t tlas_start = 0, n_nodes = co.n_nodes, tl_iters = 0, tl_levels = 0;
     bool force_exact = co.force_exact;
     if (tlas) {
         // TLAS: the same pipeline over the BLAS boxes; its "triangles" are instance slots
-        Scratch sc2;
-        sc2.reserve((size_t)n_objects * 344 + (16u << 20));
         float4 *tlo, *thi; uint32_t* tl_prim;
-        if (sc2.alloc(&tlo, (size_t)n_objects * 16) != cudaSuccess || sc2.alloc(&thi, (size_t)n_objects * 16) != cudaSuccess ||
-            sc2.alloc(&tl_prim, (size_t)n_objects * 4) != cudaSuccess) { snprintf(err, errlen, "out of device memory"); cudaGetLastError(); return bail(-2); }
+        BCU(sc.alloc(&tlo, (size_t)n_objects * 16)); BCU(sc.alloc(&thi, (size_t)n_objects * 16)); BCU(sc.alloc(&tl_prim, (size_t)n_objects * 4));
         blas_boxes_kernel<<<blocks(n_objects), TPB, 0, st>>>(pl.roots, n_objects, pl.b, tlo, thi);
         PlocOut tp;
-        rc = ploc_run(sc2, tlo, thi, n_objects, nullptr, r, st, &tp, err, errlen);
-        if (rc) return bail(rc);
-        rc = optimize_run(sc2, tp, n_objects, re_passes, re_visits, st, nullptr, err, errlen);
-        if (rc) return bail(rc);
+        rc = ploc_run(sc, tlo, thi, n_objects, nullptr, r, st, &tp, err, errlen);
+        if (rc) return rc;
+        rc = optimize_run(sc, tp, n_objects, re_passes, re_visits, re_rounds, st, nullptr, err, errlen);
+        if (rc) return rc;
         CollapseOut tc;
         tlas_start = co.n_nodes;
-        rc = collapse_run(sc2, tp, n_objects, false, max_leaf, 0, nullptr, d_nodes + (uint64_t)tlas_start * 80, tlas_cap, nullptr, tl_prim, 0, st, &tc, err, errlen);
-        if (rc) return bail(rc);
-        blas_offsets_kernel<<<blocks(n_objects), TPB, 0, st>>>(tl_prim, n_objects, d_blas);
-        if (cudaStreamSynchronize(st) != cudaSuccess) { snprintf(err, errlen, "TLAS build failed: %s", cudaGetErrorString(cudaGetLastError())); return bail(-2); }
+        rc = collapse_run(sc, tp, n_objects, false, max_leaf, 0, nullptr, d_nodes.get() + (uint64_t)tlas_start * 80, tlas_cap, nullptr, tl_prim, 0, st,
+                          &tc, err, errlen);
+        if (rc) return rc;
+        // blas_offsets in TLAS-leaf order: object k's BLAS has its root wide node at node index k (forest level 0)
+        BCU(cudaMemcpyAsync(d_blas.get(), tl_prim, (size_t)n_objects * 4, cudaMemcpyDeviceToDevice, st));
+        BCU(cudaStreamSynchronize(st));
         n_nodes += tc.n_nodes; tl_iters = tp.iters; tl_levels = tc.levels; force_exact = force_exact || tc.force_exact;
     }
     const double t_end = now_ms();
-    out->d_nodes = d_nodes; out->n_nodes = n_nodes; out->d_tris = d_tri_out; out->d_prim_indices = d_prim_idx;
-    out->d_blas_offsets = d_blas; out->n_instances = tlas ? n_objects : 0; out->tlas_start = tlas_start;
+    out->d_nodes = d_nodes.release(); out->n_nodes = n_nodes; out->d_tris = d_tri_out.release(); out->d_prim_indices = d_prim_idx.release();
+    out->d_blas_offsets = d_blas.release(); out->n_instances = tlas ? n_objects : 0; out->tlas_start = tlas_start;
     out->force_exact = force_exact;
     out->stats.n_tris = n; out->stats.n_nodes = n_nodes; out->stats.ploc_iterations = pl.iters + tl_iters; out->stats.levels = co.levels + tl_levels;
     out->stats.ms_upload = (float)(t_upload - t_begin); out->stats.ms_sort = 0.f;
@@ -1124,15 +1124,9 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     return 0;
 }
 
-void refit_free(RefitTopology* t) {
-    cudaFree(t->d_items); cudaFree(t->d_node_box); cudaFree(t->d_slot_box); cudaFree(t->d_flag);
-    *t = RefitTopology();
-}
-
 int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uint32_t* d_blas, uint32_t n_instances, uint32_t tlas_start,
                cudaStream_t st, RefitTopology* out, char* err, size_t errlen) {
     RefitTopology t;
-    auto fail = [&](int code) { refit_free(&t); return code; };
     // roots: node 0, or the distinct blas_offsets (a BLAS shared by two instances is one tree) and then the TLAS
     std::vector<uint32_t> roots;
     if (n_instances) {
@@ -1146,26 +1140,18 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
     } else if (n_nodes) {
         roots.push_back(0u);
     }
-    uint32_t* visited = nullptr;
-    uint32_t* d_walk = nullptr;                       // [0] tail, [1] error bits
-    auto walk_fail = [&](int code) { cudaFree(visited); cudaFree(d_walk); return fail(code); };
-#define WCU(call)                                                                                                  \
-    do {                                                                                                           \
-        cudaError_t e_ = (call);                                                                                   \
-        if (e_ != cudaSuccess) {                                                                                   \
-            snprintf(err, errlen, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__);     \
-            return walk_fail(-2);                                                                                  \
-        }                                                                                                          \
-    } while (0)
+    DevPtr<uint32_t> visited_buf, walk_buf;
     const uint64_t cap = n_nodes ? n_nodes : 1;
-    WCU(cudaMalloc(&t.d_items, cap * sizeof(uint2)));
-    WCU(cudaMalloc(&t.d_node_box, cap * 2 * sizeof(int4)));
-    WCU(cudaMalloc(&t.d_slot_box, (n_tris ? n_tris : 1) * 2 * sizeof(int4)));
-    WCU(cudaMalloc(&t.d_flag, 7 * 4));                // the level flag; the coordinate check's 7 words
-    WCU(cudaMalloc(&visited, cap * 4));
-    WCU(cudaMalloc(&d_walk, 8));
-    WCU(cudaMemsetAsync(visited, 0, cap * 4, st));
-    WCU(cudaMemsetAsync(d_walk, 0, 8, st));
+    BCU(dev_alloc(t.d_items, cap * sizeof(uint2)));
+    BCU(dev_alloc(t.d_node_box, cap * 2 * sizeof(int4)));
+    BCU(dev_alloc(t.d_slot_box, (n_tris ? n_tris : 1) * 2 * sizeof(int4)));
+    BCU(dev_alloc(t.d_flag, 7 * 4));                  // the level flag; the coordinate check's 7 words
+    BCU(dev_alloc(visited_buf, cap * 4));
+    BCU(dev_alloc(walk_buf, 8));
+    uint32_t *visited = visited_buf.get(), *d_walk = walk_buf.get();      // d_walk: [0] tail, [1] error bits
+    uint2* items = t.d_items.get();
+    BCU(cudaMemsetAsync(visited, 0, cap * 4, st));
+    BCU(cudaMemsetAsync(d_walk, 0, 8, st));
     const uint4* nodes = static_cast<const uint4*>(d_nodes);
     uint32_t tail = 0;
     t.level_off.push_back(0);
@@ -1176,25 +1162,25 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
         // blas_offsets entry equal to tlas_start).  Refused here, before its roots are written to the list.
         if ((uint64_t)tail + part_roots.size() > cap) {
             snprintf(err, errlen, "the tree cannot be refit: a node is reached twice");
-            return walk_fail(-1);
+            return -1;
         }
-        WCU(cudaMemcpyAsync(t.d_items + tail, part_roots.data(), part_roots.size() * sizeof(uint2), cudaMemcpyHostToDevice, st));
-        refit_roots_kernel<<<blocks(part_roots.size()), TPB, 0, st>>>(t.d_items, tail, (uint32_t)part_roots.size(), visited, d_walk + 1);
+        BCU(cudaMemcpyAsync(items + tail, part_roots.data(), part_roots.size() * sizeof(uint2), cudaMemcpyHostToDevice, st));
+        refit_roots_kernel<<<blocks(part_roots.size()), TPB, 0, st>>>(items, tail, (uint32_t)part_roots.size(), visited, d_walk + 1);
         tail += (uint32_t)part_roots.size();
-        WCU(cudaMemcpyAsync(d_walk, &tail, 4, cudaMemcpyHostToDevice, st));
+        BCU(cudaMemcpyAsync(d_walk, &tail, 4, cudaMemcpyHostToDevice, st));
         t.level_off.push_back(tail);
         for (;;) {
             const uint32_t begin = t.level_off[t.level_off.size() - 2], n = tail - begin;
-            refit_walk_kernel<<<blocks(n), TPB, 0, st>>>(nodes, t.d_items, begin, n, (uint32_t)cap, child_lo, n_nodes, leaf_limit, d_walk,
+            refit_walk_kernel<<<blocks(n), TPB, 0, st>>>(nodes, items, begin, n, (uint32_t)cap, child_lo, n_nodes, leaf_limit, d_walk,
                                                          visited, d_walk + 1);
             uint32_t w[2];
-            WCU(cudaMemcpyAsync(w, d_walk, 8, cudaMemcpyDeviceToHost, st));
-            WCU(cudaStreamSynchronize(st));
-            WCU(cudaGetLastError());
+            BCU(cudaMemcpyAsync(w, d_walk, 8, cudaMemcpyDeviceToHost, st));
+            BCU(cudaStreamSynchronize(st));
+            BCU(cudaGetLastError());
             if (w[1]) {
                 snprintf(err, errlen, "the tree cannot be refit: %s", (w[1] & WALK_TWICE) ? "a node is reached twice"
                          : (w[1] & WALK_CHILD_RANGE) ? "a child index is outside the node array" : "a leaf range is outside its array");
-                return walk_fail(-1);
+                return -1;
             }
             if (w[0] == tail) return 0;
             tail = w[0];
@@ -1209,35 +1195,31 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
         part.assign(1, make_uint2(tlas_start, tlas_start));
         if (const int rc = walk(part, tlas_start, n_instances)) return rc;
     }
-    WCU(cudaMemsetAsync(t.d_flag, 0, 4, st));
-    if (n_nodes) refit_unreached_exact_kernel<<<blocks(n_nodes), TPB, 0, st>>>(nodes, n_nodes, visited, t.d_flag);
+    BCU(cudaMemsetAsync(t.d_flag.get(), 0, 4, st));
+    if (n_nodes) refit_unreached_exact_kernel<<<blocks(n_nodes), TPB, 0, st>>>(nodes, n_nodes, visited, t.d_flag.get());
     uint32_t f = 0;
-    WCU(cudaMemcpyAsync(&f, t.d_flag, 4, cudaMemcpyDeviceToHost, st));
-    WCU(cudaStreamSynchronize(st));
-    WCU(cudaGetLastError());
-#undef WCU
-    cudaFree(visited); cudaFree(d_walk);
+    BCU(cudaMemcpyAsync(&f, t.d_flag.get(), 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    BCU(cudaGetLastError());
     t.unreached_exact = f != 0;
     t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4;
-    *out = t;
+    *out = std::move(t);
     return 0;
 }
 
 int refit_check(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, cudaStream_t st, bool* bad, char* err, size_t errlen) {
-    // flag 0; minima +max, maxima -max (ordered)
-    const int init[7] = { 0, 0x7f7fffff, 0x7f7fffff, 0x7f7fffff, (int)0x80800000, (int)0x80800000, (int)0x80800000 };
-    int scan[7];
-    BCU(cudaMemcpyAsync(t.d_flag, init, sizeof init, cudaMemcpyHostToDevice, st));
-    if (n_tris) refit_scan_kernel<<<blocks(n_tris * 9 < (1ull << 24) ? n_tris * 9 : (1ull << 24)), TPB, 0, st>>>(d_tris9, n_tris * 9,
-                                                                                                                  reinterpret_cast<int*>(t.d_flag));
-    BCU(cudaMemcpyAsync(scan, t.d_flag, sizeof scan, cudaMemcpyDeviceToHost, st));
+    int init[7] = { 0 }, scan[7];                     // flag 0, then the empty bounds
+    memcpy(init + 1, EMPTY_BOUNDS, sizeof EMPTY_BOUNDS);
+    int* d_scan = reinterpret_cast<int*>(t.d_flag.get());
+    BCU(cudaMemcpyAsync(d_scan, init, sizeof init, cudaMemcpyHostToDevice, st));
+    if (n_tris) refit_scan_kernel<<<blocks(n_tris * 9 < (1ull << 24) ? n_tris * 9 : (1ull << 24)), TPB, 0, st>>>(d_tris9, n_tris * 9, d_scan);
+    BCU(cudaMemcpyAsync(scan, d_scan, sizeof scan, cudaMemcpyDeviceToHost, st));
     BCU(cudaStreamSynchronize(st));
     BCU(cudaGetLastError());
     *bad = scan[0] != 0;
     // every node box lies inside the vertices' bounds: if their extent is finite on every axis, so is every extent the encoder sees
     for (int a = 0; a < 3 && n_tris && !*bad; a++) {
-        auto o2f_host = [](int i) { i = i >= 0 ? i : i ^ 0x7fffffff; float f; memcpy(&f, &i, 4); return f; };
-        const float ext = o2f_host(scan[4 + a]) - o2f_host(scan[1 + a]);
+        const float ext = o2f(scan[4 + a]) - o2f(scan[1 + a]);
         *bad = !std::isfinite(ext);
     }
     return 0;
@@ -1247,26 +1229,29 @@ int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, con
               void* d_nodes, void* d_tris, const uint32_t* d_blas, cudaStream_t st, bool* exact, char* err, size_t errlen) {
     const uint32_t n = (uint32_t)n_tris;
     uint8_t* tri_out = static_cast<uint8_t*>(d_tris);
-    BCU(cudaMemsetAsync(t.d_flag, 0, 4, st));
+    uint32_t* flag = t.d_flag.get();
+    BCU(cudaMemsetAsync(flag, 0, 4, st));
     if (n) {
-#define TRIS(S) refit_tris_kernel<S><<<blocks(n), TPB, 0, st>>>(d_tris9, n, d_prim_indices, tri_out, t.d_slot_box)
+#define TRIS(S) refit_tris_kernel<S><<<blocks(n), TPB, 0, st>>>(d_tris9, n, d_prim_indices, tri_out, t.d_slot_box.get())
         if (tri_stride == 64) TRIS(64); else if (tri_stride == 24) TRIS(24); else TRIS(48);
 #undef TRIS
     }
     uint4* nodes = static_cast<uint4*>(d_nodes);
     const uint32_t n_levels = (uint32_t)t.level_off.size() - 1;
+    const uint2* items = t.d_items.get();
+    int4 *node_box = t.d_node_box.get(), *slot_box = t.d_slot_box.get();
     // BLAS (or flat) levels deepest first, then the TLAS over the BLAS roots' boxes
     for (uint32_t part = 0; part < 2; part++) {
         const uint32_t first = part == 0 ? 0 : t.n_blas_levels, last = part == 0 ? t.n_blas_levels : n_levels;
         for (uint32_t L = last; L-- > first;) {
             const uint32_t begin = t.level_off[L], cnt = t.level_off[L + 1] - begin;
-            if (part == 0) refit_node_kernel<false><<<blocks(cnt), TPB, 0, st>>>(t.d_items + begin, cnt, nodes, t.d_node_box, t.d_slot_box, d_blas, t.d_flag);
-            else refit_node_kernel<true><<<blocks(cnt), TPB, 0, st>>>(t.d_items + begin, cnt, nodes, t.d_node_box, t.d_slot_box, d_blas, t.d_flag);
+            if (part == 0) refit_node_kernel<false><<<blocks(cnt), TPB, 0, st>>>(items + begin, cnt, nodes, node_box, slot_box, d_blas, flag);
+            else refit_node_kernel<true><<<blocks(cnt), TPB, 0, st>>>(items + begin, cnt, nodes, node_box, slot_box, d_blas, flag);
         }
     }
     BCU(cudaGetLastError());
     uint32_t f = 0;
-    BCU(cudaMemcpyAsync(&f, t.d_flag, 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaMemcpyAsync(&f, flag, 4, cudaMemcpyDeviceToHost, st));
     BCU(cudaStreamSynchronize(st));
     BCU(cudaGetLastError());
     *exact = f != 0 || t.unreached_exact;

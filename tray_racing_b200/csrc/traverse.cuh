@@ -58,13 +58,6 @@ constexpr uint32_t CURSOR_COUNTERS = 1, N_COUNTERS = 5, CURSOR_N_BOUNCE = 11, CU
 constexpr float F32_MAX_ = 3.402823466e+38f;
 constexpr float F32_EPS_ = 1.1920929e-7f;     // sampling.hlsl:3
 constexpr float BOX_EPS_ = 0.0001f;           // query.hlsl:274
-// The fused node test needs 2^23 * scale * |1/d| finite, i.e. below 2^105 on the x axis.  Rays with |1/d| >= 2^64 on some axis
-// (RayConst::wide) and scenes with an exponent byte >= EXACT_EXP_BYTE (scale >= 2^40) take the unfused test: together the two
-// guards keep 2^23 * A below 2^23 * 2^39 * 2^64 = 2^126, two bits short of the overflow.
-constexpr uint32_t EXACT_EXP_BYTE = 167;
-__host__ __device__ __forceinline__ bool node_needs_exact(uint32_t exp_bytes3) {    // the three exponent bytes of a node (byte 12..14)
-    return (exp_bytes3 & 0xffu) >= EXACT_EXP_BYTE || ((exp_bytes3 >> 8) & 0xffu) >= EXACT_EXP_BYTE || ((exp_bytes3 >> 16) & 0xffu) >= EXACT_EXP_BYTE;
-}
 
 struct FrameParams {
     tray_view view;

@@ -44,6 +44,10 @@ int env_int(const char* name, int dflt) {
     return v && *v ? atoi(v) : dflt;
 }
 
+// whether a scene takes the unfused node test everywhere: some node scale is >= 2^40 (tray::node_needs_exact), or
+// TRAY_CUDA_FORCE_EXACT asks for it
+bool scene_force_exact(bool nodes_need_it) { return env_int("TRAY_CUDA_FORCE_EXACT", 0) != 0 || nodes_need_it; }
+
 }  // namespace
 
 // Everything one frame in flight owns: its compact (tile-ordered) buffers, its work cursors and its stream.  Slot 0 runs on
@@ -412,7 +416,7 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     if (s->stream) cudaStreamSynchronize(s->stream);
     cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
     cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_costs); cudaFree(s->d_geom_offsets);
-    if (s->refit) { tray_build::refit_free(s->refit); delete s->refit; }
+    delete s->refit;
     free_pipeline(s);
     cudaFree(s->d_untiled);
     for (auto& f : s->slot) {
@@ -457,7 +461,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     s->device = device; s->n_nodes = n_nodes; s->n_tris = n_tris; s->tri_stride = tri_stride;
     s->n_instances = n_instances; s->tlas_start = tlas_start; s->tlas = n_instances > 0;
     s->refill_min = (uint32_t)env_int("TRAY_CUDA_REFILL_MIN", 6);       // 6: +0.3 % (C3) ... +2 % (C1) over 4 with the r2 kernel (profiles/experiments/r2_refill_min_ab.log)
-    s->force_exact = env_int("TRAY_CUDA_FORCE_EXACT", 0) != 0 || (built && built->force_exact);
+    s->force_exact = scene_force_exact(built && built->force_exact);
     for (uint64_t i = 0; !built && i < n_nodes && !s->force_exact; i++) {
         const uint8_t* e = (const uint8_t*)nodes + i * 80 + 12;
         if (tray::node_needs_exact(e[0] | (uint32_t)e[1] << 8 | (uint32_t)e[2] << 16)) s->force_exact = true;   // scale = 2^(e-127) >= 2^40
@@ -769,9 +773,9 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         const int rc = tray_build::refit_walk(s->d_nodes, s->n_nodes, s->n_tris, s->tlas ? s->d_blas : nullptr, s->tlas ? s->n_instances : 0u,
                                               s->tlas_start, s->stream, &t, msg, sizeof msg);
         if (rc) return fail(rc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "refit: %s", msg);
-        s->refit = new (std::nothrow) tray_build::RefitTopology(t);
-        if (!s->refit) { tray_build::refit_free(&t); return fail(TRAY_ERR_ARG, "out of host memory"); }
-        s->device_bytes += t.bytes;
+        s->refit = new (std::nothrow) tray_build::RefitTopology(std::move(t));
+        if (!s->refit) return fail(TRAY_ERR_ARG, "out of host memory");
+        s->device_bytes += s->refit->bytes;
     }
     const float* d_tris9 = tris9;
     float* d_upload = nullptr;
@@ -796,7 +800,7 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         CU(cudaEventRecord(s->ev[1], s->stream));
         CU(cudaEventSynchronize(s->ev[1]));
         CU(cudaEventElapsedTime(&ms_run, s->ev[0], s->ev[1]));
-        s->force_exact = env_int("TRAY_CUDA_FORCE_EXACT", 0) != 0 || exact;      // as scene creation decides it
+        s->force_exact = scene_force_exact(exact);
         if (ms_refit) *ms_refit = ms_check + ms_run;
         return TRAY_OK;
     };
