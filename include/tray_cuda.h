@@ -243,7 +243,7 @@ int tray_cuda_scene_info(const tray_scene* scene, tray_scene_info* out_info);
 
 /* *out_exact = 1 when the scene's traversal takes the unfused (exact) node test at every node — some node has an exponent byte
  * >= 167 (a scale >= 2^40, where the fused test could overflow), or TRAY_CUDA_FORCE_EXACT is set — and 0 when it takes the
- * fused one.  Decided when the scene is made and again by every tray_cuda_scene_refit. */
+ * fused one.  Decided when the scene is made and again by every tray_cuda_scene_refit and tray_cuda_scene_refit_rebuild_tlas. */
 int tray_cuda_scene_exact_node_test(const tray_scene* scene, int* out_exact);
 
 /* ---- refit: move the triangles, keep the tree -----------------------------------------------------------------------------
@@ -270,6 +270,36 @@ int tray_cuda_scene_exact_node_test(const tray_scene* scene, int* out_exact);
 int tray_cuda_scene_refit(tray_scene* scene, const float* tris9, uint64_t n_tris, float* ms_refit);
 /* the same with DEVICE memory; the refit starts after the work enqueued so far on `stream` (NULL: none) */
 int tray_cuda_scene_refit_device(tray_scene* scene, const float* d_tris9, uint64_t n_tris, void* stream, float* ms_refit);
+
+/* ---- refit every BLAS, rebuild the TLAS: objects that move as a whole ------------------------------------------------------
+ * For two-level scenes whose objects move apart: a refit keeps the TLAS grouping instances that are no longer near each other,
+ * a TLAS rebuild regroups them at a fraction of a full build's cost.
+ *   1. Every BLAS is refit exactly as tray_cuda_scene_refit refits it: the same triangle records, the same bytes for every node
+ *      below tlas_start.
+ *   2. The TLAS primitives are the instances, each with its BLAS root's exact box, in canonical order: by blas_offsets value (the
+ *      BLAS root node), ties (one BLAS under two instances) by TLAS-leaf position.  For scenes of tray_cuda_scene_build_tlas
+ *      object k's root is node k, so the canonical order is object order and the new TLAS and blas_offsets are byte for byte
+ *      those tray_cuda_scene_build_tlas builds on the moved triangles.
+ *   3. The TLAS is built as tray_cuda_scene_build_tlas builds its TLAS: PLOC with search_radius (0 = 14, 1..64), the
+ *      reinsertion passes (TRAY_CUDA_BUILD_REINSERT*), the collapse with max_prims_per_leaf (1..3).
+ *   4. It is written over nodes [tlas_start, tlas_start + m); blas_offsets[j] becomes the root of TLAS leaf j; n_nodes becomes
+ *      tlas_start + m and tlas_start stays.  A scene made by tray_cuda_scene_create holds exactly n_nodes: the first call that
+ *      needs more grows its node array to tlas_start + n_instances + 1 nodes.  The first call also allocates the TLAS build's
+ *      device scratch, n_instances x 384 B + 16 MiB, which the scene keeps: later calls allocate and free nothing on the device.
+ *      tray_scene_info.device_bytes counts both.
+ *   5. The exact node test is decided as the refit decides it, over the BLAS nodes, the new TLAS and the unreached nodes below
+ *      tlas_start.  Later refits and rebuilds work on the new TLAS.
+ *   ms   CUDA-event time on the scene stream from the coordinate check to the last TLAS write, the TLAS build's host round
+ *        trips included, the host upload and the topology walk of a first call not; a first call's also holds its growth and
+ *        scratch allocation (NULL ok)
+ * Synchronous and ordered as tray_cuda_scene_refit.  TRAY_ERR_ARG, with nothing changed: every refusal of the refit, a scene
+ * without a TLAS, max_prims_per_leaf or search_radius out of range, a node reached from a BLAS root at index >= tlas_start (the
+ * TLAS is not the tail of the node array), a BLAS that reaches no triangle, or tlas_start + n_instances + 1 beyond 32 bits. */
+int tray_cuda_scene_refit_rebuild_tlas(tray_scene* scene, const float* tris9, uint64_t n_tris, uint32_t max_prims_per_leaf,
+                                       uint32_t search_radius, float* ms);
+/* the same with DEVICE memory; starts after the work enqueued so far on `stream` (NULL: none) */
+int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* scene, const float* d_tris9, uint64_t n_tris, uint32_t max_prims_per_leaf,
+                                              uint32_t search_radius, void* stream, float* ms);
 
 /* ---- ray-batch operator: Traversable::traverse at batch grain (traversable/src/lib.rs:20) ----- */
 
@@ -509,7 +539,8 @@ int tray_cuda_hits_to_geometry(tray_scene* scene, const tray_hit* hits, uint64_t
  *                                   tray_cuda_frame_readback_begin; with two frames in flight the group alternates two targets
  *   tray_cuda_group_scene           borrow the scene of devices[i] (counters, hit downloads of its shard, set_variant ..)
  * Moving geometry: refit every replica, tray_cuda_scene_refit on tray_cuda_group_scene(i) for each i; the group has no refit
- * call of its own, as its caller would still loop over the devices.                                                          */
+ * call of its own, as its caller would still loop over the devices.  The same for tray_cuda_scene_refit_rebuild_tlas: call it
+ * on tray_cuda_group_scene(i) for each i; the replicas stay byte-identical.                                                   */
 typedef struct tray_group tray_group;
 int  tray_cuda_group_create(const void* nodes, uint64_t n_nodes, const void* tris, uint64_t n_tris, uint32_t tri_stride,
                             const uint32_t* blas_offsets, uint32_t n_instances, uint32_t tlas_start,

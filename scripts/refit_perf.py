@@ -9,7 +9,13 @@ For each config and each tree producer (the host's binned SAH, the device's PLOC
   frame_ms          render_frame_ms at the config's size, median of 10 after 3 warm-up frames: before any motion, after each
                     motion refit, and on a scene built on the device from the moved triangles
 Motions: "jitter", every vertex moved by up to 1 % of the mean triangle size; "rigid" (two-level configs), every object
-translated by up to 5 % of the scene's extent.  The first line names the GPU and its power limit."""
+translated by up to 5 % of the scene's extent.  Two-level configs also get, per motion k:
+  ms_refit_rebuild_tlas[k]   CUDA-event time of tray_cuda_scene_refit_rebuild_tlas_device on the moved triangles (every BLAS
+                             refit, the TLAS rebuilt), median of 20 after 3 warm-up calls; measured after the refit-only frames
+  frame_ms.after_k_refit_rebuild_tlas   the frame on that tree
+  per_ray[k]                 nodes, instances and triangles per primary and per bounce ray, from one TRAY_RENDER_COUNTERS frame
+                             of each tree: "refit", "refit_rebuild_tlas", "rebuild" (counts: they do not depend on the card)
+The first line names the GPU and its power limit."""
 import json
 import os
 import subprocess
@@ -28,6 +34,19 @@ def frame_ms(sc, view, w, h):
     for _ in range(3):
         sc.render_frame_ms(view, w, h, 0)
     return float(np.median([sc.render_frame_ms(view, w, h, 0) for _ in range(10)]))
+
+
+def per_ray(sc, view, w, h):
+    """nodes, instances and triangles per primary and per bounce ray of one counted frame"""
+    sc.render(view, w, h, 0, cuda.RENDER_BOUNCE | cuda.RENDER_COUNTERS, timed=False)
+    sc.sync()
+    return {which: {k: c[k] / max(c["rays"], 1) for k in ("nodes", "instances", "tris")} for which, c in zip(("primary", "bounce"), sc.counters())}
+
+
+def rebuild_tlas_ms(sc, d):
+    for _ in range(3):
+        sc.refit_rebuild_tlas_device(d.data_ptr(), d.shape[0])
+    return [sc.refit_rebuild_tlas_device(d.data_ptr(), d.shape[0], timed=True) for _ in range(20)]
 
 
 def refit_ms(sc, d):
@@ -65,10 +84,12 @@ def main():
             b = cuda.TrayCudaScene.build(tris, object_offsets=offs)
             builds.append(b.build_stats["ms_total"])
             b.close()
-        rebuilt = {}
+        rebuilt, rebuilt_counts = {}, {}
         for k, moved in motions.items():
             sc = cuda.TrayCudaScene.build(moved, object_offsets=offs)
             rebuilt[k] = frame_ms(sc, view, w, h)
+            if offs is not None:
+                rebuilt_counts[k] = per_ray(sc, view, w, h)
             sc.close()
         for producer in ("host", "device"):
             if producer == "host":
@@ -89,7 +110,18 @@ def main():
                 sc.refit_device(dm.data_ptr(), tris.shape[0])
                 line["frame_ms"][f"after_{k}_refit"] = frame_ms(sc, view, w, h)
                 line["frame_ms"][f"after_{k}_rebuild"] = rebuilt[k]
+                if offs is not None:
+                    line.setdefault("per_ray", {})[k] = {"refit": per_ray(sc, view, w, h), "rebuild": rebuilt_counts[k]}
                 sc.refit_device(d.data_ptr(), tris.shape[0])
+            if offs is not None:
+                # last: a TLAS rebuild replaces the producer's TLAS for good
+                line["ms_refit_rebuild_tlas"] = {}
+                for k, moved in motions.items():
+                    dm = torch.from_numpy(np.ascontiguousarray(slots(moved)).reshape(-1, 9)).cuda()
+                    line["ms_refit_rebuild_tlas"][k] = float(np.median(rebuild_tlas_ms(sc, dm)))
+                    line["frame_ms"][f"after_{k}_refit_rebuild_tlas"] = frame_ms(sc, view, w, h)
+                    line["per_ray"][k]["refit_rebuild_tlas"] = per_ray(sc, view, w, h)
+                    del dm
             emit(line)
             sc.close()
             del d

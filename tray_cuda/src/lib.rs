@@ -122,6 +122,11 @@ extern "C" {
     pub fn tray_cuda_scene_refit(scene: *mut TrayScene, tris9: *const f32, n_tris: u64, ms_refit: *mut f32) -> c_int;
     pub fn tray_cuda_scene_refit_device(scene: *mut TrayScene, d_tris9: *const f32, n_tris: u64, stream: *mut c_void,
         ms_refit: *mut f32) -> c_int;
+    // two-level scenes whose objects move as a whole: refit every BLAS, rebuild the TLAS over their boxes; synchronous as the refit
+    pub fn tray_cuda_scene_refit_rebuild_tlas(scene: *mut TrayScene, tris9: *const f32, n_tris: u64, max_prims_per_leaf: u32,
+        search_radius: u32, ms: *mut f32) -> c_int;
+    pub fn tray_cuda_scene_refit_rebuild_tlas_device(scene: *mut TrayScene, d_tris9: *const f32, n_tris: u64, max_prims_per_leaf: u32,
+        search_radius: u32, stream: *mut c_void, ms: *mut f32) -> c_int;
     pub fn tray_cuda_frame_download(scene: *mut TrayScene, primary: *mut TrayHit, bounce: *mut TrayHit,
         bounce_rays: *mut TrayRay, rgba: *mut u8) -> c_int;
     pub fn tray_cuda_scene_set_variant(scene: *mut TrayScene, variant_flags: u32) -> c_int;

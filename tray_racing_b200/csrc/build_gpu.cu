@@ -683,10 +683,14 @@ __global__ void collapse_emit_kernel(const int* __restrict__ items, uint32_t n_i
 
 // Device scratch of one build: ONE cudaMalloc (reserve) carved up by a bump allocator — a two-level build makes ~80 allocations,
 // and in a process that already holds a lot of device memory each cudaMalloc / cudaFree costs up to a millisecond.  Requests
-// that do not fit the arena fall back to their own cudaMalloc.  Everything is freed on scope exit.
+// that do not fit the arena fall back to their own cudaMalloc.  Everything is freed on scope exit, except an arena borrowed from
+// its owner (a TLAS rebuild works in one the scene keeps: no allocation and no device-wide cudaFree per call).
 struct Scratch {
     void* p[128]; int n = 0;
     char* arena = nullptr; size_t cap = 0, used = 0;
+    bool owned = true;
+    Scratch() = default;
+    Scratch(void* borrowed, size_t bytes) : arena(static_cast<char*>(borrowed)), cap(bytes), owned(false) {}
     cudaError_t reserve(size_t bytes) {
         if (cudaMalloc((void**)&arena, bytes) != cudaSuccess) { arena = nullptr; cap = 0; cudaGetLastError(); }   // fall back to per-array allocations
         else cap = bytes;
@@ -700,7 +704,7 @@ struct Scratch {
         if (e == cudaSuccess) { p[n++] = q; *out = (T*)q; }
         return e;
     }
-    ~Scratch() { for (int i = 0; i < n; i++) cudaFree(p[i]); if (arena) cudaFree(arena); }
+    ~Scratch() { for (int i = 0; i < n; i++) cudaFree(p[i]); if (arena && owned) cudaFree(arena); }
 };
 
 template <typename T> cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) { T* q = nullptr; const cudaError_t e = cudaMalloc(&q, bytes); p.reset(q); return e; }
@@ -828,9 +832,18 @@ int optimize_run(Scratch& sc, const PlocOut& pl, uint32_t n_leaves, uint32_t pas
     return 0;
 }
 
+// the reinsertion knobs: TRAY_CUDA_BUILD_REINSERT passes (0 = off), _VISITS node visits per move search, _ROUNDS claim / apply
+// rounds per pass (obvhs: `reinsertion_batch_ratio`, reference src/main.rs:563-587)
+struct Reinsert { uint32_t passes, visits, rounds; };
+Reinsert reinsert_knobs() {
+    const auto env_u32 = [](const char* name, uint32_t dflt) { const char* v = getenv(name); return v && *v ? (uint32_t)atoi(v) : dflt; };
+    return { env_u32("TRAY_CUDA_BUILD_REINSERT", 4u), env_u32("TRAY_CUDA_BUILD_REINSERT_VISITS", 192u), env_u32("TRAY_CUDA_BUILD_REINSERT_ROUNDS", 3u) };
+}
+
 // level-synchronous collapse of the BVH2 subtrees `roots` (one wide root node each, stored at node indices 0..n_roots-1 of
 // `nodes`, i.e. at `nodes` itself — pass the destination already offset).  forest = child indices relative to each root.
-struct CollapseOut { uint32_t n_nodes, n_prims, levels; bool force_exact; };
+// level_end[L] = the node index (relative to `nodes`) one past level L.
+struct CollapseOut { uint32_t n_nodes, n_prims, levels; bool force_exact; std::vector<uint32_t> level_end; };
 
 int collapse_run(Scratch& sc, const PlocOut& pl, uint32_t n_prims, bool forest, uint32_t max_leaf, uint32_t tri_stride,
                  const float* d_tris9, uint8_t* nodes, uint64_t node_cap, uint8_t* tri_out, uint32_t* prim_idx, uint32_t prim_base0,
@@ -845,6 +858,7 @@ int collapse_run(Scratch& sc, const PlocOut& pl, uint32_t n_prims, bool forest, 
     BCU(cudaMemsetAsync(d_flags, 0, 4, st));
     BCU(cudaMemcpyAsync(items_a, pl.roots, (size_t)pl.n_roots * 4, cudaMemcpyDeviceToDevice, st));
     uint32_t n_items = pl.n_roots, level_base = 0, prim_base = prim_base0, levels = 0;
+    out->level_end.clear();
     int* it_in = items_a; int* it_out = items_b; uint32_t* rt_in = root_a; uint32_t* rt_out = root_b;
     while (n_items) {
         if ((uint64_t)level_base + n_items > node_cap) { snprintf(err, errlen, "node count exceeds its bound"); return -3; }
@@ -859,6 +873,7 @@ int collapse_run(Scratch& sc, const PlocOut& pl, uint32_t n_prims, bool forest, 
         }, tot, err, errlen);
         if (rc) return rc;
         level_base = next_base; prim_base += tot[1]; n_items = tot[0]; levels++;
+        out->level_end.push_back(level_base);
         int* t = it_in; it_in = it_out; it_out = t;
         uint32_t* u = rt_in; rt_in = rt_out; rt_out = u;
     }
@@ -883,6 +898,44 @@ __global__ void blas_boxes_kernel(const int* __restrict__ roots, uint32_t n_obj,
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_obj) return;
     plo[i] = b.lo[roots[i]]; phi[i] = b.hi[roots[i]];
+}
+
+// The TLAS leg of a two-level build, over n instance boxes (xyz of tlo / thi): PLOC, reinsertion, collapse.  Writes the wide
+// nodes at `nodes` (child indices relative to it) and perm[j] = the instance of TLAS leaf j.
+struct TlasOut { uint32_t n_nodes, iters; CollapseOut co; };
+int tlas_run(Scratch& sc, const float4* tlo, const float4* thi, uint32_t n, uint32_t max_leaf, int r, const Reinsert& re, uint8_t* nodes,
+             uint32_t* perm, cudaStream_t st, TlasOut* out, char* err, size_t errlen) {
+    PlocOut tp;
+    int rc = ploc_run(sc, tlo, thi, n, nullptr, r, st, &tp, err, errlen);
+    if (rc) return rc;
+    rc = optimize_run(sc, tp, n, re.passes, re.visits, re.rounds, st, nullptr, err, errlen);
+    if (rc) return rc;
+    rc = collapse_run(sc, tp, n, false, max_leaf, 0, nullptr, nodes, (uint64_t)n + 1, nullptr, perm, 0, st, &out->co, err, errlen);
+    if (rc) return rc;
+    out->n_nodes = out->co.n_nodes; out->iters = tp.iters;
+    return 0;
+}
+
+// TLAS primitives of a rebuild: the exact box of the BLAS root of canonical instance i (ordered ints of the refit)
+__global__ void tlas_boxes_kernel(const uint32_t* __restrict__ canon, uint32_t n, const int4* __restrict__ node_box, float4* __restrict__ plo,
+                                  float4* __restrict__ phi) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int4 l = node_box[2ull * canon[i]], h = node_box[2ull * canon[i] + 1];
+    plo[i] = make_float4(o2f(l.x), o2f(l.y), o2f(l.z), 0.f);
+    phi[i] = make_float4(o2f(h.x), o2f(h.y), o2f(h.z), 0.f);
+}
+
+// blas_offsets of the rebuilt TLAS: leaf j holds canonical instance perm[j], whose BLAS root is canon[perm[j]]
+__global__ void blas_compose_kernel(const uint32_t* __restrict__ perm, const uint32_t* __restrict__ canon, uint32_t n, uint32_t* __restrict__ blas) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n) blas[j] = canon[perm[j]];
+}
+
+// the topology's TLAS part after a rebuild: every one of the m new nodes, in collapse order (which is level order)
+__global__ void tlas_items_kernel(uint2* __restrict__ items, uint32_t m, uint32_t tlas_start) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < m) items[k] = make_uint2(tlas_start + k, tlas_start);
 }
 
 // ---- 5. refit: the same trees, re-encoded tight over moved triangles (tray_cuda_scene_refit) ---------------------------------
@@ -922,7 +975,8 @@ __global__ void refit_roots_kernel(const uint2* __restrict__ items, uint32_t beg
     if (i < n && atomicExch(visited + items[begin + i].x, 1u) != 0u) atomicOr(err, WALK_TWICE);
 }
 
-// one level of the walk: checks every leaf range against `leaf_limit` and appends the inner children at `tail`
+// one level of the walk: checks every leaf range against `leaf_limit` and appends the inner children at `tail`.  A node with a
+// leaf entry sets bit 1 of its tree root's visited word: that tree reaches a primitive.
 __global__ void refit_walk_kernel(const uint4* __restrict__ nodes, uint2* __restrict__ items, uint32_t begin, uint32_t n, uint32_t cap,
                                   uint64_t child_lo, uint64_t child_hi, uint64_t leaf_limit, uint32_t* __restrict__ tail,
                                   uint32_t* __restrict__ visited, uint32_t* __restrict__ err) {
@@ -931,11 +985,14 @@ __global__ void refit_walk_kernel(const uint4* __restrict__ nodes, uint2* __rest
     const uint2 it = items[begin + i];
     const uint4 n0 = nodes[5ull * it.x], n1 = nodes[5ull * it.x + 1];
     const uint32_t imask = n0.w >> 24;
+    bool leaf = false;
     for (int s = 0; s < 8; s++) {
         const uint32_t meta = node_meta(n1, s);
         if (((imask >> s) & 1u) || meta == 0u) continue;
         if ((uint64_t)n1.y + (meta & 31u) + leaf_count(meta) > leaf_limit) atomicOr(err, WALK_LEAF_RANGE);
+        leaf |= leaf_count(meta) > 0u;
     }
+    if (leaf) atomicOr(visited + it.y, 2u);
     const uint32_t k = __popc(imask);
     if (!k) return;
     const uint32_t pos = atomicAdd(tail, k);
@@ -948,12 +1005,24 @@ __global__ void refit_walk_kernel(const uint4* __restrict__ nodes, uint2* __rest
     }
 }
 
-// a node that no root reaches keeps its bytes through every refit: whether one of them asks for the exact node test is fixed
-__global__ void refit_unreached_exact_kernel(const uint4* __restrict__ nodes, uint64_t n_nodes, const uint32_t* __restrict__ visited,
+// a node that no root reaches keeps its bytes through every refit: whether one of them asks for the exact node test is fixed.
+// Bit 0: such a node below `split` (tlas_start), bit 1: at or above it (nodes a TLAS rebuild overwrites or leaves past n_nodes).
+__global__ void refit_unreached_exact_kernel(const uint4* __restrict__ nodes, uint64_t n_nodes, uint64_t split, const uint32_t* __restrict__ visited,
                                              uint32_t* __restrict__ flag) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_nodes || visited[i]) return;
-    if (tray::node_needs_exact(nodes[5 * i].w)) atomicOr(flag, 1u);
+    if (tray::node_needs_exact(nodes[5 * i].w)) atomicOr(flag, i < split ? 1u : 2u);
+}
+
+// what a TLAS rebuild needs of the BLAS part, over its n walk items (the first n_roots of them its roots): bit 0 = some node
+// has an index >= tlas_start (the TLAS is not the tail of the node array), bit 1 = some BLAS reaches no primitive
+__global__ void refit_blas_check_kernel(const uint2* __restrict__ items, uint32_t n, uint32_t n_roots, const uint32_t* __restrict__ visited,
+                                        uint32_t tlas_start, uint32_t* __restrict__ flag) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t x = items[i].x;
+    if (x >= tlas_start) atomicOr(flag, 1u);
+    if (i < n_roots && !(visited[x] & 2u)) atomicOr(flag, 2u);
 }
 
 // records of slot k from triangle prim_indices[k] (k without the map), and the slot's box from the f32 vertices
@@ -1068,12 +1137,9 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     if (tlas && pl.n_roots != n_objects) { snprintf(err, errlen, "PLOC left %u roots for %u objects", pl.n_roots, n_objects); return -3; }
     BCU(cudaStreamSynchronize(st));
     const double t_ploc = now_ms();
-    // reinsertion passes (obvhs: `reinsertion_batch_ratio`, reference src/main.rs:563-587); TRAY_CUDA_BUILD_REINSERT=0 turns them off
-    const auto env_u32 = [](const char* name, uint32_t dflt) { const char* v = getenv(name); return v && *v ? (uint32_t)atoi(v) : dflt; };
-    const uint32_t re_passes = env_u32("TRAY_CUDA_BUILD_REINSERT", 4u), re_visits = env_u32("TRAY_CUDA_BUILD_REINSERT_VISITS", 192u),
-                   re_rounds = env_u32("TRAY_CUDA_BUILD_REINSERT_ROUNDS", 3u);
+    const Reinsert re = reinsert_knobs();
     OptStats os;
-    rc = optimize_run(sc, pl, n, re_passes, re_visits, re_rounds, st, &os, err, errlen);
+    rc = optimize_run(sc, pl, n, re.passes, re.visits, re.rounds, st, &os, err, errlen);
     if (rc) return rc;
     BCU(cudaStreamSynchronize(st));
     const double t_opt = now_ms();
@@ -1093,27 +1159,19 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
     uint32_t tlas_start = 0, n_nodes = co.n_nodes, tl_iters = 0, tl_levels = 0;
     bool force_exact = co.force_exact;
     if (tlas) {
-        // TLAS: the same pipeline over the BLAS boxes; its "triangles" are instance slots
-        float4 *tlo, *thi; uint32_t* tl_prim;
-        BCU(sc.alloc(&tlo, (size_t)n_objects * 16)); BCU(sc.alloc(&thi, (size_t)n_objects * 16)); BCU(sc.alloc(&tl_prim, (size_t)n_objects * 4));
+        // TLAS: the same pipeline over the BLAS boxes; its "triangles" are instance slots.  blas_offsets in TLAS-leaf order are its
+        // leaf permutation, as object k's BLAS has its root wide node at node index k (forest level 0).
+        float4 *tlo, *thi;
+        BCU(sc.alloc(&tlo, (size_t)n_objects * 16)); BCU(sc.alloc(&thi, (size_t)n_objects * 16));
         blas_boxes_kernel<<<blocks(n_objects), TPB, 0, st>>>(pl.roots, n_objects, pl.b, tlo, thi);
-        PlocOut tp;
-        rc = ploc_run(sc, tlo, thi, n_objects, nullptr, r, st, &tp, err, errlen);
-        if (rc) return rc;
-        rc = optimize_run(sc, tp, n_objects, re_passes, re_visits, re_rounds, st, nullptr, err, errlen);
-        if (rc) return rc;
-        CollapseOut tc;
         tlas_start = co.n_nodes;
-        rc = collapse_run(sc, tp, n_objects, false, max_leaf, 0, nullptr, d_nodes.get() + (uint64_t)tlas_start * 80, tlas_cap, nullptr, tl_prim, 0, st,
-                          &tc, err, errlen);
+        TlasOut to;
+        rc = tlas_run(sc, tlo, thi, n_objects, max_leaf, r, re, d_nodes.get() + (uint64_t)tlas_start * 80, d_blas.get(), st, &to, err, errlen);
         if (rc) return rc;
-        // blas_offsets in TLAS-leaf order: object k's BLAS has its root wide node at node index k (forest level 0)
-        BCU(cudaMemcpyAsync(d_blas.get(), tl_prim, (size_t)n_objects * 4, cudaMemcpyDeviceToDevice, st));
-        BCU(cudaStreamSynchronize(st));
-        n_nodes += tc.n_nodes; tl_iters = tp.iters; tl_levels = tc.levels; force_exact = force_exact || tc.force_exact;
+        n_nodes += to.n_nodes; tl_iters = to.iters; tl_levels = to.co.levels; force_exact = force_exact || to.co.force_exact;
     }
     const double t_end = now_ms();
-    out->d_nodes = d_nodes.release(); out->n_nodes = n_nodes; out->d_tris = d_tri_out.release(); out->d_prim_indices = d_prim_idx.release();
+    out->d_nodes = d_nodes.release(); out->n_nodes = n_nodes; out->node_cap = blas_cap + tlas_cap; out->d_tris = d_tri_out.release(); out->d_prim_indices = d_prim_idx.release();
     out->d_blas_offsets = d_blas.release(); out->n_instances = tlas ? n_objects : 0; out->tlas_start = tlas_start;
     out->force_exact = force_exact;
     out->stats.n_tris = n; out->stats.n_nodes = n_nodes; out->stats.ploc_iterations = pl.iters + tl_iters; out->stats.levels = co.levels + tl_levels;
@@ -1135,6 +1193,9 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
             snprintf(err, errlen, "blas_offsets download failed"); cudaGetLastError(); return -2;
         }
         std::sort(roots.begin(), roots.end());
+        // the instances' roots in canonical order (a TLAS rebuild permutes blas_offsets, so this stays what it is)
+        BCU(dev_alloc(t.d_canon, (size_t)n_instances * 4));
+        BCU(cudaMemcpyAsync(t.d_canon.get(), roots.data(), (size_t)n_instances * 4, cudaMemcpyHostToDevice, st));
         roots.erase(std::unique(roots.begin(), roots.end()), roots.end());
         if (roots.back() >= n_nodes) { snprintf(err, errlen, "blas_offsets entry %u outside %llu nodes", roots.back(), (unsigned long long)n_nodes); return -1; }
     } else if (n_nodes) {
@@ -1191,18 +1252,22 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
     for (uint32_t r : roots) part.push_back(make_uint2(r, r));
     if (const int rc = walk(part, 0, n_tris)) return rc;
     t.n_blas_levels = (uint32_t)t.level_off.size() - 1;
+    BCU(cudaMemsetAsync(t.d_flag.get(), 0, 8, st));
     if (n_instances) {
+        const uint32_t n_blas = t.level_off.back();
+        refit_blas_check_kernel<<<blocks(n_blas), TPB, 0, st>>>(items, n_blas, (uint32_t)roots.size(), visited, tlas_start, t.d_flag.get() + 1);
         part.assign(1, make_uint2(tlas_start, tlas_start));
         if (const int rc = walk(part, tlas_start, n_instances)) return rc;
     }
-    BCU(cudaMemsetAsync(t.d_flag.get(), 0, 4, st));
-    if (n_nodes) refit_unreached_exact_kernel<<<blocks(n_nodes), TPB, 0, st>>>(nodes, n_nodes, visited, t.d_flag.get());
-    uint32_t f = 0;
-    BCU(cudaMemcpyAsync(&f, t.d_flag.get(), 4, cudaMemcpyDeviceToHost, st));
+    if (n_nodes) refit_unreached_exact_kernel<<<blocks(n_nodes), TPB, 0, st>>>(nodes, n_nodes, tlas_start, visited, t.d_flag.get());
+    uint32_t f[2] = { 0, 0 };
+    BCU(cudaMemcpyAsync(f, t.d_flag.get(), 8, cudaMemcpyDeviceToHost, st));
     BCU(cudaStreamSynchronize(st));
     BCU(cudaGetLastError());
-    t.unreached_exact = f != 0;
-    t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4;
+    t.unreached_exact = f[0] != 0; t.unreached_exact_blas = (f[0] & 1u) != 0;
+    t.blas_past_tlas = (f[1] & 1u) != 0; t.blas_empty = (f[1] & 2u) != 0;
+    t.cap = cap;
+    t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4 + (uint64_t)n_instances * 4;
     *out = std::move(t);
     return 0;
 }
@@ -1226,7 +1291,7 @@ int refit_check(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, c
 }
 
 int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, const uint32_t* d_prim_indices, uint32_t tri_stride,
-              void* d_nodes, void* d_tris, const uint32_t* d_blas, cudaStream_t st, bool* exact, char* err, size_t errlen) {
+              void* d_nodes, void* d_tris, const uint32_t* d_blas, bool blas_only, cudaStream_t st, bool* exact, char* err, size_t errlen) {
     const uint32_t n = (uint32_t)n_tris;
     uint8_t* tri_out = static_cast<uint8_t*>(d_tris);
     uint32_t* flag = t.d_flag.get();
@@ -1241,7 +1306,7 @@ int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, con
     const uint2* items = t.d_items.get();
     int4 *node_box = t.d_node_box.get(), *slot_box = t.d_slot_box.get();
     // BLAS (or flat) levels deepest first, then the TLAS over the BLAS roots' boxes
-    for (uint32_t part = 0; part < 2; part++) {
+    for (uint32_t part = 0; part < (blas_only ? 1u : 2u); part++) {
         const uint32_t first = part == 0 ? 0 : t.n_blas_levels, last = part == 0 ? t.n_blas_levels : n_levels;
         for (uint32_t L = last; L-- > first;) {
             const uint32_t begin = t.level_off[L], cnt = t.level_off[L + 1] - begin;
@@ -1254,7 +1319,55 @@ int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, con
     BCU(cudaMemcpyAsync(&f, flag, 4, cudaMemcpyDeviceToHost, st));
     BCU(cudaStreamSynchronize(st));
     BCU(cudaGetLastError());
-    *exact = f != 0 || t.unreached_exact;
+    *exact = f != 0 || (blas_only ? t.unreached_exact_blas : t.unreached_exact);
+    return 0;
+}
+
+size_t tlas_arena_bytes(uint32_t n_instances) { return (size_t)n_instances * 384 + (16u << 20); }
+
+int refit_reserve(RefitTopology& t, uint64_t cap, uint32_t n_instances, cudaStream_t st, char* err, size_t errlen) {
+    if (!t.d_tlas_arena) {
+        const size_t bytes = tlas_arena_bytes(n_instances);
+        BCU(dev_alloc(t.d_tlas_arena, bytes));
+        t.tlas_arena_bytes = bytes;
+        t.bytes += bytes;
+    }
+    if (cap <= t.cap) return 0;
+    DevPtr<uint2> items; DevPtr<int4> box;
+    BCU(dev_alloc(items, cap * sizeof(uint2)));
+    BCU(dev_alloc(box, cap * 2 * sizeof(int4)));
+    BCU(cudaMemcpyAsync(items.get(), t.d_items.get(), (size_t)t.level_off.back() * sizeof(uint2), cudaMemcpyDeviceToDevice, st));
+    BCU(cudaStreamSynchronize(st));
+    t.d_items = std::move(items); t.d_node_box = std::move(box);
+    t.bytes += (cap - t.cap) * (sizeof(uint2) + 2 * sizeof(int4));
+    t.cap = cap;
+    return 0;
+}
+
+int rebuild_tlas(RefitTopology& t, void* d_nodes, uint32_t tlas_start, uint32_t n, uint32_t* d_blas, uint32_t max_leaf, uint32_t radius,
+                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen) {
+    if ((uint64_t)tlas_start + n + 1 > t.cap) { snprintf(err, errlen, "the topology holds %llu nodes", (unsigned long long)t.cap); return -3; }
+    const int r = (int)(radius < 1 ? 1 : (radius > 64 ? 64 : radius));
+    if (!t.d_tlas_arena) { snprintf(err, errlen, "no TLAS build arena (refit_reserve first)"); return -3; }
+    Scratch sc(t.d_tlas_arena.get(), t.tlas_arena_bytes);
+    float4 *tlo, *thi; uint32_t* perm;
+    BCU(sc.alloc(&tlo, (size_t)n * 16)); BCU(sc.alloc(&thi, (size_t)n * 16)); BCU(sc.alloc(&perm, (size_t)n * 4));
+    tlas_boxes_kernel<<<blocks(n), TPB, 0, st>>>(t.d_canon.get(), n, t.d_node_box.get(), tlo, thi);
+    TlasOut to;
+    if (const int rc = tlas_run(sc, tlo, thi, n, max_leaf, r, reinsert_knobs(), static_cast<uint8_t*>(d_nodes) + (uint64_t)tlas_start * 80, perm,
+                                st, &to, err, errlen)) return rc;
+    blas_compose_kernel<<<blocks(n), TPB, 0, st>>>(perm, t.d_canon.get(), n, d_blas);
+    BCU(cudaGetLastError());
+    if (written) BCU(cudaEventRecord(written, st));
+    // the BLAS levels stay; the TLAS levels become those of the new tree, every node of which is reached
+    t.level_off.resize(t.n_blas_levels + 1);
+    const uint32_t base = t.level_off.back();
+    tlas_items_kernel<<<blocks(to.n_nodes), TPB, 0, st>>>(t.d_items.get() + base, to.n_nodes, tlas_start);
+    for (uint32_t e : to.co.level_end) t.level_off.push_back(base + e);
+    t.unreached_exact = t.unreached_exact_blas;
+    BCU(cudaStreamSynchronize(st));
+    BCU(cudaGetLastError());
+    *n_tlas_nodes = to.n_nodes; *exact = to.co.force_exact;
     return 0;
 }
 

@@ -27,8 +27,8 @@ struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
 template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
 
 struct Result {
-    uint8_t* d_nodes;            // n_nodes x 80 bytes (allocation holds n_tris + 1 nodes); caller owns (cudaFree)
-    uint64_t n_nodes;
+    uint8_t* d_nodes;            // n_nodes x 80 bytes (allocation holds node_cap nodes); caller owns (cudaFree)
+    uint64_t n_nodes, node_cap;
     uint8_t* d_tris;             // n_tris x tri_stride, BVH order; caller owns
     uint32_t* d_prim_indices;    // BVH slot -> input triangle; caller owns
     uint32_t* d_blas_offsets;    // two-level builds: node index of the BLAS behind TLAS leaf k; caller owns
@@ -52,13 +52,21 @@ struct RefitTopology {
     DevPtr<int4> d_node_box;                 // per node: min, max as ordered ints (two int4)
     DevPtr<int4> d_slot_box;                 // per triangle slot: the same
     DevPtr<uint32_t> d_flag;
+    uint64_t cap = 0;                        // nodes d_items and d_node_box have room for
+    DevPtr<uint32_t> d_canon;                // two-level: blas_offsets sorted, i.e. the BLAS roots of the instances in canonical order
+    DevPtr<char> d_tlas_arena;               // device scratch of the TLAS rebuilds (refit_reserve), kept from call to call
+    size_t tlas_arena_bytes = 0;
     bool unreached_exact = false;            // a node no root reaches (never rewritten) has an exponent byte >= 167
+    bool unreached_exact_blas = false;       // ... one below tlas_start
+    bool blas_past_tlas = false;             // a node reached from a BLAS root has an index >= tlas_start
+    bool blas_empty = false;                 // some BLAS reaches no triangle
     uint64_t bytes = 0;                      // device memory held
 };
 
 // The walk: level-by-level BFS from node 0, or from the distinct blas_offsets and then tlas_start.  Returns 0, -1 (with a
 // message) for a tree it cannot refit — a node reached twice, a child or leaf index outside its array, a blas_offsets entry
-// outside the node array — or -2 for a CUDA error.  Synchronous on `st`.
+// outside the node array — or -2 for a CUDA error.  Synchronous on `st`.  blas_past_tlas and blas_empty are not refusals here:
+// a refit takes such trees, a TLAS rebuild does not.
 int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uint32_t* d_blas, uint32_t n_instances, uint32_t tlas_start,
                cudaStream_t st, RefitTopology* out, char* err, size_t errlen);
 // *bad = some coordinate of d_tris9 is not finite, or the vertices' extent on some axis (max - min in f32) is not: then a box
@@ -66,7 +74,17 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
 int refit_check(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, cudaStream_t st, bool* bad, char* err, size_t errlen);
 // Rewrites the triangle records (slot k <- d_tris9[d_prim_indices ? d_prim_indices[k] : k]) and p, exponents and used q bytes
 // of every reachable node, tight over the new triangles.  *exact = some node's exponent byte is >= 167.  Synchronous on `st`.
+// blas_only: the BLAS levels alone (a TLAS rebuild follows); *exact then leaves the TLAS nodes out.
 int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, const uint32_t* d_prim_indices, uint32_t tri_stride,
-              void* d_nodes, void* d_tris, const uint32_t* d_blas, cudaStream_t st, bool* exact, char* err, size_t errlen);
+              void* d_nodes, void* d_tris, const uint32_t* d_blas, bool blas_only, cudaStream_t st, bool* exact, char* err, size_t errlen);
+// What a TLAS rebuild of n_instances needs before its first write: room for `cap` nodes in the topology's arrays (the listed items
+// kept), and the rebuild's scratch arena (n_instances x 384 B + 16 MiB), allocated once and kept.  Synchronous on `st`.
+int refit_reserve(RefitTopology& t, uint64_t cap, uint32_t n_instances, cudaStream_t st, char* err, size_t errlen);
+// TLAS rebuild (tray_cuda_scene_refit_rebuild_tlas), after refit_run(blas_only): the TLAS leg of build_tlas over the BLAS root
+// boxes of the n instances in canonical order, written at node tlas_start of d_nodes; d_blas[j] = the root of TLAS leaf j; the
+// topology's TLAS levels become the new tree's (refit_reserve(tlas_start + n + 1) first).  `written` (optional) is recorded
+// behind the last TLAS write.  *n_tlas_nodes, and *exact = some new TLAS node's exponent byte is >= 167.  Synchronous on `st`.
+int rebuild_tlas(RefitTopology& t, void* d_nodes, uint32_t tlas_start, uint32_t n, uint32_t* d_blas, uint32_t max_leaf, uint32_t radius,
+                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen);
 
 }  // namespace tray_build

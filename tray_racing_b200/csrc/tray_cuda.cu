@@ -77,6 +77,7 @@ struct tray_scene {
     int device = 0;
     int sm_count = 0;
     uint64_t n_nodes = 0, n_tris = 0;
+    uint64_t node_cap = 0;                   // nodes d_nodes has room for (a TLAS rebuild may need more than n_nodes)
     uint32_t tri_stride = 48, n_instances = 0, tlas_start = 0;
     bool tlas = false;
     bool force_exact = false;                // some node scale >= 2^40: 2^23 * adj_inv could overflow in the fused node test
@@ -444,6 +445,21 @@ void tray_cuda_scene_destroy(tray_scene* s) {
 }  // extern "C"
 
 namespace {
+// the persisting-L2 access-policy window over the node array: `want` bytes set aside for persisting lines, windows of up to
+// `max_win` bytes
+void fit_l2_window(tray_scene* s, size_t want, size_t max_win) {
+    size_t win = (size_t)s->n_nodes * 80;
+    if (win > max_win) win = max_win;
+    memset(&s->window, 0, sizeof s->window);
+    s->window.base_ptr = s->d_nodes;
+    s->window.num_bytes = win;
+    double ratio = (double)want / (double)win;
+    s->window.hitRatio = (float)(ratio > 1.0 ? 1.0 : ratio);
+    s->window.hitProp = cudaAccessPropertyPersisting;
+    s->window.missProp = cudaAccessPropertyStreaming;
+    s->l2_persist = win < want ? win : want;
+}
+
 // `built` != NULL: adopt the device buffers of the device-side builder instead of uploading host arrays
 int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uint64_t n_tris, uint32_t tri_stride,
                       const uint32_t* blas_offsets, uint32_t n_instances, uint32_t tlas_start,
@@ -487,6 +503,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
             CU(cudaEventCreateWithFlags(&s->ev_copied[i], cudaEventDisableTiming));
         }
         const size_t nb = (size_t)(n_nodes ? n_nodes : 1) * 80, tb = (size_t)(n_tris ? n_tris : 1) * tri_stride;
+        s->node_cap = adopted ? built->node_cap : nb / 80;
         if (adopted) {
             s->d_nodes = (uint4*)built->d_nodes; s->d_tris = (uint4*)built->d_tris; s->d_prim_indices = built->d_prim_indices;
             s->d_blas = built->d_blas_offsets;
@@ -522,17 +539,8 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         if (prop.persistingL2CacheMaxSize > 0 && n_nodes) {
             size_t want = (size_t)prop.persistingL2CacheMaxSize;
             if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-                size_t win = (size_t)n_nodes * 80;
-                if (win > (size_t)prop.accessPolicyMaxWindowSize) win = (size_t)prop.accessPolicyMaxWindowSize;
-                memset(&s->window, 0, sizeof s->window);
-                s->window.base_ptr = s->d_nodes;
-                s->window.num_bytes = win;
-                double ratio = (double)want / (double)win;
-                s->window.hitRatio = (float)(ratio > 1.0 ? 1.0 : ratio);
-                s->window.hitProp = cudaAccessPropertyPersisting;
-                s->window.missProp = cudaAccessPropertyStreaming;
+                fit_l2_window(s, want, (size_t)prop.accessPolicyMaxWindowSize);
                 s->have_window = true;
-                s->l2_persist = win < want ? win : want;
             } else cudaGetLastError();
         }
         CU(cudaStreamSynchronize(s->stream));
@@ -754,12 +762,41 @@ int tray_cuda_sync(tray_scene* s) {
 }  // extern "C"
 
 namespace {
-// tray_cuda_scene_refit(_device): `tris9` is host memory unless `device_ptr`.  Every check runs before the first write, so a
-// refused call leaves nodes, records and force_exact as they were.
-int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_ptr, void* stream, float* ms_refit) {
+// the TLAS of a tray_cuda_scene_refit_rebuild_tlas(_device) call
+struct TlasRebuild { uint32_t max_leaf, radius; };
+
+// Moves the nodes of a TLAS rebuild into place: the new tree is in `nodes` (s->d_nodes, or a larger array of `cap` nodes that
+// replaces it), with m TLAS nodes at tlas_start.
+void adopt_rebuilt_tlas(tray_scene* s, uint4* nodes, uint64_t cap, uint32_t m) {
+    if (nodes != s->d_nodes) {
+        cudaFree(s->d_nodes);                 // every stream of the scene is drained: no launch reads it any more
+        s->d_nodes = nodes;
+        s->device_bytes += (cap - s->node_cap) * 80;
+        s->node_cap = cap;
+    }
+    s->n_nodes = (uint64_t)s->tlas_start + m;
+    if (s->have_window) {
+        int want = 0, max_win = 0;
+        cudaDeviceGetAttribute(&want, cudaDevAttrMaxPersistingL2CacheSize, s->device);
+        cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, s->device);
+        fit_l2_window(s, (size_t)want, (size_t)max_win);
+    }
+}
+
+// tray_cuda_scene_refit(_device), and with `rb` tray_cuda_scene_refit_rebuild_tlas(_device): `tris9` is host memory unless
+// `device_ptr`.  Every check runs before the first write, so a refused call leaves nodes, records, blas_offsets, n_nodes and
+// force_exact as they were.
+int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_ptr, void* stream, float* ms_refit, const TlasRebuild* rb = nullptr) {
     if (ms_refit) *ms_refit = 0.f;
     if (!s || !tris9) return fail(TRAY_ERR_ARG, "NULL argument");
     if (n_tris != s->n_tris) return fail(TRAY_ERR_ARG, "refit with %llu triangles, the scene has %llu", (unsigned long long)n_tris, (unsigned long long)s->n_tris);
+    if (rb) {
+        if (!s->tlas) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: the scene has no TLAS");
+        if (rb->max_leaf < 1 || rb->max_leaf > 3) return fail(TRAY_ERR_ARG, "max_prims_per_leaf must be 1..3");
+        if (rb->radius > 64) return fail(TRAY_ERR_ARG, "search_radius must be 0 (default 14) or 1..64");
+        if ((uint64_t)s->tlas_start + s->n_instances + 1 > 0xffffffffull) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: node indices are 32-bit");
+        if (n_tris == 0) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: an instance's BLAS reaches no triangle");
+    }
     CU(cudaSetDevice(s->device));
     // after every frame and batch enqueued so far: frames rendered before the refit keep their old-geometry results
     if (stream) CU(cudaStreamSynchronize((cudaStream_t)stream));
@@ -777,6 +814,8 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         if (!s->refit) return fail(TRAY_ERR_ARG, "out of host memory");
         s->device_bytes += s->refit->bytes;
     }
+    if (rb && s->refit->blas_past_tlas) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: a BLAS node lies at or past tlas_start");
+    if (rb && s->refit->blas_empty) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: an instance's BLAS reaches no triangle");
     const float* d_tris9 = tris9;
     float* d_upload = nullptr;
     if (!device_ptr) {
@@ -790,12 +829,40 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         bool bad = false, exact = false;
         CU(cudaEventRecord(s->ev[0], s->stream));
         if (tray_build::refit_check(*s->refit, d_tris9, n_tris, s->stream, &bad, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+        if (rb) {
+            // one interval, coordinate check to the last TLAS write, host round trips of the TLAS build included
+            if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
+            const uint64_t cap = (uint64_t)s->tlas_start + s->n_instances + 1;
+            tray_build::DevPtr<uint4> grown;  // a created scene's node array holds n_nodes: the first rebuild that needs more grows it
+            if (cap > s->node_cap) {
+                uint4* p = nullptr;
+                CU(cudaMalloc(&p, cap * 80));
+                grown.reset(p);
+                CU(cudaMemcpyAsync(p, s->d_nodes, (size_t)s->tlas_start * 80, cudaMemcpyDeviceToDevice, s->stream));
+            }
+            const uint64_t held = s->refit->bytes;
+            if (tray_build::refit_reserve(*s->refit, cap, s->n_instances, s->stream, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+            s->device_bytes += s->refit->bytes - held;
+            uint4* nodes = grown ? grown.get() : s->d_nodes;
+            bool tlas_exact = false;
+            uint32_t m = 0;
+            if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, nodes, s->d_tris, s->d_blas, true, s->stream,
+                                      &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+            if (tray_build::rebuild_tlas(*s->refit, nodes, s->tlas_start, s->n_instances, s->d_blas, rb->max_leaf,
+                                                         rb->radius ? rb->radius : 14u, s->stream, s->ev[1], &m, &tlas_exact, msg, sizeof msg))
+                return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", msg);     // past the first write: never a refusal
+            CU(cudaEventElapsedTime(&ms_run, s->ev[0], s->ev[1]));
+            adopt_rebuilt_tlas(s, grown ? grown.release() : s->d_nodes, cap, m);
+            s->force_exact = scene_force_exact(exact || tlas_exact);
+            if (ms_refit) *ms_refit = ms_run;
+            return TRAY_OK;
+        }
         CU(cudaEventRecord(s->ev[1], s->stream));
         CU(cudaEventSynchronize(s->ev[1]));
         CU(cudaEventElapsedTime(&ms_check, s->ev[0], s->ev[1]));
         if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
         CU(cudaEventRecord(s->ev[0], s->stream));
-        if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, s->d_nodes, s->d_tris, s->d_blas, s->stream,
+        if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, s->d_nodes, s->d_tris, s->d_blas, false, s->stream,
                                   &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
         CU(cudaEventRecord(s->ev[1], s->stream));
         CU(cudaEventSynchronize(s->ev[1]));
@@ -817,6 +884,16 @@ int tray_cuda_scene_refit(tray_scene* s, const float* tris9, uint64_t n_tris, fl
 }
 int tray_cuda_scene_refit_device(tray_scene* s, const float* d_tris9, uint64_t n_tris, void* stream, float* ms_refit) {
     return refit_impl(s, d_tris9, n_tris, true, stream, ms_refit);
+}
+int tray_cuda_scene_refit_rebuild_tlas(tray_scene* s, const float* tris9, uint64_t n_tris, uint32_t max_prims_per_leaf, uint32_t search_radius,
+                                       float* ms) {
+    const TlasRebuild rb{ max_prims_per_leaf, search_radius };
+    return refit_impl(s, tris9, n_tris, false, nullptr, ms, &rb);
+}
+int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* s, const float* d_tris9, uint64_t n_tris, uint32_t max_prims_per_leaf,
+                                              uint32_t search_radius, void* stream, float* ms) {
+    const TlasRebuild rb{ max_prims_per_leaf, search_radius };
+    return refit_impl(s, d_tris9, n_tris, true, stream, ms, &rb);
 }
 
 }  // extern "C"

@@ -34,6 +34,7 @@ EXPORTS = (
     "tray_cuda_start_multi",
     "tray_cuda_trace_cost", "tray_cuda_trace_cost_device", "tray_cuda_scene_set_ray_cost", "tray_cuda_frame_download_cost",
     "tray_cuda_scene_refit", "tray_cuda_scene_refit_device", "tray_cuda_scene_exact_node_test",
+    "tray_cuda_scene_refit_rebuild_tlas", "tray_cuda_scene_refit_rebuild_tlas_device",
 )
 # semantic switches of tray_cuda_scene_set_variant (include/tray_cuda.h TRAY_VARIANT_*)
 VARIANT_BOX_DIVIDE, VARIANT_TIE_LAST, VARIANT_BOX_TMIN_RAY, VARIANT_ZERODIR_BOX_ONLY = 1, 2, 4, 8
@@ -222,6 +223,10 @@ def lib() -> C.CDLL:
         L.tray_cuda_scene_refit_device.argtypes = [vp, vp, u64, vp, f32p]
         L.tray_cuda_scene_exact_node_test.restype = i32
         L.tray_cuda_scene_exact_node_test.argtypes = [vp, C.POINTER(i32)]
+        L.tray_cuda_scene_refit_rebuild_tlas.restype = i32
+        L.tray_cuda_scene_refit_rebuild_tlas.argtypes = [vp, vp, u64, u32, u32, f32p]
+        L.tray_cuda_scene_refit_rebuild_tlas_device.restype = i32
+        L.tray_cuda_scene_refit_rebuild_tlas_device.argtypes = [vp, vp, u64, u32, u32, vp, f32p]
         _lib = L
     return _lib
 
@@ -362,6 +367,24 @@ class TrayCudaScene:
         returns ms_refit when `timed`."""
         ms = C.c_float()
         _check(lib().tray_cuda_scene_refit_device(self._h, d_ptr, n, stream or None, C.byref(ms) if timed else None))
+        return ms.value if timed else None
+
+    def refit_rebuild_tlas(self, tris, max_prims_per_leaf=3, search_radius=0, timings: dict | None = None):
+        """Two-level scenes whose objects move as a whole: refit every BLAS as refit() does and rebuild the TLAS over the BLAS
+        roots' boxes as build() builds it (tray_cuda_scene_refit_rebuild_tlas).  `tris` in the scene's triangle order, as for
+        refit().  timings["ms_refit_rebuild_tlas"]: coordinate check to the last TLAS write."""
+        t = np.ascontiguousarray(tris, dtype=np.float32).reshape(-1, 9)
+        ms = C.c_float()
+        _check(lib().tray_cuda_scene_refit_rebuild_tlas(self._h, t.ctypes.data, t.shape[0], max_prims_per_leaf, search_radius, C.byref(ms)))
+        if timings is not None:
+            timings["ms_refit_rebuild_tlas"] = ms.value
+
+    def refit_rebuild_tlas_device(self, d_ptr: int, n: int, max_prims_per_leaf=3, search_radius=0, stream: int = 0, timed: bool = False):
+        """refit_rebuild_tlas() from n x 9 float32 in device memory, after the work enqueued so far on `stream`
+        (tray_cuda_scene_refit_rebuild_tlas_device); returns the call's ms when `timed`."""
+        ms = C.c_float()
+        _check(lib().tray_cuda_scene_refit_rebuild_tlas_device(self._h, d_ptr, n, max_prims_per_leaf, search_radius, stream or None,
+                                                                C.byref(ms) if timed else None))
         return ms.value if timed else None
 
     @classmethod
