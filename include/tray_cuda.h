@@ -301,6 +301,59 @@ int tray_cuda_scene_refit_rebuild_tlas(tray_scene* scene, const float* tris9, ui
 int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* scene, const float* d_tris9, uint64_t n_tris, uint32_t max_prims_per_leaf,
                                               uint32_t search_radius, void* stream, float* ms);
 
+/* ---- instances: place BLAS by 3x4 transforms, rebuild only the TLAS -------------------------------------------------------
+ * Makes a two-level scene INSTANCED: instance k is the BLAS whose root is blas_roots[k], placed by object_to_world + 12k (row-major
+ * 3x4 [R | t]: world = R object + t).  Rigid motion is a new transform and a TLAS build, with no triangle and no BLAS node
+ * touched; one BLAS may be placed any number of times.  Goes beyond the reference, whose runner has no instance transforms.
+ *   Instance identity  instance k is the caller's index: it stays k across calls, rebuilds and TLAS-leaf permutations.
+ *                      hits[i].prim keeps its meaning, the global triangle index; tray_cuda_trace_instance adds k.
+ *   Valid roots        the distinct blas_offsets values the scene had when it was made.  Any BLAS may be used by any number of
+ *                      instances, or by none.
+ *   Inverse            world_to_object is computed on the host in double from object_to_world, as the adjugate over the
+ *                      determinant with translation -W t, and rounded to nearest f32.
+ *   TLAS primitive of instance k, in double, with no contraction:
+ *                      1. the BLAS root's decoded box: the union over its used slots (child_meta != 0) of p + q 2^(e-127);
+ *                      2. its 8 corners mapped by object_to_world as ((M_i0 x + M_i1 y) + M_i2 z) + M_i3;
+ *                      3. the hull of the mapped corners;
+ *                      4. every face moved out by 2^-18 max |coordinate of the hull| (it covers the rounding between the
+ *                         world-space test at the TLAS and the object-space tests below it);
+ *                      5. rounded outward to f32.
+ *   Build              tray_cuda_scene_build_tlas's TLAS leg over those boxes in instance order: PLOC with search_radius (0 = 14,
+ *                      1..64), the reinsertion passes, the collapse with max_prims_per_leaf (1..3).  Written at tlas_start;
+ *                      blas_offsets[j] becomes blas_roots[leaf_instance[j]], n_nodes tlas_start + m, n_instances n_instances.
+ *                      The exact node test is decided as tray_cuda_scene_refit_rebuild_tlas decides it.
+ *   Memory             a first call, or a call with more instances than any before it, grows the node array to tlas_start + n + 1
+ *                      nodes, blas_offsets, the instance records (64 B per instance, twice) and the TLAS build's scratch, and keeps
+ *                      them: a call with no more instances than an earlier one allocates nothing on the device.
+ *                      tray_scene_info.device_bytes counts all of it.
+ *   ms                 CUDA-event time from the upload of the transforms to the last TLAS write (NULL ok)
+ * Synchronous and ordered as tray_cuda_scene_refit: a frame rendered before keeps its results.  An instanced scene stays instanced.
+ * TRAY_ERR_ARG, with nothing changed: NULL scene or pointers, n_instances == 0, a scene without a TLAS, semantic variants
+ * (tray_cuda_scene_set_variant flags), an invalid root, max_prims_per_leaf or search_radius out of range, a coordinate of
+ * object_to_world that is not finite, a zero determinant, a rounded inverse or a TLAS box that is not finite in f32, a tree the
+ * refit walk refuses, a node reached from a BLAS root at index >= tlas_start, a BLAS that reaches no triangle, or
+ * tlas_start + n_instances + 1 beyond 32 bits.
+ * On an instanced scene: tray_cuda_scene_refit and tray_cuda_scene_set_variant are refused (its TLAS leaves are transformed boxes);
+ * tray_cuda_scene_refit_rebuild_tlas(_device) refits every BLAS and then builds the TLAS as this call would, from the current roots
+ * and transforms; tray_cuda_render always takes the two-launch path (TRAY_RENDER_OVERLAP is ignored) and bounce normals go to world
+ * space through the transpose of world_to_object; the plain trace, trace_cost and render calls work and report no instances. */
+int tray_cuda_scene_set_instances(tray_scene* scene, const uint32_t* blas_roots, const float* object_to_world, uint32_t n_instances,
+                                  uint32_t max_prims_per_leaf, uint32_t search_radius, float* ms);
+/* leaf_instance[j]: the instance k of TLAS leaf j (n_instances entries); world_to_object: n_instances x 12 floats by instance, as
+ * the kernels use them.  Either may be NULL.  TRAY_ERR_ARG on a scene that is not instanced. */
+int tray_cuda_scene_download_instance_xforms(tray_scene* scene, uint32_t* leaf_instance, float* world_to_object);
+/* tray_cuda_trace / tray_cuda_trace_any (any_hit != 0) with one more output: instance_ids[i] = the instance k of hit i, 0xFFFFFFFF
+ * for a miss.  TRAY_ERR_ARG on a scene that is not instanced. */
+int tray_cuda_trace_instance(tray_scene* scene, const tray_ray* rays, uint64_t n, int any_hit, tray_hit* hits,
+                             uint32_t* instance_ids, float* ms_kernel, float* ms_total);
+/* the same with DEVICE buffers, as tray_cuda_trace_device */
+int tray_cuda_trace_instance_device(tray_scene* scene, const tray_ray* d_rays, uint64_t n, int any_hit, tray_hit* d_hits,
+                                    uint32_t* d_instance_ids, void* stream, float* ms_kernel);
+/* The last frame's instance ids, row-major (w * h each, either NULL): 0xFFFFFFFF for misses, for other shards' pixels and for
+ * pixels without a bounce ray.  TRAY_ERR_ARG on a scene that is not instanced, or for `bounce` after a frame without
+ * TRAY_RENDER_BOUNCE. */
+int tray_cuda_frame_download_instance(tray_scene* scene, uint32_t* primary, uint32_t* bounce);
+
 /* ---- ray-batch operator: Traversable::traverse at batch grain (traversable/src/lib.rs:20) ----- */
 
 /* Closest hit for `n` rays.  HOST buffers: the copy H2D of rays and D2H of hits are inside the

@@ -127,6 +127,15 @@ extern "C" {
         search_radius: u32, ms: *mut f32) -> c_int;
     pub fn tray_cuda_scene_refit_rebuild_tlas_device(scene: *mut TrayScene, d_tris9: *const f32, n_tris: u64, max_prims_per_leaf: u32,
         search_radius: u32, stream: *mut c_void, ms: *mut f32) -> c_int;
+    // instances: BLAS placed by row-major 3x4 object_to_world transforms, only the TLAS rebuilt; synchronous as the refit
+    pub fn tray_cuda_scene_set_instances(scene: *mut TrayScene, blas_roots: *const u32, object_to_world: *const f32, n_instances: u32,
+        max_prims_per_leaf: u32, search_radius: u32, ms: *mut f32) -> c_int;
+    pub fn tray_cuda_scene_download_instance_xforms(scene: *mut TrayScene, leaf_instance: *mut u32, world_to_object: *mut f32) -> c_int;
+    pub fn tray_cuda_trace_instance(scene: *mut TrayScene, rays: *const TrayRay, n: u64, any_hit: c_int, hits: *mut TrayHit,
+        instance_ids: *mut u32, ms_kernel: *mut f32, ms_total: *mut f32) -> c_int;
+    pub fn tray_cuda_trace_instance_device(scene: *mut TrayScene, d_rays: *const TrayRay, n: u64, any_hit: c_int, d_hits: *mut TrayHit,
+        d_instance_ids: *mut u32, stream: *mut c_void, ms_kernel: *mut f32) -> c_int;
+    pub fn tray_cuda_frame_download_instance(scene: *mut TrayScene, primary: *mut u32, bounce: *mut u32) -> c_int;
     pub fn tray_cuda_frame_download(scene: *mut TrayScene, primary: *mut TrayHit, bounce: *mut TrayHit,
         bounce_rays: *mut TrayRay, rgba: *mut u8) -> c_int;
     pub fn tray_cuda_scene_set_variant(scene: *mut TrayScene, variant_flags: u32) -> c_int;
@@ -252,6 +261,29 @@ impl Scene {
         let f = if any_hit { tray_cuda_trace_any } else { tray_cuda_trace };
         check(unsafe { f(self.raw, rays.as_ptr(), rays.len() as u64, hits.as_mut_ptr(), std::ptr::null_mut(), std::ptr::null_mut()) });
         hits
+    }
+
+    /// Place BLAS by transforms: instance k is the BLAS rooted at node `blas_roots[k]`, placed by the row-major 3x4
+    /// `object_to_world[k]`; only the TLAS is built.  Returns the call's ms (upload of the transforms to the last TLAS write).
+    pub fn set_instances(&mut self, blas_roots: &[u32], object_to_world: &[[f32; 12]], max_prims_per_leaf: u32, search_radius: u32) -> f32 {
+        assert_eq!(blas_roots.len(), object_to_world.len(), "one transform per instance");
+        let mut ms = 0f32;
+        check(unsafe {
+            tray_cuda_scene_set_instances(self.raw, blas_roots.as_ptr(), object_to_world.as_ptr().cast(), blas_roots.len() as u32,
+                max_prims_per_leaf, search_radius, &mut ms)
+        });
+        ms
+    }
+
+    /// Closest (or any) hit per ray of an instanced scene, with the instance of every hit (u32::MAX for a miss).
+    pub fn traverse_instance(&mut self, rays: &[TrayRay], any_hit: bool) -> (Vec<TrayHit>, Vec<u32>) {
+        let mut hits = vec![TrayHit { t: f32::INFINITY, prim: u32::MAX }; rays.len()];
+        let mut ids = vec![u32::MAX; rays.len()];
+        check(unsafe {
+            tray_cuda_trace_instance(self.raw, rays.as_ptr(), rays.len() as u64, any_hit as c_int, hits.as_mut_ptr(), ids.as_mut_ptr(),
+                std::ptr::null_mut(), std::ptr::null_mut())
+        });
+        (hits, ids)
     }
 
     /// One frame (primary + bounce rays) of shard `shard` of `shards`; returns (ms primary, ms bounce) of the kernels.

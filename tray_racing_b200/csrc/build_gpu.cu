@@ -932,6 +932,29 @@ __global__ void blas_compose_kernel(const uint32_t* __restrict__ perm, const uin
     if (j < n) blas[j] = canon[perm[j]];
 }
 
+// an instanced TLAS: leaf j holds instance perm[j], whose record (with its BLAS root) is in[perm[j]]
+__global__ void instance_compose_kernel(const uint32_t* __restrict__ perm, const uint4* __restrict__ in, uint32_t n, uint32_t* __restrict__ blas,
+                                        uint4* __restrict__ rec) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const uint4* src = in + 4ull * perm[j];
+#pragma unroll
+    for (int q = 0; q < 4; q++) rec[4ull * j + q] = src[q];
+    blas[j] = src[3].x;
+}
+
+__global__ void gather_nodes_kernel(const uint4* __restrict__ nodes, const uint32_t* __restrict__ idx, uint32_t n, uint4* __restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+#pragma unroll
+    for (int q = 0; q < 5; q++) out[5ull * i + q] = nodes[5ull * idx[i] + q];
+}
+
+__global__ void exact_scan_kernel(const uint4* __restrict__ nodes, uint32_t n, uint32_t* __restrict__ flag) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && tray::node_needs_exact(nodes[5ull * i].w)) atomicOr(flag, 1u);
+}
+
 // the topology's TLAS part after a rebuild: every one of the m new nodes, in collapse order (which is level order)
 __global__ void tlas_items_kernel(uint2* __restrict__ items, uint32_t m, uint32_t tlas_start) {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1198,6 +1221,10 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
         BCU(cudaMemcpyAsync(t.d_canon.get(), roots.data(), (size_t)n_instances * 4, cudaMemcpyHostToDevice, st));
         roots.erase(std::unique(roots.begin(), roots.end()), roots.end());
         if (roots.back() >= n_nodes) { snprintf(err, errlen, "blas_offsets entry %u outside %llu nodes", roots.back(), (unsigned long long)n_nodes); return -1; }
+        t.roots = roots;
+        BCU(dev_alloc(t.d_roots, roots.size() * 4));
+        BCU(dev_alloc(t.d_root_nodes, roots.size() * 80));
+        BCU(cudaMemcpyAsync(t.d_roots.get(), roots.data(), roots.size() * 4, cudaMemcpyHostToDevice, st));
     } else if (n_nodes) {
         roots.push_back(0u);
     }
@@ -1267,7 +1294,8 @@ int refit_walk(const void* d_nodes, uint64_t n_nodes, uint64_t n_tris, const uin
     t.unreached_exact = f[0] != 0; t.unreached_exact_blas = (f[0] & 1u) != 0;
     t.blas_past_tlas = (f[1] & 1u) != 0; t.blas_empty = (f[1] & 2u) != 0;
     t.cap = cap;
-    t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4 + (uint64_t)n_instances * 4;
+    t.bytes = cap * (sizeof(uint2) + 2 * sizeof(int4)) + (n_tris ? n_tris : 1) * 2 * sizeof(int4) + 7 * 4 + (uint64_t)n_instances * 4
+            + (uint64_t)t.roots.size() * 84;
     *out = std::move(t);
     return 0;
 }
@@ -1326,8 +1354,11 @@ int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, con
 size_t tlas_arena_bytes(uint32_t n_instances) { return (size_t)n_instances * 384 + (16u << 20); }
 
 int refit_reserve(RefitTopology& t, uint64_t cap, uint32_t n_instances, cudaStream_t st, char* err, size_t errlen) {
-    if (!t.d_tlas_arena) {
+    if (tlas_arena_bytes(n_instances) > t.tlas_arena_bytes) {
         const size_t bytes = tlas_arena_bytes(n_instances);
+        t.d_tlas_arena.reset();
+        t.bytes -= t.tlas_arena_bytes;
+        t.tlas_arena_bytes = 0;
         BCU(dev_alloc(t.d_tlas_arena, bytes));
         t.tlas_arena_bytes = bytes;
         t.bytes += bytes;
@@ -1345,18 +1376,25 @@ int refit_reserve(RefitTopology& t, uint64_t cap, uint32_t n_instances, cudaStre
 }
 
 int rebuild_tlas(RefitTopology& t, void* d_nodes, uint32_t tlas_start, uint32_t n, uint32_t* d_blas, uint32_t max_leaf, uint32_t radius,
-                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen) {
+                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen,
+                 const InstanceTlas* inst) {
     if ((uint64_t)tlas_start + n + 1 > t.cap) { snprintf(err, errlen, "the topology holds %llu nodes", (unsigned long long)t.cap); return -3; }
     const int r = (int)(radius < 1 ? 1 : (radius > 64 ? 64 : radius));
     if (!t.d_tlas_arena) { snprintf(err, errlen, "no TLAS build arena (refit_reserve first)"); return -3; }
     Scratch sc(t.d_tlas_arena.get(), t.tlas_arena_bytes);
     float4 *tlo, *thi; uint32_t* perm;
     BCU(sc.alloc(&tlo, (size_t)n * 16)); BCU(sc.alloc(&thi, (size_t)n * 16)); BCU(sc.alloc(&perm, (size_t)n * 4));
-    tlas_boxes_kernel<<<blocks(n), TPB, 0, st>>>(t.d_canon.get(), n, t.d_node_box.get(), tlo, thi);
+    if (inst) {
+        BCU(cudaMemcpyAsync(tlo, inst->h_lo, (size_t)n * 16, cudaMemcpyHostToDevice, st));
+        BCU(cudaMemcpyAsync(thi, inst->h_hi, (size_t)n * 16, cudaMemcpyHostToDevice, st));
+    } else {
+        tlas_boxes_kernel<<<blocks(n), TPB, 0, st>>>(t.d_canon.get(), n, t.d_node_box.get(), tlo, thi);
+    }
     TlasOut to;
     if (const int rc = tlas_run(sc, tlo, thi, n, max_leaf, r, reinsert_knobs(), static_cast<uint8_t*>(d_nodes) + (uint64_t)tlas_start * 80, perm,
                                 st, &to, err, errlen)) return rc;
-    blas_compose_kernel<<<blocks(n), TPB, 0, st>>>(perm, t.d_canon.get(), n, d_blas);
+    if (inst) instance_compose_kernel<<<blocks(n), TPB, 0, st>>>(perm, inst->d_in, n, d_blas, inst->d_rec);
+    else blas_compose_kernel<<<blocks(n), TPB, 0, st>>>(perm, t.d_canon.get(), n, d_blas);
     BCU(cudaGetLastError());
     if (written) BCU(cudaEventRecord(written, st));
     // the BLAS levels stay; the TLAS levels become those of the new tree, every node of which is reached
@@ -1368,6 +1406,29 @@ int rebuild_tlas(RefitTopology& t, void* d_nodes, uint32_t tlas_start, uint32_t 
     BCU(cudaStreamSynchronize(st));
     BCU(cudaGetLastError());
     *n_tlas_nodes = to.n_nodes; *exact = to.co.force_exact;
+    return 0;
+}
+
+int root_nodes(const RefitTopology& t, const void* d_nodes, cudaStream_t st, std::vector<uint4>* out, char* err, size_t errlen) {
+    const uint32_t n = (uint32_t)t.roots.size();
+    out->assign((size_t)n * 5, make_uint4(0, 0, 0, 0));
+    if (!n) return 0;
+    gather_nodes_kernel<<<blocks(n), TPB, 0, st>>>(static_cast<const uint4*>(d_nodes), t.d_roots.get(), n, t.d_root_nodes.get());
+    BCU(cudaGetLastError());
+    BCU(cudaMemcpyAsync(out->data(), t.d_root_nodes.get(), (size_t)n * 80, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int blas_exact(const RefitTopology& t, const void* d_nodes, uint32_t tlas_start, cudaStream_t st, bool* exact, char* err, size_t errlen) {
+    uint32_t* flag = t.d_flag.get();
+    BCU(cudaMemsetAsync(flag, 0, 4, st));
+    if (tlas_start) exact_scan_kernel<<<blocks(tlas_start), TPB, 0, st>>>(static_cast<const uint4*>(d_nodes), tlas_start, flag);
+    BCU(cudaGetLastError());
+    uint32_t f = 0;
+    BCU(cudaMemcpyAsync(&f, flag, 4, cudaMemcpyDeviceToHost, st));
+    BCU(cudaStreamSynchronize(st));
+    *exact = f != 0;
     return 0;
 }
 

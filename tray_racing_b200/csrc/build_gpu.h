@@ -54,6 +54,9 @@ struct RefitTopology {
     DevPtr<uint32_t> d_flag;
     uint64_t cap = 0;                        // nodes d_items and d_node_box have room for
     DevPtr<uint32_t> d_canon;                // two-level: blas_offsets sorted, i.e. the BLAS roots of the instances in canonical order
+    std::vector<uint32_t> roots;             // two-level: the distinct blas_offsets of the walk, ascending (the valid instance roots)
+    DevPtr<uint32_t> d_roots;                // the same on the device
+    DevPtr<uint4> d_root_nodes;              // room for their nodes (root_nodes)
     DevPtr<char> d_tlas_arena;               // device scratch of the TLAS rebuilds (refit_reserve), kept from call to call
     size_t tlas_arena_bytes = 0;
     bool unreached_exact = false;            // a node no root reaches (never rewritten) has an exponent byte >= 167
@@ -78,13 +81,23 @@ int refit_check(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, c
 int refit_run(const RefitTopology& t, const float* d_tris9, uint64_t n_tris, const uint32_t* d_prim_indices, uint32_t tri_stride,
               void* d_nodes, void* d_tris, const uint32_t* d_blas, bool blas_only, cudaStream_t st, bool* exact, char* err, size_t errlen);
 // What a TLAS rebuild of n_instances needs before its first write: room for `cap` nodes in the topology's arrays (the listed items
-// kept), and the rebuild's scratch arena (n_instances x 384 B + 16 MiB), allocated once and kept.  Synchronous on `st`.
+// kept), and the rebuild's scratch arena (n_instances x 384 B + 16 MiB), allocated by the first call and grown by a call with more
+// instances than any before it.  Synchronous on `st`.
 int refit_reserve(RefitTopology& t, uint64_t cap, uint32_t n_instances, cudaStream_t st, char* err, size_t errlen);
+// The TLAS of an instanced scene (tray_cuda_scene_set_instances): the boxes of instance k are h_lo[k] / h_hi[k] (host memory, xyz),
+// its InstanceRecord (traverse.cuh) d_in[4k .. 4k + 3] with the instance id k.
+struct InstanceTlas { const float4* h_lo; const float4* h_hi; const uint4* d_in; uint4* d_rec; };
 // TLAS rebuild (tray_cuda_scene_refit_rebuild_tlas), after refit_run(blas_only): the TLAS leg of build_tlas over the BLAS root
 // boxes of the n instances in canonical order, written at node tlas_start of d_nodes; d_blas[j] = the root of TLAS leaf j; the
 // topology's TLAS levels become the new tree's (refit_reserve(tlas_start + n + 1) first).  `written` (optional) is recorded
 // behind the last TLAS write.  *n_tlas_nodes, and *exact = some new TLAS node's exponent byte is >= 167.  Synchronous on `st`.
+// With `inst`: over the instances' boxes in instance order instead; d_rec[4j ..] = the InstanceRecord of TLAS leaf j.
 int rebuild_tlas(RefitTopology& t, void* d_nodes, uint32_t tlas_start, uint32_t n, uint32_t* d_blas, uint32_t max_leaf, uint32_t radius,
-                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen);
+                 cudaStream_t st, cudaEvent_t written, uint32_t* n_tlas_nodes, bool* exact, char* err, size_t errlen,
+                 const InstanceTlas* inst = nullptr);
+// The first 80-byte node of each of t.roots, as 5 uint4 per root in `out`.  Synchronous on `st`.
+int root_nodes(const RefitTopology& t, const void* d_nodes, cudaStream_t st, std::vector<uint4>* out, char* err, size_t errlen);
+// *exact = some node below tlas_start has an exponent byte >= 167 (tray::node_needs_exact).  Synchronous on `st`.
+int blas_exact(const RefitTopology& t, const void* d_nodes, uint32_t tlas_start, cudaStream_t st, bool* exact, char* err, size_t errlen);
 
 }  // namespace tray_build

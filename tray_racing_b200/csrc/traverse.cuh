@@ -103,7 +103,15 @@ struct TraceParams {
     uint32_t* __restrict__ unit_cursor;       // next tile whose bounce rays have not been claimed (zeroed by the host)
     uint32_t n_units;                         // n_work / 32: bounce work is claimed in groups of 32 items
     uint32_t gen_min;                         // idle lanes needed before the warp generates bounce rays into them
+    // INST kernels only (instanced scenes, tray_cuda_scene_set_instances).  Appended, so that the members above keep their offsets.
+    const uint4* __restrict__ inst_rec;       // per TLAS leaf, an InstanceRecord
+    uint32_t* __restrict__ inst_out;          // optional: the instance of each hit by output item (INVALID for a miss)
 };
+
+// One instance as the device reads it, 64 bytes: rows 0..2 of world_to_object ([W | -W t], 4 floats each), then {BLAS root,
+// instance id, 0, 0}.  The TLAS holds one per leaf in leaf order; the scene keeps the same records by instance id for the bounce
+// normals.
+constexpr uint32_t INST_RECORD_U4 = 4;
 
 // ---- exact float helpers (no contraction, IEEE rounding) --------------------------------------
 __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
@@ -438,10 +446,13 @@ __device__ __forceinline__ void sincos_tau(float u, float& s, float& c) {
 }
 
 // bounce ray from a primary hit (src/rt_cpu/rt_cpu.rs:61-76; basis sampling.hlsl:39-51)
-template <int TRI_STRIDE>
+// INST: `xf` is the InstanceRecord of the hit's instance; the object-space normal goes to world space through the transpose of
+// world_to_object, n'_i = W_0i n_0 + W_1i n_1 + W_2i n_2 (the inverse transpose of object_to_world), before it is normalised.
+template <int TRI_STRIDE, bool INST = false>
 __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __restrict__ tris, uint32_t px, uint32_t py,
                                            float pdx, float pdy, float pdz, float t, uint32_t prim,
-                                           float& ox, float& oy, float& oz, float& dx, float& dy, float& dz) {
+                                           float& ox, float& oy, float& oz, float& dx, float& dy, float& dz,
+                                           const uint4* __restrict__ xf = nullptr) {
     float nx, ny, nz;
     if (TRI_STRIDE == 64) {
         const uint4 g = __ldg(tris + (size_t)prim * 4u + 3);
@@ -450,6 +461,13 @@ __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __
         float v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z;
         tri_load<TRI_STRIDE>(tris, prim, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z);
         cross3(e1x, e1y, e1z, e2x, e2y, e2z, nx, ny, nz);
+    }
+    if constexpr (INST) {
+        const uint4 w0 = __ldg(xf), w1 = __ldg(xf + 1), w2 = __ldg(xf + 2);
+        const float wx = dot3(__uint_as_float(w0.x), __uint_as_float(w1.x), __uint_as_float(w2.x), nx, ny, nz);
+        const float wy = dot3(__uint_as_float(w0.y), __uint_as_float(w1.y), __uint_as_float(w2.y), nx, ny, nz);
+        const float wz = dot3(__uint_as_float(w0.z), __uint_as_float(w1.z), __uint_as_float(w2.z), nx, ny, nz);
+        nx = wx; ny = wy; nz = wz;
     }
     normalize3(nx, ny, nz);                                                    // RtTriangle::compute_normal
     const float sgn = copysignf(1.0f, dot3(nx, ny, nz, -pdx, -pdy, -pdz));     // f32::signum (rt_cpu.rs:65)
@@ -526,12 +544,14 @@ __global__ void __launch_bounds__(256) raygen_primary_kernel(const __grid_consta
 // One thread per pixel of the shard.  Hit pixels append their bounce ray to a compact list (one atomicAdd per block;
 // `ray_item` remembers the pixel); missed pixels get their final results here.
 constexpr int BOUNCE_BLOCK = 1024;    // pixels per block of raygen_bounce_kernel = the group its rays are sorted in
-template <int TRI_STRIDE>
+// INST (instanced scenes): `primary_inst` holds the instance of each primary hit, `inst_xf` the InstanceRecords by instance id.
+template <int TRI_STRIDE, bool INST = false>
 __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __grid_constant__ FrameParams F, const uint4* __restrict__ tris,
                                                             const tray_hit* __restrict__ primary, tray_ray* __restrict__ rays,
                                                             uint32_t* __restrict__ ray_item, uint32_t* __restrict__ n_rays,
                                                             tray_hit* __restrict__ bounce_out, uchar4* __restrict__ rgba_out,
-                                                            tray_ray* __restrict__ rays_by_item, uint32_t row_major) {
+                                                            tray_ray* __restrict__ rays_by_item, uint32_t row_major,
+                                                            const uint32_t* __restrict__ primary_inst, const uint4* __restrict__ inst_xf) {
     __shared__ uint32_t s_cnt[8], s_base[8];
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t px = 0, py = 0;
@@ -545,7 +565,11 @@ __global__ void __launch_bounds__(BOUNCE_BLOCK) raygen_bounce_kernel(const __gri
     if (shoot) {
         float pdx, pdy, pdz; primary_dir(F, px, py, pdx, pdy, pdz);
         float ox, oy, oz, dx, dy, dz;
-        bounce_ray<TRI_STRIDE>(F, tris, px, py, pdx, pdy, pdz, ph.t, ph.prim, ox, oy, oz, dx, dy, dz);
+        if constexpr (INST)
+            bounce_ray<TRI_STRIDE, true>(F, tris, px, py, pdx, pdy, pdz, ph.t, ph.prim, ox, oy, oz, dx, dy, dz,
+                                         inst_xf + (size_t)primary_inst[j] * INST_RECORD_U4);
+        else
+            bounce_ray<TRI_STRIDE>(F, tris, px, py, pdx, pdy, pdz, ph.t, ph.prim, ox, oy, oz, dx, dy, dz);
         a = make_float4(ox, oy, oz, 0.0f); b = make_float4(dx, dy, dz, F32_MAX_);
     }
     // The rays of the block's 1024 pixels (4 tiles: close origins) are appended grouped by direction octant, so that the
@@ -627,8 +651,14 @@ __device__ __forceinline__ void flush_counters(unsigned long long* dst, unsigned
 // (A MODE 2 — relaxed order: triangle postponing, tolerance parity — was built and measured in round 2 and is NOT in the
 // product: on CWBVHs of this shape 81 % of the nodes hold only leaves, so a lane almost never has triangles and child nodes in
 // hand at once; nothing was postponed, nothing mismatched, and the extra vote cost 3 %.  profiles/experiments/r2_relaxed_*.)
-template <bool TLAS, bool COUNT, int TRI_STRIDE, bool ANYHIT = false, bool FRAME = false, int MODE = 0>
+// INST (instanced scenes; TLAS, MODE 0, not FRAME): a TLAS leaf places its BLAS by a transform.  Entering it, the lane maps its
+// ray into object space with the leaf's world_to_object (origin o' = W o + t, direction d' = W d, not normalised, so tmin, tmax
+// and the t of a hit keep their world meaning) and prepares that ray; back at the TLAS it prepares the world ray again, re-read
+// from P.rays at its index (both callers, batch traces and the two-launch frame, hold every ray there) instead of holding six
+// more registers.  best_inst follows best_prim.
+template <bool TLAS, bool COUNT, int TRI_STRIDE, bool ANYHIT = false, bool FRAME = false, int MODE = 0, bool INST = false>
 __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(const __grid_constant__ TraceParams P) {
+    static_assert(!INST || (TLAS && !FRAME && MODE == 0), "instance transforms exist in the two-level MODE 0 batch kernels only");
     __shared__ uint8_t s_lut[LUT_BYTES];          // child_order[oct_inv][hit byte] (see node_test)
     uint2 spill[STACK_SPILL];
     child_order_fill(s_lut, threadIdx.x, BLOCK_THREADS);
@@ -654,6 +684,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
     auto stk_store = [&](uint32_t off, uint32_t x, uint32_t y) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" :: "r"(stk_base + off), "r"(x), "r"(y) : "memory"); };
     auto stk_load = [&](uint32_t off) { uint2 e; asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(e.x), "=r"(e.y) : "r"(stk_base + off) : "memory"); return e; };
     uint32_t tlas_sp = INVALID, bvh_off = 0;
+    uint32_t cur_inst = 0, best_inst = INVALID;  // INST: the instance the lane is in, the instance of best_prim
     uint32_t ray_idx = 0;
     bool exhausted = false;                      // warp-uniform
     // a lane starts fewer than 2^30 rays per launch (INDEX_MASK), so its ray and hit counts fit 32 bits
@@ -683,6 +714,11 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
         cur_x = 0; cur_y = 0x80000000u; tri_x = 0; tri_y = 0; sp &= SP_STEP - 1u;
         tlas_sp = INVALID; bvh_off = TLAS ? P.tlas_start : 0u;
         if constexpr (COUNT) { r_nodes = 0; r_tris = 0; r_insts = 0; r_peak = 0; }
+    };
+    // INST: the lane's ray becomes (o, d) with the same tmin: octant row, zero-direction patch and WIDE_BIT follow it
+    auto switch_ray = [&](float ox, float oy, float oz, float dx, float dy, float dz) {
+        prepare_ray(r, ox, oy, oz, dx, dy, dz, r.tmin, 0u, (uint32_t)__cvta_generic_to_shared(s_lut));
+        ray_idx = r.wide ? (ray_idx | WIDE_BIT) : (ray_idx & ~WIDE_BIT);
     };
     // COUNT builds, a ray retires: its counts join the warp totals of its pass, and its record goes to slot `item` of P.ray_cost
     // (`if constexpr` here and at every use of the r_* registers: the kernels that do not count compile to the code they had
@@ -716,11 +752,19 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
             const uint32_t ri = ray_idx & INDEX_MASK;
             const uint32_t item = P.ray_item ? __ldg(P.ray_item + ri) : ri;
             P.hits_out[item] = h;
+            if constexpr (INST) { if (P.inst_out) P.inst_out[item] = best_prim != INVALID ? best_inst : INVALID; }
             store_rgba(P.rgba_out, P.frame, P.row_major, item, P.shade_mode, h.t);
             if constexpr (COUNT) retire_cost(item, best_prim != INVALID);
             cur_x = 0; cur_y = 0;                                                                    // IDLE
         } else {
-            if (TLAS && sp == tlas_sp) { tlas_sp = INVALID; bvh_off = P.tlas_start; }
+            if (TLAS && sp == tlas_sp) {
+                tlas_sp = INVALID; bvh_off = P.tlas_start;
+                if constexpr (INST) {                                                    // back to the world ray
+                    const float4* rp = reinterpret_cast<const float4*>(P.rays + (ray_idx & INDEX_MASK));
+                    const float4 a = __ldg(rp), b = __ldg(rp + 1);
+                    switch_ray(a.x, a.y, a.z, b.x, b.y, b.z);
+                }
+            }
             sp -= SP_STEP;
             const uint2 e = sp < SP_SMEM_END ? stk_load(sp) : spill[sp / SP_STEP - STACK_SMEM];
             if (e.y & 0xff000000u) { cur_x = e.x; cur_y = e.y; }
@@ -856,7 +900,23 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     if (tri_y != 0u) push(tri_x, tri_y);
                     if (cur_y & 0xff000000u) push(cur_x, cur_y);
                     tlas_sp = sp;
-                    bvh_off = __ldg(P.blas_offsets + g);
+                    if constexpr (INST) {
+                        // into object space: o' = W o + t and d' = W d of the caller's direction (not the zero-patched one)
+                        const uint4* rec = P.inst_rec + (size_t)g * INST_RECORD_U4;
+                        const uint4 w0 = __ldg(rec), w1 = __ldg(rec + 1), w2 = __ldg(rec + 2), w3 = __ldg(rec + 3);
+                        const float4 d = __ldg(reinterpret_cast<const float4*>(P.rays + (ray_idx & INDEX_MASK)) + 1);
+                        bvh_off = w3.x; cur_inst = w3.y;
+                        auto row = [&](const uint4& w, float& o, float& dd) {
+                            const float m0 = __uint_as_float(w.x), m1 = __uint_as_float(w.y), m2 = __uint_as_float(w.z);
+                            o = add(add(add(mul(m0, r.ox), mul(m1, r.oy)), mul(m2, r.oz)), __uint_as_float(w.w));
+                            dd = dot3(m0, m1, m2, d.x, d.y, d.z);
+                        };
+                        float ox, oy, oz, dx, dy, dz;
+                        row(w0, ox, dx); row(w1, oy, dy); row(w2, oz, dz);
+                        switch_ray(ox, oy, oz, dx, dy, dz);
+                    } else {
+                        bvh_off = __ldg(P.blas_offsets + g);
+                    }
                     TRAY_CNT(insts);
                     cur_x = 0; cur_y = 0x80000000u; tri_y = 0;
                 } else {
@@ -875,10 +935,10 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     const float t = tri_test<TRI_STRIDE, MODE == 1>(r, best_t, P.tris, g);
                     // CPU tie rule: first of equal t wins (§8a a11); TRAY_VARIANT_TIE_LAST: the HLSL's `tt <= t` (query.hlsl:120)
                     const bool closer = (MODE == 1 && (P.variant & TRAY_VARIANT_TIE_LAST)) ? (t <= best_t && t < __int_as_float(0x7f800000)) : (t < best_t);
-                    if (closer) { best_t = t; best_prim = g; }
+                    if (closer) { best_t = t; best_prim = g; if constexpr (INST) best_inst = cur_inst; }
                     if (two && !(ANYHIT && best_prim != INVALID)) {      // (any-hit: the reference never runs the second test after a hit)
                         TRAY_CNT(tris);
-                        if (t2 < best_t) { best_t = t2; best_prim = g2; }
+                        if (t2 < best_t) { best_t = t2; best_prim = g2; if constexpr (INST) best_inst = cur_inst; }
                     }
                     if (ANYHIT && best_prim != INVALID) { sp &= SP_STEP - 1u; tri_y = 0u; cur_y = 0u; }   // drop the rest of the traversal
                     if (tri_y == 0u && cur_y < 0x01000000u) pop_or_retire();

@@ -2,7 +2,9 @@
 // No CPU fallback exists: without a CUDA device every compute entry point fails with TRAY_ERR_NO_DEVICE.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -69,6 +71,8 @@ struct FrameSlot {
     tray_ray* d_brays_item = nullptr;        // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
     tray_ray_cost* d_cost = nullptr;         // optional: ray costs by local item, 2 x f_cap: primary [0, n_items), bounce from n_items
     bool f_has_cost = false;                 // the last frame kept ray costs (tray_cuda_scene_set_ray_cost + TRAY_RENDER_COUNTERS)
+    uint32_t* d_pinst = nullptr; uint32_t* d_binst = nullptr;   // instanced scenes: the instance of each primary / bounce hit by item
+    bool f_has_inst = false;                 // the last frame was rendered on an instanced scene
     uint32_t* d_flag = nullptr;              // the device error word of this slot's launches (a word of tray_scene::d_overflow)
     tray::FrameParams last_frame{};          // width 0: no frame rendered yet
 };
@@ -100,9 +104,20 @@ struct tray_scene {
     bool counting = false;                   // tray_cuda_set_counting: batch traces count (a render counts with TRAY_RENDER_COUNTERS alone)
     bool ray_cost = false;                   // tray_cuda_scene_set_ray_cost: counted renders keep every ray's cost
     uint32_t variant = 0;                    // TRAY_VARIANT_* (tray_cuda_scene_set_variant): the MODE 1 kernels
+    // instanced scenes (tray_cuda_scene_set_instances): the INST kernels
+    bool instanced = false;
+    uint32_t inst_cap = 0, blas_cap = 0;     // instance records / blas_offsets entries the device arrays have room for
+    uint4* d_inst_in = nullptr;              // InstanceRecord (traverse.cuh) by instance id
+    uint4* d_inst_rec = nullptr;             // InstanceRecord by TLAS leaf (TraceParams::inst_rec)
+    std::vector<uint32_t> inst_roots;        // the caller's blas_roots and object_to_world of the last set_instances
+    std::vector<float> inst_o2w;
+    uint32_t* d_inst_ids = nullptr; uint64_t inst_ids_cap = 0;   // tray_cuda_trace_instance: allocated on first use
+    uint32_t* h_inst[2] = { nullptr, nullptr };                  // pinned instance-id slots of the pipelined host path
     uint32_t refill_min = 6, tri_weight = 3, gen_min = 4;
     bool overlap_default = false;            // TRAY_CUDA_OVERLAP=1: tray_cuda_render always takes the one-launch frame kernel
-    int blocks_per_sm[3] = { 0, 0, 0 };      // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1], the counting lane kernel [2]
+    // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1], the counting lane kernel [2], the INST kernel [3] and the
+    // counting INST kernel [4]
+    int blocks_per_sm[5] = { 0, 0, 0, 0, 0 };
     // ray-batch staging
     tray_ray* d_rays = nullptr; tray_hit* d_hits = nullptr; uint64_t batch_cap = 0;
     tray_ray_cost* d_costs = nullptr; uint64_t cost_cap = 0;   // tray_cuda_trace_cost: allocated on first use
@@ -134,7 +149,8 @@ void free_pipeline(tray_scene* s) {
         if (s->h_rays[i]) cudaFreeHost(s->h_rays[i]);
         if (s->h_hits[i]) cudaFreeHost(s->h_hits[i]);
         if (s->h_costs[i]) cudaFreeHost(s->h_costs[i]);
-        s->h_costs[i] = nullptr;
+        if (s->h_inst[i]) cudaFreeHost(s->h_inst[i]);
+        s->h_costs[i] = nullptr; s->h_inst[i] = nullptr;
         if (s->e_in[i]) cudaEventDestroy(s->e_in[i]);
         if (s->e_k[i]) cudaEventDestroy(s->e_k[i]);
         if (s->e_out[i]) cudaEventDestroy(s->e_out[i]);
@@ -151,20 +167,26 @@ typedef void (*kernel_fn)(const TraceParams);
 
 // The trace_kernel instantiation of a launch. MODE 0: every (tlas, count, stride) x {closest hit, any hit, frame}.
 // MODE 1 (variant) exists without counters only, so it ignores `count` (launch() rejects that combination).
+// INST (instanced scenes): two-level closest hit and any hit, with and without counters; the callers never ask it for a frame
+// kernel or a variant.
 template <bool TLAS, bool COUNT, int STRIDE>
-kernel_fn pick_kernel(bool anyhit, bool frame, bool variant) {
+kernel_fn pick_kernel(bool anyhit, bool frame, bool variant, bool inst) {
     if (variant) return (kernel_fn)trace_kernel<TLAS, false, STRIDE, false, false, 1>;
     if (frame) return (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, false, true>;
+    if constexpr (TLAS) {
+        if (inst) return anyhit ? (kernel_fn)trace_kernel<true, COUNT, STRIDE, true, false, 0, true>
+                                : (kernel_fn)trace_kernel<true, COUNT, STRIDE, false, false, 0, true>;
+    }
     return anyhit ? (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, true> : (kernel_fn)trace_kernel<TLAS, COUNT, STRIDE, false>;
 }
 template <bool TLAS, bool COUNT>
-kernel_fn pick_kernel(uint32_t stride, bool anyhit, bool frame, bool variant) {
-    return stride == 64 ? pick_kernel<TLAS, COUNT, 64>(anyhit, frame, variant)
-         : stride == 24 ? pick_kernel<TLAS, COUNT, 24>(anyhit, frame, variant) : pick_kernel<TLAS, COUNT, 48>(anyhit, frame, variant);
+kernel_fn pick_kernel(uint32_t stride, bool anyhit, bool frame, bool variant, bool inst) {
+    return stride == 64 ? pick_kernel<TLAS, COUNT, 64>(anyhit, frame, variant, inst)
+         : stride == 24 ? pick_kernel<TLAS, COUNT, 24>(anyhit, frame, variant, inst) : pick_kernel<TLAS, COUNT, 48>(anyhit, frame, variant, inst);
 }
-kernel_fn pick_kernel(bool tlas, bool count, uint32_t stride, bool anyhit, bool frame, bool variant) {
-    if (tlas) return count ? pick_kernel<true, true>(stride, anyhit, frame, variant) : pick_kernel<true, false>(stride, anyhit, frame, variant);
-    return count ? pick_kernel<false, true>(stride, anyhit, frame, variant) : pick_kernel<false, false>(stride, anyhit, frame, variant);
+kernel_fn pick_kernel(bool tlas, bool count, uint32_t stride, bool anyhit, bool frame, bool variant, bool inst) {
+    if (tlas) return count ? pick_kernel<true, true>(stride, anyhit, frame, variant, inst) : pick_kernel<true, false>(stride, anyhit, frame, variant, inst);
+    return count ? pick_kernel<false, true>(stride, anyhit, frame, variant, inst) : pick_kernel<false, false>(stride, anyhit, frame, variant, inst);
 }
 
 uint64_t local_items(uint32_t w, uint32_t h, uint32_t shard, uint32_t shards) {
@@ -179,6 +201,7 @@ void base_params(const tray_scene* s, TraceParams& P) {
     P.cursor = (uint32_t*)s->d_cursor; P.overflow = s->d_overflow;
     P.refill_min = s->refill_min; P.tri_weight = s->tri_weight; P.k4b = 0x4B000000u; P.force_exact = s->force_exact ? 1u : 0u;
     P.variant = s->variant; P.one = 1u;
+    P.inst_rec = s->d_inst_rec;
 }
 
 const char* const VARIANT_REFUSAL = "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only";
@@ -188,8 +211,8 @@ const char* const VARIANT_REFUSAL = "semantic variants (tray_cuda_scene_set_vari
 // `count`: the counting kernels (tray_scene::counting for batch traces, TRAY_RENDER_COUNTERS for the launches of one frame)
 int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* cur, int counter_slot, bool count, bool anyhit = false, bool keep_counters = false, bool frame = false) {
     if (s->variant && (anyhit || frame || count)) return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);
-    kernel_fn k = pick_kernel(s->tlas, count, s->tri_stride, anyhit, frame, s->variant != 0);
-    int& bps = s->blocks_per_sm[s->variant ? 1 : count ? 2 : 0];
+    kernel_fn k = pick_kernel(s->tlas, count, s->tri_stride, anyhit, frame, s->variant != 0, s->instanced);
+    int& bps = s->blocks_per_sm[s->variant ? 1 : s->instanced ? (count ? 4 : 3) : count ? 2 : 0];
     if (bps == 0) {
         int nb = 0;
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, BLOCK_THREADS, 0));
@@ -230,9 +253,9 @@ int sync_streams(const tray_scene* s, bool scene_stream_first) {
 // the per-frame buffers of a slot (not its cursor block); the caller has synchronised the slot's stream
 void free_frame_buffers(FrameSlot& f) {
     cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
-    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item); cudaFree(f.d_cost);
+    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item); cudaFree(f.d_cost); cudaFree(f.d_pinst); cudaFree(f.d_binst);
     f.d_primary = nullptr; f.d_bounce = nullptr; f.d_brays = nullptr; f.d_rgba = nullptr;
-    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.d_cost = nullptr; f.f_cap = 0;
+    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.d_cost = nullptr; f.d_pinst = nullptr; f.d_binst = nullptr; f.f_cap = 0;
 }
 
 int check_tri_stride(uint32_t tri_stride) {
@@ -417,6 +440,7 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     if (s->stream) cudaStreamSynchronize(s->stream);
     cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
     cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_costs); cudaFree(s->d_geom_offsets);
+    cudaFree(s->d_inst_in); cudaFree(s->d_inst_rec); cudaFree(s->d_inst_ids);
     delete s->refit;
     free_pipeline(s);
     cudaFree(s->d_untiled);
@@ -475,7 +499,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
     tray_scene* s = new (std::nothrow) tray_scene();
     if (!s) return fail(TRAY_ERR_ARG, "out of host memory");
     s->device = device; s->n_nodes = n_nodes; s->n_tris = n_tris; s->tri_stride = tri_stride;
-    s->n_instances = n_instances; s->tlas_start = tlas_start; s->tlas = n_instances > 0;
+    s->n_instances = n_instances; s->tlas_start = tlas_start; s->tlas = n_instances > 0; s->blas_cap = n_instances;
     s->refill_min = (uint32_t)env_int("TRAY_CUDA_REFILL_MIN", 6);       // 6: +0.3 % (C3) ... +2 % (C1) over 4 with the r2 kernel (profiles/experiments/r2_refill_min_ab.log)
     s->force_exact = scene_force_exact(built && built->force_exact);
     for (uint64_t i = 0; !built && i < n_nodes && !s->force_exact; i++) {
@@ -649,6 +673,7 @@ int tray_cuda_scene_set_ray_cost(tray_scene* s, int enabled) {
 int tray_cuda_scene_set_variant(tray_scene* s, uint32_t flags) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     if (flags & ~0xfu) return fail(TRAY_ERR_ARG, "unknown variant flags 0x%x", flags);
+    if (s->instanced) return fail(TRAY_ERR_ARG, "an instanced scene has no semantic variants");
     s->variant = flags;
     return TRAY_OK;
 }
@@ -783,6 +808,144 @@ void adopt_rebuilt_tlas(tray_scene* s, uint4* nodes, uint64_t cap, uint32_t m) {
     }
 }
 
+// the f32 below / above a double (rule 5 of tray_cuda_scene_set_instances: __double2float_rd / _ru)
+float f32_down(double x) { const float f = (float)x; return (double)f > x ? nextafterf(f, -INFINITY) : f; }
+float f32_up(double x) { const float f = (float)x; return (double)f < x ? nextafterf(f, INFINITY) : f; }
+
+// world_to_object of one instance: the adjugate of R over its determinant and -W t, in double, rounded to nearest f32.  False for
+// a zero determinant or a rounded inverse that is not finite.  (Host code in double: x86-64 has no fused multiply-add to contract to.)
+bool invert_xform(const float* M, float* W) {
+    double m[3][4];
+    for (int i = 0; i < 3; i++) for (int j = 0; j < 4; j++) m[i][j] = M[4 * i + j];
+    double a[3][3];
+    a[0][0] = m[1][1] * m[2][2] - m[1][2] * m[2][1]; a[0][1] = m[0][2] * m[2][1] - m[0][1] * m[2][2]; a[0][2] = m[0][1] * m[1][2] - m[0][2] * m[1][1];
+    a[1][0] = m[1][2] * m[2][0] - m[1][0] * m[2][2]; a[1][1] = m[0][0] * m[2][2] - m[0][2] * m[2][0]; a[1][2] = m[0][2] * m[1][0] - m[0][0] * m[1][2];
+    a[2][0] = m[1][0] * m[2][1] - m[1][1] * m[2][0]; a[2][1] = m[0][1] * m[2][0] - m[0][0] * m[2][1]; a[2][2] = m[0][0] * m[1][1] - m[0][1] * m[1][0];
+    const double det = (m[0][0] * a[0][0] + m[0][1] * a[1][0]) + m[0][2] * a[2][0];
+    if (det == 0.0 || !std::isfinite(det)) return false;
+    for (int i = 0; i < 3; i++) {
+        double w[3];
+        for (int j = 0; j < 3; j++) w[j] = a[i][j] / det;
+        const double t = -((w[0] * m[0][3] + w[1] * m[1][3]) + w[2] * m[2][3]);
+        for (int j = 0; j < 3; j++) W[4 * i + j] = (float)w[j];
+        W[4 * i + 3] = (float)t;
+        for (int j = 0; j < 4; j++) if (!std::isfinite(W[4 * i + j])) return false;
+    }
+    return true;
+}
+
+// The TLAS primitives of n instances (rules 1-5 of tray_cuda_scene_set_instances), over the current root nodes of the BLAS in
+// `nodes`.  1: no instance box is finite in f32 (or a root has no used slot), -2 (with *msg): a CUDA error.
+int instance_boxes(tray_scene* s, const void* nodes, const uint32_t* roots, const float* o2w, uint32_t n, std::vector<float4>& lo,
+                   std::vector<float4>& hi, char* msg, size_t len) {
+    const tray_build::RefitTopology& t = *s->refit;
+    std::vector<uint4> rn;
+    if (tray_build::root_nodes(t, nodes, s->stream, &rn, msg, len)) return -2;
+    auto u8 = [](uint32_t w, int j) { return (double)((w >> (8 * j)) & 0xffu); };
+    std::vector<double> rb(t.roots.size() * 6);
+    for (size_t r = 0; r < t.roots.size(); r++) {
+        const uint4* nd = &rn[5 * r];
+        const uint32_t pw[3] = { nd[0].x, nd[0].y, nd[0].z };
+        const uint4 q[3] = { nd[2], nd[3], nd[4] };
+        double* b = &rb[6 * r];
+        for (int a = 0; a < 3; a++) { b[a] = INFINITY; b[3 + a] = -INFINITY; }
+        for (int sl = 0; sl < 8; sl++) {
+            if (u8(sl < 4 ? nd[1].z : nd[1].w, sl & 3) == 0.0) continue;                        // child_meta == 0: an empty slot
+            for (int a = 0; a < 3; a++) {
+                float p; memcpy(&p, &pw[a], 4);
+                const double scale = ldexp(1.0, (int)((nd[0].w >> (8 * a)) & 0xffu) - 127);
+                const double l = (double)p + u8(sl < 4 ? q[a].x : q[a].y, sl & 3) * scale;
+                const double h = (double)p + u8(sl < 4 ? q[a].z : q[a].w, sl & 3) * scale;
+                b[a] = std::min(b[a], l); b[3 + a] = std::max(b[3 + a], h);
+            }
+        }
+    }
+    lo.resize(n); hi.resize(n);
+    for (uint32_t k = 0; k < n; k++) {
+        const double* b = &rb[6 * (std::lower_bound(t.roots.begin(), t.roots.end(), roots[k]) - t.roots.begin())];
+        if (!(b[0] <= b[3])) return 1;
+        const float* M = o2w + 12 * (size_t)k;
+        double mn[3] = { INFINITY, INFINITY, INFINITY }, mx[3] = { -INFINITY, -INFINITY, -INFINITY };
+        for (int c = 0; c < 8; c++) {
+            const double x = b[(c & 1) ? 3 : 0], y = b[(c & 2) ? 4 : 1], z = b[(c & 4) ? 5 : 2];
+            for (int i = 0; i < 3; i++) {
+                const double v = (((double)M[4 * i] * x + (double)M[4 * i + 1] * y) + (double)M[4 * i + 2] * z) + (double)M[4 * i + 3];
+                mn[i] = std::min(mn[i], v); mx[i] = std::max(mx[i], v);
+            }
+        }
+        double big = 0.0;
+        for (int i = 0; i < 3; i++) big = std::max(big, std::max(std::fabs(mn[i]), std::fabs(mx[i])));
+        const double pad = ldexp(big, -18);
+        lo[k] = make_float4(f32_down(mn[0] - pad), f32_down(mn[1] - pad), f32_down(mn[2] - pad), 0.f);
+        hi[k] = make_float4(f32_up(mx[0] + pad), f32_up(mx[1] + pad), f32_up(mx[2] + pad), 0.f);
+        for (float v : { lo[k].x, lo[k].y, lo[k].z, hi[k].x, hi[k].y, hi[k].z }) if (!std::isfinite(v)) return 1;
+    }
+    return 0;
+}
+
+// the refit topology of the scene, walked by the first call that needs it
+int ensure_topology(tray_scene* s, char* msg, size_t len) {
+    if (s->refit) return TRAY_OK;
+    tray_build::RefitTopology t;
+    const int rc = tray_build::refit_walk(s->d_nodes, s->n_nodes, s->n_tris, s->tlas ? s->d_blas : nullptr, s->tlas ? s->n_instances : 0u,
+                                          s->tlas_start, s->stream, &t, msg, len);
+    if (rc) return fail(rc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "refit: %s", msg);
+    s->refit = new (std::nothrow) tray_build::RefitTopology(std::move(t));
+    if (!s->refit) return fail(TRAY_ERR_ARG, "out of host memory");
+    s->device_bytes += s->refit->bytes;
+    return TRAY_OK;
+}
+
+// after every frame and batch enqueued so far (and the work on `stream`): frames rendered before keep their results
+int drain_scene(tray_scene* s, void* stream) {
+    if (stream) CU(cudaStreamSynchronize((cudaStream_t)stream));
+    if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
+    CU(cudaStreamSynchronize(s->copy_stream));
+    if (s->pipeline_ready) { CU(cudaStreamSynchronize(s->s_in)); CU(cudaStreamSynchronize(s->s_out)); }
+    return TRAY_OK;
+}
+
+// The TLAS leg of tray_cuda_scene_refit_rebuild_tlas and tray_cuda_scene_set_instances, from the first write on, for n instances:
+// the node array grown to tlas_start + n + 1 nodes, the topology's room and scratch, then `blas(nodes, &exact)` (the BLAS refit of
+// a rebuild, the exact-node scan of set_instances), then the TLAS, adopted by the scene.  An instanced scene's TLAS is over
+// `lo` / `hi`, or, when they are NULL, over the boxes of its instances on the refit roots.  ev[0] is the caller's; *ms ends at the
+// last TLAS write.  Every failure here is a CUDA error, never a refusal.
+template <typename Blas>
+int tlas_leg(tray_scene* s, uint32_t n, const TlasRebuild& rb, const std::vector<float4>* lo, const std::vector<float4>* hi, Blas blas,
+             float* ms, char* msg, size_t len) {
+    const uint64_t cap = (uint64_t)s->tlas_start + n + 1;
+    tray_build::DevPtr<uint4> grown;      // a created scene's node array holds n_nodes: the first rebuild that needs more grows it
+    if (cap > s->node_cap) {
+        uint4* p = nullptr;
+        CU(cudaMalloc(&p, cap * 80));
+        grown.reset(p);
+        CU(cudaMemcpyAsync(p, s->d_nodes, (size_t)s->tlas_start * 80, cudaMemcpyDeviceToDevice, s->stream));
+    }
+    const uint64_t held = s->refit->bytes;
+    if (tray_build::refit_reserve(*s->refit, cap, n, s->stream, msg, len)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+    s->device_bytes += s->refit->bytes - held;
+    uint4* nodes = grown ? grown.get() : s->d_nodes;
+    bool exact = false, tlas_exact = false;
+    uint32_t m = 0;
+    if (const int rc = blas(nodes, &exact)) return rc;
+    std::vector<float4> rlo, rhi;
+    if (s->instanced && !lo) {
+        const int rc = instance_boxes(s, nodes, s->inst_roots.data(), s->inst_o2w.data(), n, rlo, rhi, msg, len);
+        if (rc) return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", rc > 0 ? "an instance box is not finite in f32 after the refit" : msg);
+        lo = &rlo; hi = &rhi;
+    }
+    const tray_build::InstanceTlas it{ lo ? lo->data() : nullptr, hi ? hi->data() : nullptr, s->d_inst_in, s->d_inst_rec };
+    if (tray_build::rebuild_tlas(*s->refit, nodes, s->tlas_start, n, s->d_blas, rb.max_leaf, rb.radius ? rb.radius : 14u, s->stream, s->ev[1],
+                                 &m, &tlas_exact, msg, len, lo ? &it : nullptr))
+        return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", msg);
+    float t = 0.f;
+    CU(cudaEventElapsedTime(&t, s->ev[0], s->ev[1]));
+    adopt_rebuilt_tlas(s, grown ? grown.release() : s->d_nodes, cap, m);
+    s->force_exact = scene_force_exact(exact || tlas_exact);
+    if (ms) *ms = t;
+    return TRAY_OK;
+}
+
 // tray_cuda_scene_refit(_device), and with `rb` tray_cuda_scene_refit_rebuild_tlas(_device): `tris9` is host memory unless
 // `device_ptr`.  Every check runs before the first write, so a refused call leaves nodes, records, blas_offsets, n_nodes and
 // force_exact as they were.
@@ -790,6 +953,7 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
     if (ms_refit) *ms_refit = 0.f;
     if (!s || !tris9) return fail(TRAY_ERR_ARG, "NULL argument");
     if (n_tris != s->n_tris) return fail(TRAY_ERR_ARG, "refit with %llu triangles, the scene has %llu", (unsigned long long)n_tris, (unsigned long long)s->n_tris);
+    if (!rb && s->instanced) return fail(TRAY_ERR_ARG, "refit: an instanced scene's TLAS leaves are transformed boxes (use refit_rebuild_tlas)");
     if (rb) {
         if (!s->tlas) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: the scene has no TLAS");
         if (rb->max_leaf < 1 || rb->max_leaf > 3) return fail(TRAY_ERR_ARG, "max_prims_per_leaf must be 1..3");
@@ -798,22 +962,10 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         if (n_tris == 0) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: an instance's BLAS reaches no triangle");
     }
     CU(cudaSetDevice(s->device));
-    // after every frame and batch enqueued so far: frames rendered before the refit keep their old-geometry results
-    if (stream) CU(cudaStreamSynchronize((cudaStream_t)stream));
-    if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
-    CU(cudaStreamSynchronize(s->copy_stream));
-    if (s->pipeline_ready) { CU(cudaStreamSynchronize(s->s_in)); CU(cudaStreamSynchronize(s->s_out)); }
+    if (const int rc = drain_scene(s, stream)) return rc;
     if (n_tris == 0) return TRAY_OK;
     char msg[400] = "";
-    if (!s->refit) {
-        tray_build::RefitTopology t;
-        const int rc = tray_build::refit_walk(s->d_nodes, s->n_nodes, s->n_tris, s->tlas ? s->d_blas : nullptr, s->tlas ? s->n_instances : 0u,
-                                              s->tlas_start, s->stream, &t, msg, sizeof msg);
-        if (rc) return fail(rc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "refit: %s", msg);
-        s->refit = new (std::nothrow) tray_build::RefitTopology(std::move(t));
-        if (!s->refit) return fail(TRAY_ERR_ARG, "out of host memory");
-        s->device_bytes += s->refit->bytes;
-    }
+    if (const int rc = ensure_topology(s, msg, sizeof msg)) return rc;
     if (rb && s->refit->blas_past_tlas) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: a BLAS node lies at or past tlas_start");
     if (rb && s->refit->blas_empty) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: an instance's BLAS reaches no triangle");
     const float* d_tris9 = tris9;
@@ -832,30 +984,11 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
         if (rb) {
             // one interval, coordinate check to the last TLAS write, host round trips of the TLAS build included
             if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
-            const uint64_t cap = (uint64_t)s->tlas_start + s->n_instances + 1;
-            tray_build::DevPtr<uint4> grown;  // a created scene's node array holds n_nodes: the first rebuild that needs more grows it
-            if (cap > s->node_cap) {
-                uint4* p = nullptr;
-                CU(cudaMalloc(&p, cap * 80));
-                grown.reset(p);
-                CU(cudaMemcpyAsync(p, s->d_nodes, (size_t)s->tlas_start * 80, cudaMemcpyDeviceToDevice, s->stream));
-            }
-            const uint64_t held = s->refit->bytes;
-            if (tray_build::refit_reserve(*s->refit, cap, s->n_instances, s->stream, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
-            s->device_bytes += s->refit->bytes - held;
-            uint4* nodes = grown ? grown.get() : s->d_nodes;
-            bool tlas_exact = false;
-            uint32_t m = 0;
-            if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, nodes, s->d_tris, s->d_blas, true, s->stream,
-                                      &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
-            if (tray_build::rebuild_tlas(*s->refit, nodes, s->tlas_start, s->n_instances, s->d_blas, rb->max_leaf,
-                                                         rb->radius ? rb->radius : 14u, s->stream, s->ev[1], &m, &tlas_exact, msg, sizeof msg))
-                return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", msg);     // past the first write: never a refusal
-            CU(cudaEventElapsedTime(&ms_run, s->ev[0], s->ev[1]));
-            adopt_rebuilt_tlas(s, grown ? grown.release() : s->d_nodes, cap, m);
-            s->force_exact = scene_force_exact(exact || tlas_exact);
-            if (ms_refit) *ms_refit = ms_run;
-            return TRAY_OK;
+            return tlas_leg(s, s->n_instances, *rb, nullptr, nullptr, [&](uint4* nodes, bool* blas_exact) -> int {
+                if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, nodes, s->d_tris, s->d_blas, true, s->stream,
+                                          blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+                return TRAY_OK;
+            }, ms_refit, msg, sizeof msg);
         }
         CU(cudaEventRecord(s->ev[1], s->stream));
         CU(cudaEventSynchronize(s->ev[1]));
@@ -875,9 +1008,96 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
     cudaFree(d_upload);
     return rc;
 }
+
+// device arrays of an instanced scene with room for n instances: blas_offsets and the two record arrays grow, never shrink
+int reserve_instances(tray_scene* s, uint32_t n) {
+    if (n > s->blas_cap) {
+        uint32_t* p = nullptr;
+        CU(cudaMalloc(&p, (size_t)n * 4));
+        cudaFree(s->d_blas); s->d_blas = p;
+        s->device_bytes += (uint64_t)(n - s->blas_cap) * 4;
+        s->blas_cap = n;
+    }
+    if (n > s->inst_cap) {
+        uint4 *a = nullptr, *b = nullptr;
+        CU(cudaMalloc(&a, (size_t)n * 64));
+        if (cudaMalloc(&b, (size_t)n * 64) != cudaSuccess) { cudaFree(a); cudaGetLastError(); return fail(TRAY_ERR_CUDA, "cudaMalloc of instance records failed"); }
+        cudaFree(s->d_inst_in); cudaFree(s->d_inst_rec);
+        s->d_inst_in = a; s->d_inst_rec = b;
+        s->device_bytes += (uint64_t)(n - s->inst_cap) * 128;
+        s->inst_cap = n;
+    }
+    return TRAY_OK;
+}
 }  // namespace
 
 extern "C" {
+
+int tray_cuda_scene_set_instances(tray_scene* s, const uint32_t* blas_roots, const float* object_to_world, uint32_t n,
+                                  uint32_t max_prims_per_leaf, uint32_t search_radius, float* ms) {
+    if (ms) *ms = 0.f;
+    if (!s || !blas_roots || !object_to_world) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (n == 0) return fail(TRAY_ERR_ARG, "set_instances: no instances");
+    if (!s->tlas) return fail(TRAY_ERR_ARG, "set_instances: the scene has no TLAS");
+    if (s->variant) return fail(TRAY_ERR_ARG, "set_instances: the scene has semantic variants (tray_cuda_scene_set_variant)");
+    if (max_prims_per_leaf < 1 || max_prims_per_leaf > 3) return fail(TRAY_ERR_ARG, "max_prims_per_leaf must be 1..3");
+    if (search_radius > 64) return fail(TRAY_ERR_ARG, "search_radius must be 0 (default 14) or 1..64");
+    if ((uint64_t)s->tlas_start + n + 1 > 0xffffffffull) return fail(TRAY_ERR_ARG, "set_instances: node indices are 32-bit");
+    std::vector<uint4> in((size_t)n * INST_RECORD_U4);
+    for (uint32_t k = 0; k < n; k++) {
+        const float* M = object_to_world + 12 * (size_t)k;
+        for (int j = 0; j < 12; j++)
+            if (!std::isfinite(M[j])) return fail(TRAY_ERR_ARG, "set_instances: object_to_world of instance %u is not finite", k);
+        float W[12];
+        if (!invert_xform(M, W)) return fail(TRAY_ERR_ARG, "set_instances: object_to_world of instance %u has no finite f32 inverse", k);
+        uint4* r = &in[(size_t)k * INST_RECORD_U4];
+        memcpy(r, W, sizeof W);
+        r[3] = make_uint4(blas_roots[k], k, 0u, 0u);
+    }
+    CU(cudaSetDevice(s->device));
+    if (const int rc = drain_scene(s, nullptr)) return rc;
+    char msg[400] = "";
+    if (const int rc = ensure_topology(s, msg, sizeof msg)) return rc;
+    const tray_build::RefitTopology& t = *s->refit;
+    if (t.blas_past_tlas) return fail(TRAY_ERR_ARG, "set_instances: a BLAS node lies at or past tlas_start");
+    if (t.blas_empty) return fail(TRAY_ERR_ARG, "set_instances: a BLAS reaches no triangle");
+    for (uint32_t k = 0; k < n; k++)
+        if (!std::binary_search(t.roots.begin(), t.roots.end(), blas_roots[k]))
+            return fail(TRAY_ERR_ARG, "set_instances: blas_roots[%u] = %u is not a BLAS root of the scene", k, blas_roots[k]);
+    std::vector<float4> lo, hi;
+    if (const int rc = instance_boxes(s, s->d_nodes, blas_roots, object_to_world, n, lo, hi, msg, sizeof msg))
+        return rc > 0 ? fail(TRAY_ERR_ARG, "set_instances: an instance's TLAS box is not finite in f32") : fail(TRAY_ERR_CUDA, "set_instances: %s", msg);
+    if (const int rc = reserve_instances(s, n)) return rc;
+    CU(cudaEventRecord(s->ev[0], s->stream));
+    CU(cudaMemcpyAsync(s->d_inst_in, in.data(), (size_t)n * 64, cudaMemcpyHostToDevice, s->stream));
+    const TlasRebuild rb{ max_prims_per_leaf, search_radius };
+    const int rc = tlas_leg(s, n, rb, &lo, &hi, [&](uint4* nodes, bool* blas_exact) -> int {
+        if (tray_build::blas_exact(*s->refit, nodes, s->tlas_start, s->stream, blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "set_instances: %s", msg);
+        return TRAY_OK;
+    }, ms, msg, sizeof msg);
+    if (rc) return rc;
+    s->instanced = true;
+    s->n_instances = n;
+    s->inst_roots.assign(blas_roots, blas_roots + n);
+    s->inst_o2w.assign(object_to_world, object_to_world + 12 * (size_t)n);
+    return TRAY_OK;
+}
+
+int tray_cuda_scene_download_instance_xforms(tray_scene* s, uint32_t* leaf_instance, float* world_to_object) {
+    if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
+    if (!s->instanced) return fail(TRAY_ERR_ARG, "the scene is not instanced (tray_cuda_scene_set_instances)");
+    CU(cudaSetDevice(s->device));
+    CU(cudaStreamSynchronize(s->stream));
+    std::vector<uint4> rec((size_t)s->n_instances * INST_RECORD_U4);
+    CU(cudaMemcpy(rec.data(), s->d_inst_rec, rec.size() * 16, cudaMemcpyDeviceToHost));
+    for (uint32_t j = 0; j < s->n_instances; j++) {
+        const uint4* r = &rec[(size_t)j * INST_RECORD_U4];
+        const uint32_t k = r[3].y;
+        if (leaf_instance) leaf_instance[j] = k;
+        if (world_to_object && k < s->n_instances) memcpy(world_to_object + 12 * (size_t)k, r, 48);
+    }
+    return TRAY_OK;
+}
 
 int tray_cuda_scene_refit(tray_scene* s, const float* tris9, uint64_t n_tris, float* ms_refit) {
     return refit_impl(s, tris9, n_tris, false, nullptr, ms_refit);
@@ -900,8 +1120,9 @@ int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* s, const float* d_tris
 
 namespace {
 // d_costs != NULL: the cost calls — the counting kernels whatever tray_scene::counting says, the counters read under it alone
+// d_inst != NULL: tray_cuda_trace_instance_device, the instance of every hit goes there
 int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hit* d_hits, tray_ray_cost* d_costs, void* stream,
-                      float* ms_kernel, bool anyhit) {
+                      float* ms_kernel, bool anyhit, uint32_t* d_inst = nullptr) {
     if (!s || (n && (!d_rays || !d_hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
@@ -911,6 +1132,7 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
         TraceParams P; base_params(s, P);
         P.rays = d_rays + off; P.n_work = (uint32_t)(n - off < chunk ? n - off : chunk); P.hits_out = d_hits + off;
         P.ray_cost = d_costs ? d_costs + off : nullptr;
+        P.inst_out = d_inst ? d_inst + off : nullptr;
         int rc = launch(s, P, st, s->d_cursor, 0, s->counting || d_costs, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
         if (rc) return rc;
     }
@@ -957,8 +1179,9 @@ int ensure_pipeline(tray_scene* s) {
 // [copy stream: D2H into a pinned slot] [host threads: -> caller's hits]; chunk i+1 is staged and uploaded while chunk i is
 // traced and chunk i-1 is read back.  The caller's memory is only borrowed for the call and never registered.
 // costs != NULL: the cost calls (see trace_device_impl); the records travel like the hits
+// inst != NULL: tray_cuda_trace_instance; the instance ids travel like the hits
 int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, tray_ray_cost* costs, float* ms_kernel, float* ms_total,
-               bool anyhit) {
+               bool anyhit, uint32_t* inst = nullptr) {
     if (!s || (n && (!rays || !hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     const auto t0 = std::chrono::steady_clock::now();
@@ -973,21 +1196,30 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
         CU(cudaMalloc(&s->d_costs, n * sizeof(tray_ray_cost)));
         s->cost_cap = n;
     }
+    if (inst && n > s->inst_ids_cap) {
+        cudaFree(s->d_inst_ids); s->d_inst_ids = nullptr; s->inst_ids_cap = 0;
+        CU(cudaMalloc(&s->d_inst_ids, n * sizeof(uint32_t)));
+        s->inst_ids_cap = n;
+    }
     tray_ray_cost* const d_costs = costs ? s->d_costs : nullptr;
+    uint32_t* const d_inst = inst ? s->d_inst_ids : nullptr;
     float k = 0.f;
     int rc = TRAY_OK;
     if (n < PIPE_MIN) {
         if (n) CU(cudaMemcpyAsync(s->d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, s->stream));
-        rc = trace_device_impl(s, s->d_rays, n, s->d_hits, d_costs, s->stream, &k, anyhit);
+        rc = trace_device_impl(s, s->d_rays, n, s->d_hits, d_costs, s->stream, &k, anyhit, d_inst);
         if (rc) return rc;
         if (n) CU(cudaMemcpyAsync(hits, s->d_hits, n * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->stream));
         if (n && costs) CU(cudaMemcpyAsync(costs, d_costs, n * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->stream));
+        if (n && inst) CU(cudaMemcpyAsync(inst, d_inst, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
         CU(cudaStreamSynchronize(s->stream));
     } else {
         rc = ensure_pipeline(s);
         if (rc) return rc;
         for (int i = 0; costs && i < 2; i++)
             if (!s->h_costs[i]) CU(cudaMallocHost(&s->h_costs[i], CHUNK_MAX * sizeof(tray_ray_cost)));
+        for (int i = 0; inst && i < 2; i++)
+            if (!s->h_inst[i]) CU(cudaMallocHost(&s->h_inst[i], CHUNK_MAX * sizeof(uint32_t)));
         // chunk size: the pipeline only pays once it has a few stages, and every stage is a kernel launch with its own
         // drain phase — 2^19 rays below 4 M rays, 2^20 above
         const uint64_t chunk = n < (4ull << 20) ? (CHUNK_MAX >> 1) : CHUNK_MAX;
@@ -1007,6 +1239,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 TraceParams P; base_params(s, P);
                 P.rays = s->d_rays + off; P.n_work = (uint32_t)len; P.hits_out = s->d_hits + off;
                 P.ray_cost = d_costs ? d_costs + off : nullptr;
+                P.inst_out = d_inst ? d_inst + off : nullptr;
                 rc = launch(s, P, s->stream, s->d_cursor, 0, s->counting || costs, anyhit, /*keep_counters=*/true);
                 if (rc) return rc;
                 rc = drop_placeholder_costs(s, P.ray_cost, len, s->stream);
@@ -1018,6 +1251,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 CU(cudaStreamWaitEvent(s->s_out, s->e_k[ps], 0));
                 CU(cudaMemcpyAsync(s->h_hits[ps], s->d_hits + j * chunk, chunk_len(j) * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->s_out));
                 if (costs) CU(cudaMemcpyAsync(s->h_costs[ps], d_costs + j * chunk, chunk_len(j) * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->s_out));
+                if (inst) CU(cudaMemcpyAsync(s->h_inst[ps], d_inst + j * chunk, chunk_len(j) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->s_out));
                 CU(cudaEventRecord(s->e_out[ps], s->s_out));
             }
             if (i >= 2) {                                                               // chunk i-2: hand its hits to the caller
@@ -1025,6 +1259,7 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
                 CU(cudaEventSynchronize(s->e_out[ps]));
                 tray::par_copy(hits + j * chunk, s->h_hits[ps], chunk_len(j) * sizeof(tray_hit));
                 if (costs) tray::par_copy(costs + j * chunk, s->h_costs[ps], chunk_len(j) * sizeof(tray_ray_cost));
+                if (inst) tray::par_copy(inst + j * chunk, s->h_inst[ps], chunk_len(j) * sizeof(uint32_t));
             }
         }
         CU(cudaEventRecord(s->ev[1], s->stream));
@@ -1070,6 +1305,18 @@ int tray_cuda_trace_cost(tray_scene* s, const tray_ray* rays, uint64_t n, int an
     if (!s || (n && (!rays || !hits || !costs))) return fail(TRAY_ERR_ARG, "NULL argument");
     if (s->variant) return fail(TRAY_ERR_ARG, "%s", VARIANT_REFUSAL);
     return trace_impl(s, rays, n, hits, costs, ms_kernel, ms_total, any_hit != 0);
+}
+int tray_cuda_trace_instance(tray_scene* s, const tray_ray* rays, uint64_t n, int any_hit, tray_hit* hits, uint32_t* instance_ids,
+                             float* ms_kernel, float* ms_total) {
+    if (!s || (n && (!rays || !hits || !instance_ids))) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (!s->instanced) return fail(TRAY_ERR_ARG, "the scene is not instanced (tray_cuda_scene_set_instances)");
+    return trace_impl(s, rays, n, hits, nullptr, ms_kernel, ms_total, any_hit != 0, instance_ids);
+}
+int tray_cuda_trace_instance_device(tray_scene* s, const tray_ray* d_rays, uint64_t n, int any_hit, tray_hit* d_hits, uint32_t* d_instance_ids,
+                                    void* stream, float* ms_kernel) {
+    if (!s || (n && (!d_rays || !d_hits || !d_instance_ids))) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (!s->instanced) return fail(TRAY_ERR_ARG, "the scene is not instanced (tray_cuda_scene_set_instances)");
+    return trace_device_impl(s, d_rays, n, d_hits, nullptr, stream, ms_kernel, any_hit != 0, d_instance_ids);
 }
 
 uint64_t tray_cuda_shard_pixels(uint32_t w, uint32_t h, uint32_t shard, uint32_t shards) {
@@ -1192,9 +1439,10 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     const bool bounce = (flags & TRAY_RENDER_BOUNCE) != 0, rgba = (flags & TRAY_RENDER_RGBA) != 0;
     const bool keep_rays = (flags & TRAY_RENDER_KEEP_RAYS) != 0;
     const bool any_ao = (flags & TRAY_RENDER_ANYHIT_AO) != 0;
-    const bool overlap = bounce && !any_ao && !s->variant && ((flags & TRAY_RENDER_OVERLAP) != 0 || s->overlap_default);
+    // (instanced scenes: the one-launch frame kernel has no instance transforms)
+    const bool overlap = bounce && !any_ao && !s->variant && !s->instanced && ((flags & TRAY_RENDER_OVERLAP) != 0 || s->overlap_default);
     const bool keep_cost = want_count && s->ray_cost;
-    if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item) || (keep_cost && !f.d_cost)) {
+    if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item) || (keep_cost && !f.d_cost) || (s->instanced && !f.d_pinst)) {
         const uint64_t cap = items_cap > f.f_cap ? items_cap : f.f_cap;
         CU(cudaStreamSynchronize(st));
         free_frame_buffers(f);
@@ -1207,6 +1455,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         CU(cudaMalloc(&f.d_bitem, c1 * sizeof(uint32_t)));
         if (keep_rays) CU(cudaMalloc(&f.d_brays_item, c1 * sizeof(tray_ray)));
         if (keep_cost) CU(cudaMalloc(&f.d_cost, 2 * c1 * sizeof(tray_ray_cost)));
+        if (s->instanced) { CU(cudaMalloc(&f.d_pinst, c1 * sizeof(uint32_t))); CU(cudaMalloc(&f.d_binst, c1 * sizeof(uint32_t))); }
         CU(cudaMemsetAsync(f.d_primary, 0xff, c1 * sizeof(tray_hit), st));
         CU(cudaMemsetAsync(f.d_bounce, 0xff, c1 * sizeof(tray_hit), st));
         CU(cudaMemsetAsync(f.d_rgba, 0, c1 * sizeof(uchar4), st));
@@ -1216,6 +1465,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     f.f_has_bounce = bounce; f.f_has_rgba = rgba && !s->frame_target; f.f_has_rays = keep_rays && bounce;
     f.f_target = rgba ? s->frame_target : nullptr;
     f.f_has_cost = keep_cost;
+    f.f_has_inst = s->instanced;
     f.last_frame = F;
     if (F.n_items == 0) {                        // a shard without tiles: no launch, and nothing to count
         if (ms_primary) *ms_primary = 0.f;
@@ -1241,6 +1491,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     uchar4* const rgba_dst = s->frame_target ? s->frame_target : f.d_rgba;
     P.rgba_out = (rgba && !bounce) ? rgba_dst : nullptr; P.shade_mode = SHADE_PRIMARY;
     P.ray_cost = keep_cost ? f.d_cost : nullptr;
+    P.inst_out = s->instanced ? f.d_pinst : nullptr;
     if (overlap) {
         // one launch for the whole frame (trace_kernel<FRAME>): the bounce rays of finished tiles fill the primary pass's drain
         CU(cudaMemsetAsync(f.d_units, 0, sizeof(uint32_t), st));
@@ -1258,15 +1509,20 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     // ---- bounce: generate + compact rays of hit pixels, trace ----
     if (bounce && !overlap) {
         CU(cudaMemsetAsync(d_nbrays, 0, sizeof(uint32_t), st));
-        auto gen = s->tri_stride == 64 ? tray::raygen_bounce_kernel<64> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24> : tray::raygen_bounce_kernel<48>;
+        auto gen = s->instanced ? (s->tri_stride == 64 ? tray::raygen_bounce_kernel<64, true> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24, true>
+                                                                                                     : tray::raygen_bounce_kernel<48, true>)
+                 : s->tri_stride == 64 ? tray::raygen_bounce_kernel<64> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24> : tray::raygen_bounce_kernel<48>;
+        if (s->instanced) CU(cudaMemsetAsync(f.d_binst, 0xff, (size_t)F.n_items * sizeof(uint32_t), st));   // pixels that shoot no bounce ray
         gen<<<(F.n_items + BOUNCE_BLOCK - 1) / BOUNCE_BLOCK, BOUNCE_BLOCK, 0, st>>>(F, s->d_tris, f.d_primary, f.d_brays, f.d_bitem, d_nbrays, f.d_bounce,
-                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major);
+                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major,
+                                             f.d_pinst, s->d_inst_in);
         CU(cudaGetLastError());
         TraceParams B; base_params(s, B);
         B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
         B.overflow = f.d_flag; B.frame = F; B.row_major = P.row_major;
         B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
         B.ray_cost = d_cost_bounce;
+        B.inst_out = s->instanced ? f.d_binst : nullptr;
         rc = launch(s, B, st, f.d_cursor, 1, want_count, any_ao);
         if (rc) return rc;
         if (timed) CU(cudaEventRecord(f.ev[2], st));
@@ -1351,12 +1607,13 @@ int tray_cuda_frame_device_ptrs(tray_scene* s, void** d_primary, void** d_bounce
 }  // extern "C"
 
 namespace {
-// the last frame's compact buffer `d_src`, untiled into the row-major `d_dst` on the frame's stream
+// the last frame's compact buffer `d_src`, untiled into the row-major `d_dst` on the frame's stream; pixels of other shards are
+// bytes `fill`
 template <typename T>
-int untile_last_frame(tray_scene* s, const T* d_src, T* d_dst) {
+int untile_last_frame(tray_scene* s, const T* d_src, T* d_dst, int fill = 0) {
     const FrameParams& F = s->slot[s->cur].last_frame;
     cudaStream_t st = slot_stream(s, s->cur);
-    if (F.shard_count > 1) CU(cudaMemsetAsync(d_dst, 0, (uint64_t)F.width * F.height * sizeof(T), st));   // pixels of other shards read as zero
+    if (F.shard_count > 1) CU(cudaMemsetAsync(d_dst, fill, (uint64_t)F.width * F.height * sizeof(T), st));
     if (F.n_items) {
         tray::untile_kernel<T><<<(F.n_items + 255) / 256, 256, 0, st>>>(F, d_src, d_dst);
         CU(cudaGetLastError());
@@ -1365,7 +1622,7 @@ int untile_last_frame(tray_scene* s, const T* d_src, T* d_dst) {
 }
 
 template <typename T>
-int download(tray_scene* s, const T* d_src, T* host_dst) {
+int download(tray_scene* s, const T* d_src, T* host_dst, int fill = 0) {
     const FrameParams& F = s->slot[s->cur].last_frame;
     cudaStream_t st = slot_stream(s, s->cur);
     const uint64_t bytes = (uint64_t)F.width * F.height * sizeof(T);
@@ -1374,7 +1631,7 @@ int download(tray_scene* s, const T* d_src, T* host_dst) {
         CU(cudaMalloc(&s->d_untiled, bytes));
         s->untiled_cap = bytes;
     }
-    if (const int rc = untile_last_frame(s, d_src, (T*)s->d_untiled)) return rc;
+    if (const int rc = untile_last_frame(s, d_src, (T*)s->d_untiled, fill)) return rc;
     CU(cudaMemcpyAsync(host_dst, s->d_untiled, bytes, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return TRAY_OK;
@@ -1415,6 +1672,20 @@ int tray_cuda_frame_download_cost(tray_scene* s, tray_ray_cost* primary, tray_ra
     int rc;
     if (primary) { rc = download<tray_ray_cost>(s, f.d_cost, primary); if (rc) return rc; }
     if (bounce) { rc = download<tray_ray_cost>(s, f.d_cost + f.last_frame.n_items, bounce); if (rc) return rc; }
+    return check_overflow(f.d_flag, slot_stream(s, s->cur));
+}
+
+int tray_cuda_frame_download_instance(tray_scene* s, uint32_t* primary, uint32_t* bounce) {
+    if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
+    if (!s->instanced) return fail(TRAY_ERR_ARG, "the scene is not instanced (tray_cuda_scene_set_instances)");
+    const FrameSlot& f = s->slot[s->cur];
+    if (f.last_frame.width == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
+    if (!f.f_has_inst) return fail(TRAY_ERR_ARG, "the last frame was rendered before the scene was instanced");
+    if (bounce && !f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
+    CU(cudaSetDevice(s->device));
+    int rc;
+    if (primary) { rc = download<uint32_t>(s, f.d_pinst, primary, 0xff); if (rc) return rc; }
+    if (bounce) { rc = download<uint32_t>(s, f.d_binst, bounce, 0xff); if (rc) return rc; }
     return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 

@@ -35,6 +35,8 @@ EXPORTS = (
     "tray_cuda_trace_cost", "tray_cuda_trace_cost_device", "tray_cuda_scene_set_ray_cost", "tray_cuda_frame_download_cost",
     "tray_cuda_scene_refit", "tray_cuda_scene_refit_device", "tray_cuda_scene_exact_node_test",
     "tray_cuda_scene_refit_rebuild_tlas", "tray_cuda_scene_refit_rebuild_tlas_device",
+    "tray_cuda_scene_set_instances", "tray_cuda_scene_download_instance_xforms", "tray_cuda_trace_instance",
+    "tray_cuda_trace_instance_device", "tray_cuda_frame_download_instance",
 )
 # semantic switches of tray_cuda_scene_set_variant (include/tray_cuda.h TRAY_VARIANT_*)
 VARIANT_BOX_DIVIDE, VARIANT_TIE_LAST, VARIANT_BOX_TMIN_RAY, VARIANT_ZERODIR_BOX_ONLY = 1, 2, 4, 8
@@ -227,6 +229,16 @@ def lib() -> C.CDLL:
         L.tray_cuda_scene_refit_rebuild_tlas.argtypes = [vp, vp, u64, u32, u32, f32p]
         L.tray_cuda_scene_refit_rebuild_tlas_device.restype = i32
         L.tray_cuda_scene_refit_rebuild_tlas_device.argtypes = [vp, vp, u64, u32, u32, vp, f32p]
+        L.tray_cuda_scene_set_instances.restype = i32
+        L.tray_cuda_scene_set_instances.argtypes = [vp, vp, vp, u32, u32, u32, f32p]
+        L.tray_cuda_scene_download_instance_xforms.restype = i32
+        L.tray_cuda_scene_download_instance_xforms.argtypes = [vp, vp, vp]
+        L.tray_cuda_trace_instance.restype = i32
+        L.tray_cuda_trace_instance.argtypes = [vp, vp, u64, i32, vp, vp, f32p, f32p]
+        L.tray_cuda_trace_instance_device.restype = i32
+        L.tray_cuda_trace_instance_device.argtypes = [vp, vp, u64, i32, vp, vp, vp, f32p]
+        L.tray_cuda_frame_download_instance.restype = i32
+        L.tray_cuda_frame_download_instance.argtypes = [vp, vp, vp]
         _lib = L
     return _lib
 
@@ -386,6 +398,64 @@ class TrayCudaScene:
         _check(lib().tray_cuda_scene_refit_rebuild_tlas_device(self._h, d_ptr, n, max_prims_per_leaf, search_radius, stream or None,
                                                                 C.byref(ms) if timed else None))
         return ms.value if timed else None
+
+    def set_instances(self, blas_roots, object_to_world, max_prims_per_leaf=3, search_radius=0, timings: dict | None = None):
+        """Place BLAS by transforms (tray_cuda_scene_set_instances): instance k is the BLAS whose root node is blas_roots[k]
+        (one of the scene's blas_offsets values), placed by object_to_world[k], a row-major 3 x 4 [R | t].  Only the TLAS is
+        built; timings["ms_set_instances"]: upload of the transforms to the last TLAS write."""
+        roots = np.asarray(blas_roots)
+        xf = np.asarray(object_to_world)
+        if roots.ndim != 1 or roots.size == 0 or roots.dtype.kind not in "iu":
+            raise ValueError("blas_roots must be a non-empty 1-D integer array")
+        if (roots < 0).any() or (roots > 0xFFFFFFFF).any():
+            raise ValueError("blas_roots must be node indices (uint32)")
+        if xf.dtype.kind != "f" or xf.shape != (roots.size, 3, 4):
+            raise ValueError(f"object_to_world must be a float array of shape ({roots.size}, 3, 4), got {xf.dtype} {xf.shape}")
+        roots = np.ascontiguousarray(roots, dtype=np.uint32)
+        xf = np.ascontiguousarray(xf, dtype=np.float32)
+        ms = C.c_float()
+        _check(lib().tray_cuda_scene_set_instances(self._h, roots.ctypes.data, xf.ctypes.data, roots.size, max_prims_per_leaf,
+                                                    search_radius, C.byref(ms)))
+        if timings is not None:
+            timings["ms_set_instances"] = ms.value
+
+    def download_instance_xforms(self):
+        """(leaf_instance, world_to_object): the instance of every TLAS leaf, and every instance's world_to_object (n, 3, 4)
+        as the kernels use it (tray_cuda_scene_download_instance_xforms)."""
+        n = self.info()["n_instances"]
+        leaf, w2o = np.zeros(n, dtype=np.uint32), np.zeros((n, 3, 4), dtype=np.float32)
+        _check(lib().tray_cuda_scene_download_instance_xforms(self._h, leaf.ctypes.data, w2o.ctypes.data))
+        return leaf, w2o
+
+    def traverse_instance(self, rays: np.ndarray, any_hit: bool = False, timings: dict | None = None):
+        """(hits, instance_ids): traverse() on an instanced scene plus the instance of every hit, 0xFFFFFFFF for a miss
+        (tray_cuda_trace_instance)."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        hits = np.empty(rays.shape[0], dtype=HIT_DTYPE)
+        ids = np.empty(rays.shape[0], dtype=np.uint32)
+        k, t = C.c_float(), C.c_float()
+        _check(lib().tray_cuda_trace_instance(self._h, rays.ctypes.data, rays.shape[0], int(any_hit), hits.ctypes.data, ids.ctypes.data,
+                                              C.byref(k), C.byref(t)))
+        if timings is not None:
+            timings["ms_kernel"], timings["ms_total"] = k.value, t.value
+        return hits, ids
+
+    def traverse_instance_device(self, d_rays_ptr: int, n: int, d_hits_ptr: int, d_ids_ptr: int, stream: int = 0, timed: bool = False,
+                                 any_hit: bool = False):
+        """traverse_device() plus a uint32 instance id per ray at `d_ids_ptr` — tray_cuda_trace_instance_device."""
+        k = C.c_float()
+        _check(lib().tray_cuda_trace_instance_device(self._h, d_rays_ptr, n, int(any_hit), d_hits_ptr, d_ids_ptr, stream or None,
+                                                     C.byref(k) if timed else None))
+        return k.value if timed else None
+
+    def download_instance(self, primary=True, bounce=False) -> dict:
+        """The last frame's instance ids (uint32, row-major, w*h): "primary" and / or "bounce"; 0xFFFFFFFF for misses, other
+        shards' pixels and pixels without a bounce ray (tray_cuda_frame_download_instance)."""
+        w, h = self.frame_size
+        out = {name: np.zeros(w * h, dtype=np.uint32) for name, want in (("primary", primary), ("bounce", bounce)) if want}
+        p, b = out.get("primary"), out.get("bounce")
+        _check(lib().tray_cuda_frame_download_instance(self._h, None if p is None else p.ctypes.data, None if b is None else b.ctypes.data))
+        return out
 
     @classmethod
     def from_packed(cls, p, device=0) -> "TrayCudaScene":
