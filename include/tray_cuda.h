@@ -104,6 +104,13 @@ typedef struct tray_hit {
 
 #define TRAY_INVALID_PRIM 0xFFFFFFFFu
 
+/* The surface at a hit (tray_cuda_hit_attributes): what the triangle test computed for the hit's triangle and ray.  20 bytes.
+ * Miss record: all 20 bytes 0xFF (a NaN in every field).                                                                   */
+typedef struct tray_hit_attr {
+    float u, v;     /* barycentric weights of v1 and v2 (v0's is 1 - u - v), exactly as the triangle test computed them */
+    float ng[3];    /* geometric normal, NOT normalised, in world space */
+} tray_hit_attr;
+
 /* `ViewUniform` (src/main.rs:589-617): column-major glam Mat4s, #[repr(C)], padded to 160 bytes. */
 typedef struct tray_view {
     float    view_inv[16];
@@ -353,6 +360,43 @@ int tray_cuda_trace_instance_device(tray_scene* scene, const tray_ray* d_rays, u
  * pixels without a bounce ray.  TRAY_ERR_ARG on a scene that is not instanced, or for `bounce` after a frame without
  * TRAY_RENDER_BOUNCE. */
 int tray_cuda_frame_download_instance(tray_scene* scene, uint32_t* primary, uint32_t* bounce);
+
+/* ---- hit attributes: barycentrics and geometric normal of each hit ------------------------------------------------------------
+ * For hit i of ray i, tray_hit_attr {u, v, ng} as the triangle test computed them for triangle hits[i].prim and that ray, bit for
+ * bit (one pass over the hits after the traversal, with the test's own arithmetic):
+ *   record     {v0, e1 = v0 - v1, e2 = v2 - v0} (stride 24: e1, e2 unpacked from f16 as the test unpacks them)
+ *   direction  d = the ray's direction with zero components replaced by 2^-23 (FLT_EPSILON), as the traversal prepares it;
+ *              under TRAY_VARIANT_ZERODIR_BOX_ONLY the caller's d
+ *   u, v       det = dot(Ng, d), u = dot(cross(d, v0 - o), e2) / det (the weight of v1), v = dot(cross(d, v0 - o), e1) / det
+ *              (the weight of v2), in f32 without contraction.  They depend on neither t nor tmax: closest-hit, any-hit and
+ *              tie-variant hits all get their triangle's own values.
+ *   ng         stride 64: the record's ng; strides 48 and 24: cross(e1, e2) in f32 (= cross(v0 - v1, v2 - v0)).  Not normalised and
+ *              not flipped toward the ray.
+ *   instances  (instanced scenes) u, v from the object-space ray of the traversal, o'_i = ((W_i0 o_x + W_i1 o_y) + W_i2 o_z) + W_i3,
+ *              d'_i = (W_i0 d_x + W_i1 d_y) + W_i2 d_z then zero-patched (W = world_to_object of instance instance_ids[i]); ng
+ *              taken to world space as the bounce normal is, n'_i = (W_0i n_0 + W_1i n_1) + W_2i n_2, not normalised.  On other
+ *              scenes object space is world space.
+ *   miss       all 20 bytes 0xFF for prim == 0xFFFFFFFF, prim >= n_tris and, on an instanced scene, instance_ids[i] == 0xFFFFFFFF
+ *              or >= n_instances; nothing is read for them.
+ * instance_ids is required on an instanced scene (the output of tray_cuda_trace_instance; a plain tray_cuda_trace reports no
+ * instance, so its hits on an instanced scene cannot be attributed) and must be NULL on any other scene: TRAY_ERR_ARG otherwise.
+ * The scene's CURRENT triangles, transforms and variant flags are used: attributes of hits traced before a refit,
+ * tray_cuda_scene_set_instances or tray_cuda_scene_set_variant describe the new geometry.
+ * HOST buffers: copies in, one launch, copies out on the scene stream, then returns; n == 0 does nothing.  ms_kernel (NULL ok):
+ * CUDA-event time of the launch. */
+int tray_cuda_hit_attributes(tray_scene* scene, const tray_ray* rays, const tray_hit* hits, const uint32_t* instance_ids,
+                             uint64_t n, tray_hit_attr* attrs, float* ms_kernel);
+/* the same with DEVICE buffers, ordered as tray_cuda_trace_device: on `stream` (NULL: the scene stream), after the work enqueued
+ * so far on the scene stream (so hits of a tray_cuda_trace_device there are complete); synchronises only when ms_kernel != NULL */
+int tray_cuda_hit_attributes_device(tray_scene* scene, const tray_ray* d_rays, const tray_hit* d_hits, const uint32_t* d_instance_ids,
+                                    uint64_t n, tray_hit_attr* d_attrs, void* stream, float* ms_kernel);
+/* The last frame's attributes, row-major (w * h records each, either NULL): the primary hits' on the frame's primary rays, the
+ * bounce hits' on its bounce rays, as tray_cuda_hit_attributes computes them.  The miss record for misses, other shards' pixels
+ * and pixels without a bounce ray.  Synchronous.  TRAY_ERR_ARG, with nothing written: no frame rendered, `bounce` after a frame
+ * without TRAY_RENDER_BOUNCE, or a scene changed since the frame by tray_cuda_scene_refit(_device),
+ * tray_cuda_scene_refit_rebuild_tlas(_device), tray_cuda_scene_set_instances or tray_cuda_scene_set_variant (the attributes would
+ * no longer describe that frame's hits; the next frame's call succeeds). */
+int tray_cuda_frame_download_attributes(tray_scene* scene, tray_hit_attr* primary, tray_hit_attr* bounce);
 
 /* ---- ray-batch operator: Traversable::traverse at batch grain (traversable/src/lib.rs:20) ----- */
 

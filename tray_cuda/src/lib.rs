@@ -11,6 +11,12 @@ pub struct TrayRay { pub origin: [f32; 3], pub tmin: f32, pub dir: [f32; 3], pub
 #[derive(Clone, Copy, bytemuck::Pod, bytemuck::Zeroable)]
 pub struct TrayHit { pub t: f32, pub prim: u32 }
 
+/// `tray_hit_attr` of include/tray_cuda.h: the triangle test's barycentrics of v1 and v2 (v0's is 1 - u - v) and its geometric
+/// normal in world space, not normalised; every byte 0xFF (NaN) for a miss.  20 bytes.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, bytemuck::Pod, bytemuck::Zeroable)]
+pub struct TrayHitAttr { pub u: f32, pub v: f32, pub ng: [f32; 3] }
+
 /// `ViewUniform` of tray_racing (src/main.rs:589-597) padded to 160 bytes.
 #[repr(C)]
 #[derive(Clone, Copy, bytemuck::Pod, bytemuck::Zeroable)]
@@ -136,6 +142,12 @@ extern "C" {
     pub fn tray_cuda_trace_instance_device(scene: *mut TrayScene, d_rays: *const TrayRay, n: u64, any_hit: c_int, d_hits: *mut TrayHit,
         d_instance_ids: *mut u32, stream: *mut c_void, ms_kernel: *mut f32) -> c_int;
     pub fn tray_cuda_frame_download_instance(scene: *mut TrayScene, primary: *mut u32, bounce: *mut u32) -> c_int;
+    // hit attributes: u, v and the geometric normal of each hit, as the triangle test computed them
+    pub fn tray_cuda_hit_attributes(scene: *mut TrayScene, rays: *const TrayRay, hits: *const TrayHit, instance_ids: *const u32, n: u64,
+        attrs: *mut TrayHitAttr, ms_kernel: *mut f32) -> c_int;
+    pub fn tray_cuda_hit_attributes_device(scene: *mut TrayScene, d_rays: *const TrayRay, d_hits: *const TrayHit, d_instance_ids: *const u32,
+        n: u64, d_attrs: *mut TrayHitAttr, stream: *mut c_void, ms_kernel: *mut f32) -> c_int;
+    pub fn tray_cuda_frame_download_attributes(scene: *mut TrayScene, primary: *mut TrayHitAttr, bounce: *mut TrayHitAttr) -> c_int;
     pub fn tray_cuda_frame_download(scene: *mut TrayScene, primary: *mut TrayHit, bounce: *mut TrayHit,
         bounce_rays: *mut TrayRay, rgba: *mut u8) -> c_int;
     pub fn tray_cuda_scene_set_variant(scene: *mut TrayScene, variant_flags: u32) -> c_int;
@@ -284,6 +296,31 @@ impl Scene {
                 std::ptr::null_mut(), std::ptr::null_mut())
         });
         (hits, ids)
+    }
+
+    /// u, v and the world-space geometric normal of every hit on its ray (`hits` and `instance_ids` as `traverse` or
+    /// `traverse_instance` returned them; `instance_ids` is required on an instanced scene and must be `None` on any other).
+    pub fn hit_attributes(&mut self, rays: &[TrayRay], hits: &[TrayHit], instance_ids: Option<&[u32]>) -> Vec<TrayHitAttr> {
+        assert_eq!(rays.len(), hits.len(), "one hit per ray");
+        if let Some(ids) = instance_ids { assert_eq!(ids.len(), hits.len(), "one instance id per hit"); }
+        let mut attrs = vec![TrayHitAttr { u: f32::NAN, v: f32::NAN, ng: [f32::NAN; 3] }; hits.len()];
+        check(unsafe {
+            tray_cuda_hit_attributes(self.raw, rays.as_ptr(), hits.as_ptr(), instance_ids.map_or(std::ptr::null(), |i| i.as_ptr()),
+                hits.len() as u64, attrs.as_mut_ptr(), std::ptr::null_mut())
+        });
+        attrs
+    }
+
+    /// The last frame's hit attributes, row-major (width * height each): (primary, bounce); `bounce` needs a frame rendered with
+    /// RENDER_BOUNCE.  Panics when the scene was refit, re-instanced or given other variants since that frame.
+    pub fn download_attributes(&mut self, width: u32, height: u32, bounce: bool) -> (Vec<TrayHitAttr>, Vec<TrayHitAttr>) {
+        let n = width as usize * height as usize;
+        let nan = TrayHitAttr { u: f32::NAN, v: f32::NAN, ng: [f32::NAN; 3] };
+        let (mut p, mut b) = (vec![nan; n], if bounce { vec![nan; n] } else { Vec::new() });
+        check(unsafe {
+            tray_cuda_frame_download_attributes(self.raw, p.as_mut_ptr(), if bounce { b.as_mut_ptr() } else { std::ptr::null_mut() })
+        });
+        (p, b)
     }
 
     /// One frame (primary + bounce rays) of shard `shard` of `shards`; returns (ms primary, ms bounce) of the kernels.

@@ -345,6 +345,28 @@ __device__ __forceinline__ void tri_load(const uint4* __restrict__ tris, uint32_
 }
 
 // ---- triangle test: RtTriangle::intersect, twin query.hlsl:89-129; returns t or +inf -------------
+// The test's geometric normal (not normalised): the record's for stride 64, cross(e1, e2) otherwise (query.hlsl:93)
+template <int TRI_STRIDE>
+__device__ __forceinline__ void tri_normal(const uint4* __restrict__ tris, uint32_t prim, float e1x, float e1y, float e1z,
+                                           float e2x, float e2y, float e2z, float& ngx, float& ngy, float& ngz) {
+    if (TRI_STRIDE == 64) {
+        const uint4 g = __ldg(tris + (size_t)prim * 4u + 3);
+        ngx = __uint_as_float(g.x); ngy = __uint_as_float(g.y); ngz = __uint_as_float(g.z);
+    } else {
+        cross3(e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz);                       // :93
+    }
+}
+// The test's barycentrics for the ray (o, dd), query.hlsl:96-101: c = v0 - o, inv_det, u (the weight of v1) and v (of v2).
+// tri_test and the attribute pass (hit_attr) both take them from here, so a hit's reported u, v are the test's own bits.
+__device__ __forceinline__ void tri_uv(float ox, float oy, float oz, float ddx, float ddy, float ddz, float v0x, float v0y, float v0z,
+                                       float e1x, float e1y, float e1z, float e2x, float e2y, float e2z, float ngx, float ngy, float ngz,
+                                       float& cx, float& cy, float& cz, float& inv_det, float& u, float& v) {
+    cx = sub(v0x, ox); cy = sub(v0y, oy); cz = sub(v0z, oz);                       // :96
+    float rx, ry, rz; cross3(ddx, ddy, ddz, cx, cy, cz, rx, ry, rz);               // :97
+    inv_det = __fdiv_rn(1.0f, dot3(ngx, ngy, ngz, ddx, ddy, ddz));                 // :98
+    u = mul(dot3(rx, ry, rz, e2x, e2y, e2z), inv_det);                             // :100
+    v = mul(dot3(rx, ry, rz, e1x, e1y, e1z), inv_det);                             // :101
+}
 // VARIANT_DIR: the test reads its direction from r.tdx/tdy/tdz (MODE 1) instead of the box test's r.dx/dy/dz
 template <int TRI_STRIDE, bool VARIANT_DIR = false>
 __device__ __forceinline__ float tri_test(const RayConst& r, float tmax, const uint4* __restrict__ tris, uint32_t prim) {
@@ -352,17 +374,9 @@ __device__ __forceinline__ float tri_test(const RayConst& r, float tmax, const u
     float v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z;
     tri_load<TRI_STRIDE>(tris, prim, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z);
     float ngx, ngy, ngz;
-    if (TRI_STRIDE == 64) {
-        const uint4 g = __ldg(tris + (size_t)prim * 4u + 3);
-        ngx = __uint_as_float(g.x); ngy = __uint_as_float(g.y); ngz = __uint_as_float(g.z);
-    } else {
-        cross3(e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz);                       // :93
-    }
-    const float cx = sub(v0x, r.ox), cy = sub(v0y, r.oy), cz = sub(v0z, r.oz);     // :96
-    float rx, ry, rz; cross3(ddx, ddy, ddz, cx, cy, cz, rx, ry, rz);               // :97
-    const float inv_det = __fdiv_rn(1.0f, dot3(ngx, ngy, ngz, ddx, ddy, ddz));     // :98
-    const float u = mul(dot3(rx, ry, rz, e2x, e2y, e2z), inv_det);                 // :100
-    const float v = mul(dot3(rx, ry, rz, e1x, e1y, e1z), inv_det);                 // :101
+    tri_normal<TRI_STRIDE>(tris, prim, e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz);
+    float cx, cy, cz, inv_det, u, v;
+    tri_uv(r.ox, r.oy, r.oz, ddx, ddy, ddz, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz, cx, cy, cz, inv_det, u, v);
     const float w = sub(sub(1.0f, u), v);                                          // :102
     const uint32_t hit = __float_as_uint(u) | __float_as_uint(v) | __float_as_uint(w);   // :112
     float t = __int_as_float(0x7f800000);
@@ -445,6 +459,23 @@ __device__ __forceinline__ void sincos_tau(float u, float& s, float& c) {
     c = q == 0 ? cs : q == 1 ? -sn : q == 2 ? -cs : sn;
 }
 
+// ---- instance transforms: `xf` is an InstanceRecord, rows 0..2 of world_to_object W ([W | -W t]) -------------------------
+// The ray of a TLAS leaf in object space: o' = ((W_i0 o_x + W_i1 o_y) + W_i2 o_z) + W_i3 and d' = dot(W_i, d) for row i
+__device__ __forceinline__ void xform_row(const uint4& w, float ox, float oy, float oz, float dx, float dy, float dz, float& o, float& d) {
+    const float m0 = __uint_as_float(w.x), m1 = __uint_as_float(w.y), m2 = __uint_as_float(w.z);
+    o = add(add(add(mul(m0, ox), mul(m1, oy)), mul(m2, oz)), __uint_as_float(w.w));
+    d = dot3(m0, m1, m2, dx, dy, dz);
+}
+// An object-space normal to world space through the transpose of W, n'_i = W_0i n_0 + W_1i n_1 + W_2i n_2 (the inverse
+// transpose of object_to_world), not normalised
+__device__ __forceinline__ void normal_to_world(const uint4* __restrict__ xf, float& nx, float& ny, float& nz) {
+    const uint4 w0 = __ldg(xf), w1 = __ldg(xf + 1), w2 = __ldg(xf + 2);
+    const float wx = dot3(__uint_as_float(w0.x), __uint_as_float(w1.x), __uint_as_float(w2.x), nx, ny, nz);
+    const float wy = dot3(__uint_as_float(w0.y), __uint_as_float(w1.y), __uint_as_float(w2.y), nx, ny, nz);
+    const float wz = dot3(__uint_as_float(w0.z), __uint_as_float(w1.z), __uint_as_float(w2.z), nx, ny, nz);
+    nx = wx; ny = wy; nz = wz;
+}
+
 // bounce ray from a primary hit (src/rt_cpu/rt_cpu.rs:61-76; basis sampling.hlsl:39-51)
 // INST: `xf` is the InstanceRecord of the hit's instance; the object-space normal goes to world space through the transpose of
 // world_to_object, n'_i = W_0i n_0 + W_1i n_1 + W_2i n_2 (the inverse transpose of object_to_world), before it is normalised.
@@ -462,13 +493,7 @@ __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __
         tri_load<TRI_STRIDE>(tris, prim, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z);
         cross3(e1x, e1y, e1z, e2x, e2y, e2z, nx, ny, nz);
     }
-    if constexpr (INST) {
-        const uint4 w0 = __ldg(xf), w1 = __ldg(xf + 1), w2 = __ldg(xf + 2);
-        const float wx = dot3(__uint_as_float(w0.x), __uint_as_float(w1.x), __uint_as_float(w2.x), nx, ny, nz);
-        const float wy = dot3(__uint_as_float(w0.y), __uint_as_float(w1.y), __uint_as_float(w2.y), nx, ny, nz);
-        const float wz = dot3(__uint_as_float(w0.z), __uint_as_float(w1.z), __uint_as_float(w2.z), nx, ny, nz);
-        nx = wx; ny = wy; nz = wz;
-    }
+    if constexpr (INST) normal_to_world(xf, nx, ny, nz);
     normalize3(nx, ny, nz);                                                    // RtTriangle::compute_normal
     const float sgn = copysignf(1.0f, dot3(nx, ny, nz, -pdx, -pdy, -pdz));     // f32::signum (rt_cpu.rs:65)
     nx = mul(nx, sgn); ny = mul(ny, sgn); nz = mul(nz, sgn);
@@ -906,13 +931,10 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                         const uint4 w0 = __ldg(rec), w1 = __ldg(rec + 1), w2 = __ldg(rec + 2), w3 = __ldg(rec + 3);
                         const float4 d = __ldg(reinterpret_cast<const float4*>(P.rays + (ray_idx & INDEX_MASK)) + 1);
                         bvh_off = w3.x; cur_inst = w3.y;
-                        auto row = [&](const uint4& w, float& o, float& dd) {
-                            const float m0 = __uint_as_float(w.x), m1 = __uint_as_float(w.y), m2 = __uint_as_float(w.z);
-                            o = add(add(add(mul(m0, r.ox), mul(m1, r.oy)), mul(m2, r.oz)), __uint_as_float(w.w));
-                            dd = dot3(m0, m1, m2, d.x, d.y, d.z);
-                        };
                         float ox, oy, oz, dx, dy, dz;
-                        row(w0, ox, dx); row(w1, oy, dy); row(w2, oz, dz);
+                        xform_row(w0, r.ox, r.oy, r.oz, d.x, d.y, d.z, ox, dx);
+                        xform_row(w1, r.ox, r.oy, r.oz, d.x, d.y, d.z, oy, dy);
+                        xform_row(w2, r.ox, r.oy, r.oz, d.x, d.y, d.z, oz, dz);
                         switch_ray(ox, oy, oz, dx, dy, dz);
                     } else {
                         bvh_off = __ldg(P.blas_offsets + g);
@@ -974,6 +996,97 @@ __global__ void untile_shards_kernel(const uchar4* __restrict__ src, uint32_t wi
     const uint32_t lx = px & 31u, ly = py & 7u;
     const uint32_t j = local_tile * 256u + (((ly >> 2) * 4u + (lx >> 3)) << 5) + ((ly & 3u) << 3) + (lx & 7u);
     dst[(size_t)py * width + px] = src[(size_t)shard * items_per_shard + j];
+}
+
+// ---- hit attributes (tray_cuda_hit_attributes): one thread per hit, after the traversal -------------------------------------
+// A pass of its own rather than three more live values in trace_kernel (its INST instantiations sit at 64 registers with spills):
+// it re-reads the ray, the hit and the triangle record (and the instance's transform), rebuilds the ray the triangle test saw and
+// repeats the test's u, v and Ng through the helpers tri_test uses, so the values are the test's own bits.
+struct AttrScene {
+    const uint4* __restrict__ tris;
+    uint64_t n_tris;
+    const uint4* __restrict__ inst_xf;       // INST: InstanceRecords by instance id
+    uint32_t n_inst;
+    uint32_t variant;                        // TRAY_VARIANT_*: only ZERODIR_BOX_ONLY reaches the triangle test's direction
+};
+
+// {u, v, ng} of hit `prim` (of instance `inst`) on the ray {a = origin, tmin; b = direction, tmax}; all bytes 0xFF for a miss, a
+// prim past the triangles or an instance past the instances, with nothing read for them
+template <int TRI_STRIDE, bool INST>
+__device__ __forceinline__ void hit_attr(const AttrScene& S, const float4& a, const float4& b, uint32_t prim, uint32_t inst, tray_hit_attr* out) {
+    float* o = reinterpret_cast<float*>(out);
+    if (prim == INVALID || prim >= S.n_tris || (INST && inst >= S.n_inst)) {
+        const float nan = __uint_as_float(0xffffffffu);
+        o[0] = nan; o[1] = nan; o[2] = nan; o[3] = nan; o[4] = nan;
+        return;
+    }
+    RayConst r;
+    const uint4* xf = INST ? S.inst_xf + (size_t)inst * INST_RECORD_U4 : nullptr;
+    if constexpr (INST) {                    // the TLAS leaf's object-space ray, prepared as switch_ray prepares it
+        const uint4 w0 = __ldg(xf), w1 = __ldg(xf + 1), w2 = __ldg(xf + 2);
+        float ox, oy, oz, dx, dy, dz;
+        xform_row(w0, a.x, a.y, a.z, b.x, b.y, b.z, ox, dx);
+        xform_row(w1, a.x, a.y, a.z, b.x, b.y, b.z, oy, dy);
+        xform_row(w2, a.x, a.y, a.z, b.x, b.y, b.z, oz, dz);
+        prepare_ray(r, ox, oy, oz, dx, dy, dz, a.w, 0u);
+    } else {
+        prepare_ray(r, a.x, a.y, a.z, b.x, b.y, b.z, a.w, S.variant);
+    }
+    float v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz;
+    tri_load<TRI_STRIDE>(S.tris, prim, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z);
+    tri_normal<TRI_STRIDE>(S.tris, prim, e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz);
+    float cx, cy, cz, inv_det, u, v;       // (r.tdx: the direction of the test, zero-patched unless ZERODIR_BOX_ONLY)
+    tri_uv(r.ox, r.oy, r.oz, r.tdx, r.tdy, r.tdz, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z, ngx, ngy, ngz, cx, cy, cz, inv_det, u, v);
+    if constexpr (INST) normal_to_world(xf, ngx, ngy, ngz);
+    o[0] = u; o[1] = v; o[2] = ngx; o[3] = ngy; o[4] = ngz;
+}
+
+// n hits of a ray batch; INST: `inst_ids` holds the instance of every hit (tray_cuda_trace_instance)
+template <int TRI_STRIDE, bool INST>
+__global__ void __launch_bounds__(256) hit_attr_kernel(const AttrScene S, const tray_ray* __restrict__ rays, const tray_hit* __restrict__ hits,
+                                                       const uint32_t* __restrict__ inst_ids, uint64_t n, tray_hit_attr* __restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t prim = __ldg(&hits[i].prim);
+    const uint32_t inst = INST ? __ldg(inst_ids + i) : 0u;
+    float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+    if (prim != INVALID) {
+        const float4* rp = reinterpret_cast<const float4*>(rays + i);
+        a = __ldg(rp); b = __ldg(rp + 1);
+    }
+    hit_attr<TRI_STRIDE, INST>(S, a, b, prim, inst, out + i);
+}
+
+// The last frame's attributes by local item (compact, as the frame's hit buffers): the primary ray as generated (`prays`), the
+// bounce ray regenerated by bounce_ray from the primary hit and direction, as raygen_bounce_kernel and the FRAME kernel make it.
+// Pixels that shot no bounce ray (outside the frame, or a primary miss) get the miss record.  Either output may be NULL.
+template <int TRI_STRIDE, bool INST>
+__global__ void __launch_bounds__(256) frame_attr_kernel(const __grid_constant__ FrameParams F, const AttrScene S, const tray_ray* __restrict__ prays,
+                                                         const tray_hit* __restrict__ primary, const tray_hit* __restrict__ bounce,
+                                                         const uint32_t* __restrict__ pinst, const uint32_t* __restrict__ binst,
+                                                         tray_hit_attr* __restrict__ out_primary, tray_hit_attr* __restrict__ out_bounce) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= F.n_items) return;
+    uint32_t px = 0, py = 0;
+    const bool inside = item_to_pixel(F, j, px, py);
+    const tray_hit ph = primary[j];
+    const uint32_t pk = INST ? pinst[j] : 0u;
+    const float4* rp = reinterpret_cast<const float4*>(prays + j);
+    const float4 pa = __ldg(rp), pb = __ldg(rp + 1);
+    if (out_primary) hit_attr<TRI_STRIDE, INST>(S, pa, pb, ph.prim, pk, out_primary + j);
+    if (out_bounce) {
+        const bool shoot = inside && ph.t < F32_MAX_ && ph.prim < S.n_tris && (!INST || pk < S.n_inst);   // rt_cpu.rs:61
+        float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+        uint32_t prim = INVALID;
+        if (shoot) {
+            float ox, oy, oz, dx, dy, dz;
+            bounce_ray<TRI_STRIDE, INST>(F, S.tris, px, py, pb.x, pb.y, pb.z, ph.t, ph.prim, ox, oy, oz, dx, dy, dz,
+                                         INST ? S.inst_xf + (size_t)pk * INST_RECORD_U4 : nullptr);
+            a = make_float4(ox, oy, oz, 0.0f); b = make_float4(dx, dy, dz, F32_MAX_);   // Ray::new(o, dir, 0.0, f32::MAX)
+            prim = bounce[j].prim;
+        }
+        hit_attr<TRI_STRIDE, INST>(S, a, b, prim, INST ? binst[j] : 0u, out_bounce + j);
+    }
 }
 
 }  // namespace tray

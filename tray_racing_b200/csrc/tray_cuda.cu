@@ -21,6 +21,7 @@ static_assert(sizeof(tray_cwbvh_node) == 80, "CwBvhNode is 80 bytes (bvh_embree_
 static_assert(sizeof(tray_tri48) == 48 && sizeof(tray_tri64) == 64 && sizeof(tray_tri24) == 24, "triangle record strides");
 static_assert(sizeof(tray_ray) == 32 && sizeof(tray_hit) == 8, "ray / hit records");
 static_assert(sizeof(tray_ray_cost) == 16 && alignof(tray_ray_cost) == 4, "ray cost record: one 16-byte store per ray");
+static_assert(sizeof(tray_hit_attr) == 20 && alignof(tray_hit_attr) == 4, "hit attribute record: u, v, ng[3]");
 static_assert(sizeof(tray_view) == 160, "ViewUniform is padded to 160 bytes (main.rs:589-597)");
 
 namespace {
@@ -75,6 +76,7 @@ struct FrameSlot {
     bool f_has_inst = false;                 // the last frame was rendered on an instanced scene
     uint32_t* d_flag = nullptr;              // the device error word of this slot's launches (a word of tray_scene::d_overflow)
     tray::FrameParams last_frame{};          // width 0: no frame rendered yet
+    uint64_t geom_gen = 0;                   // tray_scene::geom_gen when the last frame was rendered
 };
 
 struct tray_scene {
@@ -138,6 +140,11 @@ struct tray_scene {
     uint32_t* h_flag = nullptr;              // pinned, one word per staging slot: the error word of the frame staging slot i was filled from
     uchar4* frame_target = nullptr;          // borrowed: row-major RGBA8 frame (this or a peer device), see tray_cuda_scene_set_frame_target
     tray_counters cnt_primary{}, cnt_bounce{};
+    // geometry generation: every refit, TLAS rebuild, set_instances and set_variant that was not refused adds one, so that a frame
+    // whose hits no longer describe the scene's triangles is not given attributes (tray_cuda_frame_download_attributes)
+    uint64_t geom_gen = 0;
+    void* d_attr_buf = nullptr; uint64_t attr_cap = 0;   // tray_cuda_hit_attributes / frame attributes: 64 B per record, on first use
+    cudaEvent_t ev_attr = nullptr;           // tray_cuda_hit_attributes_device: a caller's stream waits for the scene stream
 };
 
 namespace {
@@ -463,6 +470,8 @@ void tray_cuda_scene_destroy(tray_scene* s) {
     if (s->own_stream) cudaStreamDestroy(s->own_stream);
     if (s->h_flag) cudaFreeHost(s->h_flag);
     if (s->ev_after) cudaEventDestroy(s->ev_after);
+    if (s->ev_attr) cudaEventDestroy(s->ev_attr);
+    cudaFree(s->d_attr_buf);
     delete s;
 }
 
@@ -520,6 +529,7 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         for (auto& e : s->ev) CU(cudaEventCreate(&e));
         CU(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
         CU(cudaEventCreateWithFlags(&s->ev_after, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&s->ev_attr, cudaEventDisableTiming));
         CU(cudaMallocHost(&s->h_flag, TRAY_READBACK_SLOTS * sizeof(uint32_t)));
         for (int i = 0; i < TRAY_READBACK_SLOTS; i++) {
             s->h_flag[i] = 0u;
@@ -675,6 +685,7 @@ int tray_cuda_scene_set_variant(tray_scene* s, uint32_t flags) {
     if (flags & ~0xfu) return fail(TRAY_ERR_ARG, "unknown variant flags 0x%x", flags);
     if (s->instanced) return fail(TRAY_ERR_ARG, "an instanced scene has no semantic variants");
     s->variant = flags;
+    s->geom_gen++;
     return TRAY_OK;
 }
 
@@ -1029,6 +1040,13 @@ int reserve_instances(tray_scene* s, uint32_t n) {
     }
     return TRAY_OK;
 }
+
+// the status of a call that changes the scene's geometry: unless it was refused (nothing changed), frames rendered before it
+// no longer match the scene
+int geometry_changed(tray_scene* s, int rc) {
+    if (s && rc != TRAY_ERR_ARG) s->geom_gen++;
+    return rc;
+}
 }  // namespace
 
 extern "C" {
@@ -1071,10 +1089,10 @@ int tray_cuda_scene_set_instances(tray_scene* s, const uint32_t* blas_roots, con
     CU(cudaEventRecord(s->ev[0], s->stream));
     CU(cudaMemcpyAsync(s->d_inst_in, in.data(), (size_t)n * 64, cudaMemcpyHostToDevice, s->stream));
     const TlasRebuild rb{ max_prims_per_leaf, search_radius };
-    const int rc = tlas_leg(s, n, rb, &lo, &hi, [&](uint4* nodes, bool* blas_exact) -> int {
+    const int rc = geometry_changed(s, tlas_leg(s, n, rb, &lo, &hi, [&](uint4* nodes, bool* blas_exact) -> int {
         if (tray_build::blas_exact(*s->refit, nodes, s->tlas_start, s->stream, blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "set_instances: %s", msg);
         return TRAY_OK;
-    }, ms, msg, sizeof msg);
+    }, ms, msg, sizeof msg));
     if (rc) return rc;
     s->instanced = true;
     s->n_instances = n;
@@ -1100,20 +1118,20 @@ int tray_cuda_scene_download_instance_xforms(tray_scene* s, uint32_t* leaf_insta
 }
 
 int tray_cuda_scene_refit(tray_scene* s, const float* tris9, uint64_t n_tris, float* ms_refit) {
-    return refit_impl(s, tris9, n_tris, false, nullptr, ms_refit);
+    return geometry_changed(s, refit_impl(s, tris9, n_tris, false, nullptr, ms_refit));
 }
 int tray_cuda_scene_refit_device(tray_scene* s, const float* d_tris9, uint64_t n_tris, void* stream, float* ms_refit) {
-    return refit_impl(s, d_tris9, n_tris, true, stream, ms_refit);
+    return geometry_changed(s, refit_impl(s, d_tris9, n_tris, true, stream, ms_refit));
 }
 int tray_cuda_scene_refit_rebuild_tlas(tray_scene* s, const float* tris9, uint64_t n_tris, uint32_t max_prims_per_leaf, uint32_t search_radius,
                                        float* ms) {
     const TlasRebuild rb{ max_prims_per_leaf, search_radius };
-    return refit_impl(s, tris9, n_tris, false, nullptr, ms, &rb);
+    return geometry_changed(s, refit_impl(s, tris9, n_tris, false, nullptr, ms, &rb));
 }
 int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* s, const float* d_tris9, uint64_t n_tris, uint32_t max_prims_per_leaf,
                                               uint32_t search_radius, void* stream, float* ms) {
     const TlasRebuild rb{ max_prims_per_leaf, search_radius };
-    return refit_impl(s, d_tris9, n_tris, true, stream, ms, &rb);
+    return geometry_changed(s, refit_impl(s, d_tris9, n_tris, true, stream, ms, &rb));
 }
 
 }  // extern "C"
@@ -1467,6 +1485,7 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     f.f_has_cost = keep_cost;
     f.f_has_inst = s->instanced;
     f.last_frame = F;
+    f.geom_gen = s->geom_gen;
     if (F.n_items == 0) {                        // a shard without tiles: no launch, and nothing to count
         if (ms_primary) *ms_primary = 0.f;
         if (ms_bounce) *ms_bounce = 0.f;
@@ -1765,6 +1784,129 @@ int tray_cuda_start(const void* bvh_bytes, uint64_t bvh_len, const void* instanc
                     render_time_s, benchmark, animate, out_min_ms, out_mean_ms, out_frames);
     tray_cuda_scene_destroy(s);
     return rc;
+}
+
+}  // extern "C"
+
+// ---- hit attributes: barycentrics and geometric normal (traverse.cuh hit_attr) --------------------------------------------------
+namespace {
+AttrScene attr_scene(const tray_scene* s) {
+    AttrScene S;
+    S.tris = s->d_tris; S.n_tris = s->n_tris;
+    S.inst_xf = s->instanced ? s->d_inst_in : nullptr; S.n_inst = s->instanced ? s->n_instances : 0u;
+    S.variant = s->variant;
+    return S;
+}
+
+// the scene's attribute staging with room for n records (rays, hits, instance ids and attributes of a host batch, or the compact
+// attributes of a frame): grown, never shrunk
+int ensure_attr_buf(tray_scene* s, uint64_t n) {
+    if (n <= s->attr_cap) return TRAY_OK;
+    cudaFree(s->d_attr_buf); s->d_attr_buf = nullptr; s->attr_cap = 0;
+    CU(cudaMalloc(&s->d_attr_buf, n * 64));
+    s->attr_cap = n;
+    return TRAY_OK;
+}
+
+int check_attr_args(const tray_scene* s, const void* rays, const void* hits, const uint32_t* ids, uint64_t n, const void* attrs) {
+    if (!s || (n && (!rays || !hits || !attrs))) return fail(TRAY_ERR_ARG, "NULL argument");
+    if (s->instanced && n && !ids) return fail(TRAY_ERR_ARG, "hit attributes on an instanced scene need the instance ids of tray_cuda_trace_instance");
+    if (!s->instanced && ids) return fail(TRAY_ERR_ARG, "instance ids given, but the scene is not instanced (tray_cuda_scene_set_instances)");
+    return TRAY_OK;
+}
+
+// hit_attr_kernel over n hits on `st`, in launches of at most 2^30 hits
+int launch_hit_attr(tray_scene* s, const tray_ray* rays, const tray_hit* hits, const uint32_t* ids, uint64_t n, tray_hit_attr* out, cudaStream_t st) {
+    const uint32_t k = s->tri_stride;
+    auto fn = s->instanced ? (k == 64 ? hit_attr_kernel<64, true> : k == 24 ? hit_attr_kernel<24, true> : hit_attr_kernel<48, true>)
+                           : (k == 64 ? hit_attr_kernel<64, false> : k == 24 ? hit_attr_kernel<24, false> : hit_attr_kernel<48, false>);
+    const AttrScene S = attr_scene(s);
+    const uint64_t chunk = 1ull << 30;
+    for (uint64_t off = 0; off < n; off += chunk) {
+        const uint64_t len = n - off < chunk ? n - off : chunk;
+        fn<<<(unsigned)((len + 255) / 256), 256, 0, st>>>(S, rays + off, hits + off, ids ? ids + off : nullptr, len, out + off);
+        CU(cudaGetLastError());
+    }
+    return TRAY_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int tray_cuda_hit_attributes(tray_scene* s, const tray_ray* rays, const tray_hit* hits, const uint32_t* instance_ids, uint64_t n,
+                             tray_hit_attr* attrs, float* ms_kernel) {
+    if (ms_kernel) *ms_kernel = 0.f;
+    if (const int rc = check_attr_args(s, rays, hits, instance_ids, n, attrs)) return rc;
+    if (n == 0) return TRAY_OK;
+    CU(cudaSetDevice(s->device));
+    if (const int rc = ensure_attr_buf(s, n)) return rc;
+    // 64 bytes per record: rays (32), hits (8), attributes (20), instance ids (4)
+    uint8_t* base = (uint8_t*)s->d_attr_buf;
+    tray_ray* d_rays = (tray_ray*)base;
+    tray_hit* d_hits = (tray_hit*)(base + n * 32);
+    tray_hit_attr* d_attrs = (tray_hit_attr*)(base + n * 40);
+    uint32_t* d_ids = instance_ids ? (uint32_t*)(base + n * 60) : nullptr;
+    cudaStream_t st = s->stream;
+    CU(cudaMemcpyAsync(d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_hits, hits, n * sizeof(tray_hit), cudaMemcpyHostToDevice, st));
+    if (d_ids) CU(cudaMemcpyAsync(d_ids, instance_ids, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(s->ev[0], st));
+    if (const int rc = launch_hit_attr(s, d_rays, d_hits, d_ids, n, d_attrs, st)) return rc;
+    CU(cudaEventRecord(s->ev[1], st));
+    CU(cudaMemcpyAsync(attrs, d_attrs, n * sizeof(tray_hit_attr), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (ms_kernel) CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+    return TRAY_OK;
+}
+
+int tray_cuda_hit_attributes_device(tray_scene* s, const tray_ray* d_rays, const tray_hit* d_hits, const uint32_t* d_instance_ids, uint64_t n,
+                                    tray_hit_attr* d_attrs, void* stream, float* ms_kernel) {
+    if (ms_kernel) *ms_kernel = 0.f;
+    if (const int rc = check_attr_args(s, d_rays, d_hits, d_instance_ids, n, d_attrs)) return rc;
+    CU(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (st != s->stream) {                          // after the traces enqueued on the scene stream
+        CU(cudaEventRecord(s->ev_attr, s->stream));
+        CU(cudaStreamWaitEvent(st, s->ev_attr, 0));
+    }
+    if (ms_kernel) CU(cudaEventRecord(s->ev[0], st));
+    if (const int rc = launch_hit_attr(s, d_rays, d_hits, d_instance_ids, n, d_attrs, st)) return rc;
+    if (ms_kernel) {
+        CU(cudaEventRecord(s->ev[1], st));
+        CU(cudaEventSynchronize(s->ev[1]));
+        CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+    }
+    return TRAY_OK;
+}
+
+int tray_cuda_frame_download_attributes(tray_scene* s, tray_hit_attr* primary, tray_hit_attr* bounce) {
+    if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
+    const FrameSlot& f = s->slot[s->cur];
+    if (f.last_frame.width == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
+    if (bounce && !f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
+    if (f.geom_gen != s->geom_gen)
+        return fail(TRAY_ERR_ARG, "the scene has changed since the last frame (refit, TLAS rebuild, set_instances or set_variant): its attributes "
+                                  "would not describe that frame's hits");
+    if (!primary && !bounce) return TRAY_OK;
+    CU(cudaSetDevice(s->device));
+    const FrameParams& F = f.last_frame;
+    if (const int rc = ensure_attr_buf(s, F.n_items ? F.n_items : 1)) return rc;
+    tray_hit_attr* d_p = (tray_hit_attr*)s->d_attr_buf;
+    tray_hit_attr* d_b = d_p + F.n_items;
+    if (F.n_items) {
+        // (a frame of an instanced scene was rendered after its set_instances: the generation check above holds f_has_inst to
+        // s->instanced)
+        const uint32_t k = s->tri_stride;
+        auto fn = f.f_has_inst ? (k == 64 ? frame_attr_kernel<64, true> : k == 24 ? frame_attr_kernel<24, true> : frame_attr_kernel<48, true>)
+                               : (k == 64 ? frame_attr_kernel<64, false> : k == 24 ? frame_attr_kernel<24, false> : frame_attr_kernel<48, false>);
+        fn<<<(F.n_items + 255) / 256, 256, 0, slot_stream(s, s->cur)>>>(F, attr_scene(s), f.d_prays, f.d_primary, f.d_bounce, f.d_pinst, f.d_binst,
+                                                                         primary ? d_p : nullptr, bounce ? d_b : nullptr);
+        CU(cudaGetLastError());
+    }
+    int rc;
+    if (primary) { rc = download<tray_hit_attr>(s, d_p, primary, 0xff); if (rc) return rc; }
+    if (bounce) { rc = download<tray_hit_attr>(s, d_b, bounce, 0xff); if (rc) return rc; }
+    return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 
 }  // extern "C"

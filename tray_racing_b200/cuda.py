@@ -37,11 +37,15 @@ EXPORTS = (
     "tray_cuda_scene_refit_rebuild_tlas", "tray_cuda_scene_refit_rebuild_tlas_device",
     "tray_cuda_scene_set_instances", "tray_cuda_scene_download_instance_xforms", "tray_cuda_trace_instance",
     "tray_cuda_trace_instance_device", "tray_cuda_frame_download_instance",
+    "tray_cuda_hit_attributes", "tray_cuda_hit_attributes_device", "tray_cuda_frame_download_attributes",
 )
 # semantic switches of tray_cuda_scene_set_variant (include/tray_cuda.h TRAY_VARIANT_*)
 VARIANT_BOX_DIVIDE, VARIANT_TIE_LAST, VARIANT_BOX_TMIN_RAY, VARIANT_ZERODIR_BOX_ONLY = 1, 2, 4, 8
 # tray_ray_cost (include/tray_cuda.h): one ray's nodes fetched, triangles tested, TLAS leaf entries, peak stack entries
 COST_DTYPE = np.dtype([("nodes", "<u4"), ("tris", "<u4"), ("instances", "<u4"), ("stack", "<u4")])
+# tray_hit_attr (include/tray_cuda.h): the triangle test's barycentrics of v1 and v2 and its geometric normal (world space, not
+# normalised); every byte 0xFF for a miss
+ATTR_DTYPE = np.dtype([("u", "<f4"), ("v", "<f4"), ("ng", "<f4", 3)])
 
 
 class TrayCudaError(RuntimeError):
@@ -239,6 +243,12 @@ def lib() -> C.CDLL:
         L.tray_cuda_trace_instance_device.argtypes = [vp, vp, u64, i32, vp, vp, vp, f32p]
         L.tray_cuda_frame_download_instance.restype = i32
         L.tray_cuda_frame_download_instance.argtypes = [vp, vp, vp]
+        L.tray_cuda_hit_attributes.restype = i32
+        L.tray_cuda_hit_attributes.argtypes = [vp, vp, vp, vp, u64, vp, f32p]
+        L.tray_cuda_hit_attributes_device.restype = i32
+        L.tray_cuda_hit_attributes_device.argtypes = [vp, vp, vp, vp, u64, vp, vp, f32p]
+        L.tray_cuda_frame_download_attributes.restype = i32
+        L.tray_cuda_frame_download_attributes.argtypes = [vp, vp, vp]
         _lib = L
     return _lib
 
@@ -455,6 +465,54 @@ class TrayCudaScene:
         out = {name: np.zeros(w * h, dtype=np.uint32) for name, want in (("primary", primary), ("bounce", bounce)) if want}
         p, b = out.get("primary"), out.get("bounce")
         _check(lib().tray_cuda_frame_download_instance(self._h, None if p is None else p.ctypes.data, None if b is None else b.ctypes.data))
+        return out
+
+    def _instanced(self) -> bool:
+        """whether set_instances has made the scene instanced (the library accepts its instance-transform download)"""
+        h = getattr(self, "_h", None)
+        return bool(h is not None and h.value) and lib().tray_cuda_scene_download_instance_xforms(h, None, None) == 0
+
+    def hit_attributes(self, rays, hits, instance_ids=None, timings: dict | None = None) -> np.ndarray:
+        """{u, v, ng} (ATTR_DTYPE) of every hit on its ray, as the triangle test computed them (tray_cuda_hit_attributes).
+        `instance_ids` (from traverse_instance) is required on an instanced scene and must be None on any other."""
+        rays, hits = np.asarray(rays), np.asarray(hits)
+        if rays.dtype != RAY_DTYPE or hits.dtype != HIT_DTYPE:
+            raise ValueError(f"rays must be RAY_DTYPE and hits HIT_DTYPE, got {rays.dtype} and {hits.dtype}")
+        if rays.ndim != 1 or rays.shape != hits.shape:
+            raise ValueError(f"rays and hits must be 1-D arrays of one length, got {rays.shape} and {hits.shape}")
+        ids = None
+        if instance_ids is not None:
+            ids = np.asarray(instance_ids)
+            if ids.dtype.kind not in "iu" or ids.shape != hits.shape or (ids.size and (ids.min() < 0 or ids.max() > 0xFFFFFFFF)):
+                raise ValueError(f"instance_ids must be uint32 of shape {hits.shape}")
+            ids = np.ascontiguousarray(ids, dtype=np.uint32)
+        if (ids is None) == self._instanced():
+            raise ValueError("instance_ids are required on an instanced scene and refused on any other")
+        rays, hits = np.ascontiguousarray(rays), np.ascontiguousarray(hits)
+        out = np.empty(rays.shape[0], dtype=ATTR_DTYPE)
+        k = C.c_float()
+        _check(lib().tray_cuda_hit_attributes(self._h, rays.ctypes.data, hits.ctypes.data, None if ids is None else ids.ctypes.data,
+                                              rays.shape[0], out.ctypes.data, C.byref(k)))
+        if timings is not None:
+            timings["ms_kernel"] = k.value
+        return out
+
+    def hit_attributes_device(self, d_rays_ptr: int, d_hits_ptr: int, d_ids_ptr: int | None, n: int, d_attrs_ptr: int, stream: int = 0,
+                              timed: bool = False):
+        """hit_attributes() on device buffers (20-byte records at `d_attrs_ptr`), ordered after the scene stream's traces
+        (tray_cuda_hit_attributes_device); returns ms_kernel when `timed`."""
+        k = C.c_float()
+        _check(lib().tray_cuda_hit_attributes_device(self._h, d_rays_ptr, d_hits_ptr, d_ids_ptr or None, n, d_attrs_ptr, stream or None,
+                                                     C.byref(k) if timed else None))
+        return k.value if timed else None
+
+    def download_attributes(self, primary=True, bounce=False) -> dict:
+        """The last frame's hit attributes (ATTR_DTYPE, row-major, w*h): "primary" and / or "bounce"; every byte 0xFF for misses,
+        other shards' pixels and pixels without a bounce ray (tray_cuda_frame_download_attributes)."""
+        w, h = self.frame_size
+        out = {name: np.zeros(w * h, dtype=ATTR_DTYPE) for name, want in (("primary", primary), ("bounce", bounce)) if want}
+        p, b = out.get("primary"), out.get("bounce")
+        _check(lib().tray_cuda_frame_download_attributes(self._h, None if p is None else p.ctypes.data, None if b is None else b.ctypes.data))
         return out
 
     @classmethod
