@@ -503,6 +503,31 @@ def test_frames_of_instanced_scenes(cornell, stride, in_flight):
         sc.close()
 
 
+@gpu
+def test_frame_of_2_26_items(cornell):
+    """8192 x 8192 pixels: 2^26 items, whose attribute staging (64 B per item) is 4 GiB, past 32-bit sizes; a sample of its
+    pixels has the attributes of hit_attributes over the frame's own rays and hits"""
+    w = h = 8192
+    assert cuda.local_items(w, h) == 1 << 26
+    view = host.view_from_camera(cornell.camera, w, h)
+    sc = cuda.TrayCudaScene.from_packed(host.PackedScene(cornell))
+    try:
+        sc.render(view, w, h, 0, cuda.RENDER_BOUNCE | cuda.RENDER_KEEP_RAYS)
+        sc.sync()
+        got = sc.download_attributes(primary=True, bounce=True)
+        frame = sc.download(primary=True, bounce=True, bounce_rays=True)
+        pick = np.sort(np.random.default_rng(5).choice(w * h, 1 << 20, replace=False))
+        shoot = frame["primary"]["t"][pick] < F32_MAX
+        assert shoot.sum() > 100000
+        want_b = np.frombuffer(b"\xff" * (20 * pick.size), dtype=cuda.ATTR_DTYPE).copy()
+        want_b[shoot] = sc.hit_attributes(frame["bounce_rays"][pick][shoot], frame["bounce"][pick][shoot])
+        assert same_bytes(got["bounce"][pick], want_b)
+        prays = ob.primary_rays(view, w, h)[pick]
+        assert same_bytes(got["primary"][pick], sc.hit_attributes(prays, frame["primary"][pick]))
+    finally:
+        sc.close()
+
+
 def refused_without_writing(sc, n):
     L = cuda.lib()
     p = np.full(n * 5, 0x12345678, np.uint32)

@@ -707,8 +707,6 @@ struct Scratch {
     ~Scratch() { for (int i = 0; i < n; i++) cudaFree(p[i]); if (arena && owned) cudaFree(arena); }
 };
 
-template <typename T> cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) { T* q = nullptr; const cudaError_t e = cudaMalloc(&q, bytes); p.reset(q); return e; }
-
 // Exclusive sums of the flag arrays a and b over m + 1 entries, entry m zeroed first so that the sum there is the total.
 // `consume` enqueues the work that reads the sums; then tot = the two totals, read back once the stream has drained.
 template <typename F>
@@ -1126,7 +1124,7 @@ __global__ void __launch_bounds__(TPB) refit_node_kernel(const uint2* __restrict
 // TLAS-leaf order, triangle indices global.
 int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_offsets, uint32_t n_objects, uint32_t tri_stride,
                uint32_t max_leaf, uint32_t radius, cudaStream_t st, Result* out, char* err, size_t errlen) {
-    memset(out, 0, sizeof *out);
+    *out = Result{};
     if (n_tris == 0) return 0;
     if (n_tris >= 0x7fffffffull) { snprintf(err, errlen, "too many triangles"); return -1; }
     const bool tlas = object_offsets != nullptr;
@@ -1194,8 +1192,8 @@ int build_tlas(const float* tris9_host, uint64_t n_tris, const uint64_t* object_
         n_nodes += to.n_nodes; tl_iters = to.iters; tl_levels = to.co.levels; force_exact = force_exact || to.co.force_exact;
     }
     const double t_end = now_ms();
-    out->d_nodes = d_nodes.release(); out->n_nodes = n_nodes; out->node_cap = blas_cap + tlas_cap; out->d_tris = d_tri_out.release(); out->d_prim_indices = d_prim_idx.release();
-    out->d_blas_offsets = d_blas.release(); out->n_instances = tlas ? n_objects : 0; out->tlas_start = tlas_start;
+    out->d_nodes = std::move(d_nodes); out->n_nodes = n_nodes; out->node_cap = blas_cap + tlas_cap; out->d_tris = std::move(d_tri_out);
+    out->d_prim_indices = std::move(d_prim_idx); out->d_blas_offsets = std::move(d_blas); out->n_instances = tlas ? n_objects : 0; out->tlas_start = tlas_start;
     out->force_exact = force_exact;
     out->stats.n_tris = n; out->stats.n_nodes = n_nodes; out->stats.ploc_iterations = pl.iters + tl_iters; out->stats.levels = co.levels + tl_levels;
     out->stats.ms_upload = (float)(t_upload - t_begin); out->stats.ms_sort = 0.f;

@@ -25,16 +25,46 @@ namespace tray_build {
 // device memory freed with cudaFree when its owner goes
 struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
 template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T> cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) { T* q = nullptr; const cudaError_t e = cudaMalloc(&q, bytes); p.reset(q); return e; }
+
+// pinned host memory, freed with cudaFreeHost
+struct CudaFreeHost { void operator()(void* p) const { cudaFreeHost(p); } };
+template <typename T> using HostPtr = std::unique_ptr<T, CudaFreeHost>;
+template <typename T> cudaError_t host_alloc(HostPtr<T>& p, size_t bytes) { T* q = nullptr; const cudaError_t e = cudaMallocHost(&q, bytes); p.reset(q); return e; }
+
+// streams (non-blocking) and events, destroyed when their owner goes
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+using Stream = std::unique_ptr<CUstream_st, StreamDestroy>;
+inline cudaError_t make_stream(Stream& s) { cudaStream_t q = nullptr; const cudaError_t e = cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking); s.reset(q); return e; }
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+inline cudaError_t make_event(Event& ev, unsigned flags = cudaEventDefault) { cudaEvent_t q = nullptr; const cudaError_t e = cudaEventCreateWithFlags(&q, flags); ev.reset(q); return e; }
+
+// Device memory that grows and never shrinks, for n elements of T.  A growth frees the old allocation before it makes the new
+// one, so that the peak is the new size alone, and keeps no contents.  A failed growth leaves the buffer empty (cap 0): the next
+// call tries again.
+template <typename T> struct DevBuf {
+    DevPtr<T> p;
+    uint64_t cap = 0;
+    T* get() const { return p.get(); }
+    cudaError_t reserve(uint64_t n) {
+        if (n <= cap) return cudaSuccess;
+        p.reset(); cap = 0;
+        const cudaError_t e = dev_alloc(p, n * sizeof(T));
+        if (e == cudaSuccess) cap = n;
+        return e;
+    }
+};
 
 struct Result {
-    uint8_t* d_nodes;            // n_nodes x 80 bytes (allocation holds node_cap nodes); caller owns (cudaFree)
-    uint64_t n_nodes, node_cap;
-    uint8_t* d_tris;             // n_tris x tri_stride, BVH order; caller owns
-    uint32_t* d_prim_indices;    // BVH slot -> input triangle; caller owns
-    uint32_t* d_blas_offsets;    // two-level builds: node index of the BLAS behind TLAS leaf k; caller owns
-    uint32_t n_instances, tlas_start;
-    bool force_exact;            // some node scale >= 2^40 (see tray_scene::force_exact)
-    tray_build_stats stats;
+    DevPtr<uint8_t> d_nodes;           // n_nodes x 80 bytes (the allocation holds node_cap nodes)
+    uint64_t n_nodes = 0, node_cap = 0;
+    DevPtr<uint8_t> d_tris;            // n_tris x tri_stride, BVH order
+    DevPtr<uint32_t> d_prim_indices;   // BVH slot -> input triangle
+    DevPtr<uint32_t> d_blas_offsets;   // two-level builds: node index of the BLAS behind TLAS leaf k
+    uint32_t n_instances = 0, tlas_start = 0;
+    bool force_exact = false;          // some node scale >= 2^40 (see tray_scene::force_exact)
+    tray_build_stats stats{};
 };
 
 // Builds on the current device, synchronously with respect to `st`.  Returns 0, or a negative code with a message in `err`.

@@ -53,30 +53,55 @@ bool scene_force_exact(bool nodes_need_it) { return env_int("TRAY_CUDA_FORCE_EXA
 
 }  // namespace
 
-// Everything one frame in flight owns: its compact (tile-ordered) buffers, its work cursors and its stream.  Slot 0 runs on
+using tray_build::DevBuf;
+using tray_build::DevPtr;
+using tray_build::Event;
+using tray_build::HostPtr;
+using tray_build::Stream;
+using tray_build::dev_alloc;
+using tray_build::host_alloc;
+using tray_build::make_event;
+using tray_build::make_stream;
+
+// The compact (tile-ordered) buffers of one frame slot, allocated together for `cap` items
+struct FrameBuffers {
+    uint64_t cap = 0;
+    DevPtr<tray_hit> d_primary, d_bounce; DevPtr<uchar4> d_rgba;
+    DevPtr<tray_ray> d_prays;                // generated primary rays, local order
+    DevPtr<tray_ray> d_brays;                // generated bounce rays, COMPACT (hit pixels only)
+    DevPtr<uint32_t> d_bitem;                // local item of compact bounce ray i
+    DevPtr<tray_ray> d_brays_item;           // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
+    DevPtr<tray_ray_cost> d_cost;            // optional: ray costs by local item, 2 x cap: primary [0, n_items), bounce from n_items
+    DevPtr<uint32_t> d_pinst, d_binst;       // instanced scenes: the instance of each primary / bounce hit by item
+};
+
+// Everything one frame in flight owns: its compact buffers, its work cursors and its stream.  Slot 0 runs on
 // tray_scene::stream (the scene's own, or the caller's: tray_cuda_scene_set_stream), slot 1 on a stream of its own, so that
 // the kernels of frame k+1 fill the SM slots the drain phase of frame k leaves empty.
 struct FrameSlot {
-    cudaStream_t own_stream = nullptr;       // slot 1 only
-    unsigned long long* d_cursor = nullptr;  // cursor block (tray::CURSOR_WORDS)
-    uint32_t* d_units = nullptr;             // FRAME kernel: cursor over the 32-item groups of bounce work
-    cudaEvent_t ev[4] = { nullptr, nullptr, nullptr, nullptr };
-    cudaEvent_t done = nullptr;              // recorded behind the frame's last launch (fences, group completion)
-    uint64_t f_cap = 0;
+    Stream own_stream;                       // slot 1 only
+    DevPtr<unsigned long long> d_cursor;     // cursor block (tray::CURSOR_WORDS)
+    DevPtr<uint32_t> d_units;                // FRAME kernel: cursor over the 32-item groups of bounce work
+    Event ev[4];
+    Event done;                              // recorded behind the frame's last launch (fences, group completion)
+    FrameBuffers buf;
     bool f_has_bounce = false, f_has_rgba = false, f_has_rays = false;
     uchar4* f_target = nullptr;              // the frame target the last frame was rendered into (NULL: compact d_rgba)
-    tray_hit* d_primary = nullptr; tray_hit* d_bounce = nullptr; uchar4* d_rgba = nullptr;
-    tray_ray* d_prays = nullptr;             // generated primary rays, local order
-    tray_ray* d_brays = nullptr;             // generated bounce rays, COMPACT (hit pixels only)
-    uint32_t* d_bitem = nullptr;             // local item of compact bounce ray i
-    tray_ray* d_brays_item = nullptr;        // optional: bounce rays by local item (TRAY_RENDER_KEEP_RAYS)
-    tray_ray_cost* d_cost = nullptr;         // optional: ray costs by local item, 2 x f_cap: primary [0, n_items), bounce from n_items
     bool f_has_cost = false;                 // the last frame kept ray costs (tray_cuda_scene_set_ray_cost + TRAY_RENDER_COUNTERS)
-    uint32_t* d_pinst = nullptr; uint32_t* d_binst = nullptr;   // instanced scenes: the instance of each primary / bounce hit by item
     bool f_has_inst = false;                 // the last frame was rendered on an instanced scene
     uint32_t* d_flag = nullptr;              // the device error word of this slot's launches (a word of tray_scene::d_overflow)
     tray::FrameParams last_frame{};          // width 0: no frame rendered yet
     uint64_t geom_gen = 0;                   // tray_scene::geom_gen when the last frame was rendered
+};
+
+// host <-> device pipeline of tray_cuda_trace: two pinned staging slots per direction, copy streams, events.  Built whole by
+// ensure_pipeline or not at all: s_in is set once it is ready.
+struct Pipeline {
+    Stream s_in, s_out;
+    HostPtr<tray_ray> h_rays[2]; HostPtr<tray_hit> h_hits[2];
+    HostPtr<tray_ray_cost> h_costs[2];       // pinned cost slots, allocated by the first pipelined cost call
+    HostPtr<uint32_t> h_inst[2];             // pinned instance-id slots, allocated by the first pipelined instance call
+    Event e_in[2], e_k[2], e_out[2];
 };
 
 struct tray_scene {
@@ -87,19 +112,20 @@ struct tray_scene {
     uint32_t tri_stride = 48, n_instances = 0, tlas_start = 0;
     bool tlas = false;
     bool force_exact = false;                // some node scale >= 2^40: 2^23 * adj_inv could overflow in the fused node test
-    uint4* d_nodes = nullptr;
-    uint4* d_tris = nullptr;
-    uint32_t* d_blas = nullptr;
-    uint32_t* d_prim_indices = nullptr;      // BVH slot -> input triangle (scenes made by tray_cuda_scene_build)
-    tray_build::RefitTopology* refit = nullptr;   // the topology walk of the first tray_cuda_scene_refit, kept for the next
-    uint32_t* d_geom_offsets = nullptr; uint32_t n_geometries = 0;   // first global triangle of BLAS / object g (tray_cuda_scene_set_geometry_offsets)
-    unsigned long long* d_cursor = nullptr;     // cursor block of batch traces (tray::CURSOR_WORDS)
+    DevPtr<uint4> d_nodes;
+    DevPtr<uint4> d_tris;
+    DevPtr<uint32_t> d_blas;
+    uint32_t blas_cap = 0;                   // blas_offsets entries d_blas has room for
+    DevPtr<uint32_t> d_prim_indices;         // BVH slot -> input triangle (scenes made by tray_cuda_scene_build)
+    std::unique_ptr<tray_build::RefitTopology> refit;   // the topology walk of the first tray_cuda_scene_refit, kept for the next
+    DevPtr<uint32_t> d_geom_offsets; uint32_t n_geometries = 0;   // first global triangle of BLAS / object g (tray_cuda_scene_set_geometry_offsets)
+    DevPtr<unsigned long long> d_cursor;     // cursor block of batch traces (tray::CURSOR_WORDS)
     // device error words (TraceParams::overflow): [0] batch traces, [1 + k] the launches of frame slot k — one word per slot, so
     // that a frame's error is reported for that frame and cleared in the order of that slot's stream
-    uint32_t* d_overflow = nullptr;
-    cudaStream_t stream = nullptr;          // the stream work is enqueued on
-    cudaStream_t own_stream = nullptr;      // created with the scene
-    cudaEvent_t ev[2] = { nullptr, nullptr };
+    DevPtr<uint32_t> d_overflow;
+    cudaStream_t stream = nullptr;           // the stream work is enqueued on: own_stream, or the caller's (never owned)
+    Stream own_stream;                       // created with the scene
+    Event ev[2];
     bool have_window = false;                // persisting-L2 access-policy window over the node array, applied per launch
     cudaAccessPolicyWindow window{};
     uint64_t device_bytes = 0, l2_bytes = 0, l2_persist = 0;
@@ -108,66 +134,43 @@ struct tray_scene {
     uint32_t variant = 0;                    // TRAY_VARIANT_* (tray_cuda_scene_set_variant): the MODE 1 kernels
     // instanced scenes (tray_cuda_scene_set_instances): the INST kernels
     bool instanced = false;
-    uint32_t inst_cap = 0, blas_cap = 0;     // instance records / blas_offsets entries the device arrays have room for
-    uint4* d_inst_in = nullptr;              // InstanceRecord (traverse.cuh) by instance id
-    uint4* d_inst_rec = nullptr;             // InstanceRecord by TLAS leaf (TraceParams::inst_rec)
+    uint32_t inst_cap = 0;                   // instance records the two record arrays have room for
+    DevPtr<uint4> d_inst_in;                 // InstanceRecord (traverse.cuh) by instance id
+    DevPtr<uint4> d_inst_rec;                // InstanceRecord by TLAS leaf (TraceParams::inst_rec)
     std::vector<uint32_t> inst_roots;        // the caller's blas_roots and object_to_world of the last set_instances
     std::vector<float> inst_o2w;
-    uint32_t* d_inst_ids = nullptr; uint64_t inst_ids_cap = 0;   // tray_cuda_trace_instance: allocated on first use
-    uint32_t* h_inst[2] = { nullptr, nullptr };                  // pinned instance-id slots of the pipelined host path
+    DevBuf<uint32_t> d_inst_ids;             // tray_cuda_trace_instance: allocated on first use
     uint32_t refill_min = 6, tri_weight = 3, gen_min = 4;
     bool overlap_default = false;            // TRAY_CUDA_OVERLAP=1: tray_cuda_render always takes the one-launch frame kernel
     // resident CTAs per SM of the lane kernel [0], the MODE 1 kernel [1], the counting lane kernel [2], the INST kernel [3] and the
     // counting INST kernel [4]
     int blocks_per_sm[5] = { 0, 0, 0, 0, 0 };
     // ray-batch staging
-    tray_ray* d_rays = nullptr; tray_hit* d_hits = nullptr; uint64_t batch_cap = 0;
-    tray_ray_cost* d_costs = nullptr; uint64_t cost_cap = 0;   // tray_cuda_trace_cost: allocated on first use
-    // host <-> device pipeline of tray_cuda_trace: two pinned staging slots per direction, copy streams, events
-    tray_ray* h_rays[2] = { nullptr, nullptr }; tray_hit* h_hits[2] = { nullptr, nullptr };
-    tray_ray_cost* h_costs[2] = { nullptr, nullptr };          // pinned cost slots, allocated by the first pipelined cost call
-    cudaStream_t s_in = nullptr, s_out = nullptr; bool pipeline_ready = false;
-    cudaEvent_t e_in[2] = { nullptr, nullptr }, e_k[2] = { nullptr, nullptr }, e_out[2] = { nullptr, nullptr };
+    DevBuf<tray_ray> d_rays; DevBuf<tray_hit> d_hits;
+    DevBuf<tray_ray_cost> d_costs;           // tray_cuda_trace_cost: allocated on first use
+    Pipeline pipe;
     // frame state: one FrameSlot per frame in flight (tray_cuda_scene_set_frames_in_flight); `cur` = the slot of the last frame
     FrameSlot slot[TRAY_MAX_FRAMES_IN_FLIGHT];
     int n_slots = 1, cur = 0;
-    void* d_untiled = nullptr; uint64_t untiled_cap = 0;
+    DevBuf<uint8_t> d_untiled;
     // asynchronous RGBA readback: double-buffered row-major staging, copies on their own stream
-    cudaStream_t copy_stream = nullptr;
-    uchar4* d_stage[TRAY_READBACK_SLOTS] = {}; uint64_t stage_cap[TRAY_READBACK_SLOTS] = {}; bool stage_busy[TRAY_READBACK_SLOTS] = {};
-    cudaEvent_t ev_untiled[TRAY_READBACK_SLOTS] = {}, ev_copied[TRAY_READBACK_SLOTS] = {};
-    cudaEvent_t ev_after = nullptr;          // tray_cuda_scene_after
-    uint32_t* h_flag = nullptr;              // pinned, one word per staging slot: the error word of the frame staging slot i was filled from
+    Stream copy_stream;
+    DevBuf<uchar4> d_stage[TRAY_READBACK_SLOTS]; bool stage_busy[TRAY_READBACK_SLOTS] = {};
+    Event ev_untiled[TRAY_READBACK_SLOTS], ev_copied[TRAY_READBACK_SLOTS];
+    Event ev_after;                          // tray_cuda_scene_after
+    HostPtr<uint32_t> h_flag;                // pinned, one word per staging slot: the error word of the frame staging slot i was filled from
     uchar4* frame_target = nullptr;          // borrowed: row-major RGBA8 frame (this or a peer device), see tray_cuda_scene_set_frame_target
     tray_counters cnt_primary{}, cnt_bounce{};
     // geometry generation: every refit, TLAS rebuild, set_instances and set_variant that was not refused adds one, so that a frame
     // whose hits no longer describe the scene's triangles is not given attributes (tray_cuda_frame_download_attributes)
     uint64_t geom_gen = 0;
-    void* d_attr_buf = nullptr; uint64_t attr_cap = 0;   // tray_cuda_hit_attributes / frame attributes: 64 B per record, on first use
-    cudaEvent_t ev_attr = nullptr;           // tray_cuda_hit_attributes_device: a caller's stream waits for the scene stream
+    DevBuf<uint8_t> d_attr_buf;              // tray_cuda_hit_attributes / frame attributes: 64 B per record, on first use
+    Event ev_attr;                           // tray_cuda_hit_attributes_device: a caller's stream waits for the scene stream
 };
 
 namespace {
 
 using namespace tray;
-
-void free_pipeline(tray_scene* s) {
-    for (int i = 0; i < 2; i++) {
-        if (s->h_rays[i]) cudaFreeHost(s->h_rays[i]);
-        if (s->h_hits[i]) cudaFreeHost(s->h_hits[i]);
-        if (s->h_costs[i]) cudaFreeHost(s->h_costs[i]);
-        if (s->h_inst[i]) cudaFreeHost(s->h_inst[i]);
-        s->h_costs[i] = nullptr; s->h_inst[i] = nullptr;
-        if (s->e_in[i]) cudaEventDestroy(s->e_in[i]);
-        if (s->e_k[i]) cudaEventDestroy(s->e_k[i]);
-        if (s->e_out[i]) cudaEventDestroy(s->e_out[i]);
-        s->h_rays[i] = nullptr; s->h_hits[i] = nullptr; s->e_in[i] = s->e_k[i] = s->e_out[i] = nullptr;
-    }
-    if (s->s_in) cudaStreamDestroy(s->s_in);
-    if (s->s_out) cudaStreamDestroy(s->s_out);
-    s->s_in = s->s_out = nullptr;
-    s->pipeline_ready = false;
-}
 
 
 typedef void (*kernel_fn)(const TraceParams);
@@ -204,11 +207,11 @@ uint64_t local_items(uint32_t w, uint32_t h, uint32_t shard, uint32_t shards) {
 
 void base_params(const tray_scene* s, TraceParams& P) {
     memset(&P, 0, sizeof P);
-    P.nodes = s->d_nodes; P.tris = s->d_tris; P.blas_offsets = s->d_blas; P.tlas_start = s->tlas_start;
-    P.cursor = (uint32_t*)s->d_cursor; P.overflow = s->d_overflow;
+    P.nodes = s->d_nodes.get(); P.tris = s->d_tris.get(); P.blas_offsets = s->d_blas.get(); P.tlas_start = s->tlas_start;
+    P.cursor = (uint32_t*)s->d_cursor.get(); P.overflow = s->d_overflow.get();
     P.refill_min = s->refill_min; P.tri_weight = s->tri_weight; P.k4b = 0x4B000000u; P.force_exact = s->force_exact ? 1u : 0u;
     P.variant = s->variant; P.one = 1u;
-    P.inst_rec = s->d_inst_rec;
+    P.inst_rec = s->d_inst_rec.get();
 }
 
 const char* const VARIANT_REFUSAL = "semantic variants (tray_cuda_scene_set_variant) cover the closest-hit kernels without counters only";
@@ -247,22 +250,14 @@ int launch(tray_scene* s, TraceParams& P, cudaStream_t st, unsigned long long* c
     return TRAY_OK;
 }
 
-cudaStream_t slot_stream(const tray_scene* s, int k) { return k == 0 ? s->stream : s->slot[k].own_stream; }
+cudaStream_t slot_stream(const tray_scene* s, int k) { return k == 0 ? s->stream : s->slot[k].own_stream.get(); }
 int next_slot(const tray_scene* s) { return (s->cur + 1) % s->n_slots; }     // the slot the next tray_cuda_render takes
 // waits for the scene stream and the scene's own frame streams (slot 0 runs on tray_scene::stream), in the order asked for
 int sync_streams(const tray_scene* s, bool scene_stream_first) {
     if (scene_stream_first) CU(cudaStreamSynchronize(s->stream));
-    for (int k = 1; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) CU(cudaStreamSynchronize(s->slot[k].own_stream));
+    for (int k = 1; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) CU(cudaStreamSynchronize(s->slot[k].own_stream.get()));
     if (!scene_stream_first) CU(cudaStreamSynchronize(s->stream));
     return TRAY_OK;
-}
-
-// the per-frame buffers of a slot (not its cursor block); the caller has synchronised the slot's stream
-void free_frame_buffers(FrameSlot& f) {
-    cudaFree(f.d_primary); cudaFree(f.d_bounce); cudaFree(f.d_brays); cudaFree(f.d_rgba);
-    cudaFree(f.d_prays); cudaFree(f.d_bitem); cudaFree(f.d_brays_item); cudaFree(f.d_cost); cudaFree(f.d_pinst); cudaFree(f.d_binst);
-    f.d_primary = nullptr; f.d_bounce = nullptr; f.d_brays = nullptr; f.d_rgba = nullptr;
-    f.d_prays = nullptr; f.d_bitem = nullptr; f.d_brays_item = nullptr; f.d_cost = nullptr; f.d_pinst = nullptr; f.d_binst = nullptr; f.f_cap = 0;
 }
 
 int check_tri_stride(uint32_t tri_stride) {
@@ -393,20 +388,19 @@ int tray_cuda_l1_gather_probe(int device, uint32_t bytes, int iters, float* out_
     if (tray_cuda_device_count() == 0) return fail(TRAY_ERR_NO_DEVICE, "no CUDA device");
     CU(cudaSetDevice(device));
     cudaDeviceProp prop; CU(cudaGetDeviceProperties(&prop, device));
-    uint4* buf = nullptr; uint32_t* out = nullptr;
+    DevPtr<uint4> buf; DevPtr<uint32_t> out;
     const uint32_t n_lines = bytes / 128;
-    CU(cudaMalloc(&buf, (size_t)n_lines * 128)); CU(cudaMalloc(&out, 4));
-    CU(cudaMemset(buf, 0x5a, (size_t)n_lines * 128));
-    cudaEvent_t e0, e1; CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
+    CU(dev_alloc(buf, (size_t)n_lines * 128)); CU(dev_alloc(out, 4));
+    CU(cudaMemset(buf.get(), 0x5a, (size_t)n_lines * 128));
+    Event e0, e1; CU(make_event(e0)); CU(make_event(e1));
     const int grid = prop.multiProcessorCount * 8;
-    l1_gather_kernel<<<grid, 128>>>(buf, n_lines, 2, out);
-    CU(cudaEventRecord(e0));
-    l1_gather_kernel<<<grid, 128>>>(buf, n_lines, iters, out);
-    CU(cudaEventRecord(e1));
-    CU(cudaEventSynchronize(e1));
-    float ms = 0.f; CU(cudaEventElapsedTime(&ms, e0, e1));
+    l1_gather_kernel<<<grid, 128>>>(buf.get(), n_lines, 2, out.get());
+    CU(cudaEventRecord(e0.get()));
+    l1_gather_kernel<<<grid, 128>>>(buf.get(), n_lines, iters, out.get());
+    CU(cudaEventRecord(e1.get()));
+    CU(cudaEventSynchronize(e1.get()));
+    float ms = 0.f; CU(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
     *out_gbs = (float)((double)grid * 128.0 * 8.0 * iters * 16.0 / (ms * 1e-3) / 1e9);
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(buf); cudaFree(out);
     return TRAY_OK;
 }
 
@@ -415,20 +409,19 @@ int tray_cuda_bandwidth_probe(int device, uint64_t bytes, int iters, float* out_
     if (tray_cuda_device_count() == 0) return fail(TRAY_ERR_NO_DEVICE, "no CUDA device");
     CU(cudaSetDevice(device));
     cudaDeviceProp prop; CU(cudaGetDeviceProperties(&prop, device));
-    uint4* buf = nullptr; uint32_t* out = nullptr;
+    DevPtr<uint4> buf; DevPtr<uint32_t> out;
     const uint64_t n16 = bytes / 16;
-    CU(cudaMalloc(&buf, n16 * 16)); CU(cudaMalloc(&out, 4));
-    CU(cudaMemset(buf, 0x5a, n16 * 16));
-    cudaEvent_t e0, e1; CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
+    CU(dev_alloc(buf, n16 * 16)); CU(dev_alloc(out, 4));
+    CU(cudaMemset(buf.get(), 0x5a, n16 * 16));
+    Event e0, e1; CU(make_event(e0)); CU(make_event(e1));
     const int grid = prop.multiProcessorCount * 4;
-    bandwidth_kernel<<<grid, 512>>>(buf, n16, 2, out);      // warm-up: brings the buffer into L2 when it fits
-    CU(cudaEventRecord(e0));
-    bandwidth_kernel<<<grid, 512>>>(buf, n16, iters, out);
-    CU(cudaEventRecord(e1));
-    CU(cudaEventSynchronize(e1));
-    float ms = 0.f; CU(cudaEventElapsedTime(&ms, e0, e1));
+    bandwidth_kernel<<<grid, 512>>>(buf.get(), n16, 2, out.get());      // warm-up: brings the buffer into L2 when it fits
+    CU(cudaEventRecord(e0.get()));
+    bandwidth_kernel<<<grid, 512>>>(buf.get(), n16, iters, out.get());
+    CU(cudaEventRecord(e1.get()));
+    CU(cudaEventSynchronize(e1.get()));
+    float ms = 0.f; CU(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
     *out_gbs = (float)((double)n16 * 16.0 * iters / (ms * 1e-3) / 1e9);
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(buf); cudaFree(out);
     return TRAY_OK;
 }
 
@@ -443,35 +436,13 @@ int tray_cuda_device_count(void) {
 
 void tray_cuda_scene_destroy(tray_scene* s) {
     if (!s) return;
+    // nothing is freed while a launch or a copy may still read it
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
-    cudaFree(s->d_nodes); cudaFree(s->d_tris); cudaFree(s->d_blas); cudaFree(s->d_prim_indices); cudaFree(s->d_cursor); cudaFree(s->d_overflow);
-    cudaFree(s->d_rays); cudaFree(s->d_hits); cudaFree(s->d_costs); cudaFree(s->d_geom_offsets);
-    cudaFree(s->d_inst_in); cudaFree(s->d_inst_rec); cudaFree(s->d_inst_ids);
-    delete s->refit;
-    free_pipeline(s);
-    cudaFree(s->d_untiled);
-    for (auto& f : s->slot) {
-        if (f.own_stream) cudaStreamSynchronize(f.own_stream);
-        free_frame_buffers(f);
-        cudaFree(f.d_cursor); cudaFree(f.d_units);
-        for (auto& e : f.ev) if (e) cudaEventDestroy(e);
-        if (f.done) cudaEventDestroy(f.done);
-        if (f.own_stream) cudaStreamDestroy(f.own_stream);
-    }
-    for (auto& e : s->ev) if (e) cudaEventDestroy(e);
-    for (int i = 0; i < TRAY_READBACK_SLOTS; i++) {
-        if (s->stage_busy[i]) cudaEventSynchronize(s->ev_copied[i]);
-        cudaFree(s->d_stage[i]);
-        if (s->ev_untiled[i]) cudaEventDestroy(s->ev_untiled[i]);
-        if (s->ev_copied[i]) cudaEventDestroy(s->ev_copied[i]);
-    }
-    if (s->copy_stream) cudaStreamDestroy(s->copy_stream);
-    if (s->own_stream) cudaStreamDestroy(s->own_stream);
-    if (s->h_flag) cudaFreeHost(s->h_flag);
-    if (s->ev_after) cudaEventDestroy(s->ev_after);
-    if (s->ev_attr) cudaEventDestroy(s->ev_attr);
-    cudaFree(s->d_attr_buf);
+    for (auto& f : s->slot)
+        if (f.own_stream) cudaStreamSynchronize(f.own_stream.get());
+    for (int i = 0; i < TRAY_READBACK_SLOTS; i++)
+        if (s->stage_busy[i]) cudaEventSynchronize(s->ev_copied[i].get());
     delete s;
 }
 
@@ -484,7 +455,7 @@ void fit_l2_window(tray_scene* s, size_t want, size_t max_win) {
     size_t win = (size_t)s->n_nodes * 80;
     if (win > max_win) win = max_win;
     memset(&s->window, 0, sizeof s->window);
-    s->window.base_ptr = s->d_nodes;
+    s->window.base_ptr = s->d_nodes.get();
     s->window.num_bytes = win;
     double ratio = (double)want / (double)win;
     s->window.hitRatio = (float)(ratio > 1.0 ? 1.0 : ratio);
@@ -524,51 +495,49 @@ int scene_create_impl(const void* nodes, uint64_t n_nodes, const void* tris, uin
         CU(cudaGetDeviceProperties(&prop, device));
         s->sm_count = prop.multiProcessorCount;
         s->l2_bytes = (uint64_t)prop.l2CacheSize;
-        CU(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
-        s->stream = s->own_stream;
-        for (auto& e : s->ev) CU(cudaEventCreate(&e));
-        CU(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&s->ev_after, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&s->ev_attr, cudaEventDisableTiming));
-        CU(cudaMallocHost(&s->h_flag, TRAY_READBACK_SLOTS * sizeof(uint32_t)));
+        CU(make_stream(s->own_stream));
+        s->stream = s->own_stream.get();
+        for (auto& e : s->ev) CU(make_event(e));
+        CU(make_stream(s->copy_stream));
+        CU(make_event(s->ev_after, cudaEventDisableTiming));
+        CU(make_event(s->ev_attr, cudaEventDisableTiming));
+        CU(host_alloc(s->h_flag, TRAY_READBACK_SLOTS * sizeof(uint32_t)));
         for (int i = 0; i < TRAY_READBACK_SLOTS; i++) {
-            s->h_flag[i] = 0u;
-            CU(cudaEventCreateWithFlags(&s->ev_untiled[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->ev_copied[i], cudaEventDisableTiming));
+            s->h_flag.get()[i] = 0u;
+            CU(make_event(s->ev_untiled[i], cudaEventDisableTiming));
+            CU(make_event(s->ev_copied[i], cudaEventDisableTiming));
         }
         const size_t nb = (size_t)(n_nodes ? n_nodes : 1) * 80, tb = (size_t)(n_tris ? n_tris : 1) * tri_stride;
         s->node_cap = adopted ? built->node_cap : nb / 80;
         if (adopted) {
-            s->d_nodes = (uint4*)built->d_nodes; s->d_tris = (uint4*)built->d_tris; s->d_prim_indices = built->d_prim_indices;
-            s->d_blas = built->d_blas_offsets;
-            // ownership moves to the scene HERE: from now on tray_cuda_scene_destroy is the one place that frees them
-            built->d_nodes = nullptr; built->d_tris = nullptr; built->d_prim_indices = nullptr; built->d_blas_offsets = nullptr;
+            s->d_nodes.reset((uint4*)built->d_nodes.release()); s->d_tris.reset((uint4*)built->d_tris.release());
+            s->d_prim_indices = std::move(built->d_prim_indices); s->d_blas = std::move(built->d_blas_offsets);
         } else {
-            CU(cudaMalloc(&s->d_nodes, nb));
-            CU(cudaMalloc(&s->d_tris, tb));
+            CU(dev_alloc(s->d_nodes, nb));
+            CU(dev_alloc(s->d_tris, tb));
         }
-        if (!s->d_blas) CU(cudaMalloc(&s->d_blas, (size_t)(n_instances ? n_instances : 1) * 4));
-        CU(cudaMalloc(&s->d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
-        CU(cudaMalloc(&s->d_overflow, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t)));
-        CU(cudaMemsetAsync(s->d_cursor, 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
+        if (!s->d_blas) CU(dev_alloc(s->d_blas, (size_t)(n_instances ? n_instances : 1) * 4));
+        CU(dev_alloc(s->d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
+        CU(dev_alloc(s->d_overflow, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t)));
+        CU(cudaMemsetAsync(s->d_cursor.get(), 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
         for (int k = 0; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++) {
             FrameSlot& f = s->slot[k];
-            if (k >= 1) CU(cudaStreamCreateWithFlags(&f.own_stream, cudaStreamNonBlocking));
-            CU(cudaMalloc(&f.d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
-            CU(cudaMalloc(&f.d_units, sizeof(uint32_t)));
-            f.d_flag = s->d_overflow + 1 + k;
-            CU(cudaMemsetAsync(f.d_cursor, 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
-            for (auto& e : f.ev) CU(cudaEventCreate(&e));
-            CU(cudaEventCreateWithFlags(&f.done, cudaEventDisableTiming));
+            if (k >= 1) CU(make_stream(f.own_stream));
+            CU(dev_alloc(f.d_cursor, CURSOR_WORDS * sizeof(unsigned long long)));
+            CU(dev_alloc(f.d_units, sizeof(uint32_t)));
+            f.d_flag = s->d_overflow.get() + 1 + k;
+            CU(cudaMemsetAsync(f.d_cursor.get(), 0, CURSOR_WORDS * sizeof(unsigned long long), s->stream));
+            for (auto& e : f.ev) CU(make_event(e));
+            CU(make_event(f.done, cudaEventDisableTiming));
         }
-        CU(cudaMemsetAsync(s->d_overflow, 0, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t), s->stream));
+        CU(cudaMemsetAsync(s->d_overflow.get(), 0, (1 + TRAY_MAX_FRAMES_IN_FLIGHT) * sizeof(uint32_t), s->stream));
         s->device_bytes = nb + tb + (size_t)n_instances * 4;
         if (!adopted) {
-            if (n_nodes) CU(tray::upload_pipelined(s->d_nodes, nodes, (size_t)n_nodes * 80, s->stream));
-            else CU(cudaMemsetAsync(s->d_nodes, 0, 80, s->stream));   // empty scene: a root with no children, every ray misses
-            if (n_tris) CU(tray::upload_pipelined(s->d_tris, tris, (size_t)n_tris * tri_stride, s->stream));
+            if (n_nodes) CU(tray::upload_pipelined(s->d_nodes.get(), nodes, (size_t)n_nodes * 80, s->stream));
+            else CU(cudaMemsetAsync(s->d_nodes.get(), 0, 80, s->stream));   // empty scene: a root with no children, every ray misses
+            if (n_tris) CU(tray::upload_pipelined(s->d_tris.get(), tris, (size_t)n_tris * tri_stride, s->stream));
         }
-        if (n_instances && blas_offsets) CU(cudaMemcpyAsync(s->d_blas, blas_offsets, (size_t)n_instances * 4, cudaMemcpyHostToDevice, s->stream));
+        if (n_instances && blas_offsets) CU(cudaMemcpyAsync(s->d_blas.get(), blas_offsets, (size_t)n_instances * 4, cudaMemcpyHostToDevice, s->stream));
         // keep the node array hot in the 126 MB L2: persisting access-policy window, attached to every traversal launch
         if (prop.persistingL2CacheMaxSize > 0 && n_nodes) {
             size_t want = (size_t)prop.persistingL2CacheMaxSize;
@@ -614,8 +583,7 @@ int scene_build_impl(const float* tris9, uint64_t n_tris, const uint64_t* object
                                            search_radius ? search_radius : 14u, nullptr, &r, msg, sizeof msg);
     if (brc) return fail(brc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "device build failed: %s", msg);
     const int rc = scene_create_impl(nullptr, r.n_nodes, nullptr, n_tris, tri_stride, nullptr, r.n_instances, r.tlas_start, device, &r, out);
-    // whatever scene_create_impl did not adopt is still ours (adopted pointers are nulled in `r`): freed exactly once
-    if (rc) { cudaFree(r.d_nodes); cudaFree(r.d_tris); cudaFree(r.d_prim_indices); cudaFree(r.d_blas_offsets); return rc; }
+    if (rc) return rc;
     if (out_stats) *out_stats = r.stats;
     return TRAY_OK;
 }
@@ -638,7 +606,7 @@ int tray_cuda_scene_download_instances(tray_scene* s, uint32_t* blas_offsets) {
     if (!s || !blas_offsets) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     CU(cudaStreamSynchronize(s->stream));
-    if (s->n_instances) CU(cudaMemcpy(blas_offsets, s->d_blas, (size_t)s->n_instances * 4, cudaMemcpyDeviceToHost));
+    if (s->n_instances) CU(cudaMemcpy(blas_offsets, s->d_blas.get(), (size_t)s->n_instances * 4, cudaMemcpyDeviceToHost));
     return TRAY_OK;
 }
 
@@ -647,9 +615,9 @@ int tray_cuda_scene_download(tray_scene* s, void* nodes, void* tris, uint32_t* p
     if (prim_indices && !s->d_prim_indices && s->n_tris) return fail(TRAY_ERR_ARG, "this scene was not built on the device: it has no primitive index array");
     CU(cudaSetDevice(s->device));
     CU(cudaStreamSynchronize(s->stream));
-    if (nodes && s->n_nodes) CU(cudaMemcpy(nodes, s->d_nodes, (size_t)s->n_nodes * 80, cudaMemcpyDeviceToHost));
-    if (tris && s->n_tris) CU(cudaMemcpy(tris, s->d_tris, (size_t)s->n_tris * s->tri_stride, cudaMemcpyDeviceToHost));
-    if (prim_indices && s->n_tris) CU(cudaMemcpy(prim_indices, s->d_prim_indices, (size_t)s->n_tris * 4, cudaMemcpyDeviceToHost));
+    if (nodes && s->n_nodes) CU(cudaMemcpy(nodes, s->d_nodes.get(), (size_t)s->n_nodes * 80, cudaMemcpyDeviceToHost));
+    if (tris && s->n_tris) CU(cudaMemcpy(tris, s->d_tris.get(), (size_t)s->n_tris * s->tri_stride, cudaMemcpyDeviceToHost));
+    if (prim_indices && s->n_tris) CU(cudaMemcpy(prim_indices, s->d_prim_indices.get(), (size_t)s->n_tris * 4, cudaMemcpyDeviceToHost));
     return TRAY_OK;
 }
 
@@ -693,7 +661,7 @@ int tray_cuda_scene_set_stream(tray_scene* s, void* stream) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     CU(cudaSetDevice(s->device));
     if (const int rc = sync_streams(s, /*scene_stream_first=*/true)) return rc;
-    s->stream = stream ? (cudaStream_t)stream : s->own_stream;
+    s->stream = stream ? (cudaStream_t)stream : s->own_stream.get();
     return TRAY_OK;
 }
 
@@ -715,7 +683,7 @@ int tray_cuda_frame_push(tray_scene* s, void* d_dst) {
     const FrameSlot& f = s->slot[s->cur];
     if (f.last_frame.width == 0 || !f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA (or into a frame target)");
     CU(cudaSetDevice(s->device));
-    if (f.last_frame.n_items) CU(cudaMemcpyAsync(d_dst, f.d_rgba, (size_t)f.last_frame.n_items * sizeof(uchar4), cudaMemcpyDeviceToDevice, slot_stream(s, s->cur)));
+    if (f.last_frame.n_items) CU(cudaMemcpyAsync(d_dst, f.buf.d_rgba.get(), (size_t)f.last_frame.n_items * sizeof(uchar4), cudaMemcpyDeviceToDevice, slot_stream(s, s->cur)));
     return TRAY_OK;
 }
 
@@ -787,11 +755,11 @@ int tray_cuda_sync(tray_scene* s) {
     // every error word a launch of the scene can have set: batch traces and each frame slot; a set word is cleared on its own
     // stream, ahead of whatever is enqueued there next
     uint32_t f[1 + TRAY_MAX_FRAMES_IN_FLIGHT];
-    CU(cudaMemcpyAsync(f, s->d_overflow, sizeof f, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(f, s->d_overflow.get(), sizeof f, cudaMemcpyDeviceToHost, s->stream));
     CU(cudaStreamSynchronize(s->stream));
     uint32_t all = 0;
     for (int k = 0; k <= TRAY_MAX_FRAMES_IN_FLIGHT; k++)
-        if (f[k]) { all |= f[k]; cudaMemsetAsync(s->d_overflow + k, 0, 4, k ? slot_stream(s, k - 1) : s->stream); }
+        if (f[k]) { all |= f[k]; cudaMemsetAsync(s->d_overflow.get() + k, 0, 4, k ? slot_stream(s, k - 1) : s->stream); }
     return flag_status(all);
 }
 
@@ -801,12 +769,11 @@ namespace {
 // the TLAS of a tray_cuda_scene_refit_rebuild_tlas(_device) call
 struct TlasRebuild { uint32_t max_leaf, radius; };
 
-// Moves the nodes of a TLAS rebuild into place: the new tree is in `nodes` (s->d_nodes, or a larger array of `cap` nodes that
-// replaces it), with m TLAS nodes at tlas_start.
-void adopt_rebuilt_tlas(tray_scene* s, uint4* nodes, uint64_t cap, uint32_t m) {
-    if (nodes != s->d_nodes) {
-        cudaFree(s->d_nodes);                 // every stream of the scene is drained: no launch reads it any more
-        s->d_nodes = nodes;
+// Moves the nodes of a TLAS rebuild into place: the new tree is in s->d_nodes, or in `grown`, a larger array of `cap` nodes that
+// replaces it, with m TLAS nodes at tlas_start.
+void adopt_rebuilt_tlas(tray_scene* s, DevPtr<uint4> grown, uint64_t cap, uint32_t m) {
+    if (grown) {
+        s->d_nodes = std::move(grown);        // frees the old array: every stream of the scene is drained, no launch reads it any more
         s->device_bytes += (cap - s->node_cap) * 80;
         s->node_cap = cap;
     }
@@ -898,10 +865,10 @@ int instance_boxes(tray_scene* s, const void* nodes, const uint32_t* roots, cons
 int ensure_topology(tray_scene* s, char* msg, size_t len) {
     if (s->refit) return TRAY_OK;
     tray_build::RefitTopology t;
-    const int rc = tray_build::refit_walk(s->d_nodes, s->n_nodes, s->n_tris, s->tlas ? s->d_blas : nullptr, s->tlas ? s->n_instances : 0u,
+    const int rc = tray_build::refit_walk(s->d_nodes.get(), s->n_nodes, s->n_tris, s->tlas ? s->d_blas.get() : nullptr, s->tlas ? s->n_instances : 0u,
                                           s->tlas_start, s->stream, &t, msg, len);
     if (rc) return fail(rc == -1 ? TRAY_ERR_ARG : TRAY_ERR_CUDA, "refit: %s", msg);
-    s->refit = new (std::nothrow) tray_build::RefitTopology(std::move(t));
+    s->refit.reset(new (std::nothrow) tray_build::RefitTopology(std::move(t)));
     if (!s->refit) return fail(TRAY_ERR_ARG, "out of host memory");
     s->device_bytes += s->refit->bytes;
     return TRAY_OK;
@@ -911,8 +878,8 @@ int ensure_topology(tray_scene* s, char* msg, size_t len) {
 int drain_scene(tray_scene* s, void* stream) {
     if (stream) CU(cudaStreamSynchronize((cudaStream_t)stream));
     if (const int rc = sync_streams(s, /*scene_stream_first=*/false)) return rc;
-    CU(cudaStreamSynchronize(s->copy_stream));
-    if (s->pipeline_ready) { CU(cudaStreamSynchronize(s->s_in)); CU(cudaStreamSynchronize(s->s_out)); }
+    CU(cudaStreamSynchronize(s->copy_stream.get()));
+    if (s->pipe.s_in) { CU(cudaStreamSynchronize(s->pipe.s_in.get())); CU(cudaStreamSynchronize(s->pipe.s_out.get())); }
     return TRAY_OK;
 }
 
@@ -925,17 +892,15 @@ template <typename Blas>
 int tlas_leg(tray_scene* s, uint32_t n, const TlasRebuild& rb, const std::vector<float4>* lo, const std::vector<float4>* hi, Blas blas,
              float* ms, char* msg, size_t len) {
     const uint64_t cap = (uint64_t)s->tlas_start + n + 1;
-    tray_build::DevPtr<uint4> grown;      // a created scene's node array holds n_nodes: the first rebuild that needs more grows it
+    DevPtr<uint4> grown;                  // a created scene's node array holds n_nodes: the first rebuild that needs more grows it
     if (cap > s->node_cap) {
-        uint4* p = nullptr;
-        CU(cudaMalloc(&p, cap * 80));
-        grown.reset(p);
-        CU(cudaMemcpyAsync(p, s->d_nodes, (size_t)s->tlas_start * 80, cudaMemcpyDeviceToDevice, s->stream));
+        CU(dev_alloc(grown, cap * 80));
+        CU(cudaMemcpyAsync(grown.get(), s->d_nodes.get(), (size_t)s->tlas_start * 80, cudaMemcpyDeviceToDevice, s->stream));
     }
     const uint64_t held = s->refit->bytes;
     if (tray_build::refit_reserve(*s->refit, cap, n, s->stream, msg, len)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
     s->device_bytes += s->refit->bytes - held;
-    uint4* nodes = grown ? grown.get() : s->d_nodes;
+    uint4* nodes = grown ? grown.get() : s->d_nodes.get();
     bool exact = false, tlas_exact = false;
     uint32_t m = 0;
     if (const int rc = blas(nodes, &exact)) return rc;
@@ -945,13 +910,13 @@ int tlas_leg(tray_scene* s, uint32_t n, const TlasRebuild& rb, const std::vector
         if (rc) return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", rc > 0 ? "an instance box is not finite in f32 after the refit" : msg);
         lo = &rlo; hi = &rhi;
     }
-    const tray_build::InstanceTlas it{ lo ? lo->data() : nullptr, hi ? hi->data() : nullptr, s->d_inst_in, s->d_inst_rec };
-    if (tray_build::rebuild_tlas(*s->refit, nodes, s->tlas_start, n, s->d_blas, rb.max_leaf, rb.radius ? rb.radius : 14u, s->stream, s->ev[1],
+    const tray_build::InstanceTlas it{ lo ? lo->data() : nullptr, hi ? hi->data() : nullptr, s->d_inst_in.get(), s->d_inst_rec.get() };
+    if (tray_build::rebuild_tlas(*s->refit, nodes, s->tlas_start, n, s->d_blas.get(), rb.max_leaf, rb.radius ? rb.radius : 14u, s->stream, s->ev[1].get(),
                                  &m, &tlas_exact, msg, len, lo ? &it : nullptr))
         return fail(TRAY_ERR_CUDA, "TLAS rebuild: %s", msg);
     float t = 0.f;
-    CU(cudaEventElapsedTime(&t, s->ev[0], s->ev[1]));
-    adopt_rebuilt_tlas(s, grown ? grown.release() : s->d_nodes, cap, m);
+    CU(cudaEventElapsedTime(&t, s->ev[0].get(), s->ev[1].get()));
+    adopt_rebuilt_tlas(s, std::move(grown), cap, m);
     s->force_exact = scene_force_exact(exact || tlas_exact);
     if (ms) *ms = t;
     return TRAY_OK;
@@ -980,61 +945,57 @@ int refit_impl(tray_scene* s, const float* tris9, uint64_t n_tris, bool device_p
     if (rb && s->refit->blas_past_tlas) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: a BLAS node lies at or past tlas_start");
     if (rb && s->refit->blas_empty) return fail(TRAY_ERR_ARG, "refit_rebuild_tlas: an instance's BLAS reaches no triangle");
     const float* d_tris9 = tris9;
-    float* d_upload = nullptr;
+    DevPtr<float> d_upload;
     if (!device_ptr) {
-        CU(cudaMalloc(&d_upload, (size_t)n_tris * 36));
-        const cudaError_t e = tray::upload_pipelined(d_upload, tris9, (size_t)n_tris * 36, s->stream);
-        if (e != cudaSuccess) { cudaFree(d_upload); return fail(TRAY_ERR_CUDA, "refit upload failed: %s", cudaGetErrorString(e)); }
-        d_tris9 = d_upload;
+        CU(dev_alloc(d_upload, (size_t)n_tris * 36));
+        const cudaError_t e = tray::upload_pipelined(d_upload.get(), tris9, (size_t)n_tris * 36, s->stream);
+        if (e != cudaSuccess) return fail(TRAY_ERR_CUDA, "refit upload failed: %s", cudaGetErrorString(e));
+        d_tris9 = d_upload.get();
     }
-    auto body = [&]() -> int {
-        float ms_check = 0.f, ms_run = 0.f;
-        bool bad = false, exact = false;
-        CU(cudaEventRecord(s->ev[0], s->stream));
-        if (tray_build::refit_check(*s->refit, d_tris9, n_tris, s->stream, &bad, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
-        if (rb) {
-            // one interval, coordinate check to the last TLAS write, host round trips of the TLAS build included
-            if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
-            return tlas_leg(s, s->n_instances, *rb, nullptr, nullptr, [&](uint4* nodes, bool* blas_exact) -> int {
-                if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, nodes, s->d_tris, s->d_blas, true, s->stream,
-                                          blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
-                return TRAY_OK;
-            }, ms_refit, msg, sizeof msg);
-        }
-        CU(cudaEventRecord(s->ev[1], s->stream));
-        CU(cudaEventSynchronize(s->ev[1]));
-        CU(cudaEventElapsedTime(&ms_check, s->ev[0], s->ev[1]));
+    float ms_check = 0.f, ms_run = 0.f;
+    bool bad = false, exact = false;
+    cudaEvent_t e0 = s->ev[0].get(), e1 = s->ev[1].get();
+    CU(cudaEventRecord(e0, s->stream));
+    if (tray_build::refit_check(*s->refit, d_tris9, n_tris, s->stream, &bad, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+    if (rb) {
+        // one interval, coordinate check to the last TLAS write, host round trips of the TLAS build included
         if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
-        CU(cudaEventRecord(s->ev[0], s->stream));
-        if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices, s->tri_stride, s->d_nodes, s->d_tris, s->d_blas, false, s->stream,
-                                  &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
-        CU(cudaEventRecord(s->ev[1], s->stream));
-        CU(cudaEventSynchronize(s->ev[1]));
-        CU(cudaEventElapsedTime(&ms_run, s->ev[0], s->ev[1]));
-        s->force_exact = scene_force_exact(exact);
-        if (ms_refit) *ms_refit = ms_check + ms_run;
-        return TRAY_OK;
-    };
-    const int rc = body();
-    cudaFree(d_upload);
-    return rc;
+        return tlas_leg(s, s->n_instances, *rb, nullptr, nullptr, [&](uint4* nodes, bool* blas_exact) -> int {
+            if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices.get(), s->tri_stride, nodes, s->d_tris.get(), s->d_blas.get(), true,
+                                      s->stream, blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+            return TRAY_OK;
+        }, ms_refit, msg, sizeof msg);
+    }
+    CU(cudaEventRecord(e1, s->stream));
+    CU(cudaEventSynchronize(e1));
+    CU(cudaEventElapsedTime(&ms_check, e0, e1));
+    if (bad) return fail(TRAY_ERR_ARG, "refit: a coordinate is not finite, or the triangles' extent on some axis overflows f32");
+    CU(cudaEventRecord(e0, s->stream));
+    if (tray_build::refit_run(*s->refit, d_tris9, n_tris, s->d_prim_indices.get(), s->tri_stride, s->d_nodes.get(), s->d_tris.get(), s->d_blas.get(), false,
+                              s->stream, &exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "refit: %s", msg);
+    CU(cudaEventRecord(e1, s->stream));
+    CU(cudaEventSynchronize(e1));
+    CU(cudaEventElapsedTime(&ms_run, e0, e1));
+    s->force_exact = scene_force_exact(exact);
+    if (ms_refit) *ms_refit = ms_check + ms_run;
+    return TRAY_OK;
 }
 
-// device arrays of an instanced scene with room for n instances: blas_offsets and the two record arrays grow, never shrink
+// device arrays of an instanced scene with room for n instances: blas_offsets and the two record arrays grow, never shrink.  A
+// new array is allocated before the one it replaces is freed.
 int reserve_instances(tray_scene* s, uint32_t n) {
     if (n > s->blas_cap) {
-        uint32_t* p = nullptr;
-        CU(cudaMalloc(&p, (size_t)n * 4));
-        cudaFree(s->d_blas); s->d_blas = p;
+        DevPtr<uint32_t> p;
+        CU(dev_alloc(p, (size_t)n * 4));
+        s->d_blas = std::move(p);
         s->device_bytes += (uint64_t)(n - s->blas_cap) * 4;
         s->blas_cap = n;
     }
     if (n > s->inst_cap) {
-        uint4 *a = nullptr, *b = nullptr;
-        CU(cudaMalloc(&a, (size_t)n * 64));
-        if (cudaMalloc(&b, (size_t)n * 64) != cudaSuccess) { cudaFree(a); cudaGetLastError(); return fail(TRAY_ERR_CUDA, "cudaMalloc of instance records failed"); }
-        cudaFree(s->d_inst_in); cudaFree(s->d_inst_rec);
-        s->d_inst_in = a; s->d_inst_rec = b;
+        DevPtr<uint4> a, b;
+        CU(dev_alloc(a, (size_t)n * 64));
+        if (dev_alloc(b, (size_t)n * 64) != cudaSuccess) { cudaGetLastError(); return fail(TRAY_ERR_CUDA, "cudaMalloc of instance records failed"); }
+        s->d_inst_in = std::move(a); s->d_inst_rec = std::move(b);
         s->device_bytes += (uint64_t)(n - s->inst_cap) * 128;
         s->inst_cap = n;
     }
@@ -1083,11 +1044,11 @@ int tray_cuda_scene_set_instances(tray_scene* s, const uint32_t* blas_roots, con
         if (!std::binary_search(t.roots.begin(), t.roots.end(), blas_roots[k]))
             return fail(TRAY_ERR_ARG, "set_instances: blas_roots[%u] = %u is not a BLAS root of the scene", k, blas_roots[k]);
     std::vector<float4> lo, hi;
-    if (const int rc = instance_boxes(s, s->d_nodes, blas_roots, object_to_world, n, lo, hi, msg, sizeof msg))
+    if (const int rc = instance_boxes(s, s->d_nodes.get(), blas_roots, object_to_world, n, lo, hi, msg, sizeof msg))
         return rc > 0 ? fail(TRAY_ERR_ARG, "set_instances: an instance's TLAS box is not finite in f32") : fail(TRAY_ERR_CUDA, "set_instances: %s", msg);
     if (const int rc = reserve_instances(s, n)) return rc;
-    CU(cudaEventRecord(s->ev[0], s->stream));
-    CU(cudaMemcpyAsync(s->d_inst_in, in.data(), (size_t)n * 64, cudaMemcpyHostToDevice, s->stream));
+    CU(cudaEventRecord(s->ev[0].get(), s->stream));
+    CU(cudaMemcpyAsync(s->d_inst_in.get(), in.data(), (size_t)n * 64, cudaMemcpyHostToDevice, s->stream));
     const TlasRebuild rb{ max_prims_per_leaf, search_radius };
     const int rc = geometry_changed(s, tlas_leg(s, n, rb, &lo, &hi, [&](uint4* nodes, bool* blas_exact) -> int {
         if (tray_build::blas_exact(*s->refit, nodes, s->tlas_start, s->stream, blas_exact, msg, sizeof msg)) return fail(TRAY_ERR_CUDA, "set_instances: %s", msg);
@@ -1107,7 +1068,7 @@ int tray_cuda_scene_download_instance_xforms(tray_scene* s, uint32_t* leaf_insta
     CU(cudaSetDevice(s->device));
     CU(cudaStreamSynchronize(s->stream));
     std::vector<uint4> rec((size_t)s->n_instances * INST_RECORD_U4);
-    CU(cudaMemcpy(rec.data(), s->d_inst_rec, rec.size() * 16, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(rec.data(), s->d_inst_rec.get(), rec.size() * 16, cudaMemcpyDeviceToHost));
     for (uint32_t j = 0; j < s->n_instances; j++) {
         const uint4* r = &rec[(size_t)j * INST_RECORD_U4];
         const uint32_t k = r[3].y;
@@ -1144,27 +1105,27 @@ int trace_device_impl(tray_scene* s, const tray_ray* d_rays, uint64_t n, tray_hi
     if (!s || (n && (!d_rays || !d_hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
-    if (ms_kernel) CU(cudaEventRecord(s->ev[0], st));
+    if (ms_kernel) CU(cudaEventRecord(s->ev[0].get(), st));
     const uint64_t chunk = INDEX_MASK + 1ull;             // inside the kernel a ray index keeps two tag bits above INDEX_MASK
     for (uint64_t off = 0; off < n; off += chunk) {
         TraceParams P; base_params(s, P);
         P.rays = d_rays + off; P.n_work = (uint32_t)(n - off < chunk ? n - off : chunk); P.hits_out = d_hits + off;
         P.ray_cost = d_costs ? d_costs + off : nullptr;
         P.inst_out = d_inst ? d_inst + off : nullptr;
-        int rc = launch(s, P, st, s->d_cursor, 0, s->counting || d_costs, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
+        int rc = launch(s, P, st, s->d_cursor.get(), 0, s->counting || d_costs, anyhit, /*keep_counters=*/off > 0);      // counters accumulate over the chunks of one batch
         if (rc) return rc;
     }
     if (const int rc = drop_placeholder_costs(s, d_costs, n, st)) return rc;
     if (ms_kernel) {
-        CU(cudaEventRecord(s->ev[1], st));
-        CU(cudaEventSynchronize(s->ev[1]));
-        CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+        CU(cudaEventRecord(s->ev[1].get(), st));
+        CU(cudaEventSynchronize(s->ev[1].get()));
+        CU(cudaEventElapsedTime(ms_kernel, s->ev[0].get(), s->ev[1].get()));
         if (s->counting) {                                // synchronised: the batch's counters, summed over its launches
-            const int rc = read_counters(s->d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
+            const int rc = read_counters(s->d_cursor.get(), st, 0, &s->cnt_primary); if (rc) return rc;
             memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
             drop_placeholder_root(s);
         }
-        return check_overflow(s->d_overflow, st);         // synchronised: an overflow of this batch is reported by this call
+        return check_overflow(s->d_overflow.get(), st);         // synchronised: an overflow of this batch is reported by this call
     }
     return TRAY_OK;
 }
@@ -1173,22 +1134,18 @@ constexpr uint64_t CHUNK_MAX = 1ull << 20;        // rays per pipeline stage (32
 constexpr uint64_t PIPE_MIN = 1ull << 18;         // smaller batches take the plain copy-launch-copy path
 
 int ensure_pipeline(tray_scene* s) {
-    if (s->pipeline_ready) return TRAY_OK;
-    auto body = [&]() -> int {
-        CU(cudaStreamCreateWithFlags(&s->s_in, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&s->s_out, cudaStreamNonBlocking));
-        for (int i = 0; i < 2; i++) {
-            CU(cudaMallocHost(&s->h_rays[i], CHUNK_MAX * sizeof(tray_ray)));
-            CU(cudaMallocHost(&s->h_hits[i], CHUNK_MAX * sizeof(tray_hit)));
-            CU(cudaEventCreateWithFlags(&s->e_in[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->e_k[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->e_out[i], cudaEventDisableTiming));
-        }
-        return TRAY_OK;
-    };
-    const int rc = body();
-    if (rc) { free_pipeline(s); return rc; }      // a half-built pipeline must not look ready to the next call
-    s->pipeline_ready = true;
+    if (s->pipe.s_in) return TRAY_OK;
+    Pipeline p;                                   // a half-built pipeline must not look ready to the next call: it goes on return
+    CU(make_stream(p.s_in));
+    CU(make_stream(p.s_out));
+    for (int i = 0; i < 2; i++) {
+        CU(host_alloc(p.h_rays[i], CHUNK_MAX * sizeof(tray_ray)));
+        CU(host_alloc(p.h_hits[i], CHUNK_MAX * sizeof(tray_hit)));
+        CU(make_event(p.e_in[i], cudaEventDisableTiming));
+        CU(make_event(p.e_k[i], cudaEventDisableTiming));
+        CU(make_event(p.e_out[i], cudaEventDisableTiming));
+    }
+    s->pipe = std::move(p);
     return TRAY_OK;
 }
 
@@ -1203,93 +1160,84 @@ int trace_impl(tray_scene* s, const tray_ray* rays, uint64_t n, tray_hit* hits, 
     if (!s || (n && (!rays || !hits))) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
     const auto t0 = std::chrono::steady_clock::now();
-    if (n > s->batch_cap) {
-        cudaFree(s->d_rays); cudaFree(s->d_hits); s->d_rays = nullptr; s->d_hits = nullptr; s->batch_cap = 0;
-        CU(cudaMalloc(&s->d_rays, n * sizeof(tray_ray)));
-        CU(cudaMalloc(&s->d_hits, n * sizeof(tray_hit)));
-        s->batch_cap = n;
-    }
-    if (costs && n > s->cost_cap) {
-        cudaFree(s->d_costs); s->d_costs = nullptr; s->cost_cap = 0;
-        CU(cudaMalloc(&s->d_costs, n * sizeof(tray_ray_cost)));
-        s->cost_cap = n;
-    }
-    if (inst && n > s->inst_ids_cap) {
-        cudaFree(s->d_inst_ids); s->d_inst_ids = nullptr; s->inst_ids_cap = 0;
-        CU(cudaMalloc(&s->d_inst_ids, n * sizeof(uint32_t)));
-        s->inst_ids_cap = n;
-    }
-    tray_ray_cost* const d_costs = costs ? s->d_costs : nullptr;
-    uint32_t* const d_inst = inst ? s->d_inst_ids : nullptr;
+    CU(s->d_rays.reserve(n));
+    CU(s->d_hits.reserve(n));
+    if (costs) CU(s->d_costs.reserve(n));
+    if (inst) CU(s->d_inst_ids.reserve(n));
+    tray_ray* const d_rays = s->d_rays.get();
+    tray_hit* const d_hits = s->d_hits.get();
+    tray_ray_cost* const d_costs = costs ? s->d_costs.get() : nullptr;
+    uint32_t* const d_inst = inst ? s->d_inst_ids.get() : nullptr;
     float k = 0.f;
     int rc = TRAY_OK;
     if (n < PIPE_MIN) {
-        if (n) CU(cudaMemcpyAsync(s->d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, s->stream));
-        rc = trace_device_impl(s, s->d_rays, n, s->d_hits, d_costs, s->stream, &k, anyhit, d_inst);
+        if (n) CU(cudaMemcpyAsync(d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, s->stream));
+        rc = trace_device_impl(s, d_rays, n, d_hits, d_costs, s->stream, &k, anyhit, d_inst);
         if (rc) return rc;
-        if (n) CU(cudaMemcpyAsync(hits, s->d_hits, n * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->stream));
+        if (n) CU(cudaMemcpyAsync(hits, d_hits, n * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->stream));
         if (n && costs) CU(cudaMemcpyAsync(costs, d_costs, n * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->stream));
         if (n && inst) CU(cudaMemcpyAsync(inst, d_inst, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
         CU(cudaStreamSynchronize(s->stream));
     } else {
         rc = ensure_pipeline(s);
         if (rc) return rc;
+        Pipeline& p = s->pipe;
         for (int i = 0; costs && i < 2; i++)
-            if (!s->h_costs[i]) CU(cudaMallocHost(&s->h_costs[i], CHUNK_MAX * sizeof(tray_ray_cost)));
+            if (!p.h_costs[i]) CU(host_alloc(p.h_costs[i], CHUNK_MAX * sizeof(tray_ray_cost)));
         for (int i = 0; inst && i < 2; i++)
-            if (!s->h_inst[i]) CU(cudaMallocHost(&s->h_inst[i], CHUNK_MAX * sizeof(uint32_t)));
+            if (!p.h_inst[i]) CU(host_alloc(p.h_inst[i], CHUNK_MAX * sizeof(uint32_t)));
         // chunk size: the pipeline only pays once it has a few stages, and every stage is a kernel launch with its own
         // drain phase — 2^19 rays below 4 M rays, 2^20 above
         const uint64_t chunk = n < (4ull << 20) ? (CHUNK_MAX >> 1) : CHUNK_MAX;
         const uint64_t n_chunks = (n + chunk - 1) / chunk;
         auto chunk_len = [&](uint64_t i) { return i + 1 < n_chunks ? chunk : n - i * chunk; };
-        if (s->counting) CU(cudaMemsetAsync(s->d_cursor + CURSOR_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), s->stream));
-        CU(cudaEventRecord(s->ev[0], s->stream));
+        if (s->counting) CU(cudaMemsetAsync(s->d_cursor.get() + CURSOR_COUNTERS, 0, N_COUNTERS * sizeof(unsigned long long), s->stream));
+        CU(cudaEventRecord(s->ev[0].get(), s->stream));
         for (uint64_t i = 0; i < n_chunks + 2; i++) {
             const int slot = (int)(i & 1);
             if (i < n_chunks) {
                 const uint64_t off = i * chunk, len = chunk_len(i);
-                if (i >= 2) CU(cudaEventSynchronize(s->e_in[slot]));                 // the slot's previous upload has left it
-                tray::par_copy(s->h_rays[slot], rays + off, len * sizeof(tray_ray));
-                CU(cudaMemcpyAsync(s->d_rays + off, s->h_rays[slot], len * sizeof(tray_ray), cudaMemcpyHostToDevice, s->s_in));
-                CU(cudaEventRecord(s->e_in[slot], s->s_in));
-                CU(cudaStreamWaitEvent(s->stream, s->e_in[slot], 0));
+                if (i >= 2) CU(cudaEventSynchronize(p.e_in[slot].get()));                 // the slot's previous upload has left it
+                tray::par_copy(p.h_rays[slot].get(), rays + off, len * sizeof(tray_ray));
+                CU(cudaMemcpyAsync(d_rays + off, p.h_rays[slot].get(), len * sizeof(tray_ray), cudaMemcpyHostToDevice, p.s_in.get()));
+                CU(cudaEventRecord(p.e_in[slot].get(), p.s_in.get()));
+                CU(cudaStreamWaitEvent(s->stream, p.e_in[slot].get(), 0));
                 TraceParams P; base_params(s, P);
-                P.rays = s->d_rays + off; P.n_work = (uint32_t)len; P.hits_out = s->d_hits + off;
+                P.rays = d_rays + off; P.n_work = (uint32_t)len; P.hits_out = d_hits + off;
                 P.ray_cost = d_costs ? d_costs + off : nullptr;
                 P.inst_out = d_inst ? d_inst + off : nullptr;
-                rc = launch(s, P, s->stream, s->d_cursor, 0, s->counting || costs, anyhit, /*keep_counters=*/true);
+                rc = launch(s, P, s->stream, s->d_cursor.get(), 0, s->counting || costs, anyhit, /*keep_counters=*/true);
                 if (rc) return rc;
                 rc = drop_placeholder_costs(s, P.ray_cost, len, s->stream);
                 if (rc) return rc;
-                CU(cudaEventRecord(s->e_k[slot], s->stream));
+                CU(cudaEventRecord(p.e_k[slot].get(), s->stream));
             }
             if (i >= 1 && i - 1 < n_chunks) {                                           // chunk i-1: start its read-back
                 const uint64_t j = i - 1; const int ps = (int)(j & 1);
-                CU(cudaStreamWaitEvent(s->s_out, s->e_k[ps], 0));
-                CU(cudaMemcpyAsync(s->h_hits[ps], s->d_hits + j * chunk, chunk_len(j) * sizeof(tray_hit), cudaMemcpyDeviceToHost, s->s_out));
-                if (costs) CU(cudaMemcpyAsync(s->h_costs[ps], d_costs + j * chunk, chunk_len(j) * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, s->s_out));
-                if (inst) CU(cudaMemcpyAsync(s->h_inst[ps], d_inst + j * chunk, chunk_len(j) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->s_out));
-                CU(cudaEventRecord(s->e_out[ps], s->s_out));
+                CU(cudaStreamWaitEvent(p.s_out.get(), p.e_k[ps].get(), 0));
+                CU(cudaMemcpyAsync(p.h_hits[ps].get(), d_hits + j * chunk, chunk_len(j) * sizeof(tray_hit), cudaMemcpyDeviceToHost, p.s_out.get()));
+                if (costs) CU(cudaMemcpyAsync(p.h_costs[ps].get(), d_costs + j * chunk, chunk_len(j) * sizeof(tray_ray_cost), cudaMemcpyDeviceToHost, p.s_out.get()));
+                if (inst) CU(cudaMemcpyAsync(p.h_inst[ps].get(), d_inst + j * chunk, chunk_len(j) * sizeof(uint32_t), cudaMemcpyDeviceToHost, p.s_out.get()));
+                CU(cudaEventRecord(p.e_out[ps].get(), p.s_out.get()));
             }
             if (i >= 2) {                                                               // chunk i-2: hand its hits to the caller
                 const uint64_t j = i - 2; const int ps = (int)(j & 1);
-                CU(cudaEventSynchronize(s->e_out[ps]));
-                tray::par_copy(hits + j * chunk, s->h_hits[ps], chunk_len(j) * sizeof(tray_hit));
-                if (costs) tray::par_copy(costs + j * chunk, s->h_costs[ps], chunk_len(j) * sizeof(tray_ray_cost));
-                if (inst) tray::par_copy(inst + j * chunk, s->h_inst[ps], chunk_len(j) * sizeof(uint32_t));
+                CU(cudaEventSynchronize(p.e_out[ps].get()));
+                tray::par_copy(hits + j * chunk, p.h_hits[ps].get(), chunk_len(j) * sizeof(tray_hit));
+                if (costs) tray::par_copy(costs + j * chunk, p.h_costs[ps].get(), chunk_len(j) * sizeof(tray_ray_cost));
+                if (inst) tray::par_copy(inst + j * chunk, p.h_inst[ps].get(), chunk_len(j) * sizeof(uint32_t));
             }
         }
-        CU(cudaEventRecord(s->ev[1], s->stream));
+        CU(cudaEventRecord(s->ev[1].get(), s->stream));
         CU(cudaStreamSynchronize(s->stream));
-        CU(cudaEventElapsedTime(&k, s->ev[0], s->ev[1]));       // span of the GPU work, uploads it waited for included
+        CU(cudaEventElapsedTime(&k, s->ev[0].get(), s->ev[1].get()));       // span of the GPU work, uploads it waited for included
     }
     if (s->counting) {
-        rc = read_counters(s->d_cursor, s->stream, 0, &s->cnt_primary); if (rc) return rc;
+        rc = read_counters(s->d_cursor.get(), s->stream, 0, &s->cnt_primary); if (rc) return rc;
         memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
         drop_placeholder_root(s);
     }
-    rc = check_overflow(s->d_overflow, s->stream);
+    rc = check_overflow(s->d_overflow.get(), s->stream);
     if (rc) return rc;
     if (ms_kernel) *ms_kernel = k;
     if (ms_total) *ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1384,8 +1332,8 @@ int tray_cuda_scene_fence(tray_scene* s, void* stream) {
     for (int k = 0; k < s->n_slots; k++) {
         cudaStream_t fs = slot_stream(s, k);
         if (fs == st) continue;
-        CU(cudaEventRecord(s->slot[k].done, fs));
-        CU(cudaStreamWaitEvent(st, s->slot[k].done, 0));
+        CU(cudaEventRecord(s->slot[k].done.get(), fs));
+        CU(cudaStreamWaitEvent(st, s->slot[k].done.get(), 0));
     }
     return TRAY_OK;
 }
@@ -1438,9 +1386,9 @@ int tray_cuda_frame_wait_flag(tray_scene* s, const void* d_flag, uint32_t value,
 int tray_cuda_scene_after(tray_scene* s, void* stream) {
     if (!s || !stream) return fail(TRAY_ERR_ARG, "NULL argument");
     CU(cudaSetDevice(s->device));
-    CU(cudaEventRecord(s->ev_after, (cudaStream_t)stream));
+    CU(cudaEventRecord(s->ev_after.get(), (cudaStream_t)stream));
     for (int k = 0; k < TRAY_MAX_FRAMES_IN_FLIGHT; k++)
-        if (slot_stream(s, k) != (cudaStream_t)stream) CU(cudaStreamWaitEvent(slot_stream(s, k), s->ev_after, 0));
+        if (slot_stream(s, k) != (cudaStream_t)stream) CU(cudaStreamWaitEvent(slot_stream(s, k), s->ev_after.get(), 0));
     return TRAY_OK;
 }
 
@@ -1460,24 +1408,25 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
     // (instanced scenes: the one-launch frame kernel has no instance transforms)
     const bool overlap = bounce && !any_ao && !s->variant && !s->instanced && ((flags & TRAY_RENDER_OVERLAP) != 0 || s->overlap_default);
     const bool keep_cost = want_count && s->ray_cost;
-    if (items_cap > f.f_cap || (keep_rays && !f.d_brays_item) || (keep_cost && !f.d_cost) || (s->instanced && !f.d_pinst)) {
-        const uint64_t cap = items_cap > f.f_cap ? items_cap : f.f_cap;
+    FrameBuffers& fb = f.buf;
+    if (items_cap > fb.cap || (keep_rays && !fb.d_brays_item) || (keep_cost && !fb.d_cost) || (s->instanced && !fb.d_pinst)) {
+        const uint64_t cap = items_cap > fb.cap ? items_cap : fb.cap;
         CU(cudaStreamSynchronize(st));
-        free_frame_buffers(f);
+        fb = FrameBuffers{};                     // all of them, before the new ones are allocated
         const uint64_t c1 = cap ? cap : 1;
-        CU(cudaMalloc(&f.d_primary, c1 * sizeof(tray_hit)));
-        CU(cudaMalloc(&f.d_bounce, c1 * sizeof(tray_hit)));
-        CU(cudaMalloc(&f.d_rgba, c1 * sizeof(uchar4)));
-        CU(cudaMalloc(&f.d_prays, c1 * sizeof(tray_ray)));
-        CU(cudaMalloc(&f.d_brays, c1 * sizeof(tray_ray)));
-        CU(cudaMalloc(&f.d_bitem, c1 * sizeof(uint32_t)));
-        if (keep_rays) CU(cudaMalloc(&f.d_brays_item, c1 * sizeof(tray_ray)));
-        if (keep_cost) CU(cudaMalloc(&f.d_cost, 2 * c1 * sizeof(tray_ray_cost)));
-        if (s->instanced) { CU(cudaMalloc(&f.d_pinst, c1 * sizeof(uint32_t))); CU(cudaMalloc(&f.d_binst, c1 * sizeof(uint32_t))); }
-        CU(cudaMemsetAsync(f.d_primary, 0xff, c1 * sizeof(tray_hit), st));
-        CU(cudaMemsetAsync(f.d_bounce, 0xff, c1 * sizeof(tray_hit), st));
-        CU(cudaMemsetAsync(f.d_rgba, 0, c1 * sizeof(uchar4), st));
-        f.f_cap = cap;
+        CU(dev_alloc(fb.d_primary, c1 * sizeof(tray_hit)));
+        CU(dev_alloc(fb.d_bounce, c1 * sizeof(tray_hit)));
+        CU(dev_alloc(fb.d_rgba, c1 * sizeof(uchar4)));
+        CU(dev_alloc(fb.d_prays, c1 * sizeof(tray_ray)));
+        CU(dev_alloc(fb.d_brays, c1 * sizeof(tray_ray)));
+        CU(dev_alloc(fb.d_bitem, c1 * sizeof(uint32_t)));
+        if (keep_rays) CU(dev_alloc(fb.d_brays_item, c1 * sizeof(tray_ray)));
+        if (keep_cost) CU(dev_alloc(fb.d_cost, 2 * c1 * sizeof(tray_ray_cost)));
+        if (s->instanced) { CU(dev_alloc(fb.d_pinst, c1 * sizeof(uint32_t))); CU(dev_alloc(fb.d_binst, c1 * sizeof(uint32_t))); }
+        CU(cudaMemsetAsync(fb.d_primary.get(), 0xff, c1 * sizeof(tray_hit), st));
+        CU(cudaMemsetAsync(fb.d_bounce.get(), 0xff, c1 * sizeof(tray_hit), st));
+        CU(cudaMemsetAsync(fb.d_rgba.get(), 0, c1 * sizeof(uchar4), st));
+        fb.cap = cap;
     }
     FrameParams F; frame_params(F, view, w, h, frame_count, shard, shards);
     f.f_has_bounce = bounce; f.f_has_rgba = rgba && !s->frame_target; f.f_has_rays = keep_rays && bounce;
@@ -1493,37 +1442,37 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         return TRAY_OK;
     }
     const unsigned gen_grid = (F.n_items + 255) / 256;
-    uint32_t* d_nbrays = (uint32_t*)(f.d_cursor + CURSOR_N_BOUNCE);
+    uint32_t* d_nbrays = (uint32_t*)(f.d_cursor.get() + CURSOR_N_BOUNCE);
     const bool timed = ms_primary || ms_bounce;
 
     // ---- primary: generate rays, trace ----
     // ray costs: primary records at d_cost[item], bounce records at d_cost[n_items + item]; a pixel that shoots no bounce ray
     // writes no bounce record, so that half starts zeroed
-    tray_ray_cost* const d_cost_bounce = keep_cost ? f.d_cost + F.n_items : nullptr;
+    tray_ray_cost* const d_cost_bounce = keep_cost ? fb.d_cost.get() + F.n_items : nullptr;
     if (keep_cost && bounce) CU(cudaMemsetAsync(d_cost_bounce, 0, (size_t)F.n_items * sizeof(tray_ray_cost), st));
-    if (timed) CU(cudaEventRecord(f.ev[0], st));
-    tray::raygen_primary_kernel<<<gen_grid, 256, 0, st>>>(F, f.d_prays);
+    if (timed) CU(cudaEventRecord(f.ev[0].get(), st));
+    tray::raygen_primary_kernel<<<gen_grid, 256, 0, st>>>(F, fb.d_prays.get());
     CU(cudaGetLastError());
     TraceParams P; base_params(s, P);
-    P.rays = f.d_prays; P.n_work = F.n_items; P.hits_out = f.d_primary; P.overflow = f.d_flag;
+    P.rays = fb.d_prays.get(); P.n_work = F.n_items; P.hits_out = fb.d_primary.get(); P.overflow = f.d_flag;
     P.frame = F; P.row_major = s->frame_target ? 1u : 0u;
-    uchar4* const rgba_dst = s->frame_target ? s->frame_target : f.d_rgba;
+    uchar4* const rgba_dst = s->frame_target ? s->frame_target : fb.d_rgba.get();
     P.rgba_out = (rgba && !bounce) ? rgba_dst : nullptr; P.shade_mode = SHADE_PRIMARY;
-    P.ray_cost = keep_cost ? f.d_cost : nullptr;
-    P.inst_out = s->instanced ? f.d_pinst : nullptr;
+    P.ray_cost = keep_cost ? fb.d_cost.get() : nullptr;
+    P.inst_out = s->instanced ? fb.d_pinst.get() : nullptr;
     if (overlap) {
         // one launch for the whole frame (trace_kernel<FRAME>): the bounce rays of finished tiles fill the primary pass's drain
-        CU(cudaMemsetAsync(f.d_units, 0, sizeof(uint32_t), st));
-        CU(cudaMemsetAsync(f.d_primary, 0xff, (size_t)F.n_items * sizeof(tray_hit), st));     // "not there yet" for every primary hit
+        CU(cudaMemsetAsync(f.d_units.get(), 0, sizeof(uint32_t), st));
+        CU(cudaMemsetAsync(fb.d_primary.get(), 0xff, (size_t)F.n_items * sizeof(tray_hit), st));     // "not there yet" for every primary hit
         P.rgba_out = rgba ? rgba_dst : nullptr;
-        P.bounce_out = f.d_bounce; P.rays_by_item = keep_rays ? f.d_brays_item : nullptr; P.gen_min = s->gen_min;
-        P.gen_rays = f.d_brays;
-        P.unit_cursor = f.d_units; P.n_units = (uint32_t)(F.n_items / 32);
+        P.bounce_out = fb.d_bounce.get(); P.rays_by_item = keep_rays ? fb.d_brays_item.get() : nullptr; P.gen_min = s->gen_min;
+        P.gen_rays = fb.d_brays.get();
+        P.unit_cursor = f.d_units.get(); P.n_units = (uint32_t)(F.n_items / 32);
     }
-    int rc = launch(s, P, st, f.d_cursor, 0, want_count, false, false, overlap);
+    int rc = launch(s, P, st, f.d_cursor.get(), 0, want_count, false, false, overlap);
     if (rc) return rc;
-    if (timed) CU(cudaEventRecord(f.ev[1], st));
-    if (overlap && timed) CU(cudaEventRecord(f.ev[2], st));
+    if (timed) CU(cudaEventRecord(f.ev[1].get(), st));
+    if (overlap && timed) CU(cudaEventRecord(f.ev[2].get(), st));
 
     // ---- bounce: generate + compact rays of hit pixels, trace ----
     if (bounce && !overlap) {
@@ -1531,34 +1480,34 @@ int render_slot(tray_scene* s, const tray_view* view, uint32_t w, uint32_t h, ui
         auto gen = s->instanced ? (s->tri_stride == 64 ? tray::raygen_bounce_kernel<64, true> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24, true>
                                                                                                      : tray::raygen_bounce_kernel<48, true>)
                  : s->tri_stride == 64 ? tray::raygen_bounce_kernel<64> : s->tri_stride == 24 ? tray::raygen_bounce_kernel<24> : tray::raygen_bounce_kernel<48>;
-        if (s->instanced) CU(cudaMemsetAsync(f.d_binst, 0xff, (size_t)F.n_items * sizeof(uint32_t), st));   // pixels that shoot no bounce ray
-        gen<<<(F.n_items + BOUNCE_BLOCK - 1) / BOUNCE_BLOCK, BOUNCE_BLOCK, 0, st>>>(F, s->d_tris, f.d_primary, f.d_brays, f.d_bitem, d_nbrays, f.d_bounce,
-                                             rgba ? rgba_dst : nullptr, keep_rays ? f.d_brays_item : nullptr, P.row_major,
-                                             f.d_pinst, s->d_inst_in);
+        if (s->instanced) CU(cudaMemsetAsync(fb.d_binst.get(), 0xff, (size_t)F.n_items * sizeof(uint32_t), st));   // pixels that shoot no bounce ray
+        gen<<<(F.n_items + BOUNCE_BLOCK - 1) / BOUNCE_BLOCK, BOUNCE_BLOCK, 0, st>>>(F, s->d_tris.get(), fb.d_primary.get(), fb.d_brays.get(), fb.d_bitem.get(), d_nbrays, fb.d_bounce.get(),
+                                             rgba ? rgba_dst : nullptr, keep_rays ? fb.d_brays_item.get() : nullptr, P.row_major,
+                                             fb.d_pinst.get(), s->d_inst_in.get());
         CU(cudaGetLastError());
         TraceParams B; base_params(s, B);
-        B.rays = f.d_brays; B.ray_item = f.d_bitem; B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
+        B.rays = fb.d_brays.get(); B.ray_item = fb.d_bitem.get(); B.n_work = F.n_items; B.n_work_dev = d_nbrays;   // count stays on the device
         B.overflow = f.d_flag; B.frame = F; B.row_major = P.row_major;
-        B.hits_out = f.d_bounce; B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
+        B.hits_out = fb.d_bounce.get(); B.rgba_out = rgba ? rgba_dst : nullptr; B.shade_mode = any_ao ? SHADE_OCCLUSION : SHADE_BOUNCE;
         B.ray_cost = d_cost_bounce;
-        B.inst_out = s->instanced ? f.d_binst : nullptr;
-        rc = launch(s, B, st, f.d_cursor, 1, want_count, any_ao);
+        B.inst_out = s->instanced ? fb.d_binst.get() : nullptr;
+        rc = launch(s, B, st, f.d_cursor.get(), 1, want_count, any_ao);
         if (rc) return rc;
-        if (timed) CU(cudaEventRecord(f.ev[2], st));
+        if (timed) CU(cudaEventRecord(f.ev[2].get(), st));
     }
-    if (keep_cost) { rc = drop_placeholder_costs(s, f.d_cost, F.n_items, st); if (rc) return rc; }   // (an empty scene shoots no bounce ray)
+    if (keep_cost) { rc = drop_placeholder_costs(s, fb.d_cost.get(), F.n_items, st); if (rc) return rc; }   // (an empty scene shoots no bounce ray)
     if (timed) {
         CU(cudaStreamSynchronize(st));
         float a = 0.f, b = 0.f;
-        CU(cudaEventElapsedTime(&a, f.ev[0], f.ev[1]));
-        if (bounce) CU(cudaEventElapsedTime(&b, f.ev[1], f.ev[2]));
+        CU(cudaEventElapsedTime(&a, f.ev[0].get(), f.ev[1].get()));
+        if (bounce) CU(cudaEventElapsedTime(&b, f.ev[1].get(), f.ev[2].get()));
         if (ms_primary) *ms_primary = a;
         if (ms_bounce) *ms_bounce = b;
         rc = check_overflow(f.d_flag, st); if (rc) return rc;
     }
     if (want_count) {
-        rc = read_counters(f.d_cursor, st, 0, &s->cnt_primary); if (rc) return rc;
-        if (bounce) { rc = read_counters(f.d_cursor, st, 1, &s->cnt_bounce); if (rc) return rc; }
+        rc = read_counters(f.d_cursor.get(), st, 0, &s->cnt_primary); if (rc) return rc;
+        if (bounce) { rc = read_counters(f.d_cursor.get(), st, 1, &s->cnt_bounce); if (rc) return rc; }
         else memset(&s->cnt_bounce, 0, sizeof s->cnt_bounce);
         // rays generated for pixels outside the frame (tmax = 0) are not rays of the workload
         const uint64_t pad = (uint64_t)F.n_items - tray_cuda_shard_pixels(w, h, shard, shards);
@@ -1598,12 +1547,12 @@ int tray_cuda_render_timed(tray_scene* s, const tray_view* view, uint32_t w, uin
     CU(cudaSetDevice(s->device));
     const int k = next_slot(s);                                               // the slot tray_cuda_render is about to take
     cudaStream_t st = slot_stream(s, k);
-    CU(cudaEventRecord(s->slot[k].ev[0], st));
+    CU(cudaEventRecord(s->slot[k].ev[0].get(), st));
     int rc = tray_cuda_render(s, view, w, h, frame_count, flags, shard, shards, nullptr, nullptr);
     if (rc) return rc;
-    CU(cudaEventRecord(s->slot[k].ev[3], st));
-    CU(cudaEventSynchronize(s->slot[k].ev[3]));
-    CU(cudaEventElapsedTime(ms_frame, s->slot[k].ev[0], s->slot[k].ev[3]));
+    CU(cudaEventRecord(s->slot[k].ev[3].get(), st));
+    CU(cudaEventSynchronize(s->slot[k].ev[3].get()));
+    CU(cudaEventElapsedTime(ms_frame, s->slot[k].ev[0].get(), s->slot[k].ev[3].get()));
     return check_overflow(s->slot[k].d_flag, st);    // synchronising point: a stack overflow / watchdog flag must not pass as TRAY_OK
 }
 
@@ -1617,9 +1566,9 @@ int tray_cuda_counters(tray_scene* s, tray_counters* primary, tray_counters* bou
 int tray_cuda_frame_device_ptrs(tray_scene* s, void** d_primary, void** d_bounce, void** d_rgba) {
     if (!s) return fail(TRAY_ERR_ARG, "NULL scene");
     const FrameSlot& f = s->slot[s->cur];
-    if (d_primary) *d_primary = f.d_primary;
-    if (d_bounce) *d_bounce = f.d_bounce;
-    if (d_rgba) *d_rgba = f.d_rgba;
+    if (d_primary) *d_primary = f.buf.d_primary.get();
+    if (d_bounce) *d_bounce = f.buf.d_bounce.get();
+    if (d_rgba) *d_rgba = f.buf.d_rgba.get();
     return TRAY_OK;
 }
 
@@ -1645,13 +1594,9 @@ int download(tray_scene* s, const T* d_src, T* host_dst, int fill = 0) {
     const FrameParams& F = s->slot[s->cur].last_frame;
     cudaStream_t st = slot_stream(s, s->cur);
     const uint64_t bytes = (uint64_t)F.width * F.height * sizeof(T);
-    if (bytes > s->untiled_cap) {
-        cudaFree(s->d_untiled); s->d_untiled = nullptr; s->untiled_cap = 0;
-        CU(cudaMalloc(&s->d_untiled, bytes));
-        s->untiled_cap = bytes;
-    }
-    if (const int rc = untile_last_frame(s, d_src, (T*)s->d_untiled, fill)) return rc;
-    CU(cudaMemcpyAsync(host_dst, s->d_untiled, bytes, cudaMemcpyDeviceToHost, st));
+    CU(s->d_untiled.reserve(bytes));
+    if (const int rc = untile_last_frame(s, d_src, (T*)s->d_untiled.get(), fill)) return rc;
+    CU(cudaMemcpyAsync(host_dst, s->d_untiled.get(), bytes, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     return TRAY_OK;
 }
@@ -1665,18 +1610,18 @@ int tray_cuda_frame_download(tray_scene* s, tray_hit* primary, tray_hit* bounce,
     if (f.last_frame.width == 0) return fail(TRAY_ERR_ARG, "no frame has been rendered");
     CU(cudaSetDevice(s->device));
     int rc;
-    if (primary) { rc = download<tray_hit>(s, f.d_primary, primary); if (rc) return rc; }
+    if (primary) { rc = download<tray_hit>(s, f.buf.d_primary.get(), primary); if (rc) return rc; }
     if (bounce) {
         if (!f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
-        rc = download<tray_hit>(s, f.d_bounce, bounce); if (rc) return rc;
+        rc = download<tray_hit>(s, f.buf.d_bounce.get(), bounce); if (rc) return rc;
     }
     if (bounce_rays) {
         if (!f.f_has_rays) return fail(TRAY_ERR_ARG, "last frame was rendered without the keep-bounce-rays flag (0x8)");
-        rc = download<tray_ray>(s, f.d_brays_item, bounce_rays); if (rc) return rc;
+        rc = download<tray_ray>(s, f.buf.d_brays_item.get(), bounce_rays); if (rc) return rc;
     }
     if (rgba) {
         if (!f.f_has_rgba) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_RGBA");
-        rc = download<uchar4>(s, f.d_rgba, (uchar4*)rgba); if (rc) return rc;
+        rc = download<uchar4>(s, f.buf.d_rgba.get(), (uchar4*)rgba); if (rc) return rc;
     }
     return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
@@ -1689,8 +1634,8 @@ int tray_cuda_frame_download_cost(tray_scene* s, tray_ray_cost* primary, tray_ra
     if (bounce && !f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
     CU(cudaSetDevice(s->device));
     int rc;
-    if (primary) { rc = download<tray_ray_cost>(s, f.d_cost, primary); if (rc) return rc; }
-    if (bounce) { rc = download<tray_ray_cost>(s, f.d_cost + f.last_frame.n_items, bounce); if (rc) return rc; }
+    if (primary) { rc = download<tray_ray_cost>(s, f.buf.d_cost.get(), primary); if (rc) return rc; }
+    if (bounce) { rc = download<tray_ray_cost>(s, f.buf.d_cost.get() + f.last_frame.n_items, bounce); if (rc) return rc; }
     return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 
@@ -1703,8 +1648,8 @@ int tray_cuda_frame_download_instance(tray_scene* s, uint32_t* primary, uint32_t
     if (bounce && !f.f_has_bounce) return fail(TRAY_ERR_ARG, "last frame was rendered without TRAY_RENDER_BOUNCE");
     CU(cudaSetDevice(s->device));
     int rc;
-    if (primary) { rc = download<uint32_t>(s, f.d_pinst, primary, 0xff); if (rc) return rc; }
-    if (bounce) { rc = download<uint32_t>(s, f.d_binst, bounce, 0xff); if (rc) return rc; }
+    if (primary) { rc = download<uint32_t>(s, f.buf.d_pinst.get(), primary, 0xff); if (rc) return rc; }
+    if (bounce) { rc = download<uint32_t>(s, f.buf.d_binst.get(), bounce, 0xff); if (rc) return rc; }
     return check_overflow(f.d_flag, slot_stream(s, s->cur));
 }
 
@@ -1716,29 +1661,26 @@ int tray_cuda_frame_readback_begin(tray_scene* s, uint8_t* rgba, uint32_t slot) 
     CU(cudaSetDevice(s->device));
     const uint64_t bytes = (uint64_t)f.last_frame.width * f.last_frame.height * sizeof(uchar4);
     if (s->stage_busy[slot]) {                       // the previous copy out of this staging buffer must have landed
-        CU(cudaEventSynchronize(s->ev_copied[slot]));
+        CU(cudaEventSynchronize(s->ev_copied[slot].get()));
         s->stage_busy[slot] = false;
     }
-    if (bytes > s->stage_cap[slot]) {
-        cudaFree(s->d_stage[slot]); s->d_stage[slot] = nullptr; s->stage_cap[slot] = 0;
-        CU(cudaMalloc(&s->d_stage[slot], bytes));
-        s->stage_cap[slot] = bytes;
-    }
+    CU(s->d_stage[slot].reserve(bytes / sizeof(uchar4)));
+    uchar4* const stage = s->d_stage[slot].get();
     if (f.f_target) {
         // the frame was rendered into a row-major frame target (all shards' pixels, once the caller's barrier has passed):
         // snapshot it, so that the next frame may overwrite the target while this one travels to the host
-        CU(cudaMemcpyAsync(s->d_stage[slot], f.f_target, bytes, cudaMemcpyDeviceToDevice, st));
-    } else if (const int rc = untile_last_frame(s, f.d_rgba, s->d_stage[slot])) {
+        CU(cudaMemcpyAsync(stage, f.f_target, bytes, cudaMemcpyDeviceToDevice, st));
+    } else if (const int rc = untile_last_frame(s, f.buf.d_rgba.get(), stage)) {
         return rc;
     }
     // the error word travels with the frame (a stream synchronise here would undo the overlap): taken on the frame's stream,
     // behind the frame's launches and ahead of the next frame on that slot, and reported by _wait
-    CU(cudaMemcpyAsync(s->h_flag + slot, f.d_flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(s->h_flag.get() + slot, f.d_flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     CU(cudaMemsetAsync(f.d_flag, 0, sizeof(uint32_t), st));
-    CU(cudaEventRecord(s->ev_untiled[slot], st));
-    CU(cudaStreamWaitEvent(s->copy_stream, s->ev_untiled[slot], 0));
-    CU(cudaMemcpyAsync(rgba, s->d_stage[slot], bytes, cudaMemcpyDeviceToHost, s->copy_stream));
-    CU(cudaEventRecord(s->ev_copied[slot], s->copy_stream));
+    CU(cudaEventRecord(s->ev_untiled[slot].get(), st));
+    CU(cudaStreamWaitEvent(s->copy_stream.get(), s->ev_untiled[slot].get(), 0));
+    CU(cudaMemcpyAsync(rgba, stage, bytes, cudaMemcpyDeviceToHost, s->copy_stream.get()));
+    CU(cudaEventRecord(s->ev_copied[slot].get(), s->copy_stream.get()));
     s->stage_busy[slot] = true;
     return TRAY_OK;
 }
@@ -1747,10 +1689,10 @@ int tray_cuda_frame_readback_wait(tray_scene* s, uint32_t slot) {
     if (!s || slot >= TRAY_READBACK_SLOTS) return fail(TRAY_ERR_ARG, "bad argument");
     if (!s->stage_busy[slot]) return TRAY_OK;
     CU(cudaSetDevice(s->device));
-    CU(cudaEventSynchronize(s->ev_copied[slot]));
+    CU(cudaEventSynchronize(s->ev_copied[slot].get()));
     s->stage_busy[slot] = false;
-    const uint32_t fl = s->h_flag[slot];
-    s->h_flag[slot] = 0u;
+    const uint32_t fl = s->h_flag.get()[slot];
+    s->h_flag.get()[slot] = 0u;
     return flag_status(fl);
 }
 
@@ -1792,20 +1734,10 @@ int tray_cuda_start(const void* bvh_bytes, uint64_t bvh_len, const void* instanc
 namespace {
 AttrScene attr_scene(const tray_scene* s) {
     AttrScene S;
-    S.tris = s->d_tris; S.n_tris = s->n_tris;
-    S.inst_xf = s->instanced ? s->d_inst_in : nullptr; S.n_inst = s->instanced ? s->n_instances : 0u;
+    S.tris = s->d_tris.get(); S.n_tris = s->n_tris;
+    S.inst_xf = s->instanced ? s->d_inst_in.get() : nullptr; S.n_inst = s->instanced ? s->n_instances : 0u;
     S.variant = s->variant;
     return S;
-}
-
-// the scene's attribute staging with room for n records (rays, hits, instance ids and attributes of a host batch, or the compact
-// attributes of a frame): grown, never shrunk
-int ensure_attr_buf(tray_scene* s, uint64_t n) {
-    if (n <= s->attr_cap) return TRAY_OK;
-    cudaFree(s->d_attr_buf); s->d_attr_buf = nullptr; s->attr_cap = 0;
-    CU(cudaMalloc(&s->d_attr_buf, n * 64));
-    s->attr_cap = n;
-    return TRAY_OK;
 }
 
 int check_attr_args(const tray_scene* s, const void* rays, const void* hits, const uint32_t* ids, uint64_t n, const void* attrs) {
@@ -1839,9 +1771,9 @@ int tray_cuda_hit_attributes(tray_scene* s, const tray_ray* rays, const tray_hit
     if (const int rc = check_attr_args(s, rays, hits, instance_ids, n, attrs)) return rc;
     if (n == 0) return TRAY_OK;
     CU(cudaSetDevice(s->device));
-    if (const int rc = ensure_attr_buf(s, n)) return rc;
     // 64 bytes per record: rays (32), hits (8), attributes (20), instance ids (4)
-    uint8_t* base = (uint8_t*)s->d_attr_buf;
+    CU(s->d_attr_buf.reserve(n * 64));
+    uint8_t* base = s->d_attr_buf.get();
     tray_ray* d_rays = (tray_ray*)base;
     tray_hit* d_hits = (tray_hit*)(base + n * 32);
     tray_hit_attr* d_attrs = (tray_hit_attr*)(base + n * 40);
@@ -1850,12 +1782,12 @@ int tray_cuda_hit_attributes(tray_scene* s, const tray_ray* rays, const tray_hit
     CU(cudaMemcpyAsync(d_rays, rays, n * sizeof(tray_ray), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(d_hits, hits, n * sizeof(tray_hit), cudaMemcpyHostToDevice, st));
     if (d_ids) CU(cudaMemcpyAsync(d_ids, instance_ids, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    CU(cudaEventRecord(s->ev[0], st));
+    CU(cudaEventRecord(s->ev[0].get(), st));
     if (const int rc = launch_hit_attr(s, d_rays, d_hits, d_ids, n, d_attrs, st)) return rc;
-    CU(cudaEventRecord(s->ev[1], st));
+    CU(cudaEventRecord(s->ev[1].get(), st));
     CU(cudaMemcpyAsync(attrs, d_attrs, n * sizeof(tray_hit_attr), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    if (ms_kernel) CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+    if (ms_kernel) CU(cudaEventElapsedTime(ms_kernel, s->ev[0].get(), s->ev[1].get()));
     return TRAY_OK;
 }
 
@@ -1866,15 +1798,15 @@ int tray_cuda_hit_attributes_device(tray_scene* s, const tray_ray* d_rays, const
     CU(cudaSetDevice(s->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (st != s->stream) {                          // after the traces enqueued on the scene stream
-        CU(cudaEventRecord(s->ev_attr, s->stream));
-        CU(cudaStreamWaitEvent(st, s->ev_attr, 0));
+        CU(cudaEventRecord(s->ev_attr.get(), s->stream));
+        CU(cudaStreamWaitEvent(st, s->ev_attr.get(), 0));
     }
-    if (ms_kernel) CU(cudaEventRecord(s->ev[0], st));
+    if (ms_kernel) CU(cudaEventRecord(s->ev[0].get(), st));
     if (const int rc = launch_hit_attr(s, d_rays, d_hits, d_instance_ids, n, d_attrs, st)) return rc;
     if (ms_kernel) {
-        CU(cudaEventRecord(s->ev[1], st));
-        CU(cudaEventSynchronize(s->ev[1]));
-        CU(cudaEventElapsedTime(ms_kernel, s->ev[0], s->ev[1]));
+        CU(cudaEventRecord(s->ev[1].get(), st));
+        CU(cudaEventSynchronize(s->ev[1].get()));
+        CU(cudaEventElapsedTime(ms_kernel, s->ev[0].get(), s->ev[1].get()));
     }
     return TRAY_OK;
 }
@@ -1890,8 +1822,8 @@ int tray_cuda_frame_download_attributes(tray_scene* s, tray_hit_attr* primary, t
     if (!primary && !bounce) return TRAY_OK;
     CU(cudaSetDevice(s->device));
     const FrameParams& F = f.last_frame;
-    if (const int rc = ensure_attr_buf(s, F.n_items ? F.n_items : 1)) return rc;
-    tray_hit_attr* d_p = (tray_hit_attr*)s->d_attr_buf;
+    CU(s->d_attr_buf.reserve((uint64_t)(F.n_items ? F.n_items : 1) * 64));   // 64 B per item: its primary and bounce attributes
+    tray_hit_attr* d_p = (tray_hit_attr*)s->d_attr_buf.get();
     tray_hit_attr* d_b = d_p + F.n_items;
     if (F.n_items) {
         // (a frame of an instanced scene was rendered after its set_instances: the generation check above holds f_has_inst to
@@ -1899,7 +1831,7 @@ int tray_cuda_frame_download_attributes(tray_scene* s, tray_hit_attr* primary, t
         const uint32_t k = s->tri_stride;
         auto fn = f.f_has_inst ? (k == 64 ? frame_attr_kernel<64, true> : k == 24 ? frame_attr_kernel<24, true> : frame_attr_kernel<48, true>)
                                : (k == 64 ? frame_attr_kernel<64, false> : k == 24 ? frame_attr_kernel<24, false> : frame_attr_kernel<48, false>);
-        fn<<<(F.n_items + 255) / 256, 256, 0, slot_stream(s, s->cur)>>>(F, attr_scene(s), f.d_prays, f.d_primary, f.d_bounce, f.d_pinst, f.d_binst,
+        fn<<<(F.n_items + 255) / 256, 256, 0, slot_stream(s, s->cur)>>>(F, attr_scene(s), f.buf.d_prays.get(), f.buf.d_primary.get(), f.buf.d_bounce.get(), f.buf.d_pinst.get(), f.buf.d_binst.get(),
                                                                          primary ? d_p : nullptr, bounce ? d_b : nullptr);
         CU(cudaGetLastError());
     }
@@ -1940,10 +1872,10 @@ int tray_cuda_scene_set_geometry_offsets(tray_scene* s, const uint32_t* tri_offs
     }
     CU(cudaSetDevice(s->device));
     CU(cudaStreamSynchronize(s->stream));
-    cudaFree(s->d_geom_offsets); s->d_geom_offsets = nullptr; s->n_geometries = 0;
+    s->d_geom_offsets.reset(); s->n_geometries = 0;
     if (n_geometries) {
-        CU(cudaMalloc(&s->d_geom_offsets, (size_t)(n_geometries + 1) * 4));
-        CU(cudaMemcpy(s->d_geom_offsets, tri_offsets, (size_t)(n_geometries + 1) * 4, cudaMemcpyHostToDevice));
+        CU(dev_alloc(s->d_geom_offsets, (size_t)(n_geometries + 1) * 4));
+        CU(cudaMemcpy(s->d_geom_offsets.get(), tri_offsets, (size_t)(n_geometries + 1) * 4, cudaMemcpyHostToDevice));
         s->n_geometries = n_geometries;
     }
     return TRAY_OK;
@@ -1953,21 +1885,16 @@ int tray_cuda_hits_to_geometry(tray_scene* s, const tray_hit* hits, uint64_t n, 
     if (!s || (n && (!hits || !geometry_id || !primitive_id))) return fail(TRAY_ERR_ARG, "NULL argument");
     if (n == 0) return TRAY_OK;
     CU(cudaSetDevice(s->device));
-    tray_hit* d_h = nullptr; uint32_t* d_o = nullptr;
-    CU(cudaMalloc(&d_h, n * sizeof(tray_hit)));
-    if (cudaMalloc(&d_o, n * 8) != cudaSuccess) { cudaFree(d_h); return fail(TRAY_ERR_CUDA, "cudaMalloc failed"); }
-    auto body = [&]() -> int {
-        CU(cudaMemcpyAsync(d_h, hits, n * sizeof(tray_hit), cudaMemcpyHostToDevice, s->stream));
-        hits_to_geometry_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s->stream>>>(d_h, n, s->d_geom_offsets, s->n_geometries, d_o, d_o + n);
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(geometry_id, d_o, n * 4, cudaMemcpyDeviceToHost, s->stream));
-        CU(cudaMemcpyAsync(primitive_id, d_o + n, n * 4, cudaMemcpyDeviceToHost, s->stream));
-        CU(cudaStreamSynchronize(s->stream));
-        return TRAY_OK;
-    };
-    const int rc = body();
-    cudaFree(d_h); cudaFree(d_o);
-    return rc;
+    DevPtr<tray_hit> d_h; DevPtr<uint32_t> d_o;
+    CU(dev_alloc(d_h, n * sizeof(tray_hit)));
+    if (dev_alloc(d_o, n * 8) != cudaSuccess) return fail(TRAY_ERR_CUDA, "cudaMalloc failed");
+    CU(cudaMemcpyAsync(d_h.get(), hits, n * sizeof(tray_hit), cudaMemcpyHostToDevice, s->stream));
+    hits_to_geometry_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s->stream>>>(d_h.get(), n, s->d_geom_offsets.get(), s->n_geometries, d_o.get(), d_o.get() + n);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(geometry_id, d_o.get(), n * 4, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaMemcpyAsync(primitive_id, d_o.get() + n, n * 4, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    return TRAY_OK;
 }
 
 }  // extern "C"
@@ -1981,47 +1908,45 @@ int tray_cuda_hits_to_geometry(tray_scene* s, const tray_hit* hits, uint64_t n, 
 struct tray_group {
     std::vector<tray_scene*> scenes;
     std::vector<int> devices;
-    uchar4* target[TRAY_MAX_FRAMES_IN_FLIGHT] = {};    // row-major frames on devices[0], one per frame in flight
-    uint64_t target_bytes = 0;
+    DevBuf<uchar4> target[TRAY_MAX_FRAMES_IN_FLIGHT];  // row-major frames on devices[0], one per frame in flight
     int in_flight = 1, cur = 0;
-    cudaEvent_t ev_snap[TRAY_MAX_FRAMES_IN_FLIGHT] = {};   // devices[0]: the frame in target[i] has been copied out (readback)
+    Event ev_snap[TRAY_MAX_FRAMES_IN_FLIGHT];          // devices[0]: the frame in target[i] has been copied out (readback)
     bool snap_pending[TRAY_MAX_FRAMES_IN_FLIGHT] = {};
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;      // devices[0]: frame timing
+    Event ev_t0, ev_t1;                                // devices[0]: frame timing
     // exchange 1 ("push", default): every device keeps its compact shard and moves it with one peer DMA copy into staging[] on
     // devices[0], which untiles all shards in one launch; exchange 0: the kernels store pixels straight into the frame
     int exchange = 1;
-    uchar4* staging[TRAY_MAX_FRAMES_IN_FLIGHT] = {};
-    uint64_t staging_bytes = 0;
-    cudaEvent_t ev_staged[TRAY_MAX_FRAMES_IN_FLIGHT] = {};  // devices[0]: staging[i] has been untiled (it may be overwritten)
+    DevBuf<uchar4> staging[TRAY_MAX_FRAMES_IN_FLIGHT];
+    Event ev_staged[TRAY_MAX_FRAMES_IN_FLIGHT];        // devices[0]: staging[i] has been untiled (it may be overwritten)
     bool staged_pending[TRAY_MAX_FRAMES_IN_FLIGHT] = {};
 };
 
 namespace {
+// whether every one of the frames' buffers `b` has room for n pixels
+bool have_room(const DevBuf<uchar4> (&b)[TRAY_MAX_FRAMES_IN_FLIGHT], uint64_t n) {
+    return std::all_of(std::begin(b), std::end(b), [n](const DevBuf<uchar4>& x) { return n <= x.cap; });
+}
 int group_ensure_target(tray_group* g, uint32_t w, uint32_t h) {
-    const uint64_t bytes = (uint64_t)w * h * 4;
-    if (bytes <= g->target_bytes) return TRAY_OK;
+    const uint64_t n = (uint64_t)w * h;
+    if (have_room(g->target, n)) return TRAY_OK;
     CU(cudaSetDevice(g->devices[0]));
     for (auto* sc : g->scenes) { int rc = tray_cuda_sync(sc); if (rc) return rc; }
     CU(cudaSetDevice(g->devices[0]));
-    for (int i = 0; i < TRAY_MAX_FRAMES_IN_FLIGHT; i++) {
-        cudaFree(g->target[i]); g->target[i] = nullptr;
-        CU(cudaMalloc(&g->target[i], bytes));
-        CU(cudaMemset(g->target[i], 0, bytes));
+    for (auto& t : g->target) {
+        CU(t.reserve(n));
+        CU(cudaMemset(t.get(), 0, n * 4));
     }
-    g->target_bytes = bytes;
     return TRAY_OK;
 }
 int group_ensure_staging(tray_group* g, uint32_t w, uint32_t h) {
-    const uint64_t bytes = (uint64_t)g->scenes.size() * local_items(w, h, 0, (uint32_t)g->scenes.size()) * 4;
-    if (bytes <= g->staging_bytes) return TRAY_OK;
+    const uint64_t n = (uint64_t)g->scenes.size() * local_items(w, h, 0, (uint32_t)g->scenes.size());
+    if (have_room(g->staging, n)) return TRAY_OK;
     for (auto* sc : g->scenes) { int rc = tray_cuda_sync(sc); if (rc) return rc; }
     CU(cudaSetDevice(g->devices[0]));
     for (int i = 0; i < TRAY_MAX_FRAMES_IN_FLIGHT; i++) {
-        cudaFree(g->staging[i]); g->staging[i] = nullptr;
-        CU(cudaMalloc(&g->staging[i], bytes));
+        CU(g->staging[i].reserve(n));
         g->staged_pending[i] = false;
     }
-    g->staging_bytes = bytes;
     return TRAY_OK;
 }
 }  // namespace
@@ -2030,17 +1955,8 @@ extern "C" {
 
 void tray_cuda_group_destroy(tray_group* g) {
     if (!g) return;
-    for (auto* sc : g->scenes) tray_cuda_scene_destroy(sc);
-    if (!g->devices.empty()) {
-        cudaSetDevice(g->devices[0]);
-        for (int i = 0; i < TRAY_MAX_FRAMES_IN_FLIGHT; i++) {
-            cudaFree(g->target[i]); cudaFree(g->staging[i]);
-            if (g->ev_snap[i]) cudaEventDestroy(g->ev_snap[i]);
-            if (g->ev_staged[i]) cudaEventDestroy(g->ev_staged[i]);
-        }
-        if (g->ev_t0) cudaEventDestroy(g->ev_t0);
-        if (g->ev_t1) cudaEventDestroy(g->ev_t1);
-    }
+    for (auto* sc : g->scenes) tray_cuda_scene_destroy(sc);      // each with its own device current, its streams drained first
+    if (!g->devices.empty()) cudaSetDevice(g->devices[0]);       // the frames, staging and events live there
     delete g;
 }
 
@@ -2078,11 +1994,11 @@ int tray_cuda_group_create(const void* nodes, uint64_t n_nodes, const void* tris
         }
         CU(cudaSetDevice(g->devices[0]));
         for (int i = 0; i < TRAY_MAX_FRAMES_IN_FLIGHT; i++) {
-            CU(cudaEventCreateWithFlags(&g->ev_snap[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&g->ev_staged[i], cudaEventDisableTiming));
+            CU(make_event(g->ev_snap[i], cudaEventDisableTiming));
+            CU(make_event(g->ev_staged[i], cudaEventDisableTiming));
         }
         g->exchange = env_int("TRAY_CUDA_GROUP_EXCHANGE", 1) ? 1 : 0;
-        CU(cudaEventCreate(&g->ev_t0)); CU(cudaEventCreate(&g->ev_t1));
+        CU(make_event(g->ev_t0)); CU(make_event(g->ev_t1));
         return TRAY_OK;
     };
     const int rc = body();
@@ -2121,7 +2037,7 @@ int tray_cuda_group_render(tray_group* g, const tray_view* view, uint32_t w, uin
     const bool push = g->exchange == 1 && n > 1;
     if (push) { rc = group_ensure_staging(g, w, h); if (rc) return rc; }
     g->cur = (g->cur + 1) % g->in_flight;
-    uchar4* const target = g->target[g->cur];
+    uchar4* const target = g->target[g->cur].get();
     const uint64_t items = local_items(w, h, 0, (uint32_t)n);
     const bool snap = g->snap_pending[g->cur];             // the frame this target held last is still being copied out
     for (int i = 0; i < n; i++) {
@@ -2129,7 +2045,7 @@ int tray_cuda_group_render(tray_group* g, const tray_view* view, uint32_t w, uin
         const int k = next_slot(sc);                       // the slot this frame will take on device i
         if (!push && i > 0 && snap) {                      // the previous frame in this target must have been copied out first
             CU(cudaSetDevice(sc->device));
-            CU(cudaStreamWaitEvent(slot_stream(sc, k), g->ev_snap[g->cur], 0));
+            CU(cudaStreamWaitEvent(slot_stream(sc, k), g->ev_snap[g->cur].get(), 0));
         }
         sc->frame_target = push ? nullptr : target;
         rc = tray_cuda_render(sc, view, w, h, frame_count, flags | TRAY_RENDER_RGBA, (uint32_t)i, (uint32_t)n, nullptr, nullptr);
@@ -2137,24 +2053,24 @@ int tray_cuda_group_render(tray_group* g, const tray_view* view, uint32_t w, uin
         cudaStream_t st = slot_stream(sc, sc->cur);
         if (push) {
             // one DMA copy of the compact shard into devices[0]'s staging (behind the untile of the frame that used it last)
-            if (g->staged_pending[g->cur]) CU(cudaStreamWaitEvent(st, g->ev_staged[g->cur], 0));
+            if (g->staged_pending[g->cur]) CU(cudaStreamWaitEvent(st, g->ev_staged[g->cur].get(), 0));
             const FrameSlot& f = sc->slot[sc->cur];
             if (f.last_frame.n_items)
-                CU(cudaMemcpyPeerAsync(g->staging[g->cur] + (uint64_t)i * items, g->devices[0], f.d_rgba, sc->device, (size_t)f.last_frame.n_items * sizeof(uchar4), st));
+                CU(cudaMemcpyPeerAsync(g->staging[g->cur].get() + (uint64_t)i * items, g->devices[0], f.buf.d_rgba.get(), sc->device, (size_t)f.last_frame.n_items * sizeof(uchar4), st));
         }
-        if (i > 0) CU(cudaEventRecord(sc->slot[sc->cur].done, st));
+        if (i > 0) CU(cudaEventRecord(sc->slot[sc->cur].done.get(), st));
     }
     g->snap_pending[g->cur] = false;
     // frame complete on devices[0]: its stream waits for every other device's last launch / copy
     tray_scene* s0 = g->scenes[0];
     cudaStream_t st0 = slot_stream(s0, s0->cur);
     CU(cudaSetDevice(s0->device));
-    for (int i = 1; i < n; i++) CU(cudaStreamWaitEvent(st0, g->scenes[i]->slot[g->scenes[i]->cur].done, 0));
+    for (int i = 1; i < n; i++) CU(cudaStreamWaitEvent(st0, g->scenes[i]->slot[g->scenes[i]->cur].done.get(), 0));
     if (push) {
-        if (snap) CU(cudaStreamWaitEvent(st0, g->ev_snap[g->cur], 0));
-        tray::untile_shards_kernel<<<dim3((w + 255) / 256, h), 256, 0, st0>>>(g->staging[g->cur], w, h, (w + 31) / 32, (uint32_t)n, items, target);
+        if (snap) CU(cudaStreamWaitEvent(st0, g->ev_snap[g->cur].get(), 0));
+        tray::untile_shards_kernel<<<dim3((w + 255) / 256, h), 256, 0, st0>>>(g->staging[g->cur].get(), w, h, (w + 31) / 32, (uint32_t)n, items, target);
         CU(cudaGetLastError());
-        CU(cudaEventRecord(g->ev_staged[g->cur], st0));
+        CU(cudaEventRecord(g->ev_staged[g->cur].get(), st0));
         g->staged_pending[g->cur] = true;
         FrameSlot& f0 = s0->slot[s0->cur];               // the readback of devices[0]'s scene reads the assembled frame
         f0.f_target = target; f0.f_has_rgba = false;
@@ -2168,18 +2084,18 @@ int tray_cuda_group_render_timed(tray_group* g, const tray_view* view, uint32_t 
     if (rc) return rc;
     tray_scene* s0 = g->scenes[0];
     CU(cudaSetDevice(s0->device));
-    CU(cudaEventRecord(g->ev_t0, slot_stream(s0, next_slot(s0))));
+    CU(cudaEventRecord(g->ev_t0.get(), slot_stream(s0, next_slot(s0))));
     for (size_t i = 1; i < g->scenes.size(); i++) {      // nobody starts before the clock does
         tray_scene* sc = g->scenes[i];
         CU(cudaSetDevice(sc->device));
-        CU(cudaStreamWaitEvent(slot_stream(sc, next_slot(sc)), g->ev_t0, 0));
+        CU(cudaStreamWaitEvent(slot_stream(sc, next_slot(sc)), g->ev_t0.get(), 0));
     }
     rc = tray_cuda_group_render(g, view, w, h, frame_count, flags);
     if (rc) return rc;
     CU(cudaSetDevice(s0->device));
-    CU(cudaEventRecord(g->ev_t1, slot_stream(s0, s0->cur)));
-    CU(cudaEventSynchronize(g->ev_t1));
-    CU(cudaEventElapsedTime(ms_frame, g->ev_t0, g->ev_t1));
+    CU(cudaEventRecord(g->ev_t1.get(), slot_stream(s0, s0->cur)));
+    CU(cudaEventSynchronize(g->ev_t1.get()));
+    CU(cudaEventElapsedTime(ms_frame, g->ev_t0.get(), g->ev_t1.get()));
     for (auto* sc : g->scenes) { CU(cudaSetDevice(sc->device)); rc = check_overflow(sc->slot[sc->cur].d_flag, slot_stream(sc, sc->cur)); if (rc) return rc; }
     return TRAY_OK;
 }
@@ -2189,7 +2105,7 @@ int tray_cuda_group_readback_begin(tray_group* g, uint8_t* rgba_host, uint32_t s
     tray_scene* s0 = g->scenes[0];
     int rc = tray_cuda_frame_readback_begin(s0, rgba_host, slot);       // snapshots the frame target on devices[0], D2H on the copy stream
     if (rc) return rc;
-    CU(cudaEventRecord(g->ev_snap[g->cur], slot_stream(s0, s0->cur)));
+    CU(cudaEventRecord(g->ev_snap[g->cur].get(), slot_stream(s0, s0->cur)));
     g->snap_pending[g->cur] = true;
     return TRAY_OK;
 }
@@ -2201,7 +2117,7 @@ int tray_cuda_group_readback_wait(tray_group* g, uint32_t slot) {
 
 int tray_cuda_group_frame_ptr(tray_group* g, void** d_frame) {
     if (!g || !d_frame) return fail(TRAY_ERR_ARG, "NULL argument");
-    *d_frame = g->target[g->cur];
+    *d_frame = g->target[g->cur].get();
     return TRAY_OK;
 }
 
