@@ -334,6 +334,14 @@ int tray_cuda_scene_refit_rebuild_tlas_device(tray_scene* scene, const float* d_
  *                      them: a call with no more instances than an earlier one allocates nothing on the device.
  *                      tray_scene_info.device_bytes counts all of it.
  *   ms                 CUDA-event time from the upload of the transforms to the last TLAS write (NULL ok)
+ *   Scale              the tests hold objects of size 2^k placed at world size ~1, |k| <= 32 (strides 48 and 64; stride 24 keeps its
+ *                      edges in f16, |k| <= 8), under powers of two, rotations, signed axis permutations, diag(2^-12, 1, 2^12),
+ *                      strong shear and translations of 1e4, to a float64 world-space evaluation.  The object-space triangle
+ *                      test's determinant grows as ~s^3 in the object size s and bounds the range: it leaves f32 near |k| = 42.
+ *                      An object-space direction's zero components are patched at the instance's scale: with
+ *                      2^r = the largest |W_ij| of row i rounded down to a power of two, component i becomes 2^-23 * 2^r where
+ *                      |r| > 3, and 2^-23 (the patch of a plain scene) where |r| <= 3.  A bounce normal is brought to [1, 2) by a power of two before and after the transpose
+ *                      of W, so its squared length (~s^6 otherwise) stays in f32.
  * Synchronous and ordered as tray_cuda_scene_refit: a frame rendered before keeps its results.  An instanced scene stays instanced.
  * TRAY_ERR_ARG, with nothing changed: NULL scene or pointers, n_instances == 0, a scene without a TLAS, semantic variants
  * (tray_cuda_scene_set_variant flags), an invalid root, max_prims_per_leaf or search_radius out of range, a coordinate of
@@ -373,7 +381,8 @@ int tray_cuda_frame_download_instance(tray_scene* scene, uint32_t* primary, uint
  *   ng         stride 64: the record's ng; strides 48 and 24: cross(e1, e2) in f32 (= cross(v0 - v1, v2 - v0)).  Not normalised and
  *              not flipped toward the ray.
  *   instances  (instanced scenes) u, v from the object-space ray of the traversal, o'_i = ((W_i0 o_x + W_i1 o_y) + W_i2 o_z) + W_i3,
- *              d'_i = (W_i0 d_x + W_i1 d_y) + W_i2 d_z then zero-patched (W = world_to_object of instance instance_ids[i]); ng
+ *              d'_i = (W_i0 d_x + W_i1 d_y) + W_i2 d_z then zero-patched at the instance's scale (tray_cuda_scene_set_instances,
+ *              Scale) (W = world_to_object of instance instance_ids[i]); ng
  *              taken to world space as the bounce normal is, n'_i = (W_0i n_0 + W_1i n_1) + W_2i n_2, not normalised.  On other
  *              scenes object space is world space.
  *   miss       all 20 bytes 0xFF for prim == 0xFFFFFFFF, prim >= n_tris and, on an instanced scene, instance_ids[i] == 0xFFFFFFFF

@@ -62,15 +62,20 @@ __global__ void k_primary_dir(tray::FrameParams F, const uint32_t* px, const uin
     tray::primary_dir(F, px[i], py[i], out[3 * i], out[3 * i + 1], out[3 * i + 2]);
 }
 
-// case i: record prim[i] of `tris`, primary direction pd[3i..], hit distance t[i], pixel (px[i], py[i]), frame F.frame_count + fc[i]
+// case i: record prim[i] of `tris`, primary direction pd[3i..], hit distance t[i], pixel (px[i], py[i]), frame F.frame_count + fc[i];
+// with `inst` (64-byte InstanceRecords, one per case), the instanced form with record i
 template <int S>
 __global__ void k_bounce_ray(tray::FrameParams F, const uint4* tris, const uint32_t* px, const uint32_t* py, const float* pd,
-                             const float* t, const uint32_t* prim, const uint32_t* fc, uint32_t n, float* out) {
+                             const float* t, const uint32_t* prim, const uint32_t* fc, const uint4* inst, uint32_t n, float* out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     F.frame_count = fc[i];
     float* o = out + 6u * i;
-    tray::bounce_ray<S>(F, tris, px[i], py[i], pd[3 * i], pd[3 * i + 1], pd[3 * i + 2], t[i], prim[i], o[0], o[1], o[2], o[3], o[4], o[5]);
+    if (inst)
+        tray::bounce_ray<S, true>(F, tris, px[i], py[i], pd[3 * i], pd[3 * i + 1], pd[3 * i + 2], t[i], prim[i], o[0], o[1], o[2], o[3], o[4],
+                                  o[5], inst + tray::INST_RECORD_U4 * i);
+    else
+        tray::bounce_ray<S>(F, tris, px[i], py[i], pd[3 * i], pd[3 * i + 1], pd[3 * i + 2], t[i], prim[i], o[0], o[1], o[2], o[3], o[4], o[5]);
 }
 
 __global__ void k_uhash(const uint32_t* a, const uint32_t* b, uint32_t n, uint32_t* out) {
@@ -184,10 +189,10 @@ int probe_primary_dir(const tray_view* view, uint32_t w, uint32_t h, const uint3
     return (int)d.err;
 }
 
-// out: n x {ox, oy, oz, dx, dy, dz}
-int probe_bounce_ray(uint32_t stride, const void* records, uint32_t n_records, const tray_view* view, const uint32_t* px,
-                     const uint32_t* py, const float* pd, const float* t, const uint32_t* prim, const uint32_t* frame_count,
-                     uint32_t n, float* out) {
+// out: n x {ox, oy, oz, dx, dy, dz}; inst_records: NULL, or n x 64 B (case i's instance)
+static int bounce_ray_cases(uint32_t stride, const void* records, uint32_t n_records, const tray_view* view, const uint32_t* px,
+                            const uint32_t* py, const float* pd, const float* t, const uint32_t* prim, const uint32_t* frame_count,
+                            const void* inst_records, uint32_t n, float* out) {
     Dev d;
     const uint4* tr = d.in<uint4>(records, (size_t)n_records * stride);
     const uint32_t* x = d.in<uint32_t>(px, n * 4u);
@@ -196,17 +201,31 @@ int probe_bounce_ray(uint32_t stride, const void* records, uint32_t n_records, c
     const float* tt = d.in<float>(t, n * 4u);
     const uint32_t* pp = d.in<uint32_t>(prim, n * 4u);
     const uint32_t* fc = d.in<uint32_t>(frame_count, n * 4u);
+    const uint4* ir = inst_records ? d.in<uint4>(inst_records, (size_t)n * 64u) : nullptr;
     float* o = d.alloc<float>(n * 24u);
     const tray::FrameParams F = frame(view, 1, 1, 0);
     if (d.err == cudaSuccess && n) {
         const unsigned g = blocks(n);
-        if (stride == 24) k_bounce_ray<24><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, n, o);
-        else if (stride == 48) k_bounce_ray<48><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, n, o);
-        else if (stride == 64) k_bounce_ray<64><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, n, o);
+        if (stride == 24) k_bounce_ray<24><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, ir, n, o);
+        else if (stride == 48) k_bounce_ray<48><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, ir, n, o);
+        else if (stride == 64) k_bounce_ray<64><<<g, 128>>>(F, tr, x, y, dd, tt, pp, fc, ir, n, o);
         else return (int)cudaErrorInvalidValue;
     }
     d.back(out, o, n * 24u);
     return (int)d.err;
+}
+
+int probe_bounce_ray(uint32_t stride, const void* records, uint32_t n_records, const tray_view* view, const uint32_t* px,
+                     const uint32_t* py, const float* pd, const float* t, const uint32_t* prim, const uint32_t* frame_count,
+                     uint32_t n, float* out) {
+    return bounce_ray_cases(stride, records, n_records, view, px, py, pd, t, prim, frame_count, nullptr, n, out);
+}
+
+// the instanced form (bounce_ray<S, true>): inst_records = n x 64-byte InstanceRecords, case i takes record i
+int probe_bounce_ray_inst(uint32_t stride, const void* records, uint32_t n_records, const tray_view* view, const uint32_t* px,
+                          const uint32_t* py, const float* pd, const float* t, const uint32_t* prim, const uint32_t* frame_count,
+                          const void* inst_records, uint32_t n, float* out) {
+    return bounce_ray_cases(stride, records, n_records, view, px, py, pd, t, prim, frame_count, inst_records, n, out);
 }
 
 int probe_uhash(const uint32_t* a, const uint32_t* b, uint32_t n, uint32_t* out) {

@@ -35,8 +35,15 @@ static void attr_one(const uint8_t* rec, uint32_t stride, const float* W, const 
         } else {
             o[i] = ray->o[i]; d[i] = ray->d[i];
         }
-        if (!zerodir_box_only && d[i] == 0.0f) d[i] = F32_EPSILON;
     }
+    if (W) {                  /* object space: zero components patched at the instance's scale (traverse.cuh object_zero_patch) */
+        for (int i = 0; i < 3; i++) {
+            int e;
+            frexpf(fmaxf(fmaxf(fabsf(W[4 * i]), fabsf(W[4 * i + 1])), fabsf(W[4 * i + 2])), &e);
+            if (d[i] == 0.0f) d[i] = (e - 1 > 3 || e - 1 < -3) ? ldexpf(F32_EPSILON, e - 1) : F32_EPSILON;
+        }
+    }
+    for (int i = 0; i < 3; i++) if (!zerodir_box_only && d[i] == 0.0f) d[i] = F32_EPSILON;
     float v0[3], e1[3], e2[3], ng[3];
     memcpy(v0, rec, 12);
     if (stride == 24) {

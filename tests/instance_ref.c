@@ -4,7 +4,8 @@
  * The oracle's two-level loop (oracle/tray_oracle.c trace_one_ex: the same node order, triangle order, stack and tie rule) with
  * the one thing the oracle does not have: a transform per TLAS leaf.  Entering leaf j, the ray becomes
  *     o'_i = ((W_i0 o_x + W_i1 o_y) + W_i2 o_z) + W_i3,   d'_i = (W_i0 d_x + W_i1 d_y) + W_i2 d_z
- * (W = world_to_object of the leaf's instance, d the caller's direction, tmin and the running tmax unchanged), and back at the
+ * (W = world_to_object of the leaf's instance, d the caller's direction, tmin and the running tmax unchanged; zero components of d'
+ * patched at the instance's scale, object_zero_patch), and back at the
  * TLAS it is the world ray again.  Node and triangle tests are the oracle's own exported ones (orc_node_intersect,
  * orc_intersect_tri), so everything the oracle decides about one ray against one node or triangle is decided here the same way.
  * The bounce ray of a frame takes the object-space normal to world space through the transpose of W before it is normalised.
@@ -19,6 +20,16 @@
 
 static uint32_t firstbithigh(uint32_t x) { return 31u - (uint32_t)__builtin_clz(x); }
 
+/* d' = W d with its zero components patched at the instance's scale (traverse.cuh object_zero_patch): component i becomes 2^-23
+ * times 2^r, r = floor(log2 max_j |W_ij|), where |r| > 3, and 2^-23 itself where |r| <= 3 */
+static void object_zero_patch(float d[3], const float* W) {
+    for (int i = 0; i < 3; i++) {
+        int e;
+        frexpf(fmaxf(fmaxf(fabsf(W[4 * i]), fabsf(W[4 * i + 1])), fabsf(W[4 * i + 2])), &e);
+        if (d[i] == 0.0f) d[i] = (e - 1 > 3 || e - 1 < -3) ? ldexpf(1.1920929e-7f, e - 1) : 1.1920929e-7f;
+    }
+}
+
 static void xform_ray(const float* W, const orc_ray* in, orc_ray* out) {
     for (int i = 0; i < 3; i++) {
         const float* m = W + 4 * i;
@@ -26,6 +37,7 @@ static void xform_ray(const float* W, const orc_ray* in, orc_ray* out) {
         out->d[i] = (m[0] * in->d[0] + m[1] * in->d[1]) + m[2] * in->d[2];
     }
     out->tmin = in->tmin; out->tmax = in->tmax;
+    object_zero_patch(out->d, W);
 }
 
 /* One ray of scene `s` (two-level: blas_offsets[j] = the BLAS root of TLAS leaf j) with world_to_object w2o[12 j ..] and instance
@@ -133,8 +145,16 @@ int inst_trace(const orc_scene* s, const float* w2o, const uint32_t* leaf_inst, 
     return rc;
 }
 
+/* v times the power of two that puts its largest |component| in [1, 2); a zero vector stays zero (traverse.cuh scale_pow2) */
+static void scale_pow2(float v[3]) {
+    int e;
+    frexpf(fmaxf(fmaxf(fabsf(v[0]), fabsf(v[1])), fabsf(v[2])), &e);
+    for (int k = 0; k < 3; k++) v[k] = ldexpf(v[k], 1 - e);
+}
+
 /* The bounce ray of pixel (px, py) after primary ray `pr` hit `hit` in instance `k` (world_to_object w2o[12 k ..]; NULL: no
- * transform): oracle/tray_oracle.c orc_bounce_ray with the normal taken to world space, n'_i = (W_0i n_0 + W_1i n_1) + W_2i n_2. */
+ * transform): oracle/tray_oracle.c orc_bounce_ray with the normal taken to world space, n'_i = (W_0i n_0 + W_1i n_1) + W_2i n_2,
+ * brought to [1, 2) by a power of two before and after that product. */
 static void bounce_one(const orc_scene* s, const orc_view* vw, const orc_ray* pr, const orc_hit* hit, const float* W, uint32_t px, uint32_t py,
                        uint32_t frame_count, orc_ray* out) {
     memset(out, 0, sizeof *out);
@@ -156,8 +176,10 @@ static void bounce_one(const orc_scene* s, const orc_view* vw, const orc_ray* pr
     else { n[0] = e1[1] * e2[2] - e1[2] * e2[1]; n[1] = e1[2] * e2[0] - e1[0] * e2[2]; n[2] = e1[0] * e2[1] - e1[1] * e2[0]; }
     if (W) {
         float w[3];
+        scale_pow2(n);
         for (int i = 0; i < 3; i++) w[i] = (W[i] * n[0] + W[4 + i] * n[1]) + W[8 + i] * n[2];
         n[0] = w[0]; n[1] = w[1]; n[2] = w[2];
+        scale_pow2(n);
     }
     float len = sqrtf((n[0] * n[0] + n[1] * n[1]) + n[2] * n[2]);
     n[0] = n[0] / len; n[1] = n[1] / len; n[2] = n[2] / len;

@@ -54,7 +54,8 @@ class Probe:
         vp, u32, i32 = C.c_void_p, C.c_uint32, C.c_int
         sig = {"probe_prepare_ray": [vp, u32, u32, vp], "probe_node_test": [vp, vp, u32, u32, u32, vp],
                "probe_tri_test": [vp, u32, vp, u32, u32, u32, vp], "probe_primary_dir": [vp, u32, u32, vp, vp, u32, vp],
-               "probe_bounce_ray": [u32, vp, u32, vp, vp, vp, vp, vp, vp, vp, u32, vp], "probe_uhash": [vp, vp, u32, vp],
+               "probe_bounce_ray": [u32, vp, u32, vp, vp, vp, vp, vp, vp, vp, u32, vp],
+               "probe_bounce_ray_inst": [u32, vp, u32, vp, vp, vp, vp, vp, vp, vp, vp, u32, vp], "probe_uhash": [vp, vp, u32, vp],
                "probe_hash_noise": [vp, vp, vp, u32, vp], "probe_sincos_tau": [vp, u32, vp, vp], "probe_shade": [u32, vp, u32, vp],
                "probe_child_order": [vp]}
         for name, args in sig.items():
@@ -94,12 +95,18 @@ class Probe:
         self._call("probe_primary_dir", C.addressof(view), w, h, px, py, len(px), out)
         return out
 
-    def bounce_ray(self, stride, records, view, px, py, pd, t, prim, frame_count):
+    def bounce_ray(self, stride, records, view, px, py, pd, t, prim, frame_count, w2o=None):
+        """w2o: None, or one world_to_object (3, 4) per case: the instanced form, with case i's InstanceRecord"""
         rec = np.ascontiguousarray(records, np.uint8).reshape(-1)
         a = [np.ascontiguousarray(x, dt) for x, dt in ((px, np.uint32), (py, np.uint32), (pd, np.float32), (t, np.float32),
                                                        (prim, np.uint32), (frame_count, np.uint32))]
         out = np.zeros((len(a[0]), 6), np.float32)
-        self._call("probe_bounce_ray", stride, rec, rec.size // stride, C.addressof(view), *a, len(a[0]), out)
+        if w2o is None:
+            self._call("probe_bounce_ray", stride, rec, rec.size // stride, C.addressof(view), *a, len(a[0]), out)
+        else:
+            inst = np.zeros((len(a[0]), 16), np.float32)
+            inst[:, :12] = np.asarray(w2o, np.float32).reshape(-1, 12)
+            self._call("probe_bounce_ray_inst", stride, rec, rec.size // stride, C.addressof(view), *a, inst, len(a[0]), out)
         return out
 
     def uhash(self, a, b):
@@ -685,6 +692,40 @@ def test_uhash_and_hash_noise(probe):
     L = ob.lib()
     for i in range(0, len(a), 997):
         assert L.orc_uhash(int(a[i]), int(b[i])) == uhash_np(a[i], b[i])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("stride", [24, 48, 64])
+def test_instanced_bounce_normals_at_exponent_edges(probe, stride):
+    """bounce_ray<S, true> on the records of normal_records scaled by 2^k (k = -32 .. 32; stride 24 keeps f16 edges, |k| <= 8)
+    under W = 2^k P (P a signed axis permutation, optionally composed with a rotation): every direction finite and of unit
+    length and in the hemisphere of the float64 world normal (instance_ref.c's bounce_one is held to the kernel's frames bit for
+    bit in test_instance_kernels.py)"""
+    tris, _, ns = normal_records(stride)
+    keep = np.nonzero(np.abs(ns[:, 2] + 1) > 1e-3)[0]
+    view = host.view_from_camera(CAMERA, 64, 64)
+    rng = np.random.default_rng(stride)
+    ks = (-8, 8) if stride == 24 else (-32, -24, -16, -8, 8, 16, 24, 32)
+    for k in ks:
+        for rotate in (False, True):
+            P = np.eye(3)[rng.permutation(3)] * rng.choice([-1.0, 1.0], 3)[:, None]
+            A = (np.linalg.qr(rng.normal(size=(3, 3)))[0] if rotate else np.eye(3)) @ P             # object_to_world = 2^-k A
+            obj = (tris.astype(np.float64).reshape(-1, 3) @ np.linalg.inv(A).T * 2.0 ** k).astype(np.float32).reshape(tris.shape)
+            rec = np.ascontiguousarray(host.tri_records(obj, stride)).view(np.uint8).reshape(-1)
+            W = np.zeros((3, 4)); W[:, :3] = np.linalg.inv(A) * 2.0 ** k
+            n = 4096
+            prim = keep[np.arange(n) % len(keep)].astype(np.uint32)
+            pd = rng.normal(size=(n, 3)); pd /= np.linalg.norm(pd, axis=1, keepdims=True)
+            px, py = rng.integers(0, 2048, n), rng.integers(0, 2048, n)
+            got = probe.bounce_ray(stride, rec, view, px, py, pd, np.full(n, 2.0), prim, np.zeros(n), np.tile(W, (n, 1, 1)))
+            d = got[:, 3:6].astype(np.float64)
+            assert np.isfinite(d).all(), (k, rotate)
+            assert np.abs(np.linalg.norm(d, axis=1) - 1).max() <= 1e-6, (k, rotate)
+            t3 = obj.astype(np.float64)[prim]
+            nf = np.cross(t3[:, 0] - t3[:, 1], t3[:, 2] - t3[:, 0]) @ W[:, :3]                 # W^T n, by rows
+            nf /= np.linalg.norm(nf, axis=1, keepdims=True)
+            nf *= np.where((nf * -pd).sum(1) >= 0, 1.0, -1.0)[:, None]
+            assert ((d * nf).sum(1) >= -1e-6).all(), (k, rotate)
 
 
 # ---- float64 checks of the sampler ------------------------------------------------------------------------------------------

@@ -466,6 +466,20 @@ __device__ __forceinline__ void xform_row(const uint4& w, float ox, float oy, fl
     o = add(add(add(mul(m0, ox), mul(m1, oy)), mul(m2, oz)), __uint_as_float(w.w));
     d = dot3(m0, m1, m2, dx, dy, dz);
 }
+// The zero components of an object-space direction d' = W d, patched as prepare_ray patches a world direction (query.hlsl:334)
+// but at the instance's scale.  Row i of W has scale 2^r, r = floor(log2 max_j |W_ij|).  A patch of 2^-23 tilts the object-space
+// ray by ~2^-23 / 2^r, which for an object placed at scale 2^-r is a tilt the world ray does not have (at 2^r = 2^-16, 10 % in t
+// for an axis-parallel ray; at 2^-32 a miss).  Rows with |r| > 3 get 2^-23 * 2^r, the image of the world-space patch on that
+// row.  Rows with |r| <= 3 keep prepare_ray's own 2^-23, which tilts them by at most 2^-20: every transform of ordinary scale
+// (W = I among them) traces exactly as before, and identity instances as the plain two-level scene.
+__device__ __forceinline__ float row_eps(const uint4& w) {
+    int e;
+    frexpf(fmaxf(fmaxf(fabsf(__uint_as_float(w.x)), fabsf(__uint_as_float(w.y))), fabsf(__uint_as_float(w.z))), &e);
+    return (e - 1 > 3 || e - 1 < -3) ? ldexpf(F32_EPS_, e - 1) : F32_EPS_;
+}
+__device__ __forceinline__ void object_zero_patch(float& x, float& y, float& z, const uint4& w0, const uint4& w1, const uint4& w2) {
+    x = x == 0.0f ? row_eps(w0) : x; y = y == 0.0f ? row_eps(w1) : y; z = z == 0.0f ? row_eps(w2) : z;
+}
 // An object-space normal to world space through the transpose of W, n'_i = W_0i n_0 + W_1i n_1 + W_2i n_2 (the inverse
 // transpose of object_to_world), not normalised
 __device__ __forceinline__ void normal_to_world(const uint4* __restrict__ xf, float& nx, float& ny, float& nz) {
@@ -475,10 +489,20 @@ __device__ __forceinline__ void normal_to_world(const uint4* __restrict__ xf, fl
     const float wz = dot3(__uint_as_float(w0.z), __uint_as_float(w1.z), __uint_as_float(w2.z), nx, ny, nz);
     nx = wx; ny = wy; nz = wz;
 }
+// v times the power of two that puts its largest |component| in [1, 2); a zero vector stays zero.  Scaling by 2^k commutes with
+// IEEE rounding while nothing is subnormal or overflows, so normalize3 of the result is normalize3(v) bit for bit wherever that
+// was computed in the normal range, and finite and unit length where the squared length of v under- or overflows.
+__device__ __forceinline__ void scale_pow2(float& x, float& y, float& z) {
+    int e;
+    frexpf(fmaxf(fmaxf(fabsf(x), fabsf(y)), fabsf(z)), &e);
+    x = ldexpf(x, 1 - e); y = ldexpf(y, 1 - e); z = ldexpf(z, 1 - e);
+}
 
 // bounce ray from a primary hit (src/rt_cpu/rt_cpu.rs:61-76; basis sampling.hlsl:39-51)
 // INST: `xf` is the InstanceRecord of the hit's instance; the object-space normal goes to world space through the transpose of
 // world_to_object, n'_i = W_0i n_0 + W_1i n_1 + W_2i n_2 (the inverse transpose of object_to_world), before it is normalised.
+// The normal is brought to [1, 2) by a power of two before and after that product (scale_pow2): the cross product of an object
+// of size s placed at world size 1 goes to world space with a squared length ~ s^6, which leaves f32 for s < 1e-7 or s > 1e6.
 template <int TRI_STRIDE, bool INST = false>
 __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __restrict__ tris, uint32_t px, uint32_t py,
                                            float pdx, float pdy, float pdz, float t, uint32_t prim,
@@ -493,7 +517,11 @@ __device__ __forceinline__ void bounce_ray(const FrameParams& P, const uint4* __
         tri_load<TRI_STRIDE>(tris, prim, v0x, v0y, v0z, e1x, e1y, e1z, e2x, e2y, e2z);
         cross3(e1x, e1y, e1z, e2x, e2y, e2z, nx, ny, nz);
     }
-    if constexpr (INST) normal_to_world(xf, nx, ny, nz);
+    if constexpr (INST) {
+        scale_pow2(nx, ny, nz);
+        normal_to_world(xf, nx, ny, nz);
+        scale_pow2(nx, ny, nz);
+    }
     normalize3(nx, ny, nz);                                                    // RtTriangle::compute_normal
     const float sgn = copysignf(1.0f, dot3(nx, ny, nz, -pdx, -pdy, -pdz));     // f32::signum (rt_cpu.rs:65)
     nx = mul(nx, sgn); ny = mul(ny, sgn); nz = mul(nz, sgn);
@@ -926,7 +954,8 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                     if (cur_y & 0xff000000u) push(cur_x, cur_y);
                     tlas_sp = sp;
                     if constexpr (INST) {
-                        // into object space: o' = W o + t and d' = W d of the caller's direction (not the zero-patched one)
+                        // into object space: o' = W o + t and d' = W d of the caller's direction (not the zero-patched one), its zero
+                        // components patched at the instance's scale
                         const uint4* rec = P.inst_rec + (size_t)g * INST_RECORD_U4;
                         const uint4 w0 = __ldg(rec), w1 = __ldg(rec + 1), w2 = __ldg(rec + 2), w3 = __ldg(rec + 3);
                         const float4 d = __ldg(reinterpret_cast<const float4*>(P.rays + (ray_idx & INDEX_MASK)) + 1);
@@ -935,6 +964,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, TRAY_MIN_BLOCKS) trace_kernel(c
                         xform_row(w0, r.ox, r.oy, r.oz, d.x, d.y, d.z, ox, dx);
                         xform_row(w1, r.ox, r.oy, r.oz, d.x, d.y, d.z, oy, dy);
                         xform_row(w2, r.ox, r.oy, r.oz, d.x, d.y, d.z, oz, dz);
+                        object_zero_patch(dx, dy, dz, w0, w1, w2);
                         switch_ray(ox, oy, oz, dx, dy, dz);
                     } else {
                         bvh_off = __ldg(P.blas_offsets + g);
@@ -1028,6 +1058,7 @@ __device__ __forceinline__ void hit_attr(const AttrScene& S, const float4& a, co
         xform_row(w0, a.x, a.y, a.z, b.x, b.y, b.z, ox, dx);
         xform_row(w1, a.x, a.y, a.z, b.x, b.y, b.z, oy, dy);
         xform_row(w2, a.x, a.y, a.z, b.x, b.y, b.z, oz, dz);
+        object_zero_patch(dx, dy, dz, w0, w1, w2);
         prepare_ray(r, ox, oy, oz, dx, dy, dz, a.w, 0u);
     } else {
         prepare_ray(r, a.x, a.y, a.z, b.x, b.y, b.z, a.w, S.variant);
